@@ -25,6 +25,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 os.environ.setdefault("DESMO_KERNEL_EVENTS", "1")  # lets the library time its dominant kernel with CUDA events
 
 WORKLOADS = {
@@ -41,6 +42,7 @@ WORKLOADS = {
 }
 METRIC = "train_iters_per_s"  # weak scaling: slab-iterations per second (N slabs per step at N GPUs); strong: whole-job iterations per second
 UNIT = "it/s"
+DUMP_BYTES = 64 * 2 ** 20  # --dump-outputs writes at most this much
 
 
 def load_peaks():
@@ -228,6 +230,30 @@ def count_graph_kernels(torch, engine):
         return per, f"formula ({type(ex).__name__})"
 
 
+def step_outputs(torch, engine, budget=DUMP_BYTES):
+    """What a caller of the train step holds after it, as host float32 arrays: the updated parameters in the packed layout, the losses
+    the step computed (mse, ortho, l1, total) and the learning rates the scheduler left.  phi (r x points) is the only array that grows
+    with the mesh: when everything does not fit in `budget` bytes, phi is cut to a fixed, seeded sample of points (same sample for the
+    same shape in every run), whose indices are written beside it as phi_points (float64)."""
+    import numpy as np
+
+    e = engine
+    out = {"losses": e.losses, "gates": e.gates, "omega": e.omega, "lrs": e.hyper[:5 if e.nF else 4]}
+    if e.nF:
+        out.update(coefs=e.coefs, periods=e.periods)
+    else:
+        out["rows"] = e.rows[:, :e.m]
+    out = {k: v.detach().cpu().numpy() for k, v in out.items()}
+    room = budget - sum(v.nbytes for v in out.values())
+    if 4 * e.r * e.n <= room:
+        out["phi"] = e.phi[:, :e.n].cpu().numpy()
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(e.n, room // (4 * e.r + 8), replace=False))
+        out["phi"] = e.phi[:, torch.from_numpy(idx).to(e.device)].cpu().numpy()
+        out["phi_points"] = idx.astype(np.float64)
+    return out
+
+
 def sharded_parity(torch, dist, dev, rank, world, m, r, p, nF, path):
     """One small sharded fused pass (slabs of points + all-reduce of `red`) against the unsharded pass over the same global data on rank 0."""
     from desmo_b200 import DesmoEngine
@@ -287,7 +313,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-pod", action="store_true", help="profiling runs: random orthonormal-scale modes instead of the POD init")
     ap.add_argument("--cpu-sample", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the parameters, losses and learning rates of the last timed step as DIR/<name>.npy "
+                         "(at most 64 MB; rank 0's slab of phi): the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     n, m, r, p, nF, sched_every, patience, beta = WORKLOADS[args.workload]
     if args.modes:
@@ -422,6 +453,8 @@ def main():
                 ms_total += ev0.elapsed_time(ev1)
                 sample_graph_kernel()
             barrier()
+    # the measurements below run more steps: keep the state of the last timed one
+    dumped = step_outputs(torch, e) if args.dump_outputs and rank == 0 else None
     # The dominant kernel's launch durations over a SECOND timed region of the same K steps (the 64 most recent at most), launched eagerly and back to back
     # (the library brackets the kernel with one CUDA event pair per launch on the launching stream; the events of a captured
     # step can only keep the last replay).  The region starts from the same state as the first one: synchronised, after a pause
@@ -585,6 +618,12 @@ def main():
                                              "gpu": small_gpu_pair(torch, dev, 27000, 1000, 4, 2)}
             except Exception as ex:
                 line["cpu_baseline"] = {"value": None, "error": str(ex)[:200]}
+        if dumped is not None:
+            import numpy as np
+
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         print(json.dumps(line), flush=True)
     if world > 1:
         # tear-down of a process group whose collectives were captured in a CUDA graph can block; everything is measured and
