@@ -15,6 +15,7 @@ PATH_NAMES = {1: "fp32 ffma", 2: "fused tcgen05 (bf16-split)", 3: "tcgen05 GEMM 
 HYP_LR_GATES, HYP_LR_PHI, HYP_LR_Z, HYP_LR_OMEGA, HYP_LR_PERIOD, HYP_BETA, HYP_L1_LAMBDA, HYP_COUNT = range(8)
 MAX_R, MAX_P, MAX_K = 64, 7, 4096
 PRE_MAGNITUDE, PRE_SUBTRACT_MEAN, PRE_SCALE_SQRT_M = 1, 2, 4
+DTYPE_F32, DTYPE_F64, DTYPE_BF16 = 0, 1, 2
 
 
 class DesmoError(RuntimeError):
@@ -43,6 +44,9 @@ SIGNATURES: Dict[str, tuple] = {
     "desmo_recon_backward": (C.c_int, [_SP] + [_vp] * 9),
     "desmo_fused_residual_grad_begin": (C.c_int, [_SP] + [_vp] * 9),
     "desmo_fused_residual_grad_finish": (C.c_int, [_SP] + [_vp] * 9),
+    "desmo_fused_residual_grad_ex": (C.c_int, [_SP, _vp, _i32] + [_vp] * 8),
+    "desmo_fused_residual_grad_begin_ex": (C.c_int, [_SP, _vp, _i32] + [_vp] * 8),
+    "desmo_fused_residual_grad_finish_ex": (C.c_int, [_SP, _vp, _i32] + [_vp] * 8),
     "desmo_adamax_update": (C.c_int, [_SP] + [_vp] * 26),
     "desmo_assemble_grads": (C.c_int, [_SP] + [_vp] * 17),
     "desmo_reconstruct": (C.c_int, [_SP] + [_vp] * 6),
@@ -58,7 +62,11 @@ SIGNATURES: Dict[str, tuple] = {
     "desmo_pod_gram": (C.c_int, [_SP] + [_vp] * 4),
     "desmo_pod_eig": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, C.c_size_t, _vp]),
     "desmo_pod_project": (C.c_int, [_SP] + [_vp] * 5),
+    "desmo_pod_gram_ex": (C.c_int, [_SP, _vp, _i32, _vp, _vp, _vp]),
+    "desmo_pod_project_ex": (C.c_int, [_SP, _vp, _i32, _vp, _vp, _vp, _vp]),
     "desmo_preprocess": (C.c_int, [_SP, _vp, _i32, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "desmo_preprocess_ex": (C.c_int, [_SP, _vp, _i32, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _i32, _vp, _vp, _vp]),
+    "desmo_snapshot_to_bf16": (C.c_int, [_SP, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
     "desmo_plateau_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "desmo_peer_begin_step": (C.c_int, [_vp, _vp]),
     "desmo_peer_allreduce": (C.c_int, [_vp, _i64, _vp, _vp]),
@@ -142,6 +150,17 @@ def torch_allreduce_hook(group=None):
             return 1
 
     return ALLREDUCE_FN(hook)
+
+
+def u_dtype_code(dtype) -> int:
+    """DESMO_DTYPE_* of a snapshot matrix's torch dtype: fp32 or bf16 storage; anything else raises before a launch."""
+    import torch
+
+    if dtype == torch.float32:
+        return DTYPE_F32
+    if dtype == torch.bfloat16:
+        return DTYPE_BF16
+    raise DesmoError(f"the snapshot matrix U must be float32 or bfloat16, got {dtype}")
 
 
 def check(rc: int, what: str = "") -> None:

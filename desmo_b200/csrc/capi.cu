@@ -153,6 +153,13 @@ int carve_workspace(const desmo_shape* s, const Dims& d, void* base, Workspace* 
 
 bool use_tc_path(const desmo_shape* s, const Dims& d) { return select_path(s, d) == DESMO_PATH_TC; }
 
+// element type of the snapshot matrix U: fp32 or bf16 storage
+static int check_u_dtype(int32_t u_dtype, const char* who) {
+    if (u_dtype == DESMO_DTYPE_F32 || u_dtype == DESMO_DTYPE_BF16) return DESMO_OK;
+    set_error("%s: u_dtype %d is not DESMO_DTYPE_F32 (%d) or DESMO_DTYPE_BF16 (%d)", who, (int)u_dtype, DESMO_DTYPE_F32, DESMO_DTYPE_BF16);
+    return DESMO_ERR_ARG;
+}
+
 }  // namespace desmo
 
 using namespace desmo;
@@ -211,45 +218,62 @@ int desmo_build_w(const desmo_shape* s, const float* gates, float* rows, const f
                    step_dev, ws.l1, (cudaStream_t)stream);
 }
 
-static int fused_dispatch(const desmo_shape* s, const float* U, const float* P, const float* phi, const float* omega, const float* W,
-                          float* dphi, float* red, void* workspace, void* stream, bool supplied, const char* who, int phase = 0) {
+static int fused_dispatch(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                          const float* W, float* dphi, float* red, void* workspace, void* stream, bool supplied, const char* who,
+                          int phase = 0) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
+    if ((rc = check_u_dtype(u_dtype, who))) return rc;
     if ((rc = device_ok())) return rc;
     if (!U || !P || !phi || !omega || !W || !dphi || !red || !workspace) { set_error("%s: null pointer", who); return DESMO_ERR_ARG; }
     Workspace ws;
     if ((rc = carve_workspace(s, d, workspace, &ws))) return rc;
     switch (select_path(s, d)) {
-        case DESMO_PATH_TC: return fused_tc(s, d.mt, d.T, d.Kp, U, P, phi, omega, W, dphi, red, ws, (cudaStream_t)stream, supplied, phase);
+        case DESMO_PATH_TC: return fused_tc(s, d.mt, d.T, d.Kp, U, u_dtype, P, phi, omega, W, dphi, red, ws, (cudaStream_t)stream, supplied, phase);
         case DESMO_PATH_FP32:
             if (phase == 2) return DESMO_OK;  // the other paths do everything in the first phase
-            return fused_fp32(s, d.mt, d.T, d.Kp, U, P, phi, omega, W, dphi, red, ws, (cudaStream_t)stream, supplied);
+            return fused_fp32(s, d.mt, d.T, d.Kp, U, u_dtype, P, phi, omega, W, dphi, red, ws, (cudaStream_t)stream, supplied);
         case DESMO_PATH_GEMM:
             if (phase == 2) return DESMO_OK;
-            return fused_gemm_path(s, d.T, d.K, d.Kp, U, P, phi, omega, W, dphi, red, ws.Dacc, ws.gemm, (cudaStream_t)stream, supplied);
+            return fused_gemm_path(s, d.T, d.K, d.Kp, U, u_dtype, P, phi, omega, W, dphi, red, ws.Dacc, ws.gemm, (cudaStream_t)stream, supplied);
         default: return DESMO_ERR_UNSUPPORTED;
     }
 }
 
 int desmo_fused_residual_grad(const desmo_shape* s, const float* U, const float* P, const float* phi, const float* omega,
                               const float* W, float* dphi, float* red, void* workspace, void* stream) {
-    return fused_dispatch(s, U, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad");
+    return fused_dispatch(s, U, DESMO_DTYPE_F32, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad");
 }
 
 int desmo_fused_residual_grad_begin(const desmo_shape* s, const float* U, const float* P, const float* phi, const float* omega,
                                     const float* W, float* dphi, float* red, void* workspace, void* stream) {
-    return fused_dispatch(s, U, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad_begin", 1);
+    return fused_dispatch(s, U, DESMO_DTYPE_F32, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad_begin", 1);
 }
 
 int desmo_fused_residual_grad_finish(const desmo_shape* s, const float* U, const float* P, const float* phi, const float* omega,
                                      const float* W, float* dphi, float* red, void* workspace, void* stream) {
-    return fused_dispatch(s, U, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad_finish", 2);
+    return fused_dispatch(s, U, DESMO_DTYPE_F32, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad_finish", 2);
+}
+
+int desmo_fused_residual_grad_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                 const float* omega, const float* W, float* dphi, float* red, void* workspace, void* stream) {
+    return fused_dispatch(s, U, u_dtype, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad_ex");
+}
+
+int desmo_fused_residual_grad_begin_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                       const float* omega, const float* W, float* dphi, float* red, void* workspace, void* stream) {
+    return fused_dispatch(s, U, u_dtype, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad_begin_ex", 1);
+}
+
+int desmo_fused_residual_grad_finish_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                        const float* omega, const float* W, float* dphi, float* red, void* workspace, void* stream) {
+    return fused_dispatch(s, U, u_dtype, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad_finish_ex", 2);
 }
 
 int desmo_recon_backward(const desmo_shape* s, const float* grad_recon, const float* P, const float* phi, const float* omega,
                          const float* W, float* dphi, float* red, void* workspace, void* stream) {
-    return fused_dispatch(s, grad_recon, P, phi, omega, W, dphi, red, workspace, stream, true, "desmo_recon_backward");
+    return fused_dispatch(s, grad_recon, DESMO_DTYPE_F32, P, phi, omega, W, dphi, red, workspace, stream, true, "desmo_recon_backward");
 }
 
 static int fill_update(const desmo_shape* s, const Dims& d, const Workspace& ws, UpdateArgs* a) {
@@ -405,19 +429,24 @@ int desmo_debug_timers(const desmo_shape* s, void* workspace, uint64_t* out_host
     return DESMO_OK;
 }
 
-int desmo_pod_gram(const desmo_shape* s, const float* U, float* C, void* workspace, void* stream) {
+int desmo_pod_gram_ex(const desmo_shape* s, const void* U, int32_t u_dtype, float* C, void* workspace, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
+    if ((rc = check_u_dtype(u_dtype, "desmo_pod_gram"))) return rc;
     if ((rc = device_ok())) return rc;
     if (!U || !C) { set_error("desmo_pod_gram: null pointer"); return DESMO_ERR_ARG; }
     if (s->path != DESMO_PATH_FP32 && workspace) {
         Workspace ws;
         if ((rc = carve_workspace(s, d, workspace, &ws))) return rc;
-        rc = pod_gram_tc(s, U, C, ws.gram, (cudaStream_t)stream);
+        rc = pod_gram_tc(s, U, u_dtype, C, ws.gram, (cudaStream_t)stream);
         if (rc != DESMO_ERR_UNSUPPORTED) return rc;  // shapes the tensor-core Gram does not cover run on the FFMA Gram kernel
     }
-    return pod_gram_fp32(s, U, C, (cudaStream_t)stream);
+    return pod_gram_fp32(s, U, u_dtype, C, (cudaStream_t)stream);
+}
+
+int desmo_pod_gram(const desmo_shape* s, const float* U, float* C, void* workspace, void* stream) {
+    return desmo_pod_gram_ex(s, U, DESMO_DTYPE_F32, C, workspace, stream);
 }
 
 int desmo_pod_eig(int32_t m, int32_t r, const float* C, float* V, float* sigma, void* workspace, size_t workspace_bytes, void* stream) {
@@ -427,21 +456,49 @@ int desmo_pod_eig(int32_t m, int32_t r, const float* C, float* V, float* sigma, 
     return pod_eig(m, r, C, V, sigma, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
-int desmo_pod_project(const desmo_shape* s, const float* U, const float* V, const float* sigma, float* P, void* stream) {
+int desmo_pod_project_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* V, const float* sigma, float* P, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
+    if ((rc = check_u_dtype(u_dtype, "desmo_pod_project"))) return rc;
     if ((rc = device_ok())) return rc;
     if (!U || !V || !sigma || !P) { set_error("desmo_pod_project: null pointer"); return DESMO_ERR_ARG; }
-    return pod_project(s, U, V, sigma, P, (cudaStream_t)stream);
+    return pod_project(s, U, u_dtype, V, sigma, P, (cudaStream_t)stream);
+}
+
+int desmo_pod_project(const desmo_shape* s, const float* U, const float* V, const float* sigma, float* P, void* stream) {
+    return desmo_pod_project_ex(s, U, DESMO_DTYPE_F32, V, sigma, P, stream);
+}
+
+int desmo_snapshot_to_bf16(const desmo_shape* s, const float* src, int64_t src_ld, int32_t t0, int32_t rows, void* U, double* qsums,
+                           void* stream) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if (!src || !U) { set_error("desmo_snapshot_to_bf16: null pointer"); return DESMO_ERR_ARG; }
+    if (src_ld < s->n || rows < 0 || t0 < 0 || (int64_t)t0 + rows > s->m) {
+        set_error("desmo_snapshot_to_bf16: need src_ld >= n and 0 <= t0 <= t0 + rows <= m (got src_ld=%lld t0=%d rows=%d n=%lld m=%d)",
+                  (long long)src_ld, t0, rows, (long long)s->n, s->m);
+        return DESMO_ERR_ARG;
+    }
+    if ((rc = device_ok())) return rc;
+    if (rows == 0) return DESMO_OK;
+    return snapshot_to_bf16(s, src, src_ld, t0, rows, static_cast<__nv_bfloat16*>(U), qsums, (cudaStream_t)stream);
 }
 
 int desmo_preprocess(const desmo_shape* s, const void* V, int32_t v_dtype, int64_t v_ld, int32_t m_in, int32_t t_stride, int32_t d_in,
                      int32_t d_use, int32_t flags, float* U, double* mean, void* stream) {
+    return desmo_preprocess_ex(s, V, v_dtype, v_ld, m_in, t_stride, d_in, d_use, flags, U, DESMO_DTYPE_F32, nullptr, mean, stream);
+}
+
+int desmo_preprocess_ex(const desmo_shape* s, const void* V, int32_t v_dtype, int64_t v_ld, int32_t m_in, int32_t t_stride, int32_t d_in,
+                        int32_t d_use, int32_t flags, void* U, int32_t u_dtype, double* qsums, double* mean, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
     if (!V || !U) { set_error("desmo_preprocess: null pointer"); return DESMO_ERR_ARG; }
+    if ((rc = check_u_dtype(u_dtype, "desmo_preprocess"))) return rc;
+    if (qsums && u_dtype != DESMO_DTYPE_BF16) { set_error("desmo_preprocess: qsums needs bf16 output (fp32 output is not quantised)"); return DESMO_ERR_ARG; }
     if (v_dtype != DESMO_DTYPE_F32 && v_dtype != DESMO_DTYPE_F64) { set_error("desmo_preprocess: v_dtype must be F32 or F64"); return DESMO_ERR_ARG; }
     if (d_in < 1 || d_in > 3 || d_use < 1 || d_use > d_in) { set_error("desmo_preprocess: need 1 <= d_use <= d_in <= 3"); return DESMO_ERR_ARG; }
     if (!(flags & DESMO_PRE_MAGNITUDE) && d_in != 1) {
@@ -454,7 +511,7 @@ int desmo_preprocess(const desmo_shape* s, const void* V, int32_t v_dtype, int64
     }
     if (v_ld < s->n * d_in) { set_error("desmo_preprocess: v_ld < n * d_in"); return DESMO_ERR_ARG; }
     if ((rc = device_ok())) return rc;
-    return preprocess(s, V, v_dtype, v_ld, m_in, t_stride, d_in, d_use, flags, U, mean, (cudaStream_t)stream);
+    return preprocess(s, V, v_dtype, v_ld, m_in, t_stride, d_in, d_use, flags, U, u_dtype, qsums, mean, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -1,5 +1,6 @@
 // Shared definitions for the desmo_b200 kernels (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -76,10 +77,11 @@ struct EvalArgs {
 // host-side launchers (one per translation unit)
 int build_w(const desmo_shape* s, int K, int Kp, const float* gates, float* rows, const float* coefs, const float* periods,
             float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st);
-// supplied = true: U holds dL/drecon ([m][ld]) and R := (n_global m / 2) * U instead of G W - U (desmo_recon_backward)
-int fused_fp32(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const float* U, const float* P, const float* phi,
+// U is [m][ld] in the element type u_dtype names (DESMO_DTYPE_F32 or DESMO_DTYPE_BF16; validated by the C ABI).
+// supplied = true: U holds dL/drecon ([m][ld], fp32) and R := (n_global m / 2) * U instead of G W - U (desmo_recon_backward)
+int fused_fp32(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
                const float* omega, const float* W, float* dphi, float* red, const Workspace& ws, cudaStream_t st, bool supplied = false);
-int fused_tc(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const float* U, const float* P, const float* phi,
+int fused_tc(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
              const float* omega, const float* W, float* dphi, float* red, const Workspace& ws, cudaStream_t st, bool supplied = false,
              int phase = 0);
 int fused_tc_supported(const desmo_shape* s, int Kp);
@@ -97,18 +99,23 @@ int launch_reconstruct(const EvalArgs& a, cudaStream_t st);
 int launch_colnorm2(const EvalArgs& a, cudaStream_t st);
 int launch_term_norms(const float* g2, const float* gates, const float* rows, int T, int K, int m, int mld, int fourier_quirk, double* out,
                       cudaStream_t st);
-int pod_gram_fp32(const desmo_shape* s, const float* U, float* C, cudaStream_t st);
-int pod_gram_tc(const desmo_shape* s, const float* U, float* C, void* workspace, cudaStream_t st);
+int pod_gram_fp32(const desmo_shape* s, const void* U, int u_dtype, float* C, cudaStream_t st);
+int pod_gram_tc(const desmo_shape* s, const void* U, int u_dtype, float* C, void* workspace, cudaStream_t st);
 int pod_eig(int m, int r, const float* C, float* V, float* sigma, void* workspace, size_t workspace_bytes, cudaStream_t st);
-int pod_project(const desmo_shape* s, const float* U, const float* V, const float* sigma, float* P, cudaStream_t st);
+int pod_project(const desmo_shape* s, const void* U, int u_dtype, const float* V, const float* sigma, float* P, cudaStream_t st);
+// U is written as fp32 or, for u_dtype == DESMO_DTYPE_BF16, as bf16_rn of the fp32 value; qsums (optional, fp64 [2]) accumulates
+// sum (u - q)^2 and sum u^2 over the n real points, u = the fp32 value, q = the stored one
 int preprocess(const desmo_shape* s, const void* V, int v_dtype, long long v_ld, int m_in, int t_stride, int d_in, int d_use, int flags,
-               float* U, double* mean, cudaStream_t st);
+               void* U, int u_dtype, double* qsums, double* mean, cudaStream_t st);
+// src [rows][src_ld] fp32 -> U[t0 .. t0 + rows)[ld] bf16 (round to nearest even, pad columns zeroed); qsums as above (may be NULL)
+int snapshot_to_bf16(const desmo_shape* s, const float* src, long long src_ld, int t0, int rows, __nv_bfloat16* U, double* qsums,
+                     cudaStream_t st);
 
 struct Dims { int T, K, Kp; bool small; MonoTable mt; };  // small: within the fused kernels' limits (mt valid)
 int count_terms(int r, int p);  // T = C(r+p, p) for 1 <= r <= DESMO_MAX_R, 0 <= p <= DESMO_MAX_P and T + 3r <= DESMO_MAX_K, else -1
 struct GemmWorkspace;
 size_t gemm_workspace_bytes(const desmo_shape* s, int T, int K, int Kp, uint8_t* base, GemmWorkspace* w);
-int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const float* U, const float* P, const float* phi, const float* omega,
+int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi, const float* omega,
                     const float* W, float* dphi, float* red, float* Dacc, void* gemm_ws, cudaStream_t st, bool supplied);
 int reconstruct_gemm_path(const desmo_shape* s, int T, int K, int Kp, const float* P, const float* phi, const float* omega, const float* W,
                           float* out, cudaStream_t st);
@@ -129,6 +136,12 @@ int device_ok();
         int _rc = ::desmo::check_cuda((call), #call);      \
         if (_rc) return _rc;                               \
     } while (0)
+
+// Snapshot element loads: bf16 -> fp32 is exact (the bf16 bits are the upper half of the fp32 word).
+__device__ __forceinline__ float ldg_u(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ldg_u(const __nv_bfloat16* p) {
+    return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
+}
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -21,7 +21,7 @@ constexpr int kGS = 260;    // smem row pitch of G_s / R_s (float4-aligned, rows
 constexpr int kBT = 16;     // snapshots per slab
 
 struct FusedArgs {
-    const float* U;
+    const void* U;  // [m][ld] fp32, or bf16 (fused_fp32_kernel<KP, __nv_bfloat16>)
     const float* P;
     const float* phi;
     const float* omega;
@@ -53,7 +53,7 @@ struct FusedSmem {
     static size_t bytes(int mc) { return red_doubles * sizeof(double) + (size_t)(e_off + KP * mc) * sizeof(float); }
 };
 
-template <int KP>
+template <int KP, class UT>
 __global__ void __launch_bounds__(kTile, 1) fused_fp32_kernel(const FusedArgs a) {
     using L = FusedSmem<KP>;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -122,7 +122,7 @@ __global__ void __launch_bounds__(kTile, 1) fused_fp32_kernel(const FusedArgs a)
 #pragma unroll
             for (int tt = 0; tt < kBT; ++tt) {
                 const int t = t0 + tt;
-                u[tt] = (xin && t < a.m) ? __ldg(a.U + (long long)t * a.ld + x) : 0.0f;
+                u[tt] = (xin && t < a.m) ? ldg_u(static_cast<const UT*>(a.U) + (long long)t * a.ld + x) : 0.0f;
             }
             const float* Wb = Wt_s + buf * kBT * KP;
             float lsum = 0.0f;
@@ -754,7 +754,7 @@ int chain_rule_launch(const desmo_shape* s, const MonoTable& mt, int T, int Kp, 
     return DESMO_OK;
 }
 
-template <int KP>
+template <int KP, class UT>
 static int launch_fused(const FusedArgs& a, int sms, size_t smem_cap, cudaStream_t st, int* gx_out, int* nslots_out) {
     using L = FusedSmem<KP>;
     // smallest number of time chunks whose E chunk fits next to the staging buffers
@@ -782,10 +782,10 @@ static int launch_fused(const FusedArgs& a, int sms, size_t smem_cap, cudaStream
     b.mc = mc;
     const int per_chunk = sms / nchunk > 0 ? sms / nchunk : 1;
     const int gx = (int)(ntiles < per_chunk ? ntiles : per_chunk);
-    DESMO_CUDA(cudaFuncSetAttribute(fused_fp32_kernel<KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::bytes(mc)));
+    DESMO_CUDA(cudaFuncSetAttribute(fused_fp32_kernel<KP, UT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::bytes(mc)));
     if (nchunk > 1) DESMO_CUDA(cudaMemsetAsync(b.Dacc, 0, sizeof(float) * (size_t)KP * a.ld, st));
     fused_event_record(0, st);
-    fused_fp32_kernel<KP><<<dim3(gx, nchunk), kTile, L::bytes(mc), st>>>(b);
+    fused_fp32_kernel<KP, UT><<<dim3(gx, nchunk), kTile, L::bytes(mc), st>>>(b);
     fused_event_record(1, st);
     DESMO_CUDA(cudaGetLastError());
     int nslots = gx * nchunk;
@@ -799,7 +799,13 @@ static int launch_fused(const FusedArgs& a, int sms, size_t smem_cap, cudaStream
     return DESMO_OK;
 }
 
-int fused_fp32(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const float* U, const float* P, const float* phi,
+template <int KP>
+static int launch_fused_u(const FusedArgs& a, int u_dtype, int sms, size_t smem_cap, cudaStream_t st, int* gx_out, int* nslots_out) {
+    return u_dtype == DESMO_DTYPE_BF16 ? launch_fused<KP, __nv_bfloat16>(a, sms, smem_cap, st, gx_out, nslots_out)
+                                       : launch_fused<KP, float>(a, sms, smem_cap, st, gx_out, nslots_out);
+}
+
+int fused_fp32(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
                const float* omega, const float* W, float* dphi, float* red, const Workspace& ws, cudaStream_t st, bool supplied) {
     int dev = 0, sms = 0, smem_cap = 0;
     DESMO_CUDA(cudaGetDevice(&dev));
@@ -814,11 +820,11 @@ int fused_fp32(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const f
     a.mt = mt;
     int gx = 0, nslots = 0, rc = 0;
     switch (Kp) {
-        case 16: rc = launch_fused<16>(a, sms, smem_cap, st, &gx, &nslots); break;
-        case 32: rc = launch_fused<32>(a, sms, smem_cap, st, &gx, &nslots); break;
-        case 48: rc = launch_fused<48>(a, sms, smem_cap, st, &gx, &nslots); break;
-        case 64: rc = launch_fused<64>(a, sms, smem_cap, st, &gx, &nslots); break;
-        case 80: rc = launch_fused<80>(a, sms, smem_cap, st, &gx, &nslots); break;  // r = 8, p = 2 (K = 69): BASELINE's "8 modes"
+        case 16: rc = launch_fused_u<16>(a, u_dtype, sms, smem_cap, st, &gx, &nslots); break;
+        case 32: rc = launch_fused_u<32>(a, u_dtype, sms, smem_cap, st, &gx, &nslots); break;
+        case 48: rc = launch_fused_u<48>(a, u_dtype, sms, smem_cap, st, &gx, &nslots); break;
+        case 64: rc = launch_fused_u<64>(a, u_dtype, sms, smem_cap, st, &gx, &nslots); break;
+        case 80: rc = launch_fused_u<80>(a, u_dtype, sms, smem_cap, st, &gx, &nslots); break;  // r = 8, p = 2 (K = 69): BASELINE's "8 modes"
         default: set_error("fused_fp32: padded K=%d not instantiated", Kp); return DESMO_ERR_UNSUPPORTED;
     }
     if (rc) return rc;

@@ -69,7 +69,8 @@ constexpr uint32_t W_OFF = R_OFF + NPR * R_PLANE;
 constexpr uint32_t G_OFF = W_OFF + 2 * W_SLAB;        // two planes (B of G4); G1 reads its three planes from TMEM
 constexpr uint32_t LAT_OFF = G_OFF + 2 * G_PLANE;     // phi tile [kMaxR][128] then P tile [kMaxR][128] of the tile whose library is next
 constexpr uint32_t LAT_HALF = kMaxR * BP * 4;
-// U staging: each snapshot quarter of the epilogue owns a private ring of U_RING TMA stages of [U_ROWS snapshots][128 points] fp32.
+// U staging: each snapshot quarter of the epilogue owns a private ring of U_RING TMA stages of [U_ROWS snapshots][128 points] fp32
+// (bf16 snapshots: the same stages at half the bytes, in the first half of the fp32-sized region).
 // Private rings matter: mbarrier parity waits are only sound if a waiter is never two phases away from the barrier, which a
 // ring shared by independently progressing consumer groups cannot guarantee.
 constexpr uint32_t U_OFF = LAT_OFF + 2 * LAT_HALF;
@@ -83,12 +84,14 @@ constexpr int U_PER = QT / U_ROWS;                     // stages a quarter consu
 #endif
 constexpr int U_RING = DESMO_U_RING;                   // stages in a quarter's ring
 constexpr uint32_t U_STAGE = U_ROWS * BP * 4;          // must be a multiple of 128 B, the TMA destination alignment
+template <bool kU16>
+constexpr uint32_t u_stage() { return U_ROWS * BP * (kU16 ? 2 : 4); }  // bytes of one stage of U's element type
 constexpr uint32_t TRACE_OFF = U_OFF + NQ * U_RING * U_STAGE;  // debug builds only: 6 event logs of TRACE_LEN entries
 constexpr int TRACE_LEN = 384;
 constexpr uint32_t SMEM_BYTES = TRACE_OFF + 1024;  // + alignment slack
 constexpr uint32_t SMEM_BYTES_DEBUG = SMEM_BYTES + 6 * TRACE_LEN * 8;
 static_assert(SMEM_BYTES + 2048 <= 232448, "dynamic + static shared memory must fit the 227 KB of an sm_100 CTA");
-static_assert(QT % U_ROWS == 0 && U_STAGE % 128 == 0 && U_RING >= U_PER, "U stage shape");
+static_assert(QT % U_ROWS == 0 && u_stage<true>() % 128 == 0 && U_RING >= U_PER, "U stage shape");
 constexpr uint32_t TMEM_REC = 0, TMEM_D = 128, TMEM_G = 192, TMEM_E = 256;  // D: NPR column blocks of 32 (N-stacked B planes), summed in the epilogue
 // G1's A operand (the three bf16 planes of the library tile, [point = lane][lib pair = column], 16 columns per plane) lives in
 // TMEM: an SS-mode MMA re-reads its 4 KB A tile from shared memory for every instruction, and shared-memory bandwidth is what
@@ -96,7 +99,7 @@ constexpr uint32_t TMEM_REC = 0, TMEM_D = 128, TMEM_G = 192, TMEM_E = 256;  // D
 }  // namespace tc
 
 struct TcArgs {
-    const float* U;
+    const void* U;
     const float* P;
     const float* phi;
     const float* omega;
@@ -276,12 +279,16 @@ constexpr uint32_t kDescHi = (1024u >> 4) | (1u << 14) | (2u << 29);  // SBO = 1
 
 // kSupplied: backward of forward()'s reconstruction for an arbitrary upstream gradient (desmo_recon_backward): the buffer read through
 // the U path holds dL/drecon, R := seed_scale * (that) instead of G W - U, G1 is skipped; G3 / G4 / hand-overs are unchanged.
-template <bool kDebug, bool kSupplied>
+// kU16: U holds bf16 snapshots; the epilogue widens each one exactly to fp32 (a 16-bit shift), all arithmetic after the load is the same.
+template <bool kDebug, bool kSupplied, bool kU16>
 __global__ void __launch_bounds__(tc::THREADS, 1) fused_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmW,
                                                                           const __grid_constant__ CUtensorMap tmU,
                                                                           const __grid_constant__ CUtensorMap tmPhi,
                                                                           const __grid_constant__ CUtensorMap tmP) {
     using namespace tc;
+    static_assert(!(kSupplied && kU16), "recon_backward reads an fp32 upstream gradient");
+    constexpr uint32_t US = u_stage<kU16>();  // bytes per U stage
+    constexpr uint32_t UB = kU16 ? 2 : 4;     // bytes per snapshot element
     extern __shared__ uint8_t smem_raw[];
     enum { W_FULL0 = 0, W_FULL1, W_EMPTY0, W_EMPTY1, REC_FULL, REC_EMPTY, R_FULL, GT_FULL, LAT_FULL, LAT_EMPTY, D_FULL, D_EMPTY,
            R_EMPTYQ0, U_FULL0 = R_EMPTYQ0 + 4, U_EMPTY0 = U_FULL0 + NQ * U_RING, NBARS = U_EMPTY0 + NQ * U_RING };
@@ -425,8 +432,8 @@ __global__ void __launch_bounds__(tc::THREADS, 1) fused_tc_kernel(const TcArgs a
 #ifdef EXP_NO_UTMA
                         mbar_arrive(bar(U_FULL0 + b));
 #else
-                        mbar_expect_tx(bar(U_FULL0 + b), U_STAGE);
-                        tma_load_2d(sbase + U_OFF + b * U_STAGE, &tmU, (int)(tile * BP), slab * BT + (h0 + hh) * QT + k * U_ROWS, bar(U_FULL0 + b));
+                        mbar_expect_tx(bar(U_FULL0 + b), US);
+                        tma_load_2d(sbase + U_OFF + b * US, &tmU, (int)(tile * BP), slab * BT + (h0 + hh) * QT + k * U_ROWS, bar(U_FULL0 + b));
 #endif
                     }
                     if (++st == U_RING) { st = 0; ++use; }
@@ -748,14 +755,20 @@ __global__ void __launch_bounds__(tc::THREADS, 1) fused_tc_kernel(const TcArgs a
                         const int sk = (it * U_PER + k) % U_RING;
                         const int st = h * U_RING + sk;
                         if (k > 0) mbar_wait(bar(U_FULL0 + st), ((it * U_PER + k) / U_RING) & 1, 11, it);
-                        const uint32_t us = sbase + U_OFF + st * U_STAGE + p * 4;
+                        const uint32_t us = sbase + U_OFF + st * US + p * UB;
 #pragma unroll
                         for (int j = 0; j < U_ROWS; ++j) {
                             float uv;
 #ifdef EXP_NO_ULDS
                             uv = __uint_as_float(us);
 #else
-                            asm volatile("ld.shared.f32 %0, [%1];" : "=f"(uv) : "r"(us + j * (BP * 4)));
+                            if constexpr (kU16) {
+                                uint32_t hv;
+                                asm volatile("ld.shared.u16 %0, [%1];" : "=r"(hv) : "r"(us + j * (BP * UB)));
+                                uv = __uint_as_float(hv << 16);
+                            } else {
+                                asm volatile("ld.shared.f32 %0, [%1];" : "=f"(uv) : "r"(us + j * (BP * 4)));
+                            }
 #endif
                             float rr = kSupplied ? uv * a.seed_scale : __uint_as_float(u[k * U_ROWS + j]) - uv;
                             if (decltype(masked)::value) rr = (xin && t0 + k * U_ROWS + j < a.m) ? rr : 0.0f;
@@ -960,7 +973,15 @@ int chain_rule_launch(const desmo_shape* s, const MonoTable& mt, int T, int Kp, 
 
 // phase: 0 = the whole pass; 1 = the dominant kernel + the E part of `red` (final for this rank when it returns); 2 = chain rule + the
 // scalar tail of `red` (needs the per-CTA partials phase 1 left in the workspace).
-int fused_tc(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const float* U, const float* P, const float* phi,
+template <bool kDebug, bool kSupplied, bool kU16>
+static int launch_tc(int grid, uint32_t smem, const TcArgs& a, const CUtensorMap& tm, const CUtensorMap& tmu, const CUtensorMap& tmphi,
+                     const CUtensorMap& tmp, cudaStream_t st) {
+    DESMO_CUDA(cudaFuncSetAttribute(fused_tc_kernel<kDebug, kSupplied, kU16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fused_tc_kernel<kDebug, kSupplied, kU16><<<grid, tc::THREADS, smem, st>>>(a, tm, tmu, tmphi, tmp);
+    return DESMO_OK;
+}
+
+int fused_tc(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
              const float* omega, const float* W, float* dphi, float* red, const Workspace& ws, cudaStream_t st, bool supplied, int phase) {
     (void)W;
     if (!fused_tc_supported(s, Kp)) { set_error("tcgen05 path: unsupported shape"); return DESMO_ERR_UNSUPPORTED; }
@@ -991,12 +1012,15 @@ int fused_tc(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const flo
     CUresult cr = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)ws.tc, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                       CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (cr != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed (%d)", (int)cr); return DESMO_ERR_CUDA; }
+    const bool u16 = u_dtype == DESMO_DTYPE_BF16;
+    if (u16 && supplied) { set_error("tcgen05 path: recon_backward takes an fp32 upstream gradient"); return DESMO_ERR_ARG; }
     CUtensorMap tmu;
     {
         const cuuint64_t udims[2] = {(cuuint64_t)s->ld, (cuuint64_t)s->m};
-        const cuuint64_t ustr[1] = {(cuuint64_t)s->ld * 4};
+        const cuuint64_t ustr[1] = {(cuuint64_t)s->ld * (u16 ? 2 : 4)};
         const cuuint32_t ubox[2] = {(cuuint32_t)tc::BP, (cuuint32_t)tc::U_ROWS};
-        cr = enc(&tmu, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)U, udims, ustr, ubox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+        cr = enc(&tmu, u16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)U, udims, ustr, ubox, estr,
+                 CU_TENSOR_MAP_INTERLEAVE_NONE,
                  CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (cr != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(U) failed (%d)", (int)cr); return DESMO_ERR_CUDA; }
     }
@@ -1032,16 +1056,13 @@ int fused_tc(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const flo
     const long long ntiles = s->ld / tc::BP;
     const int grid = (int)(ntiles < sms ? ntiles : sms);
     fused_event_record(0, st);
-    if (supplied) {
-        DESMO_CUDA(cudaFuncSetAttribute(fused_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES));
-        fused_tc_kernel<false, true><<<grid, tc::THREADS, tc::SMEM_BYTES, st>>>(a, tm, tmu, tmphi, tmp);
-    } else if (a.dbg) {
-        DESMO_CUDA(cudaFuncSetAttribute(fused_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES_DEBUG));
-        fused_tc_kernel<true, false><<<grid, tc::THREADS, tc::SMEM_BYTES_DEBUG, st>>>(a, tm, tmu, tmphi, tmp);
-    } else {
-        DESMO_CUDA(cudaFuncSetAttribute(fused_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES));
-        fused_tc_kernel<false, false><<<grid, tc::THREADS, tc::SMEM_BYTES, st>>>(a, tm, tmu, tmphi, tmp);
-    }
+    int lrc;
+    if (supplied) lrc = launch_tc<false, true, false>(grid, tc::SMEM_BYTES, a, tm, tmu, tmphi, tmp, st);
+    else if (a.dbg) lrc = u16 ? launch_tc<true, false, true>(grid, tc::SMEM_BYTES_DEBUG, a, tm, tmu, tmphi, tmp, st)
+                              : launch_tc<true, false, false>(grid, tc::SMEM_BYTES_DEBUG, a, tm, tmu, tmphi, tmp, st);
+    else lrc = u16 ? launch_tc<false, false, true>(grid, tc::SMEM_BYTES, a, tm, tmu, tmphi, tmp, st)
+                   : launch_tc<false, false, false>(grid, tc::SMEM_BYTES, a, tm, tmu, tmphi, tmp, st);
+    if (lrc) return lrc;
     fused_event_record(1, st);
     DESMO_CUDA(cudaGetLastError());
     if (phase == 1) {

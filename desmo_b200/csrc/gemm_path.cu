@@ -21,6 +21,8 @@
 #include <cuda_bf16.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace desmo {
@@ -32,7 +34,7 @@ constexpr int EPI_WARPS = 8;
 constexpr int THREADS = 64 + EPI_WARPS * 32;
 constexpr int kChunkPoints = 16384;
 
-enum { EPI_RESID = 0, EPI_D = 1, EPI_E = 2, EPI_RECON = 3 };
+enum { EPI_RESID = 0, EPI_D = 1, EPI_E = 2, EPI_RECON = 3, EPI_RESID_BF16 = 4 };  // EPI_RESID_BF16: EPI_RESID reading bf16 snapshots
 
 // ------------------------------------------------------------------------------------------------- PTX helpers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -108,7 +110,7 @@ struct GemmArgs {
     int a_rows, b_rows;        // rows per plane of the 2-D maps (planes are stacked along rows)
     int n_lib16;               // valid extent of the library dimension rounded up to 16 (N of the last tile, EPI_D / EPI_E)
     // epilogue
-    const float* U;            // EPI_RESID: snapshots [m][ld]
+    const void* U;             // EPI_RESID: snapshots [m][ld] fp32 (EPI_RESID_BF16: bf16)
     float* out;                // EPI_RECON: [m][ld]
     __nv_bfloat16* Rp;         // EPI_RESID: [2][rows_r][mp]
     float* Dacc;               // EPI_D: [K][ld]
@@ -138,6 +140,8 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
     constexpr uint32_t STAGE = (NPA + NPB) * PLANE_TILE;
     constexpr int NSTAGE = (NPA + NPB) >= 6 ? 2 : 3;
     static_assert(NPA == NPB, "plane pairs are defined for equal plane counts");
+    constexpr bool kResid = EPI == EPI_RESID || EPI == EPI_RESID_BF16;
+    using UT = typename std::conditional<EPI == EPI_RESID_BF16, __nv_bfloat16, float>::type;
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bars[2 * NSTAGE + 4];
     __shared__ uint32_t tmem_base_s;
@@ -271,7 +275,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
             }
             // ---- finalize the output tile (tm, tn) ----
             const int col0 = tn * BN + c * 64;
-            if (EPI == EPI_RESID) {
+            if (kResid) {
                 // rows = points of the chunk, columns = snapshots: r = Rec - U, loss, two bf16 planes of r (row-major, t contiguous)
                 const long long pl = (long long)tm * BM + row;  // chunk-local point
                 const long long x = g.x0 + pl;
@@ -283,7 +287,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
 #pragma unroll
                     for (int j = 0; j < 16; ++j) {
                         const int t = col0 + blk * 16 + j;
-                        u[j] = (xin && t < g.m) ? __ldg(g.U + (long long)t * g.ld + x) : 0.0f;
+                        u[j] = (xin && t < g.m) ? ldg_u(static_cast<const UT*>(g.U) + (long long)t * g.ld + x) : 0.0f;
                     }
                     uint32_t w1[8], w2[8];
 #pragma unroll
@@ -331,14 +335,14 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
                 }
             }
         }
-        if (EPI == EPI_RESID) {
+        if (kResid) {
             loss_acc = warp_sum(loss_acc);
             if (lane == 0) loss_s[warp - 2] = loss_acc;
         }
         tc_fence_before();
     }
     __syncthreads();
-    if (EPI == EPI_RESID && tid == 0) {
+    if (kResid && tid == 0) {
         double s = 0.0;
         for (int i = 0; i < EPI_WARPS; ++i) s += loss_s[i];
         g.loss_part[blockIdx.x] = g.first_chunk ? s : g.loss_part[blockIdx.x] + s;
@@ -722,7 +726,7 @@ __global__ void __launch_bounds__(256) supplied_planes_kernel(const float* __res
     }
 }
 
-int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const float* U, const float* P, const float* phi, const float* omega,
+int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi, const float* omega,
                     const float* W, float* dphi, float* red, float* Dacc, void* gemm_ws, cudaStream_t st, bool supplied) {
     using namespace gp;
     int dev = 0, sms = 0;
@@ -771,12 +775,15 @@ int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const float* U, 
             // GEMM 1: Rec[p x t] = G W; A = G (MN-major: p contiguous), B = W (MN-major: t contiguous), contraction over the library
             g.tiles_m = tiles_p; g.tiles_n = mp / 128; g.nslice = 1; g.kblocks = (K + 63) / 64; g.kb_per_slice = g.kblocks; g.kgroup = 4;
             g.a_rows = Kr; g.b_rows = Kr;
-            if ((rc = launch_gemm<true, true, 3, 3, EPI_RESID>(g, tmG_mn, tmW_mn, sms, st))) return rc;
+            rc = u_dtype == DESMO_DTYPE_BF16 ? launch_gemm<true, true, 3, 3, EPI_RESID_BF16>(g, tmG_mn, tmW_mn, sms, st)
+                                             : launch_gemm<true, true, 3, 3, EPI_RESID>(g, tmG_mn, tmW_mn, sms, st);
+            if (rc) return rc;
             const int items = g.tiles_m * g.tiles_n;
             nloss = nloss > (items < sms ? items : sms) ? nloss : (items < sms ? items : sms);
         } else {
             dim3 grid((unsigned)((rows_c + 255) / 256), 16);
-            supplied_planes_kernel<<<grid, 256, 0, st>>>(U, s->n, s->ld, x0, rows_c, s->m, mp, seed, w.Rp);
+            if (u_dtype != DESMO_DTYPE_F32) { set_error("GEMM path: recon_backward takes an fp32 upstream gradient"); return DESMO_ERR_ARG; }
+            supplied_planes_kernel<<<grid, 256, 0, st>>>(static_cast<const float*>(U), s->n, s->ld, x0, rows_c, s->m, mp, seed, w.Rp);
             DESMO_CUDA(cudaGetLastError());
         }
         // GEMM 3: D[p x lib] = R W^T; A = R (K-major: t contiguous), B = W (K-major), contraction over the snapshots

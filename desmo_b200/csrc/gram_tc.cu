@@ -8,6 +8,9 @@
 //   warp 1 (one elected thread): 24 MMAs per chunk (6 plane pairs x 4 k-steps of 16 points), accumulator in TMEM (128 columns);
 //   end: TMEM -> registers -> atomicAdd into C (and the mirrored tile).
 // Both operands are K-major because the time-major layout keeps mesh points contiguous.
+// bf16 snapshots (gram_tc_kernel<true>): the rows already are bf16 MMA operands, so the converters copy them into plane 1 as they are
+// and the issuer runs only the plane-1 x plane-1 products (4 MMAs per chunk), in the same k-step order and with the same FLUSH
+// cadence: for such data the fp32 kernel's planes 2 and 3 are exactly zero, so the result equals the fp32 Gram of U_q.float().
 #include <cuda_bf16.h>
 
 #include "common.cuh"
@@ -64,6 +67,11 @@ __device__ __forceinline__ float4 ldg_nc_v4(const float4* p) {
     asm volatile("ld.global.nc.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
     return v;
 }
+__device__ __forceinline__ uint4 ldg_nc_u4(const uint4* p) {
+    uint4 v;
+    asm volatile("ld.global.nc.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
+    return v;
+}
 __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
     asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
@@ -75,7 +83,8 @@ __device__ __forceinline__ void split3_pair(float x0, float x1, uint32_t& w1, ui
     asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(w3) : "f"(f1), "f"(f0));
 }
 
-__global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const float* __restrict__ U, long long ld, int m, int ntile, long long xchunk,
+template <bool kU16>
+__global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const void* __restrict__ Uv, long long ld, int m, int ntile, long long xchunk,
                                                              long long xtotal, float* __restrict__ C, float* __restrict__ part,
                                                              unsigned* __restrict__ pace) {
     extern __shared__ uint8_t smem_raw[];
@@ -86,6 +95,8 @@ __global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const float* __rest
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     enum { FULL0 = 0, FULL1, EMPTY0, EMPTY1, ACC_FULL, ACC_EMPTY };
     auto bar = [&](int i) { return smem_u32(&bars[i]); };
+    const float* __restrict__ U = static_cast<const float*>(Uv);
+    const __nv_bfloat16* __restrict__ U16 = static_cast<const __nv_bfloat16*>(Uv);
 
     int pair = blockIdx.x, bi = 0;
     while (pair >= ntile - bi) { pair -= ntile - bi; ++bi; }
@@ -130,7 +141,11 @@ __global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const float* __rest
                  ((uint64_t)desc_hi << 32) | (b_lo + ((PB * PLANE + ks * 32) >> 4)), idesc, acc);                            \
         acc = 1;                                                                                                             \
     }
-                GRAM_PAIR(2, 0) GRAM_PAIR(0, 2) GRAM_PAIR(1, 1) GRAM_PAIR(1, 0) GRAM_PAIR(0, 1) GRAM_PAIR(0, 0)
+                if constexpr (kU16) {
+                    GRAM_PAIR(0, 0)
+                } else {
+                    GRAM_PAIR(2, 0) GRAM_PAIR(0, 2) GRAM_PAIR(1, 1) GRAM_PAIR(1, 0) GRAM_PAIR(0, 1) GRAM_PAIR(0, 0)
+                }
 #undef GRAM_PAIR
                 umma_commit(bar(EMPTY0 + st));
                 if ((c + 1) % FLUSH == 0 || c == nchunks - 1) umma_commit(bar(ACC_FULL));
@@ -141,8 +156,21 @@ __global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const float* __rest
         //                  cover the 256 contiguous bytes of one row, so every warp-level load is four full 256 B segments ----------------
         const int ct = tid - 128;            // 0..255
         float4 ra[8], rb[8];
+        uint4 qa[4], qb[4];  // bf16: one 16 B load = the 8 points of an item
         auto load_chunk = [&](int c) {
             const long long xo = x0 + (long long)c * BK;
+            if constexpr (kU16) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const int idx = k * 256 + ct, row = idx >> 3, g8 = idx & 7;
+                    const long long x = xo + g8 * 8;
+                    const int ta = bi * BM + row, tb = bj * BM + row;
+                    const uint4 z = make_uint4(0u, 0u, 0u, 0u);
+                    qa[k] = (ta < m && x < x1) ? ldg_nc_u4(reinterpret_cast<const uint4*>(U16 + (long long)ta * ld + x)) : z;
+                    if (!diag) qb[k] = (tb < m && x < x1) ? ldg_nc_u4(reinterpret_cast<const uint4*>(U16 + (long long)tb * ld + x)) : z;
+                }
+                return;
+            }
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
                 const int idx = k * 256 + ct, row = idx >> 3, g8 = idx & 7;
@@ -178,6 +206,14 @@ __global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const float* __rest
                 st_shared_v4(base + 2 * PLANE + off, w3[0], w3[1], w3[2], w3[3]);
             }
         };
+        auto store_plane16 = [&](uint32_t base, const uint4 (&q)[4]) {  // same rows and swizzle, plane 1 only
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int idx = k * 256 + ct, row = idx >> 3, g8 = idx & 7;
+                const uint32_t off = row * 128 + ((uint32_t)(g8 ^ (row & 7)) << 4);
+                st_shared_v4(base + off, q[k].x, q[k].y, q[k].z, q[k].w);
+            }
+        };
         const int q = warp & 3, hcol = (warp - 4) >> 2;
         float* mypart = part + (long long)(blockIdx.y * gridDim.x + blockIdx.x) * (BM * BM);  // [col][row]: lanes -> consecutive rows
         if (nchunks > 0) load_chunk(0);
@@ -199,8 +235,13 @@ __global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const float* __rest
                 asm volatile("bar.sync 1, %0;" ::"n"(CONV_WARPS * 32) : "memory");
             }
             if (c >= 2) mbar_wait(bar(EMPTY0 + st), ((c >> 1) - 1) & 1);
-            store_planes(sbase + st * STAGE, ra);
-            if (!diag) store_planes(sbase + st * STAGE + OPERAND, rb);
+            if constexpr (kU16) {
+                store_plane16(sbase + st * STAGE, qa);
+                if (!diag) store_plane16(sbase + st * STAGE + OPERAND, qb);
+            } else {
+                store_planes(sbase + st * STAGE, ra);
+                if (!diag) store_planes(sbase + st * STAGE + OPERAND, rb);
+            }
             if (c + 1 < nchunks) load_chunk(c + 1);  // next chunk's loads fly while this chunk's MMAs run
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             mbar_arrive(bar(FULL0 + st));
@@ -258,7 +299,7 @@ __global__ void __launch_bounds__(256) gram_reduce_kernel(const float* __restric
 
 }  // namespace gram
 
-int pod_gram_tc(const desmo_shape* s, const float* U, float* C, void* workspace, cudaStream_t st) {
+int pod_gram_tc(const desmo_shape* s, const void* U, int u_dtype, float* C, void* workspace, cudaStream_t st) {
     float* part = static_cast<float*>(workspace);  // [SMs][128*128]
     using namespace gram;
     const int m = s->m, ntile = (m + BM - 1) / BM;
@@ -275,11 +316,14 @@ int pod_gram_tc(const desmo_shape* s, const float* U, float* C, void* workspace,
     if (nsplit > maxsplit) nsplit = maxsplit;
     long long xchunk = ((xtotal + nsplit - 1) / nsplit + BK - 1) / BK * BK;
     nsplit = (xtotal + xchunk - 1) / xchunk;
-    DESMO_CUDA(cudaFuncSetAttribute(gram_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
+    const bool u16 = u_dtype == DESMO_DTYPE_BF16;
+    DESMO_CUDA(cudaFuncSetAttribute(u16 ? gram_tc_kernel<true> : gram_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)SMEM_BYTES));
     if ((long long)npairs * nsplit > sms || nsplit > 256) return DESMO_ERR_UNSUPPORTED;  // one partial tile per SM in the workspace
     unsigned* pace = reinterpret_cast<unsigned*>(part + (size_t)sms * BM * BM);            // pacing counters, one per point range
     DESMO_CUDA(cudaMemsetAsync(pace, 0, 1024, st));
-    gram_tc_kernel<<<dim3(npairs, (unsigned)nsplit), THREADS, SMEM_BYTES, st>>>(U, s->ld, m, ntile, xchunk, xtotal, C, part, pace);
+    if (u16) gram_tc_kernel<true><<<dim3(npairs, (unsigned)nsplit), THREADS, SMEM_BYTES, st>>>(U, s->ld, m, ntile, xchunk, xtotal, C, part, pace);
+    else gram_tc_kernel<false><<<dim3(npairs, (unsigned)nsplit), THREADS, SMEM_BYTES, st>>>(U, s->ld, m, ntile, xchunk, xtotal, C, part, pace);
     DESMO_CUDA(cudaGetLastError());
     gram_reduce_kernel<<<npairs, 256, 0, st>>>(part, npairs, (int)nsplit, m, ntile, C);
     DESMO_CUDA(cudaGetLastError());

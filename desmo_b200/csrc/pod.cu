@@ -13,7 +13,9 @@ constexpr int kGT = 64;   // output tile edge
 constexpr int kGX = 32;   // points per smem stage
 constexpr int kGP = 68;   // smem pitch
 
-__global__ void __launch_bounds__(256) gram_fp32_kernel(const float* __restrict__ U, long long ld, long long n, int m,
+// UT = float or __nv_bfloat16 (snapshots stored in bf16 are widened exactly; the products and sums are the same fp32 FFMAs)
+template <class UT>
+__global__ void __launch_bounds__(256) gram_fp32_kernel(const UT* __restrict__ U, long long ld, long long n, int m,
                                                         int ntile, long long xchunk, float* __restrict__ C) {
     __shared__ __align__(16) float As[kGX][kGP];
     __shared__ __align__(16) float Bs[kGX][kGP];
@@ -34,8 +36,8 @@ __global__ void __launch_bounds__(256) gram_fp32_kernel(const float* __restrict_
             const int t = e / kGX, xx = e % kGX;
             const long long x = xb + xx;
             const int ta = bi * kGT + t, tb = bj * kGT + t;
-            As[xx][t] = (ta < m && x < x1) ? U[(long long)ta * ld + x] : 0.0f;
-            Bs[xx][t] = (tb < m && x < x1) ? U[(long long)tb * ld + x] : 0.0f;
+            As[xx][t] = (ta < m && x < x1) ? (float)U[(long long)ta * ld + x] : 0.0f;
+            Bs[xx][t] = (tb < m && x < x1) ? (float)U[(long long)tb * ld + x] : 0.0f;
         }
         __syncthreads();
 #pragma unroll 8
@@ -62,7 +64,7 @@ __global__ void __launch_bounds__(256) gram_fp32_kernel(const float* __restrict_
         }
 }
 
-int pod_gram_fp32(const desmo_shape* s, const float* U, float* C, cudaStream_t st) {
+int pod_gram_fp32(const desmo_shape* s, const void* U, int u_dtype, float* C, cudaStream_t st) {
     const int m = s->m, ntile = (m + kGT - 1) / kGT;
     const int npairs = ntile * (ntile + 1) / 2;
     DESMO_CUDA(cudaMemsetAsync(C, 0, sizeof(float) * (size_t)m * m, st));
@@ -72,7 +74,10 @@ int pod_gram_fp32(const desmo_shape* s, const float* U, float* C, cudaStream_t s
     if (nsplit < 1) nsplit = 1;
     long long xchunk = ((s->n + nsplit - 1) / nsplit + kGX - 1) / kGX * kGX;
     nsplit = (s->n + xchunk - 1) / xchunk;
-    gram_fp32_kernel<<<dim3(npairs, (unsigned)nsplit), 256, 0, st>>>(U, s->ld, s->n, m, ntile, xchunk, C);
+    if (u_dtype == DESMO_DTYPE_BF16)
+        gram_fp32_kernel<<<dim3(npairs, (unsigned)nsplit), 256, 0, st>>>(static_cast<const __nv_bfloat16*>(U), s->ld, s->n, m, ntile, xchunk, C);
+    else
+        gram_fp32_kernel<<<dim3(npairs, (unsigned)nsplit), 256, 0, st>>>(static_cast<const float*>(U), s->ld, s->n, m, ntile, xchunk, C);
     DESMO_CUDA(cudaGetLastError());
     return DESMO_OK;
 }
@@ -282,7 +287,17 @@ int pod_eig(int m, int r, const float* C, float* V, float* sigma, void* workspac
 // ---------------------------------------------------------------------------------------------------------------
 // Back-projection: P[i][x] = sum_t U[t][x] V[i][t] / sigma_i   (streams U once, HBM-bound)
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) pod_project_kernel(const float* __restrict__ U, long long ld, long long n, int m, int r,
+__device__ __forceinline__ float4 ldg_u4(const float* U, long long t, long long ld, long long xv) {
+    return __ldg(reinterpret_cast<const float4*>(U + t * ld) + xv);
+}
+__device__ __forceinline__ float4 ldg_u4(const __nv_bfloat16* U, long long t, long long ld, long long xv) {  // one 8-byte load
+    const uint2 q = __ldg(reinterpret_cast<const uint2*>(U + t * ld) + xv);
+    return make_float4(__uint_as_float(q.x << 16), __uint_as_float(q.x & 0xffff0000u), __uint_as_float(q.y << 16),
+                       __uint_as_float(q.y & 0xffff0000u));
+}
+
+template <class UT>
+__global__ void __launch_bounds__(256) pod_project_kernel(const UT* __restrict__ U, long long ld, long long n, int m, int r,
                                                           const float* __restrict__ V, const float* __restrict__ sigma,
                                                           float* __restrict__ P) {
     extern __shared__ float Vs[];  // [m][kMaxR]
@@ -298,7 +313,7 @@ __global__ void __launch_bounds__(256) pod_project_kernel(const float* __restric
         for (int i = 0; i < kMaxR; ++i) acc[i][0] = acc[i][1] = acc[i][2] = acc[i][3] = 0.0f;
 #pragma unroll 4
         for (int t = 0; t < m; ++t) {
-            const float4 u = __ldg(reinterpret_cast<const float4*>(U + (long long)t * ld) + xv);
+            const float4 u = ldg_u4(U, t, ld, xv);
             const float4 v0 = *reinterpret_cast<const float4*>(Vs + t * kMaxR);
             const float4 v1 = *reinterpret_cast<const float4*>(Vs + t * kMaxR + 4);
             const float vv[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
@@ -325,12 +340,20 @@ __global__ void __launch_bounds__(256) pod_project_kernel(const float* __restric
     }
 }
 
-int pod_project(const desmo_shape* s, const float* U, const float* V, const float* sigma, float* P, cudaStream_t st) {
+template <class UT>
+static int launch_project(const desmo_shape* s, const UT* U, const float* V, const float* sigma, float* P, cudaStream_t st) {
     const size_t smem = sizeof(float) * (size_t)s->m * kMaxR;
-    DESMO_CUDA(cudaFuncSetAttribute(pod_project_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    DESMO_CUDA(cudaFuncSetAttribute(pod_project_kernel<UT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     long long g = (s->ld / 4 + 255) / 256;
     if (g > 148 * 4) g = 148 * 4;
-    pod_project_kernel<<<(unsigned)g, 256, smem, st>>>(U, s->ld, s->n, s->m, s->r, V, sigma, P);
+    pod_project_kernel<UT><<<(unsigned)g, 256, smem, st>>>(U, s->ld, s->n, s->m, s->r, V, sigma, P);
+    return DESMO_OK;
+}
+
+int pod_project(const desmo_shape* s, const void* U, int u_dtype, const float* V, const float* sigma, float* P, cudaStream_t st) {
+    const int rc = u_dtype == DESMO_DTYPE_BF16 ? launch_project(s, static_cast<const __nv_bfloat16*>(U), V, sigma, P, st)
+                                               : launch_project(s, static_cast<const float*>(U), V, sigma, P, st);
+    if (rc) return rc;
     DESMO_CUDA(cudaGetLastError());
     return DESMO_OK;
 }

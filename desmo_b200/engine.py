@@ -16,6 +16,7 @@ from . import _lib
 from ._lib import check, make_shape, round_up
 
 REFERENCE_LRS = (1e-2, 1e-3, 1e-2, 1e3, 1e-2)  # gates, phi, z, omega, periods  (CYL:592-612, FCYL:628-631)
+SNAPSHOT_CHUNK_BYTES = 256 << 20  # fp32 staging per chunk when set_snapshot converts into bf16 storage
 
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
@@ -27,9 +28,17 @@ class _PeerDesc(C.Structure):  # desmo_peer (include/desmo_b200.h)
 
 
 class DesmoEngine:
+    """``snapshot_dtype``: storage of the snapshot matrix U -- torch.float32 (default) or torch.bfloat16.  bf16 storage halves U's
+    memory and HBM traffic; every kernel widens it exactly to fp32, so training on it is bit-identical to fp32 storage of
+    U_q.float(), U_q = the snapshot rounded to bf16 (see snapshot_quantization_error).  fp16 is rejected: snapshots in physical units
+    would need a per-tensor scale to stay clear of its overflow / subnormal range; bf16 has fp32's range."""
+
     def __init__(self, n: int, m: int, polyorder: int, r: int, omega_init: float = 10000.0, nF: Optional[int] = None,
                  period_init: float = 60.0, device: Optional[torch.device] = None, n_global: Optional[int] = None,
-                 path: int = _lib.PATH_AUTO, process_group=None):
+                 path: int = _lib.PATH_AUTO, process_group=None, snapshot_dtype: torch.dtype = torch.float32):
+        if snapshot_dtype not in (torch.float32, torch.bfloat16):
+            raise _lib.DesmoError(f"snapshot_dtype must be torch.float32 or torch.bfloat16, got {snapshot_dtype}")
+        self.snapshot_dtype = snapshot_dtype
         self.lib = _lib.load()
         if device is None:
             device = torch.device("cuda", torch.cuda.current_device()) if torch.cuda.is_available() else None
@@ -53,6 +62,7 @@ class DesmoEngine:
         f32 = dict(dtype=torch.float32, device=self.device)
         z = lambda *s: torch.zeros(*s, **f32)  # noqa: E731
         self.U: Optional[torch.Tensor] = None
+        self._qsums: Optional[torch.Tensor] = None  # fp64 [sum (u - q)^2, sum u^2] of the last bf16 conversion of U
         self.P = z(self.r, self.ld)
         self.phi, self.phi_m, self.phi_u, self.dphi = z(self.r, self.ld), z(self.r, self.ld), z(self.r, self.ld), z(self.r, self.ld)
         self.phi[:, :self.n] = 1.0
@@ -95,12 +105,53 @@ class DesmoEngine:
         self.P[:, :self.n] = pm.to(torch.float32).t().to(self.device)
 
     def set_snapshot(self, snapshot: torch.Tensor, non_blocking: bool = True) -> None:
-        """The reference's (m, n) batch (CYL:708).  Host tensors are uploaded; any float dtype is cast to fp32."""
+        """The reference's (m, n) batch (CYL:708).  Host tensors are uploaded; any float dtype is cast to fp32.
+
+        bf16 storage: bf16 input is stored as it is; fp32 / fp64 input is rounded to bf16 (nearest even) by desmo_snapshot_to_bf16
+        in chunks of at most SNAPSHOT_CHUNK_BYTES of fp32, so the device never holds an fp32 copy of the whole matrix."""
         if tuple(snapshot.shape) != (self.m, self.n):
             raise ValueError(f"snapshot must be ({self.m}, {self.n}) like the reference batch, got {tuple(snapshot.shape)}")
+        if self.U is None or self.U.dtype != self.snapshot_dtype:
+            self.U = torch.zeros(self.m, self.ld, dtype=self.snapshot_dtype, device=self.device)
+        if self.snapshot_dtype == torch.float32:
+            self.U[:, :self.n].copy_(snapshot, non_blocking=non_blocking)
+            return
+        if snapshot.dtype == torch.bfloat16:
+            self.U[:, :self.n].copy_(snapshot, non_blocking=non_blocking)
+            self._qsums = None  # nothing was rounded
+            return
+        if snapshot.dtype not in (torch.float32, torch.float64):
+            raise _lib.DesmoError(f"bf16 storage takes fp32, fp64 or bf16 snapshots, got {snapshot.dtype}")
+        self._qsums = torch.zeros(2, dtype=torch.float64, device=self.device)
+        rows = max(1, min(self.m, SNAPSHOT_CHUNK_BYTES // (4 * self.n)))
+        with torch.cuda.device(self.device):
+            for t0 in range(0, self.m, rows):
+                part = snapshot[t0:t0 + rows]
+                if part.dtype != torch.float32 and part.device.type == "cpu":
+                    part = part.to(torch.float32)  # cast on the host: only fp32 crosses the bus
+                src = part.to(self.device, torch.float32, non_blocking=non_blocking).contiguous()
+                check(self.lib.desmo_snapshot_to_bf16(C.byref(self.shape), src.data_ptr(), src.stride(0), t0, src.shape[0],
+                                                      self.U.data_ptr(), self._qsums.data_ptr(), self._stream()),
+                      "desmo_snapshot_to_bf16")
+                del part, src  # the next chunk reuses this block: at most one chunk is resident
+
+    def snapshot_quantization_error(self) -> float:
+        """||U - U_q||_F / ||U||_F of the bf16 snapshot storage (fp64; over all ranks when point-sharded): U the fp32 snapshot the
+        fp32 path would train on, U_q what is stored.  0.0 for fp32 storage or a snapshot given in bf16."""
         if self.U is None:
-            self.U = torch.zeros(self.m, self.ld, dtype=torch.float32, device=self.device)
-        self.U[:, :self.n].copy_(snapshot, non_blocking=non_blocking)
+            raise _lib.DesmoError("no snapshot matrix set")
+        if self._qsums is None or self.U.dtype != torch.bfloat16:
+            return 0.0
+        q = self._qsums.clone()
+        if self._sharded():
+            torch.distributed.all_reduce(q, group=self.pg)
+        e2, u2 = q.tolist()
+        return (e2 / u2) ** 0.5 if u2 > 0 else 0.0
+
+    def _u_dtype(self) -> int:
+        if self.U is None:
+            raise _lib.DesmoError("no snapshot matrix set (call set_snapshot)")
+        return _lib.u_dtype_code(self.U.dtype)
 
     def set_hyper(self, lrs: Sequence[float], beta: float, l1_lambda: float) -> None:
         vals = list(lrs) + [REFERENCE_LRS[4]] * (5 - len(lrs)) + [beta, l1_lambda]
@@ -134,11 +185,10 @@ class DesmoEngine:
                                      self._stream()), "desmo_build_w")
 
     def fused_residual_grad(self, red: Optional[torch.Tensor] = None) -> None:
-        if self.U is None:
-            raise _lib.DesmoError("no snapshot matrix set (call set_snapshot)")
-        check(self.lib.desmo_fused_residual_grad(C.byref(self.shape), _ptr(self.U), _ptr(self.P), _ptr(self.phi), _ptr(self.omega),
-                                                 _ptr(self.W), _ptr(self.dphi), _ptr(self.red if red is None else red),
-                                                 _ptr(self.workspace), self._stream()),
+        ud = self._u_dtype()
+        check(self.lib.desmo_fused_residual_grad_ex(C.byref(self.shape), _ptr(self.U), ud, _ptr(self.P), _ptr(self.phi), _ptr(self.omega),
+                                                    _ptr(self.W), _ptr(self.dphi), _ptr(self.red if red is None else red),
+                                                    _ptr(self.workspace), self._stream()),
               "desmo_fused_residual_grad")
 
     def enable_peer_allreduce(self, group=None) -> bool:
@@ -219,19 +269,17 @@ class DesmoEngine:
                 self.fused_residual_grad(self.red_local)
                 check(self.lib.desmo_peer_allreduce(C.byref(self._peer), self._red_pad.numel(), _ptr(self._red_pad), st), "desmo_peer_allreduce")
             else:
-                if self.U is None:
-                    raise _lib.DesmoError("no snapshot matrix set (call set_snapshot)")
-                args = (C.byref(self.shape), _ptr(self.U), _ptr(self.P), _ptr(self.phi), _ptr(self.omega), _ptr(self.W), _ptr(self.dphi),
+                args = (C.byref(self.shape), _ptr(self.U), self._u_dtype(), _ptr(self.P), _ptr(self.phi), _ptr(self.omega), _ptr(self.W), _ptr(self.dphi),
                         _ptr(self.red), _ptr(self.workspace))
                 main = torch.cuda.current_stream(self.device)
                 if self._side is None:
                     self._side = torch.cuda.Stream(device=self.device)
                 ecount = self.Kp * self.mld
-                check(self.lib.desmo_fused_residual_grad_begin(*args, main.cuda_stream), "desmo_fused_residual_grad_begin")
+                check(self.lib.desmo_fused_residual_grad_begin_ex(*args, main.cuda_stream), "desmo_fused_residual_grad_begin")
                 self._side.wait_stream(main)
                 with torch.cuda.stream(self._side):
                     torch.distributed.all_reduce(self.red[:ecount], group=self.pg)
-                check(self.lib.desmo_fused_residual_grad_finish(*args, main.cuda_stream), "desmo_fused_residual_grad_finish")
+                check(self.lib.desmo_fused_residual_grad_finish_ex(*args, main.cuda_stream), "desmo_fused_residual_grad_finish")
                 torch.distributed.all_reduce(self.red[ecount:], group=self.pg)
                 main.wait_stream(self._side)
             self.adamax_update()
@@ -343,26 +391,28 @@ class DesmoEngine:
         """Reader output -> resident snapshot U on the device (desmo_preprocess): magnitude of the first ``d_use`` of ``d_in``
         velocity components (CYL:88-133), temporal-mean removal (CYL:136-149), optional 1/sqrt(m) (ANEU:143) and every
         ``t_stride``-th snapshot (TURB:189).  ``raw`` is X.T as read: [m_in, n*d_in], fp32 or fp64, on this device.
+        bf16 storage receives the fp32 result rounded once more (and the quantisation error is recorded).
         Returns the fp64 temporal mean [n] (the reference's X_mean)."""
         d_use = d_in if d_use is None else d_use
         if raw.device != self.device or raw.dtype not in (torch.float32, torch.float64) or raw.dim() != 2 or raw.stride(1) != 1:
             raise ValueError("raw must be a [m_in, n*d_in] fp32/fp64 tensor on the engine's device with unit inner stride")
         if raw.shape[1] != self.n * d_in:
             raise ValueError(f"raw has {raw.shape[1]} columns, expected n*d_in = {self.n * d_in}")
-        if self.U is None:
-            self.U = torch.empty(self.m, self.ld, dtype=torch.float32, device=self.device)
+        if self.U is None or self.U.dtype != self.snapshot_dtype:
+            self.U = torch.empty(self.m, self.ld, dtype=self.snapshot_dtype, device=self.device)
         mean = torch.empty(self.n, dtype=torch.float64, device=self.device)
         flags = (_lib.PRE_MAGNITUDE if magnitude else 0) | (_lib.PRE_SUBTRACT_MEAN if subtract_mean else 0) | \
                 (_lib.PRE_SCALE_SQRT_M if scale_sqrt_m else 0)
-        _lib.check(self.lib.desmo_preprocess(C.byref(self.shape), raw.data_ptr(), 1 if raw.dtype == torch.float64 else 0, raw.stride(0),
-                                             raw.shape[0], t_stride, d_in, d_use, flags, self.U.data_ptr(), mean.data_ptr(),
-                                             self._stream()), "desmo_preprocess")
+        bf16 = self.snapshot_dtype == torch.bfloat16
+        self._qsums = torch.zeros(2, dtype=torch.float64, device=self.device) if bf16 else None
+        _lib.check(self.lib.desmo_preprocess_ex(C.byref(self.shape), raw.data_ptr(), 1 if raw.dtype == torch.float64 else 0, raw.stride(0),
+                                                raw.shape[0], t_stride, d_in, d_use, flags, self.U.data_ptr(), self._u_dtype(),
+                                                _ptr(self._qsums), mean.data_ptr(), self._stream()), "desmo_preprocess")
         return mean
 
     def pod_from_snapshot(self) -> torch.Tensor:
         """Replaces POD_analysis (CYL:197-205) for the resident snapshot matrix: returns singular values (r,), fills self.P."""
-        if self.U is None:
-            raise _lib.DesmoError("no snapshot matrix set")
+        ud = self._u_dtype()
         f32 = dict(dtype=torch.float32, device=self.device)
         Cm = torch.zeros(self.m, self.m, **f32)
         V, sigma = torch.zeros(self.r, self.m, **f32), torch.zeros(self.r, **f32)
@@ -370,14 +420,15 @@ class DesmoEngine:
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
         with torch.cuda.device(self.device):
             ev[0].record()
-            check(self.lib.desmo_pod_gram(C.byref(self.shape), _ptr(self.U), _ptr(Cm), _ptr(self.workspace), self._stream()), "desmo_pod_gram")
+            check(self.lib.desmo_pod_gram_ex(C.byref(self.shape), _ptr(self.U), ud, _ptr(Cm), _ptr(self.workspace), self._stream()),
+                  "desmo_pod_gram")
             ev[1].record()
             if self.n_global != self.n and torch.distributed.is_initialized():
                 torch.distributed.all_reduce(Cm, group=self.pg)
             trace = Cm.diagonal().sum(dtype=torch.float64)  # = sum of all sigma^2 = ||X||_F^2 (the all-reduced Gram's trace)
             check(self.lib.desmo_pod_eig(self.m, self.r, _ptr(Cm), _ptr(V), _ptr(sigma), _ptr(ws), ws.numel(), self._stream()), "desmo_pod_eig")
             ev[2].record()
-            check(self.lib.desmo_pod_project(C.byref(self.shape), _ptr(self.U), _ptr(V), _ptr(sigma), _ptr(self.P), self._stream()),
+            check(self.lib.desmo_pod_project_ex(C.byref(self.shape), _ptr(self.U), ud, _ptr(V), _ptr(sigma), _ptr(self.P), self._stream()),
                   "desmo_pod_project")
             ev[3].record()
         torch.cuda.synchronize(self.device)

@@ -86,9 +86,10 @@ def _slice_grad(eng: DesmoEngine, g: dict, kind: str, idx) -> torch.Tensor:
 
 
 class _DesmoBase(nn.Module):
-    def _build(self, n, m, polyorder, r_DESMO, omega_init, nF, period_init, pod_modes, device, n_global, path, process_group):
+    def _build(self, n, m, polyorder, r_DESMO, omega_init, nF, period_init, pod_modes, device, n_global, path, process_group,
+               snapshot_dtype):
         self.engine = DesmoEngine(n, m, polyorder, r_DESMO, omega_init, nF, period_init, device=device, n_global=n_global,
-                                  path=path, process_group=process_group)
+                                  path=path, process_group=process_group, snapshot_dtype=snapshot_dtype)
         e = self.engine
         T, r = e.T, e.r
         print('Number of terms in polynomial library:', T)  # CYL:510
@@ -220,14 +221,19 @@ class _DesmoBase(nn.Module):
 
 
 class DESMO(_DesmoBase):
+    """``snapshot_dtype=torch.bfloat16`` stores the snapshot matrix in bf16 (see DesmoEngine)."""
+
     def __init__(self, n, m, polyorder, r_DESMO, omega_init=10000, *, pod_modes=None, device=None, n_global=None,
-                 path=_lib.PATH_AUTO, process_group=None):
+                 path=_lib.PATH_AUTO, process_group=None, snapshot_dtype=torch.float32):
         super().__init__()
-        self._build(n, m, polyorder, r_DESMO, omega_init, None, 0.0, pod_modes, device, n_global, path, process_group)
+        self._build(n, m, polyorder, r_DESMO, omega_init, None, 0.0, pod_modes, device, n_global, path, process_group, snapshot_dtype)
 
 
 class DESMOFourier(_DesmoBase):
+    """``snapshot_dtype=torch.bfloat16`` stores the snapshot matrix in bf16 (see DesmoEngine)."""
+
     def __init__(self, n, m, polyorder, r_DESMO, omega_init=10000, nF=10, *, period_init=60.0, pod_modes=None, device=None,
-                 n_global=None, path=_lib.PATH_AUTO, process_group=None):
+                 n_global=None, path=_lib.PATH_AUTO, process_group=None, snapshot_dtype=torch.float32):
         super().__init__()
-        self._build(n, m, polyorder, r_DESMO, omega_init, nF, period_init, pod_modes, device, n_global, path, process_group)
+        self._build(n, m, polyorder, r_DESMO, omega_init, nF, period_init, pod_modes, device, n_global, path, process_group,
+                    snapshot_dtype)

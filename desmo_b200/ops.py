@@ -1,11 +1,12 @@
 """torch custom ops over the C ABI: one ``torch.ops.desmo_b200.*`` op per hot-path entry point of include/desmo_b200.h.
 
   build_w, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, library_colnorm2, term_norms,
-  pod_gram, pod_eig, pod_project, preprocess, plateau_step, peer_begin_step, peer_allreduce
+  pod_gram, pod_eig, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce
 
 They take the packed device tensors of a DesmoEngine (layout: include/desmo_b200.h) plus the shape integers and launch the
 sm_100a kernels on the current stream.  CUDA only: no CPU implementation is registered and every op checks its tensors, so a call
-with CPU tensors fails loudly."""
+with CPU tensors fails loudly.  The ops that read the snapshot matrix U take it in fp32 or bf16 (dispatched on U.dtype); any other
+dtype raises before a launch."""
 from __future__ import annotations
 
 import ctypes as C
@@ -46,10 +47,11 @@ def fused_residual_grad(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, ome
                         red: torch.Tensor, workspace: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int, nF: int,
                         path: int) -> None:
     _require_cuda(U, P, phi, omega, W, dphi, red)
+    ud = _lib.u_dtype_code(U.dtype)
     s = make_shape(n, m, r, polyorder, nF, n_global, path)
     with torch.cuda.device(U.device):
-        check(_lib.load().desmo_fused_residual_grad(C.byref(s), _p(U), _p(P), _p(phi), _p(omega), _p(W), _p(dphi), _p(red),
-                                                    _p(workspace), _stream(U)), "desmo_fused_residual_grad")
+        check(_lib.load().desmo_fused_residual_grad_ex(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), _p(dphi), _p(red),
+                                                       _p(workspace), _stream(U)), "desmo_fused_residual_grad")
 
 
 @torch.library.custom_op("desmo_b200::recon_backward", mutates_args=("dphi", "red", "workspace"))
@@ -128,9 +130,10 @@ def term_norms(g2: torch.Tensor, gates: torch.Tensor, rows: torch.Tensor, fourie
 def pod_gram(U: torch.Tensor, Cm: torch.Tensor, workspace: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int, nF: int,
              path: int) -> None:
     _require_cuda(U, Cm, workspace)
+    ud = _lib.u_dtype_code(U.dtype)
     s = make_shape(n, m, r, polyorder, nF, n_global, path)
     with torch.cuda.device(U.device):
-        check(_lib.load().desmo_pod_gram(C.byref(s), _p(U), _p(Cm), _p(workspace), _stream(U)), "desmo_pod_gram")
+        check(_lib.load().desmo_pod_gram_ex(C.byref(s), _p(U), ud, _p(Cm), _p(workspace), _stream(U)), "desmo_pod_gram")
 
 
 @torch.library.custom_op("desmo_b200::pod_eig", mutates_args=("V", "sigma", "workspace"))
@@ -145,21 +148,42 @@ def pod_eig(Cm: torch.Tensor, V: torch.Tensor, sigma: torch.Tensor, workspace: t
 def pod_project(U: torch.Tensor, V: torch.Tensor, sigma: torch.Tensor, P: torch.Tensor, n: int, n_global: int, m: int, r: int,
                 polyorder: int, nF: int, path: int) -> None:
     _require_cuda(U, V, sigma, P)
+    ud = _lib.u_dtype_code(U.dtype)
     s = make_shape(n, m, r, polyorder, nF, n_global, path)
     with torch.cuda.device(U.device):
-        check(_lib.load().desmo_pod_project(C.byref(s), _p(U), _p(V), _p(sigma), _p(P), _stream(U)), "desmo_pod_project")
+        check(_lib.load().desmo_pod_project_ex(C.byref(s), _p(U), ud, _p(V), _p(sigma), _p(P), _stream(U)), "desmo_pod_project")
 
 
 @torch.library.custom_op("desmo_b200::preprocess", mutates_args=("U", "mean"))
 def preprocess(V: torch.Tensor, U: torch.Tensor, mean: Optional[torch.Tensor], m_in: int, t_stride: int, d_in: int, d_use: int, flags: int,
                n: int, n_global: int, m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """U is written in its own dtype: fp32, or bf16 (the fp32 result rounded to nearest even once more)."""
     _require_cuda(V, U, mean)
     if V.dtype not in (torch.float32, torch.float64) or V.dim() != 2 or V.stride(1) != 1:
         raise ValueError("V must be a [m_in, n*d_in] fp32/fp64 tensor with unit inner stride")
+    ud = _lib.u_dtype_code(U.dtype)
     s = make_shape(n, m, r, polyorder, nF, n_global, path)
     with torch.cuda.device(V.device):
-        check(_lib.load().desmo_preprocess(C.byref(s), _p(V), 1 if V.dtype == torch.float64 else 0, V.stride(0), m_in, t_stride, d_in, d_use,
-                                           flags, _p(U), _p(mean), _stream(V)), "desmo_preprocess")
+        check(_lib.load().desmo_preprocess_ex(C.byref(s), _p(V), 1 if V.dtype == torch.float64 else 0, V.stride(0), m_in, t_stride, d_in,
+                                              d_use, flags, _p(U), ud, None, _p(mean), _stream(V)), "desmo_preprocess")
+
+
+@torch.library.custom_op("desmo_b200::snapshot_to_bf16", mutates_args=("U", "qsums"))
+def snapshot_to_bf16(src: torch.Tensor, U: torch.Tensor, qsums: Optional[torch.Tensor], t0: int, n: int, n_global: int, m: int, r: int,
+                     polyorder: int, nF: int, path: int) -> None:
+    """fp32 rows src [rows, >= n] -> bf16 U[t0 : t0 + rows, :] (round to nearest even, pad columns zeroed); qsums (fp64 [2], optional)
+    += {sum (u - q)^2, sum u^2} (desmo_snapshot_to_bf16)."""
+    _require_cuda(src, U, qsums)
+    if src.dtype != torch.float32 or src.dim() != 2 or src.stride(1) != 1:
+        raise ValueError("src must be a [rows, >= n] fp32 tensor with unit inner stride")
+    if U.dtype != torch.bfloat16:
+        raise _lib.DesmoError(f"snapshot_to_bf16 writes a bfloat16 U, got {U.dtype}")
+    if qsums is not None and (qsums.dtype != torch.float64 or qsums.numel() < 2):
+        raise ValueError("qsums must be a float64 tensor of 2 elements")
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(U.device):
+        check(_lib.load().desmo_snapshot_to_bf16(C.byref(s), _p(src), src.stride(0), t0, src.shape[0], _p(U), _p(qsums), _stream(U)),
+              "desmo_snapshot_to_bf16")
 
 
 @torch.library.custom_op("desmo_b200::plateau_step", mutates_args=("state", "hyper"))

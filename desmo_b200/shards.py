@@ -206,9 +206,10 @@ class ShardReader:
 
 def model_from_shards(shard_dir: str, polyorder: int, r_DESMO: int, omega_init: float = 10000.0, *, d_use: Optional[int] = None,
                       magnitude: bool = True, subtract_mean: bool = True, scale_sqrt_m: bool = False, t_stride: int = 1, nF: Optional[int] = None,
-                      period_init: float = 60.0, device=None, path: int = 0):
+                      period_init: float = 60.0, device=None, path: int = 0, snapshot_dtype=None):
     """Data ingest + pre-processing + POD init of the scripts (CYL:157-205, ANEU:143, TURB:189) for this rank's slab: returns
-    (model, X_mean [n_local] fp64, singular values).  Under torch.distributed every rank calls it; the Gram is all-reduced."""
+    (model, X_mean [n_local] fp64, singular values).  Under torch.distributed every rank calls it; the Gram is all-reduced.
+    ``snapshot_dtype=torch.bfloat16`` pre-processes straight into bf16 storage (default: fp32)."""
     import torch
     import torch.distributed as dist
 
@@ -224,7 +225,7 @@ def model_from_shards(shard_dir: str, polyorder: int, r_DESMO: int, omega_init: 
     n_local, n_global = hi - lo, rd.n_points
     m = (rd.m_in + t_stride - 1) // t_stride
     dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
-    kw = dict(device=dev, n_global=n_global, path=path)
+    kw = dict(device=dev, n_global=n_global, path=path, snapshot_dtype=snapshot_dtype or torch.float32)
     model = (DESMOFourier(n_local, m, polyorder, r_DESMO, omega_init, nF, period_init=period_init, **kw) if nF
              else DESMO(n_local, m, polyorder, r_DESMO, omega_init, **kw))
     raw = rd.load_slab(rank, world, pinned=True).to(dev, non_blocking=True)

@@ -13,9 +13,11 @@
  *     synchronise, except the *_host entry points, which return after their results are in host memory.
  *   - no CPU fallback: every entry point fails (DESMO_ERR_CUDA) if no sm_100 device is usable.
  *
- * Device data layout (all fp32, row pitch in elements)
+ * Device data layout (all fp32 except U, row pitch in elements)
  *   U      [m][ld]      snapshot matrix, time-major like the reference's `snapshot` batch (CYL:708); ld >= n, ld % 128 == 0,
- *                        columns n..ld-1 must be zero.
+ *                        columns n..ld-1 must be zero.  fp32, or bf16 through the *_ex entry points (u_dtype =
+ *                        DESMO_DTYPE_BF16): the kernels widen each element exactly to fp32 and compute exactly what the fp32
+ *                        entry points compute on U_q.float(); half the memory and the HBM traffic of the snapshot.
  *   P      [r][ld]      POD modes, mode-major (POD_modes[:, i] of CYL:204,538-541), zero in the padding.
  *   phi    [r][ld]      phi_list[i] (CYL:506); likewise its Adamax state exp_avg / exp_inf.
  *   gates  [K]          [c_coef (T) | sin_coef (r) | cos_coef (r) | tanh_coef (r)]              (CYL:513,524-526)
@@ -105,6 +107,15 @@ int desmo_fused_residual_grad_begin(const desmo_shape* s, const float* U, const 
 int desmo_fused_residual_grad_finish(const desmo_shape* s, const float* U, const float* P, const float* phi, const float* omega,
                                      const float* W, float* dphi, float* red, void* workspace, void* stream);
 
+/* The three calls above for a snapshot matrix of element type u_dtype (DESMO_DTYPE_F32 or DESMO_DTYPE_BF16; anything else is
+ * DESMO_ERR_ARG).  The fp32 entry points are these with DESMO_DTYPE_F32.  Path selection does not depend on u_dtype. */
+int desmo_fused_residual_grad_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                 const float* omega, const float* W, float* dphi, float* red, void* workspace, void* stream);
+int desmo_fused_residual_grad_begin_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                       const float* omega, const float* W, float* dphi, float* red, void* workspace, void* stream);
+int desmo_fused_residual_grad_finish_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                        const float* omega, const float* W, float* dphi, float* red, void* workspace, void* stream);
+
 /* Backward of forward()'s reconstruction for an ARBITRARY upstream gradient (what autograd runs when the reference loop does
  * `recon, _, _ = model(snapshot); loss = criterion(recon, snapshot); total_loss.backward()`, CYL:711,722,766): grad_recon[m][ld]
  * = dL/drecon in the layout of U (pad columns zero).  Same kernels and outputs as desmo_fused_residual_grad with R := (n_global *
@@ -183,6 +194,10 @@ int desmo_pod_gram(const desmo_shape* s, const float* U, float* C, void* workspa
 int desmo_pod_eig(int32_t m, int32_t r, const float* C, float* V, float* sigma, void* workspace, size_t workspace_bytes,
                   void* stream);
 int desmo_pod_project(const desmo_shape* s, const float* U, const float* V, const float* sigma, float* P, void* stream);
+/* ... for a snapshot matrix of element type u_dtype (DESMO_DTYPE_F32 / DESMO_DTYPE_BF16).  The bf16 tcgen05 Gram feeds the stored
+ * rows to the tensor core as they are (one plane, 4 instead of 24 MMAs per chunk) and equals the fp32 Gram of U_q.float(). */
+int desmo_pod_gram_ex(const desmo_shape* s, const void* U, int32_t u_dtype, float* C, void* workspace, void* stream);
+int desmo_pod_project_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* V, const float* sigma, float* P, void* stream);
 
 /* Snapshot pre-processing between the reader and POD/training, on the device (reference: numpy on the host).  V is X.T as
  * read: V[m_in][v_ld] with v_ld >= n * d_in, a point's d_in components adjacent.  Replaces convert3Dto2D_data (CYL:88-106:
@@ -192,11 +207,23 @@ int desmo_pod_project(const desmo_shape* s, const float* U, const float* V, cons
  * if mean != NULL, the fp64 temporal mean[n] (X_mean). */
 #define DESMO_DTYPE_F32 0
 #define DESMO_DTYPE_F64 1
+#define DESMO_DTYPE_BF16 2
 #define DESMO_PRE_MAGNITUDE 1
 #define DESMO_PRE_SUBTRACT_MEAN 2
 #define DESMO_PRE_SCALE_SQRT_M 4
 int desmo_preprocess(const desmo_shape* s, const void* V, int32_t v_dtype, int64_t v_ld, int32_t m_in, int32_t t_stride,
                      int32_t d_in, int32_t d_use, int32_t flags, float* U, double* mean, void* stream);
+/* ... writing U in u_dtype: DESMO_DTYPE_F32 as above, or DESMO_DTYPE_BF16 = the fp32 value rounded to nearest even once more (what
+ * fp32 output followed by a bf16 cast stores).  qsums (bf16 output only, may be NULL): fp64 [2] += {sum (u - q)^2, sum u^2} over the
+ * n real points and s->m snapshots, u the fp32 value and q the stored one; summed in a fixed order (reproducible). */
+int desmo_preprocess_ex(const desmo_shape* s, const void* V, int32_t v_dtype, int64_t v_ld, int32_t m_in, int32_t t_stride,
+                        int32_t d_in, int32_t d_use, int32_t flags, void* U, int32_t u_dtype, double* qsums, double* mean, void* stream);
+
+/* fp32 snapshot rows -> bf16 storage: src[rows][src_ld] (device, fp32, src_ld >= n) -> U[t0 .. t0 + rows)[ld] (bf16), each value
+ * rounded to nearest even (cvt.rn.bf16x2.f32, = torch's .bfloat16()), columns n..ld-1 zeroed.  Lets a caller fill a bf16 U in
+ * chunks without holding an fp32 copy of the whole matrix.  qsums (may be NULL) as for desmo_preprocess_ex over these rows. */
+int desmo_snapshot_to_bf16(const desmo_shape* s, const float* src, int64_t src_ld, int32_t t0, int32_t rows, void* U, double* qsums,
+                           void* stream);
 
 /* torch.optim.lr_scheduler.ReduceLROnPlateau (mode 'min', relative threshold, cooldown 0; CYL:614,776-778, ANEU:613) ON THE DEVICE:
  * the reference steps it on the host with `total_loss`, i.e. one device->host round trip per scheduler epoch.  desmo_plateau_step is
