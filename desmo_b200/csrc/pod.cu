@@ -2,6 +2,8 @@
 //   C = U U^T (m x m Gram over mesh points; the one dense contraction)  ->  top-r eigenpairs (lambda_i, v_i) on device
 //   ->  POD mode i = X v_i / sqrt(lambda_i), i.e. P[i][x] = sum_t U[t][x] v_i[t] / sigma_i.
 // Point-sharded: each rank forms the Gram of its slab, one all-reduce of C, replicated eigensolve, local projection.
+#include <algorithm>
+
 #include "common.cuh"
 
 namespace desmo {
@@ -83,14 +85,35 @@ int pod_gram_fp32(const desmo_shape* s, const void* U, int u_dtype, float* C, cu
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Top-r eigenpairs of the (all-reduced) Gram: block subspace iteration with b = r + 8 vectors in fp64,
-// modified Gram-Schmidt each sweep, Rayleigh-Ritz (cyclic Jacobi on the b x b projection) at the end.
+// Top-r eigenpairs of the (all-reduced) Gram: block subspace iteration with b = min(r + 8, 16, m) vectors in fp64, CGS2 each
+// sweep, Rayleigh-Ritz (cyclic Jacobi on the b x b projection).  After kEigMinIters sweeps, and every kEigCheckEvery sweeps after
+// that, a Rayleigh-Ritz pass emits the top r pairs and measures their residuals ||C x_i - theta_i x_i||; the iteration stops once
+// every mode above the floor has a residual <= 2^-27 lambda_1, at the latest after a cap of 240 (r <= 8) or 600 sweeps.  The stop is a device
+// flag: the launches of the capped loop that follow it return at once, so the solver stays stream-ordered and capturable.
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kEigMaxB = 16;
+constexpr int kEigMinIters = 120;    // sweeps before the first check: r <= 8 results stay those of the fixed 120-sweep solver
+constexpr int kEigCheckEvery = 20;
+// Cap.  Every sweep enqueued after convergence still costs two launches that return at once (~1.2 us each on a B200), so the cap
+// follows the number of guard vectors: with 8 (r <= 8) a spectrum as flat as sigma_i ~ (i+1)^-0.15 converges within 120 sweeps;
+// with 2 (r = 14) it needs ~300.
+constexpr int kEigMaxItersSmallR = 240, kEigMaxIters = 600;
+constexpr double kEigTol = 0x1p-27;  // residual / lambda_1 (7.5e-9): 2x below the fp32 rounding of C
 
-__global__ void __launch_bounds__(256) eig_init_kernel(int m, int b, double* V) {
+// workspace head: written by the solver, read by the caller after the stream has passed the eigensolve (include/desmo_b200.h)
+struct EigState {
+    int32_t iterations;  // sweeps run before the emitted Rayleigh-Ritz pass
+    int32_t converged;   // 1: every mode above the floor met the residual bound
+    int32_t done;        // stop flag of the capped loop
+    int32_t pad;
+    double residual;     // max_i ||C x_i - theta_i x_i|| / lambda_1 over the modes above the floor
+};
+constexpr size_t kEigStateBytes = 256;
+
+__global__ void __launch_bounds__(256) eig_init_kernel(int m, int b, double* V, EigState* st) {
     // deterministic, well-spread start: V[j][t] = cos(pi (j+1)(t+0.5)/m) + small hash noise
     const int t = blockIdx.x * 256 + threadIdx.x;
+    if (t == 0) *st = EigState{0, 0, 0, 0, 0.0};
     if (t >= m) return;
     for (int j = 0; j < b; ++j) {
         unsigned h = (unsigned)(t * 2654435761u) ^ (unsigned)((j + 1) * 40503u);
@@ -99,9 +122,10 @@ __global__ void __launch_bounds__(256) eig_init_kernel(int m, int b, double* V) 
     }
 }
 
-// Y[j][t] = sum_s C[t][s] V[j][s]   (one warp per row t)
+// Y[j][t] = sum_s C[t][s] V[j][s]   (one warp per row t).  done: the stop flag, NULL for the sweeps before the first check.
 __global__ void __launch_bounds__(256) eig_matvec_kernel(int m, int b, const float* __restrict__ C, const double* __restrict__ V,
-                                                         double* __restrict__ Y) {
+                                                         double* __restrict__ Y, const int32_t* done) {
+    if (done && *done) return;
     const int t = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (t >= m) return;
     double acc[kEigMaxB];
@@ -134,7 +158,9 @@ __device__ double block_sum_d(double v, double* sh) {  // blockDim.x == 1024
 // Classical Gram-Schmidt with re-orthogonalisation (CGS2) of Y (b vectors of length m) -> V, single CTA.  All projections of a
 // column onto the previous ones are formed in ONE pass and ONE block reduction (a modified Gram-Schmidt needs one reduction per
 // pair: 4x more barriers for the same numerical quality once every column is orthogonalised twice).
-__global__ void __launch_bounds__(1024) eig_orth_kernel(int m, int b, const double* __restrict__ Y, double* __restrict__ V) {
+__global__ void __launch_bounds__(1024) eig_orth_kernel(int m, int b, const double* __restrict__ Y, double* __restrict__ V,
+                                                        const int32_t* done) {
+    if (done && *done) return;
     __shared__ double sh[32];
     __shared__ double part[32][kEigMaxB];
     __shared__ double dsum[kEigMaxB];
@@ -181,9 +207,13 @@ __global__ void __launch_bounds__(1024) eig_orth_kernel(int m, int b, const doub
     }
 }
 
-// Rayleigh-Ritz: H = V^T (C V) = V^T Y (b x b), Jacobi eigen-decomposition, rotate, sort, sign-normalise, emit top r.
-__global__ void __launch_bounds__(1024) eig_ritz_kernel(int m, int b, int r, const double* __restrict__ V, const double* __restrict__ Y,
-                                                        float* __restrict__ Vout, float* __restrict__ sigma) {
+// Rayleigh-Ritz: H = V^T (C V) = V^T Y (b x b), Jacobi eigen-decomposition, rotate, sort, sign-normalise, emit top r, and the
+// residuals ||Y q_i - theta_i V q_i|| = ||C x_i - theta_i x_i|| of the emitted pairs.  Floor: a Ritz value theta_i <= 2^-23 trace(C)
+// is at the rounding level of the fp32 Gram (its eigenvector is noise); it is emitted as sigma_i = 0 and left out of the stop test.
+__global__ void __launch_bounds__(1024) eig_ritz_kernel(int m, int b, int r, const float* __restrict__ C, const double* __restrict__ V,
+                                                        const double* __restrict__ Y, float* __restrict__ Vout, float* __restrict__ sigma,
+                                                        EigState* __restrict__ state, int iteration, int last) {
+    if (state->done) return;
     __shared__ double sh[32];
     __shared__ double H[kEigMaxB][kEigMaxB], Q[kEigMaxB][kEigMaxB];
     __shared__ int order[kEigMaxB];
@@ -194,10 +224,16 @@ __global__ void __launch_bounds__(1024) eig_ritz_kernel(int m, int b, int r, con
             d = block_sum_d(d, sh);
             if (threadIdx.x == 0) { H[i][j] = d; H[j][i] = d; }
         }
+    double trace = 0.0;
+    for (int t = threadIdx.x; t < m; t += 1024) trace += (double)C[(size_t)t * m + t];
+    trace = block_sum_d(trace, sh);
     __syncthreads();
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < b; ++i)
-            for (int j = 0; j < b; ++j) Q[i][j] = (i == j) ? 1.0 : 0.0;
+    if (threadIdx.x < 32) {
+        // cyclic Jacobi, one warp: every lane derives the same rotation, lane k updates row / column k (the serial sweep's arithmetic)
+        const int k = threadIdx.x;
+        if (k < b)
+            for (int j = 0; j < b; ++j) Q[k][j] = (k == j) ? 1.0 : 0.0;
+        __syncwarp();
         for (int sweep = 0; sweep < 30; ++sweep) {
             double off = 0.0;
             for (int p = 0; p < b; ++p)
@@ -209,38 +245,49 @@ __global__ void __launch_bounds__(1024) eig_ritz_kernel(int m, int b, int r, con
                     const double theta = (H[q][q] - H[p][p]) / (2.0 * H[p][q]);
                     const double tt = (theta >= 0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
                     const double c = 1.0 / sqrt(tt * tt + 1.0), s2 = tt * c;
-                    for (int k = 0; k < b; ++k) {
+                    __syncwarp();
+                    if (k < b) {
                         const double hkp = H[k][p], hkq = H[k][q];
                         H[k][p] = c * hkp - s2 * hkq;
                         H[k][q] = s2 * hkp + c * hkq;
                     }
-                    for (int k = 0; k < b; ++k) {
+                    __syncwarp();
+                    if (k < b) {
                         const double hpk = H[p][k], hqk = H[q][k];
                         H[p][k] = c * hpk - s2 * hqk;
                         H[q][k] = s2 * hpk + c * hqk;
-                    }
-                    for (int k = 0; k < b; ++k) {
                         const double qkp = Q[k][p], qkq = Q[k][q];
                         Q[k][p] = c * qkp - s2 * qkq;
                         Q[k][q] = s2 * qkp + c * qkq;
                     }
+                    __syncwarp();
                 }
         }
-        for (int i = 0; i < b; ++i) order[i] = i;
-        for (int i = 0; i < b; ++i)
-            for (int j = i + 1; j < b; ++j)
-                if (H[order[j]][order[j]] > H[order[i]][order[i]]) { const int tmp = order[i]; order[i] = order[j]; order[j] = tmp; }
+        if (k == 0) {
+            for (int i = 0; i < b; ++i) order[i] = i;
+            for (int i = 0; i < b; ++i)
+                for (int j = i + 1; j < b; ++j)
+                    if (H[order[j]][order[j]] > H[order[i]][order[i]]) { const int tmp = order[i]; order[i] = order[j]; order[j] = tmp; }
+        }
     }
     __syncthreads();
+    const double lam1 = H[order[0]][order[0]], floor_lam = 0x1p-23 * trace;
+    double worst = 0.0;
     for (int i = 0; i < r; ++i) {
         const int col = order[i];
+        const double th = H[col][col];
         // ritz vector = sum_j Q[j][col] V[j]; find the largest-|.| entry for the sign convention
-        double best = 0.0;
+        double best = 0.0, res2 = 0.0;
         for (int t = threadIdx.x; t < m; t += 1024) {
-            double v = 0.0;
-            for (int j = 0; j < b; ++j) v += Q[j][col] * V[(size_t)j * m + t];
+            double v = 0.0, cv = 0.0;
+            for (int j = 0; j < b; ++j) {
+                v += Q[j][col] * V[(size_t)j * m + t];
+                cv += Q[j][col] * Y[(size_t)j * m + t];
+            }
             if (fabs(v) > fabs(best)) best = v;
+            res2 += (cv - th * v) * (cv - th * v);
         }
+        res2 = block_sum_d(res2, sh);
         // block arg-max of |best|
         __syncthreads();
         double cand = best;
@@ -259,33 +306,53 @@ __global__ void __launch_bounds__(1024) eig_ritz_kernel(int m, int b, int r, con
             for (int j = 0; j < b; ++j) v += Q[j][col] * V[(size_t)j * m + t];
             Vout[(size_t)i * m + t] = (float)(flip * v);
         }
-        if (threadIdx.x == 0) sigma[i] = (float)sqrt(fmax(H[col][col], 0.0));
+        const bool floored = !(th > floor_lam);
+        if (!floored) worst = fmax(worst, sqrt(res2) / lam1);
+        if (threadIdx.x == 0) sigma[i] = floored ? 0.0f : (float)sqrt(th);
         __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        const int ok = worst <= kEigTol;
+        state->iterations = iteration;
+        state->converged = ok;
+        state->residual = worst;
+        state->done = ok || last;
     }
 }
 
 int pod_eig(int m, int r, const float* C, float* V, float* sigma, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-    const int b = (r + 8 <= kEigMaxB) ? r + 8 : kEigMaxB;
-    if (r > kEigMaxB - 2 || b > m) { set_error("pod_eig: r=%d unsupported for m=%d", r, m); return DESMO_ERR_UNSUPPORTED; }
-    const size_t need = 2 * sizeof(double) * (size_t)b * m;
-    if (workspace_bytes < need) { set_error("pod_eig: workspace too small (%zu < %zu)", workspace_bytes, need); return DESMO_ERR_ARG; }
-    double* Vd = static_cast<double*>(workspace);
-    double* Yd = Vd + (size_t)b * m;
-    eig_init_kernel<<<(m + 255) / 256, 256, 0, st>>>(m, b, Yd);
-    eig_orth_kernel<<<1, 1024, 0, st>>>(m, b, Yd, Vd);
-    const int iters = 120;
-    for (int it = 0; it < iters; ++it) {
-        eig_matvec_kernel<<<(m + 7) / 8, 256, 0, st>>>(m, b, C, Vd, Yd);
-        eig_orth_kernel<<<1, 1024, 0, st>>>(m, b, Yd, Vd);
+    if (r > kEigMaxB - 2) {
+        set_error("pod_eig: r=%d exceeds the on-device eigensolver's limit r <= %d", r, kEigMaxB - 2);
+        return DESMO_ERR_UNSUPPORTED;
     }
-    eig_matvec_kernel<<<(m + 7) / 8, 256, 0, st>>>(m, b, C, Vd, Yd);
-    eig_ritz_kernel<<<1, 1024, 0, st>>>(m, b, r, Vd, Yd, V, sigma);
+    if (r > m) { set_error("pod_eig: r=%d modes of an m=%d Gram", r, m); return DESMO_ERR_ARG; }
+    const int b = std::min(std::min(r + 8, kEigMaxB), m);
+    const size_t need = kEigStateBytes + 2 * sizeof(double) * (size_t)b * m;
+    if (workspace_bytes < need) { set_error("pod_eig: workspace too small (%zu < %zu)", workspace_bytes, need); return DESMO_ERR_ARG; }
+    EigState* state = static_cast<EigState*>(workspace);
+    const int32_t* done = &state->done;
+    double* Vd = reinterpret_cast<double*>(static_cast<char*>(workspace) + kEigStateBytes);
+    double* Yd = Vd + (size_t)b * m;
+    eig_init_kernel<<<(m + 255) / 256, 256, 0, st>>>(m, b, Yd, state);
+    eig_orth_kernel<<<1, 1024, 0, st>>>(m, b, Yd, Vd, nullptr);
+    const int max_iters = r <= 8 ? kEigMaxItersSmallR : kEigMaxIters;
+    for (int it = 0;; ++it) {
+        const bool checked = it >= kEigMinIters;
+        eig_matvec_kernel<<<(m + 7) / 8, 256, 0, st>>>(m, b, C, Vd, Yd, checked ? done : nullptr);
+        if (checked && (it - kEigMinIters) % kEigCheckEvery == 0) {
+            const int last = it >= max_iters;
+            eig_ritz_kernel<<<1, 1024, 0, st>>>(m, b, r, C, Vd, Yd, V, sigma, state, it, last);
+            if (last) break;
+        }
+        eig_orth_kernel<<<1, 1024, 0, st>>>(m, b, Yd, Vd, checked ? done : nullptr);
+    }
     DESMO_CUDA(cudaGetLastError());
     return DESMO_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Back-projection: P[i][x] = sum_t U[t][x] V[i][t] / sigma_i   (streams U once, HBM-bound)
+// Back-projection: P[i][x] = sum_t U[t][x] V[i][t] / sigma_i   (HBM-bound; one pass over U per group of kMaxR modes, the groups
+// are blockIdx.y; a floored mode, sigma_i = 0, gets a zero row)
 // ---------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float4 ldg_u4(const float* U, long long t, long long ld, long long xv) {
     return __ldg(reinterpret_cast<const float4*>(U + t * ld) + xv);
@@ -300,7 +367,12 @@ template <class UT>
 __global__ void __launch_bounds__(256) pod_project_kernel(const UT* __restrict__ U, long long ld, long long n, int m, int r,
                                                           const float* __restrict__ V, const float* __restrict__ sigma,
                                                           float* __restrict__ P) {
-    extern __shared__ float Vs[];  // [m][kMaxR]
+    extern __shared__ float Vs[];  // [m][kMaxR]: modes g0 .. g0 + kMaxR - 1
+    const int g0 = blockIdx.y * kMaxR;
+    V += (size_t)g0 * m;
+    sigma += g0;
+    P += (long long)g0 * ld;
+    r -= g0;
     for (int e = threadIdx.x; e < m * kMaxR; e += 256) {
         const int t = e / kMaxR, i = e % kMaxR;
         Vs[e] = (i < r) ? V[(size_t)i * m + t] : 0.0f;
@@ -328,7 +400,7 @@ __global__ void __launch_bounds__(256) pod_project_kernel(const UT* __restrict__
 #pragma unroll
         for (int i = 0; i < kMaxR; ++i)
             if (i < r) {
-                const float inv = 1.0f / sigma[i];
+                const float inv = sigma[i] > 0.0f ? 1.0f / sigma[i] : 0.0f;
                 const long long x = xv * 4;
                 float4 o;
                 o.x = (x + 0 < n) ? acc[i][0] * inv : 0.0f;
@@ -346,7 +418,8 @@ static int launch_project(const desmo_shape* s, const UT* U, const float* V, con
     DESMO_CUDA(cudaFuncSetAttribute(pod_project_kernel<UT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     long long g = (s->ld / 4 + 255) / 256;
     if (g > 148 * 4) g = 148 * 4;
-    pod_project_kernel<UT><<<(unsigned)g, 256, smem, st>>>(U, s->ld, s->n, s->m, s->r, V, sigma, P);
+    const unsigned groups = (unsigned)((s->r + kMaxR - 1) / kMaxR);
+    pod_project_kernel<UT><<<dim3((unsigned)g, groups), 256, smem, st>>>(U, s->ld, s->n, s->m, s->r, V, sigma, P);
     return DESMO_OK;
 }
 

@@ -411,7 +411,11 @@ class DesmoEngine:
         return mean
 
     def pod_from_snapshot(self) -> torch.Tensor:
-        """Replaces POD_analysis (CYL:197-205) for the resident snapshot matrix: returns singular values (r,), fills self.P."""
+        """Replaces POD_analysis (CYL:197-205) for the resident snapshot matrix: returns singular values (r,), fills self.P.
+
+        r <= 14 (the on-device eigensolver's limit; a larger r raises before P is touched).  A mode whose eigenvalue is at the rounding
+        level of the fp32 Gram (lambda_i <= 2^-23 trace) comes back as sigma_i = 0 with a zero row of P.  Raises DesmoError when the
+        eigensolver does not converge (P then holds the projection of the unconverged modes)."""
         ud = self._u_dtype()
         f32 = dict(dtype=torch.float32, device=self.device)
         Cm = torch.zeros(self.m, self.m, **f32)
@@ -434,6 +438,11 @@ class DesmoEngine:
         torch.cuda.synchronize(self.device)
         self.pod_timing = {"gram_ms": ev[0].elapsed_time(ev[1]), "eig_ms": ev[1].elapsed_time(ev[2]), "project_ms": ev[2].elapsed_time(ev[3])}
         self.pod_V, self.pod_gram = V, Cm
+        # the eigensolver's report at the head of its workspace (desmo_pod_eig): sweeps, converged flag, worst residual / lambda_1
+        iterations, converged = ws[:8].view(torch.int32).tolist()
+        self.pod_eig_iterations, self.pod_eig_residual = iterations, float(ws[16:24].view(torch.float64).item())
+        if not converged:
+            raise _lib.DesmoError(f"desmo_pod_eig did not converge in {iterations} sweeps (residual {self.pod_eig_residual:.2e} lambda_1)")
         # POD_analysis' diagnostics (CYL:200-211) without forming X_approx: energy_content = S^2 / sum(S^2) of the r leading modes, its
         # running sum, and err_POD = ||X - X_r|| / ||X|| = sqrt(1 - sum_{i<r} sigma_i^2 / ||X||_F^2) (Eckart-Young)
         s2 = sigma.double() ** 2

@@ -188,8 +188,15 @@ int desmo_debug_timers(const desmo_shape* s, void* workspace, uint64_t* out_host
 
 /* POD by the method of snapshots (replaces np.linalg.svd, CYL:197-205):
  *   gram    C[m][m] = U U^T  (local partial; tcgen05 tiles with every fp32 operand split into three bf16 planes) -- all-reduce it across ranks
- *   eig     top-r eigenpairs of C (replicated, on device): sigma[r] = sqrt(lambda), V[r][m]
- *   project P[i][x] = sum_t U[t][x] V[i][t] / sigma_i, sign-normalised so that the largest-|.| entry of V_i is positive */
+ *   eig     top-r eigenpairs of C (replicated, on device): sigma[r] = sqrt(lambda), V[r][m]; 1 <= r <= 14 and r <= m
+ *           (DESMO_ERR_UNSUPPORTED above 14).  Block subspace iteration in fp64 with b = min(r + 8, 16, m) vectors, at least 120
+ *           and at most 240 (r <= 8) or 600 sweeps: it stops once every Ritz pair above the floor has
+ *           ||C v_i - lambda_i v_i|| <= 2^-27 lambda_1.
+ *           Floor: lambda_i <= 2^-23 trace(C) is the rounding level of the fp32 Gram; such a mode is reported as sigma_i = 0.
+ *           workspace_bytes >= 256 + 16 b m.  Its first 24 bytes receive {int32 sweeps, int32 converged (1 / 0), int32, int32,
+ *           double worst residual / lambda_1}; read them once the stream has passed the call (it never synchronises).
+ *   project P[i][x] = sum_t U[t][x] V[i][t] / sigma_i for every r <= DESMO_MAX_R (one pass over U per 8 modes), sign-normalised so
+ *           that the largest-|.| entry of V_i is positive; a row with sigma_i = 0 is written as zeros */
 int desmo_pod_gram(const desmo_shape* s, const float* U, float* C, void* workspace, void* stream);
 int desmo_pod_eig(int32_t m, int32_t r, const float* C, float* V, float* sigma, void* workspace, size_t workspace_bytes,
                   void* stream);
