@@ -51,6 +51,7 @@ SIGNATURES: Dict[str, tuple] = {
     "desmo_assemble_grads": (C.c_int, [_SP] + [_vp] * 17),
     "desmo_reconstruct": (C.c_int, [_SP] + [_vp] * 6),
     "desmo_library_colnorm2": (C.c_int, [_SP] + [_vp] * 5),
+    "desmo_residual_profile": (C.c_int, [_SP, _vp, _i32] + [_vp] * 7),
     "desmo_term_norms": (C.c_int, [_SP, _vp, _vp, _vp, _i32, _vp, _vp]),
     "desmo_selftest_tables": (C.c_int, []),
     "desmo_selftest_chain_sweep": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float)]),

@@ -352,6 +352,18 @@ int desmo_reconstruct(const desmo_shape* s, const float* P, const float* phi, co
     return launch_reconstruct(a, (cudaStream_t)stream);
 }
 
+int desmo_residual_profile(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                           const float* W, double* snap, float* point, void* stream) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if ((rc = device_ok())) return rc;
+    if (!U || !P || !phi || !omega || !W || !snap || !point) { set_error("desmo_residual_profile: null pointer"); return DESMO_ERR_ARG; }
+    if ((rc = check_u_dtype(u_dtype, "desmo_residual_profile"))) return rc;
+    // one route for every library: the GEMM path's GEMM 1 (also for the shapes the fused kernels train)
+    return residual_profile_gemm_path(s, d.T, d.K, d.Kp, U, u_dtype, P, phi, omega, W, snap, point, (cudaStream_t)stream);
+}
+
 int desmo_library_colnorm2(const desmo_shape* s, const float* P, const float* phi, const float* omega, float* out_k, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);

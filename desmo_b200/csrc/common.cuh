@@ -119,6 +119,10 @@ int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, i
                     const float* W, float* dphi, float* red, float* Dacc, void* gemm_ws, cudaStream_t st, bool supplied);
 int reconstruct_gemm_path(const desmo_shape* s, int T, int K, int Kp, const float* P, const float* phi, const float* omega, const float* W,
                           float* out, cudaStream_t st);
+// snap [2][m] fp64 = {sum_x r^2, sum_x u^2}, point [2][ld] fp32 = {sum_t r^2, sum_t u^2} (pad columns 0), r = G W - U; scratch from the
+// stream-ordered allocator
+int residual_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
+                               const float* omega, const float* W, double* snap, float* point, cudaStream_t st);
 int colnorm2_gemm_path(const desmo_shape* s, int T, int K, const float* P, const float* phi, const float* omega, float* out_k, cudaStream_t st);
 int launch_update_phi_generic(const UpdateArgs& a, cudaStream_t st);
 int select_path(const desmo_shape* s, const Dims& d);  // DESMO_PATH_FP32 / _TC / _GEMM actually used, or <0 (error set)

@@ -34,7 +34,13 @@ constexpr int EPI_WARPS = 8;
 constexpr int THREADS = 64 + EPI_WARPS * 32;
 constexpr int kChunkPoints = 16384;
 
-enum { EPI_RESID = 0, EPI_D = 1, EPI_E = 2, EPI_RECON = 3, EPI_RESID_BF16 = 4 };  // EPI_RESID_BF16: EPI_RESID reading bf16 snapshots
+// EPI_RESID_BF16: EPI_RESID reading bf16 snapshots.  EPI_PROFILE (_BF16): r = Rec - U as EPI_RESID forms it, reduced to the two marginals of
+// r^2 and u^2 (per point, per snapshot) instead of being written out (desmo_residual_profile).
+enum { EPI_RESID = 0, EPI_D = 1, EPI_E = 2, EPI_RECON = 3, EPI_RESID_BF16 = 4, EPI_PROFILE = 5, EPI_PROFILE_BF16 = 6 };
+// EPI_PROFILE scratch behind the operand stages (dynamic shared memory), two buffers used by alternate tiles:
+// [4 lane quadrants][2 column halves][4 blocks of 16 columns][32] per-warp column sums, then [2][128] per-point sums of column half 1
+constexpr int kProfSlab = 4 * 2 * 4 * 32 + 2 * 128;
+constexpr size_t kProfSmem = 2 * sizeof(float) * kProfSlab;
 
 // ------------------------------------------------------------------------------------------------- PTX helpers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -111,11 +117,11 @@ struct GemmArgs {
     int n_lib16;               // valid extent of the library dimension rounded up to 16 (N of the last tile, EPI_D / EPI_E)
     // epilogue
     const void* U;             // EPI_RESID: snapshots [m][ld] fp32 (EPI_RESID_BF16: bf16)
-    float* out;                // EPI_RECON: [m][ld]
+    float* out;                // EPI_RECON: [m][ld]; EPI_PROFILE: per-point partials [tiles_n][2][rows_r] of the chunk
     __nv_bfloat16* Rp;         // EPI_RESID: [2][rows_r][mp]
     float* Dacc;               // EPI_D: [K][ld]
     float* Epart;              // EPI_E: [nslice_alloc][Kp][mld]
-    double* loss_part;         // EPI_RESID: [gridDim.x]
+    double* loss_part;         // EPI_RESID: [gridDim.x]; EPI_PROFILE: per-CTA snapshot partials [gridDim.x][2][mp], accumulated
     long long n, ld, x0;       // points of this rank, pitch, first point of the chunk
     long long rows_r;          // rows per plane of Rp (chunk points padded to 128)
     int m, mld, mp, K, Kp;
@@ -141,7 +147,8 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
     constexpr int NSTAGE = (NPA + NPB) >= 6 ? 2 : 3;
     static_assert(NPA == NPB, "plane pairs are defined for equal plane counts");
     constexpr bool kResid = EPI == EPI_RESID || EPI == EPI_RESID_BF16;
-    using UT = typename std::conditional<EPI == EPI_RESID_BF16, __nv_bfloat16, float>::type;
+    constexpr bool kProfile = EPI == EPI_PROFILE || EPI == EPI_PROFILE_BF16;
+    using UT = typename std::conditional<EPI == EPI_RESID_BF16 || EPI == EPI_PROFILE_BF16, __nv_bfloat16, float>::type;
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bars[2 * NSTAGE + 4];
     __shared__ uint32_t tmem_base_s;
@@ -320,6 +327,63 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
                 for (int j = 0; j < 64; ++j) {
                     const int k = col0 + j;
                     if (k < g.K && x < g.ld) g.Dacc[(long long)k * g.ld + x] = sum[j];
+                }
+            } else if (kProfile) {
+                // rows = points of the chunk, columns = snapshots: r = Rec - U exactly as EPI_RESID forms it; r^2 and u^2 are summed over
+                // this thread's 64 columns (per point) and over the tile's 128 rows (per snapshot), in a fixed order
+                const long long pl = (long long)tm * BM + row;  // chunk-local point
+                const long long x = g.x0 + pl;
+                const bool xin = x < g.n;
+                float* prof = reinterpret_cast<float*>(smem + NSTAGE * STAGE) + (((w - (int)blockIdx.x) / (int)gridDim.x) & 1) * kProfSlab;
+                float pr = 0.0f, pu = 0.0f;
+#pragma unroll
+                for (int blk = 0; blk < 4; ++blk) {
+                    float u[16];
+#pragma unroll
+                    for (int j = 0; j < 16; ++j) {
+                        const int t = col0 + blk * 16 + j;
+                        u[j] = (xin && t < g.m) ? ldg_u(static_cast<const UT*>(g.U) + (long long)t * g.ld + x) : 0.0f;
+                    }
+                    float v[32];  // [0, 16): r^2, [16, 32): u^2 of the block's 16 columns
+#pragma unroll
+                    for (int j = 0; j < 16; ++j) {
+                        const int t = col0 + blk * 16 + j;
+                        const float rr = (xin && t < g.m) ? sum[blk * 16 + j] - u[j] : 0.0f;
+                        v[j] = __fmul_rn(rr, rr);
+                        v[16 + j] = __fmul_rn(u[j], u[j]);
+                        pr += v[j];
+                        pu += v[16 + j];
+                    }
+                    // column sums over the warp's 32 points: halving exchange, lane l ends with the sum of v[l]
+#pragma unroll
+                    for (int o = 16; o >= 1; o >>= 1) {
+                        const bool hi = (lane & o) != 0;
+#pragma unroll
+                        for (int i = 0; i < o; ++i) {
+                            const float send = hi ? v[i] : v[i + o];
+                            const float keep = hi ? v[i + o] : v[i];
+                            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+                        }
+                    }
+                    prof[((q * 2 + c) * 4 + blk) * 32 + lane] = v[0];
+                }
+                float* pts = prof + 4 * 2 * 4 * 32;
+                if (c == 1) { pts[row] = pr; pts[128 + row] = pu; }
+                asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");  // the epilogue warps only
+                if (c == 0) {  // this tile's per-point partial: column half 0 + column half 1
+                    float* dst = g.out + (long long)tn * 2 * g.rows_r;
+                    dst[pl] = pr + pts[row];
+                    dst[g.rows_r + pl] = pu + pts[128 + row];
+                }
+                {   // per snapshot: the four lane quadrants in order, in fp64, into this CTA's partial
+                    const int e = (warp - 2) * 32 + lane;
+                    const int ch = e >> 7, blk = (e >> 5) & 3, l = e & 31;
+                    double sq = 0.0;
+#pragma unroll
+                    for (int qq = 0; qq < 4; ++qq) sq += (double)prof[((qq * 2 + ch) * 4 + blk) * 32 + l];
+                    const int t = tn * BN + ch * 64 + blk * 16 + (l & 15);
+                    double* dst = g.loss_part + ((long long)blockIdx.x * 2 + (l >> 4)) * g.mp + t;
+                    *dst += sq;
                 }
             } else {  // EPI_E: rows = snapshots, columns = library terms; this slice's partial of E^T, accumulated over the chunks
                 const int t = tm * BM + row;
@@ -646,7 +710,8 @@ template <bool A_MN, bool B_MN, int NPA, int NPB, int EPI>
 static int launch_gemm(const GemmArgs& g, const CUtensorMap& tmA, const CUtensorMap& tmB, int sms, cudaStream_t st) {
     constexpr size_t stage = (size_t)(NPA + NPB) * PLANE_TILE;
     constexpr int nstage = (NPA + NPB) >= 6 ? 2 : 3;
-    const size_t smem = nstage * stage + 1024;
+    constexpr size_t extra = (EPI == EPI_PROFILE || EPI == EPI_PROFILE_BF16) ? kProfSmem : 0;
+    const size_t smem = nstage * stage + 1024 + extra;
     auto kern = gemm_planes_kernel<A_MN, B_MN, NPA, NPB, EPI>;
     DESMO_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int items = g.tiles_m * g.tiles_n * g.nslice;
@@ -856,6 +921,92 @@ int reconstruct_gemm_path(const desmo_shape* s, int T, int K, int Kp, const floa
         g.tiles_m = (int)(pts / 128); g.tiles_n = mp / 128; g.nslice = 1; g.kblocks = (K + 63) / 64; g.kb_per_slice = g.kblocks; g.kgroup = 4;
         g.a_rows = Kr; g.b_rows = Kr; g.first_chunk = 1;
         rc = launch_gemm<true, true, 3, 3, EPI_RECON>(g, tmG_mn, tmW_mn, sms, st);
+    }
+    cudaFreeAsync(scratch, st);
+    return rc;
+}
+
+// Residual profile (desmo_residual_profile): library planes + GEMM 1 with the profile epilogue, then fixed-order sums of the partials.
+// Points per chunk: the chunk's G planes and per-point partials take about kProfileChunkBytes, so that they stay in L2 while U streams.
+constexpr size_t kProfileChunkBytes = 32u << 20;
+
+// point[0][x] = sum_t r^2, point[1][x] = sum_t u^2 for the chunk's points: the tiles_n partials in order, in fp64, rounded once
+__global__ void __launch_bounds__(256) profile_points_kernel(const float* __restrict__ pp, int tiles_n, long long rows_c, long long pts,
+                                                             long long n, long long ld, long long x0, float* __restrict__ point) {
+    const long long xl = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (xl >= pts) return;
+    double a = 0.0, b = 0.0;
+    for (int tn = 0; tn < tiles_n; ++tn) {
+        a += (double)pp[(long long)(2 * tn) * rows_c + xl];
+        b += (double)pp[(long long)(2 * tn + 1) * rows_c + xl];
+    }
+    const long long x = x0 + xl;
+    point[x] = x < n ? (float)a : 0.0f;
+    point[ld + x] = x < n ? (float)b : 0.0f;
+}
+
+// snap[q][t] = sum over the CTAs, in order, of their partials [nparts][2][mp]
+__global__ void __launch_bounds__(256) profile_snapshots_kernel(const double* __restrict__ part, int nparts, int m, int mp,
+                                                                double* __restrict__ snap) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= 2 * m) return;
+    const int q = i / m, t = i - q * m;
+    double s = 0.0;
+    for (int b = 0; b < nparts; ++b) s += part[((long long)b * 2 + q) * mp + t];
+    snap[i] = s;
+}
+
+int residual_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
+                               const float* omega, const float* W, double* snap, float* point, cudaStream_t st) {
+    using namespace gp;
+    int dev = 0, sms = 0;
+    DESMO_CUDA(cudaGetDevice(&dev));
+    DESMO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    // GEMM 1 reads (K + 63) / 64 k-blocks: planes of that many rows give the same products as reconstruct_gemm_path's
+    const int Kr = (K + 63) / 64 * 64;
+    const int mp = (s->m + 127) / 128 * 128, tiles_n = mp / 128;
+    const size_t per_point = (size_t)3 * Kr * 2 + (size_t)tiles_n * 2 * 4;
+    long long rows_c = (long long)(kProfileChunkBytes / per_point) / 128 * 128;
+    if (rows_c < 128) rows_c = 128;
+    if (rows_c > s->ld) rows_c = s->ld;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off = align_up_g(off + bytes, 1024); return o; };
+    const size_t o_idx = take((size_t)T * 8), o_deg = take((size_t)T), o_gp = take((size_t)3 * Kr * rows_c * 2),
+                 o_wp = take((size_t)3 * Kr * mp * 2), o_pp = take((size_t)tiles_n * 2 * rows_c * 4),
+                 o_part = take((size_t)sms * 2 * mp * sizeof(double));
+    uint8_t* scratch = nullptr;
+    DESMO_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&scratch), off, st));
+    __nv_bfloat16* Gp = reinterpret_cast<__nv_bfloat16*>(scratch + o_gp);
+    __nv_bfloat16* Wp = reinterpret_cast<__nv_bfloat16*>(scratch + o_wp);
+    float* pp = reinterpret_cast<float*>(scratch + o_pp);
+    double* part = reinterpret_cast<double*>(scratch + o_part);
+    TermTable tab{scratch + o_idx, scratch + o_deg};
+    int rc = check_cuda(cudaMemsetAsync(part, 0, (size_t)sms * 2 * mp * sizeof(double), st), "cudaMemsetAsync");
+    CUtensorMap tmG_mn, tmW_mn;
+    if (!rc) {
+        term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab);
+        w_planes_kernel<<<Kr, 256, 0, st>>>(W, K, Kr, s->m, s->mld, mp, Wp);
+        rc = check_cuda(cudaGetLastError(), "w_planes_kernel");
+    }
+    if (!rc && !(rc = make_map(&tmG_mn, Gp, rows_c, 3LL * Kr, 64))) rc = make_map(&tmW_mn, Wp, mp, 3LL * Kr, 64);
+    for (long long x0 = 0; x0 < s->ld && !rc; x0 += rows_c) {
+        const long long pts = (s->ld - x0 < rows_c) ? s->ld - x0 : rows_c;  // multiple of 128
+        dim3 grid((unsigned)((rows_c + 255) / 256), 64u);
+        library_planes_kernel<<<grid, 256, 0, st>>>(P, phi, omega, tab, s->r, T, K, Kr, s->n, s->ld, x0, rows_c, Gp);
+        GemmArgs g{};
+        g.U = U; g.out = pp; g.loss_part = part;
+        g.n = s->n; g.ld = s->ld; g.x0 = x0; g.rows_r = rows_c; g.m = s->m; g.mld = s->mld; g.mp = mp; g.K = K; g.Kp = Kp;
+        g.tiles_m = (int)(pts / 128); g.tiles_n = tiles_n; g.nslice = 1; g.kblocks = (K + 63) / 64; g.kb_per_slice = g.kblocks; g.kgroup = 4;
+        g.a_rows = Kr; g.b_rows = Kr; g.first_chunk = 1;
+        rc = u_dtype == DESMO_DTYPE_BF16 ? launch_gemm<true, true, 3, 3, EPI_PROFILE_BF16>(g, tmG_mn, tmW_mn, sms, st)
+                                         : launch_gemm<true, true, 3, 3, EPI_PROFILE>(g, tmG_mn, tmW_mn, sms, st);
+        if (rc) break;
+        profile_points_kernel<<<(unsigned)((pts + 255) / 256), 256, 0, st>>>(pp, tiles_n, rows_c, pts, s->n, s->ld, x0, point);
+        rc = check_cuda(cudaGetLastError(), "profile_points_kernel");
+    }
+    if (!rc) {
+        profile_snapshots_kernel<<<(2 * s->m + 255) / 256, 256, 0, st>>>(part, sms, s->m, mp, snap);
+        rc = check_cuda(cudaGetLastError(), "profile_snapshots_kernel");
     }
     cudaFreeAsync(scratch, st);
     return rc;

@@ -359,6 +359,30 @@ class DesmoEngine:
                                              _ptr(out), self._stream()), "desmo_reconstruct")
         return out[:, :self.n]
 
+    def residual_profile(self) -> dict:
+        """Where and when the model misfits: the marginals of r^2, r = recon - U (the training step's residual for the current
+        parameters; U as stored), in one pass over U without materialising recon (desmo_residual_profile).  Nothing else is written.
+
+          snapshot_residual2 (m,) fp64  sum_x r(x, t)^2      summed over ranks when point-sharded
+          snapshot_norm2     (m,) fp64  sum_x U(x, t)^2      summed over ranks when point-sharded
+          point_residual2    (n,) fp32  sum_t r(x, t)^2      this rank's points
+          point_norm2        (n,) fp32  sum_t U(x, t)^2      this rank's points
+
+        Relative error per snapshot (over the cardiac cycle / shedding period): e(t) = sqrt(snapshot_residual2 / snapshot_norm2).
+        Misfit map over the mesh: point_residual2, or sqrt(point_residual2 / point_norm2) for the relative error of each point.
+        The totals equal residual_norm2() up to the order of the sums.  Bit-identical from call to call."""
+        ud = self._u_dtype()
+        snap = torch.empty(2, self.m, dtype=torch.float64, device=self.device)
+        point = torch.empty(2, self.ld, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            self.build_w(False)
+            check(self.lib.desmo_residual_profile(C.byref(self.shape), _ptr(self.U), ud, _ptr(self.P), _ptr(self.phi), _ptr(self.omega),
+                                                  _ptr(self.W), _ptr(snap), _ptr(point), self._stream()), "desmo_residual_profile")
+            if self.n_global != self.n and torch.distributed.is_initialized():
+                torch.distributed.all_reduce(snap, group=self.pg)
+        return {"snapshot_residual2": snap[0], "snapshot_norm2": snap[1], "point_residual2": point[0, :self.n],
+                "point_norm2": point[1, :self.n]}
+
     def term_norms(self, physical: bool = False) -> torch.Tensor:
         """Per-term norms of the post-hoc sweep, K order, fp64 (poly_norm / nonlinear_norm, CYL:624-692; FCYL:644-720).
 

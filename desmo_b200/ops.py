@@ -1,6 +1,6 @@
 """torch custom ops over the C ABI: one ``torch.ops.desmo_b200.*`` op per hot-path entry point of include/desmo_b200.h.
 
-  build_w, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, library_colnorm2, term_norms,
+  build_w, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, library_colnorm2, term_norms,
   pod_gram, pod_eig, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce
 
 They take the packed device tensors of a DesmoEngine (layout: include/desmo_b200.h) plus the shape integers and launch the
@@ -106,6 +106,22 @@ def reconstruct(P: torch.Tensor, phi: torch.Tensor, omega: torch.Tensor, W: torc
     s = make_shape(n, m, r, polyorder, nF, n_global, path)
     with torch.cuda.device(P.device):
         check(_lib.load().desmo_reconstruct(C.byref(s), _p(P), _p(phi), _p(omega), _p(W), _p(out), _stream(P)), "desmo_reconstruct")
+
+
+@torch.library.custom_op("desmo_b200::residual_profile", mutates_args=("snap", "point"))
+def residual_profile(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, omega: torch.Tensor, W: torch.Tensor, snap: torch.Tensor,
+                     point: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """snap (fp64 [2, m]) = {sum_x r^2, sum_x U^2}, point (fp32 [2, ld]) = {sum_t r^2, sum_t U^2}, r = G W - U (desmo_residual_profile)."""
+    _require_cuda(U, P, phi, omega, W, snap, point)
+    ud = _lib.u_dtype_code(U.dtype)
+    if snap.dtype != torch.float64 or point.dtype != torch.float32:
+        raise _lib.DesmoError("residual_profile: snap must be float64 and point float32")
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    if snap.numel() < 2 * m or point.numel() < 2 * s.ld or not (snap.is_contiguous() and point.is_contiguous()):
+        raise _lib.DesmoError(f"residual_profile: need contiguous snap [2, {m}] and point [2, {s.ld}]")
+    with torch.cuda.device(U.device):
+        check(_lib.load().desmo_residual_profile(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), _p(snap), _p(point), _stream(U)),
+              "desmo_residual_profile")
 
 
 @torch.library.custom_op("desmo_b200::library_colnorm2", mutates_args=("out",))
@@ -241,6 +257,19 @@ def engine_term_norms_via_ops(e, physical: bool = False) -> torch.Tensor:
     torch.ops.desmo_b200.library_colnorm2(e.P if physical else None, e.phi, e.omega, g2, *sa)
     torch.ops.desmo_b200.term_norms(g2, e.gates, e.rows, 1 if (e.nF and not physical) else 0, out, *sa)
     return out
+
+
+def engine_residual_profile_via_ops(e) -> dict:
+    """DesmoEngine.residual_profile() through the registered build_w / residual_profile ops (the optimizer's step counter is not moved)."""
+    sa = _shape_args(e)
+    snap = torch.empty(2, e.m, dtype=torch.float64, device=e.device)
+    point = torch.empty(2, e.ld, dtype=torch.float32, device=e.device)
+    scratch_step = e.step_dev.clone()
+    torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, scratch_step, e.workspace, *sa)
+    torch.ops.desmo_b200.residual_profile(e.U, e.P, e.phi, e.omega, e.W, snap, point, *sa)
+    if e.n_global != e.n and torch.distributed.is_initialized():
+        torch.distributed.all_reduce(snap, group=e.pg)
+    return {"snapshot_residual2": snap[0], "snapshot_norm2": snap[1], "point_residual2": point[0, :e.n], "point_norm2": point[1, :e.n]}
 
 
 def engine_pod_via_ops(e) -> torch.Tensor:

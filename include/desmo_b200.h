@@ -144,6 +144,21 @@ int desmo_assemble_grads(const desmo_shape* s, const float* red, float* dphi, co
 int desmo_reconstruct(const desmo_shape* s, const float* P, const float* phi, const float* omega, const float* W,
                       float* out, void* stream);
 
+/* Residual profile of the current parameters, without materialising the reconstruction (evaluation only; writes nothing else).
+ * r(x, t) = (G(Phi) W)(x, t) - U(x, t) with Phi = phi * P, W as desmo_build_w builds it and U as stored (u_dtype = DESMO_DTYPE_F32 or
+ * DESMO_DTYPE_BF16; anything else is DESMO_ERR_ARG).  Outputs, for this rank's points:
+ *   snap   [2][m]   fp64: snap[0][t] = sum_x r^2, snap[1][t] = sum_x U^2    (local partial -- all-reduce them across ranks)
+ *   point  [2][ld]  fp32: point[0][x] = sum_t r^2, point[1][x] = sum_t U^2  (pad columns n..ld-1 are 0)
+ * so that e(t) = sqrt(snap[0][t] / snap[1][t]) is the relative error of snapshot t and point[0] is a spatial map of the misfit.
+ * Every library goes through GEMM 1 of the general path (six split-bf16 products, about 2^-24 relative, as desmo_reconstruct for
+ * K > 80 or r > 8; for those shapes each r is bit for bit the fp32 difference desmo_reconstruct - U).  Each thread sums r^2 over its
+ * 64 snapshots of a 128 x 128 tile in fp32; the per-snapshot sums over the tile's 128 points are fp32 trees of 32 plus fp64 over the
+ * rest; all partials are summed in a fixed order, so the result is bit-identical from call to call (no float atomics).  Accuracy:
+ * |snap - exact| <= 9 * 2^-24 * snap, |point - exact| <= 70 * 2^-24 * point, relative to the exact sums of the fp32 r.  Scratch
+ * (about 32 MB plus 16 m bytes per SM) comes from the stream-ordered allocator on `stream`, so the call stays capturable. */
+int desmo_residual_profile(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                           const float* W, double* snap, float* point, void* stream);
+
 /* Post-hoc sparsification inputs: squared column norms of G (K floats, local partial -- all-reduce them across ranks).
  * P == NULL evaluates the library on the raw phi_list, which is what the reference's sweep passes to poly_norm /
  * nonlinear_norm (CYL:1192-1194; the functions, CYL:624-692, never multiply by POD_modes); P != NULL gives the columns of
