@@ -40,6 +40,7 @@ SIGNATURES: Dict[str, tuple] = {
     "desmo_selected_path": (_i32, [_SP]),
     "desmo_workspace_bytes": (C.c_int, [_SP, C.POINTER(C.c_size_t)]),
     "desmo_build_w": (C.c_int, [_SP] + [_vp] * 8),
+    "desmo_build_w_at": (C.c_int, [_SP] + [_vp] * 4 + [_i32, _i32] + [_vp] * 5),
     "desmo_fused_residual_grad": (C.c_int, [_SP] + [_vp] * 9),
     "desmo_recon_backward": (C.c_int, [_SP] + [_vp] * 9),
     "desmo_fused_residual_grad_begin": (C.c_int, [_SP] + [_vp] * 9),

@@ -218,6 +218,35 @@ int desmo_build_w(const desmo_shape* s, const float* gates, float* rows, const f
                    step_dev, ws.l1, (cudaStream_t)stream);
 }
 
+int desmo_build_w_at(const desmo_shape* s, const float* gates, const float* rows, const float* coefs, const float* periods, int32_t m_out,
+                     int32_t mld_out, const int32_t* index, const float* times, float* W_out, float* rows_out, void* stream) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if (m_out < 1 || mld_out < m_out || mld_out % 16 != 0) {
+        set_error("desmo_build_w_at: need m_out >= 1 and mld_out >= m_out, a multiple of 16 (got m_out=%d mld_out=%d)", m_out, mld_out);
+        return DESMO_ERR_ARG;
+    }
+    if ((index == nullptr) == (times == nullptr)) { set_error("desmo_build_w_at: pass exactly one of index / times"); return DESMO_ERR_ARG; }
+    if (times && s->nF == 0) {
+        set_error("desmo_build_w_at: times need a Fourier model (nF > 0); DESMO's free rows exist only at the m training snapshots");
+        return DESMO_ERR_ARG;
+    }
+    if (!gates || !W_out || (s->nF == 0 && !rows) || (s->nF > 0 && (!coefs || !periods))) {
+        set_error("desmo_build_w_at: null pointer");
+        return DESMO_ERR_ARG;
+    }
+    for (int i = 0; i < m_out; ++i) {  // host arrays: every instant is checked before anything is launched
+        if (index && (index[i] < 0 || index[i] >= s->m)) {
+            set_error("desmo_build_w_at: index[%d] = %d outside 0 .. m-1 = %d", i, index[i], s->m - 1);
+            return DESMO_ERR_ARG;
+        }
+        if (times && !isfinite(times[i])) { set_error("desmo_build_w_at: times[%d] is not finite", i); return DESMO_ERR_ARG; }
+    }
+    if ((rc = device_ok())) return rc;
+    return build_w_at(s, d.K, d.Kp, gates, rows, coefs, periods, m_out, mld_out, index, times, W_out, rows_out, (cudaStream_t)stream);
+}
+
 static int fused_dispatch(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
                           const float* W, float* dphi, float* red, void* workspace, void* stream, bool supplied, const char* who,
                           int phase = 0) {

@@ -77,6 +77,11 @@ struct EvalArgs {
 // host-side launchers (one per translation unit)
 int build_w(const desmo_shape* s, int K, int Kp, const float* gates, float* rows, const float* coefs, const float* periods,
             float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st);
+// W_out[Kp][mld_out] (and rows_out[K][mld_out] if non-null) at m_out host-given instants, one launch per kAtBatch of them; the
+// arguments are validated by desmo_build_w_at
+constexpr int kAtBatch = 512;
+int build_w_at(const desmo_shape* s, int K, int Kp, const float* gates, const float* rows, const float* coefs, const float* periods,
+               int m_out, int mld_out, const int32_t* index, const float* times, float* W_out, float* rows_out, cudaStream_t st);
 // U is [m][ld] in the element type u_dtype names (DESMO_DTYPE_F32 or DESMO_DTYPE_BF16; validated by the C ABI).
 // supplied = true: U holds dL/drecon ([m][ld], fp32) and R := (n_global m / 2) * U instead of G W - U (desmo_recon_backward)
 int fused_fp32(const desmo_shape* s, const MonoTable& mt, int T, int Kp, const void* U, int u_dtype, const float* P, const float* phi,

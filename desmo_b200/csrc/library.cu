@@ -81,4 +81,55 @@ int build_w(const desmo_shape* s, int K, int Kp, const float* gates, float* rows
     return DESMO_OK;
 }
 
+// Instants of one build_w_at launch, passed by value (2 KB of kernel parameters): no device copy of the caller's host arrays, so the
+// call needs no allocation and stays capturable.  Launch b writes columns [c0, c1) of W_out; the instants of columns c0 .. m_out-1.
+struct AtBatch {
+    int c0, c1, m_out, use_times;
+    union { int32_t index[kAtBatch]; float time[kAtBatch]; };
+};
+
+// grid = Kp blocks (one library term each), 256 threads over the batch's columns.  Same z and gate * z as build_w_kernel at an
+// instant t_point(index, m) or a given time; rows is only read.
+__global__ void build_w_at_kernel(int K, int m, int mld, int nF, const float* __restrict__ gates, const float* __restrict__ rows,
+                                  const float* __restrict__ coefs, const float* __restrict__ periods, int mld_out,
+                                  float* __restrict__ W_out, float* __restrict__ rows_out, const AtBatch b) {
+    const int k = blockIdx.x;
+    const float gate = (k < K) ? gates[k] : 0.0f;
+    const float period = (nF > 0 && k < K) ? periods[k] : 1.0f;
+    for (int c = b.c0 + threadIdx.x; c < b.c1; c += blockDim.x) {
+        float z = 0.0f, w = 0.0f;
+        if (k < K && c < b.m_out) {
+            const int i = c - b.c0;
+            if (nF > 0) {
+                const float t = b.use_times ? b.time[i] : t_point(b.index[i], m);
+                z = fourier_value(coefs + (size_t)k * (2 * nF + 1), nF, t, period);
+            } else {
+                z = rows[(size_t)k * mld + b.index[i]];
+            }
+            w = gate * z;
+        }
+        W_out[(size_t)k * mld_out + c] = w;
+        if (rows_out && k < K) rows_out[(size_t)k * mld_out + c] = z;
+    }
+}
+
+int build_w_at(const desmo_shape* s, int K, int Kp, const float* gates, const float* rows, const float* coefs, const float* periods,
+               int m_out, int mld_out, const int32_t* index, const float* times, float* W_out, float* rows_out, cudaStream_t st) {
+    AtBatch b;
+    b.m_out = m_out;
+    b.use_times = times != nullptr;
+    for (int c0 = 0; c0 < m_out; c0 += kAtBatch) {
+        const int cnt = (m_out - c0 < kAtBatch) ? m_out - c0 : kAtBatch;
+        b.c0 = c0;
+        b.c1 = (c0 + cnt == m_out) ? mld_out : c0 + cnt;  // the last launch also zeroes the pad columns
+        for (int i = 0; i < cnt; ++i) {
+            if (times) b.time[i] = times[c0 + i];
+            else b.index[i] = index[c0 + i];
+        }
+        build_w_at_kernel<<<Kp, 256, 0, st>>>(K, s->m, s->mld, s->nF, gates, rows, coefs, periods, mld_out, W_out, rows_out, b);
+        DESMO_CUDA(cudaGetLastError());
+    }
+    return DESMO_OK;
+}
+
 }  // namespace desmo

@@ -23,6 +23,47 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
 
+def time_points(index, m: int) -> np.ndarray:
+    """The fp32 times at which a model with m snapshots evaluates training snapshot k = index[i]: t_point of csrc/library.cu, i.e.
+    torch.linspace(0, m, m)[k] as ATen computes it (FCYL:485).  step = m / (m - 1); k < m / 2 gives step * k, otherwise
+    m - step * (m - 1 - k).  k >= m continues the grid as step * k, so time_points(range(m, 2 * m), m) is the next window at the
+    training spacing.  Every operation is one fp32 rounding, as on the device."""
+    m = int(m)
+    if m < 2:
+        raise _lib.DesmoError(f"time_points needs m >= 2, got {m}")
+    k = np.asarray(index, dtype=np.int64).reshape(-1)
+    if k.size and int(k.min()) < 0:
+        raise _lib.DesmoError("time_points: negative snapshot index")
+    step = np.float32(m) / np.float32(m - 1)
+    up = step * k.astype(np.float32)
+    down = np.float32(m) - step * (m - 1 - k).astype(np.float32)
+    return np.where((k < m // 2) | (k >= m), up, down).astype(np.float32)
+
+
+def _instants(index, times, m: int, nF: int):
+    """Host arrays for desmo_build_w_at: (int32 index or None, fp32 times or None).  Raises DesmoError before any launch."""
+    if (index is None) == (times is None):
+        raise _lib.DesmoError("pass exactly one of index= (training snapshot indices) or times= (Fourier model times)")
+    if times is not None:
+        if not nF:
+            raise _lib.DesmoError("times= needs a Fourier model: DESMO's free temporal rows exist only at the m training snapshots")
+        t = np.ascontiguousarray((times.detach().cpu().numpy() if torch.is_tensor(times) else np.asarray(times)), dtype=np.float32).reshape(-1)
+        if t.size == 0:
+            raise _lib.DesmoError("times= is empty")
+        if not np.isfinite(t).all():
+            raise _lib.DesmoError("times= must be finite")
+        return None, t
+    raw = index.detach().cpu().numpy() if torch.is_tensor(index) else np.asarray(index)
+    if raw.size == 0:
+        raise _lib.DesmoError("index= is empty")
+    if not np.issubdtype(raw.dtype, np.integer):
+        raise _lib.DesmoError(f"index= must hold integers, got {raw.dtype}")
+    k = raw.astype(np.int64).reshape(-1)
+    if int(k.min()) < 0 or int(k.max()) >= m:
+        raise _lib.DesmoError(f"index= must lie in 0 .. {m - 1} (training snapshots; use times= to evaluate elsewhere)")
+    return np.ascontiguousarray(k, dtype=np.int32), None
+
+
 class _PeerDesc(C.Structure):  # desmo_peer (include/desmo_b200.h)
     _fields_ = [("world", C.c_int32), ("rank", C.c_int32), ("red_ptrs", C.c_void_p), ("flag_ptrs", C.c_void_p), ("state", C.c_void_p)]
 
@@ -122,18 +163,24 @@ class DesmoEngine:
             return
         if snapshot.dtype not in (torch.float32, torch.float64):
             raise _lib.DesmoError(f"bf16 storage takes fp32, fp64 or bf16 snapshots, got {snapshot.dtype}")
-        self._qsums = torch.zeros(2, dtype=torch.float64, device=self.device)
-        rows = max(1, min(self.m, SNAPSHOT_CHUNK_BYTES // (4 * self.n)))
+        self._qsums = self._snapshot_to_bf16(snapshot, self.U, self.shape, non_blocking)
+
+    def _snapshot_to_bf16(self, snapshot: torch.Tensor, U: torch.Tensor, shape, non_blocking: bool) -> torch.Tensor:
+        """fp32 / fp64 snapshot (rows, n) -> bf16 U[0 .. rows)[ld] of `shape` by desmo_snapshot_to_bf16, in chunks of at most
+        SNAPSHOT_CHUNK_BYTES of fp32.  Returns the fp64 quantisation sums [sum (u - q)^2, sum u^2]."""
+        qsums = torch.zeros(2, dtype=torch.float64, device=self.device)
+        rows = max(1, min(snapshot.shape[0], SNAPSHOT_CHUNK_BYTES // (4 * self.n)))
         with torch.cuda.device(self.device):
-            for t0 in range(0, self.m, rows):
+            for t0 in range(0, snapshot.shape[0], rows):
                 part = snapshot[t0:t0 + rows]
                 if part.dtype != torch.float32 and part.device.type == "cpu":
                     part = part.to(torch.float32)  # cast on the host: only fp32 crosses the bus
                 src = part.to(self.device, torch.float32, non_blocking=non_blocking).contiguous()
-                check(self.lib.desmo_snapshot_to_bf16(C.byref(self.shape), src.data_ptr(), src.stride(0), t0, src.shape[0],
-                                                      self.U.data_ptr(), self._qsums.data_ptr(), self._stream()),
+                check(self.lib.desmo_snapshot_to_bf16(C.byref(shape), src.data_ptr(), src.stride(0), t0, src.shape[0],
+                                                      U.data_ptr(), qsums.data_ptr(), self._stream()),
                       "desmo_snapshot_to_bf16")
                 del part, src  # the next chunk reuses this block: at most one chunk is resident
+        return qsums
 
     def snapshot_quantization_error(self) -> float:
         """||U - U_q||_F / ||U||_F of the bf16 snapshot storage (fp64; over all ranks when point-sharded): U the fp32 snapshot the
@@ -381,6 +428,79 @@ class DesmoEngine:
             if self.n_global != self.n and torch.distributed.is_initialized():
                 torch.distributed.all_reduce(snap, group=self.pg)
         return {"snapshot_residual2": snap[0], "snapshot_norm2": snap[1], "point_residual2": point[0, :self.n],
+                "point_norm2": point[1, :self.n]}
+
+    # ------------------------------------------------------------------ evaluation at chosen instants
+    # Each of these takes exactly one of index= (training snapshot indices, any order, repeats allowed) or times= (fp32 times in the
+    # model's own time coordinate, Fourier models only, any finite value: between grid points, before 0, beyond the window).  They
+    # write nothing the model owns: parameters, optimizer state, rows, W, red, dphi, losses, step_dev and U stay as they are.
+    def time_points(self, index) -> np.ndarray:
+        """fp32 times of the given snapshot indices (k >= m continues the grid): times=time_points(range(m, 2 * m)) is the next
+        window at the training spacing, and times=time_points(index) gives the same bits as index=index."""
+        return time_points(index, self.m)
+
+    def _w_at(self, idx: Optional[np.ndarray], t: Optional[np.ndarray], mld_out: int, rows_out: Optional[torch.Tensor] = None):
+        """W' [Kp][mld_out] at the instants _instants() validated (desmo_build_w_at); rows_out [K][mld_out] receives z(t_i)."""
+        m_out = (idx if idx is not None else t).size
+        W = torch.empty(self.Kp, mld_out, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.lib.desmo_build_w_at(C.byref(self.shape), _ptr(self.gates), _ptr(self.rows), _ptr(self.coefs), _ptr(self.periods),
+                                            m_out, mld_out, None if idx is None else idx.ctypes.data, None if t is None else t.ctypes.data,
+                                            _ptr(W), _ptr(rows_out), self._stream()), "desmo_build_w_at")
+        return W
+
+    def _shape_at(self, m_out: int):
+        """The engine's shape with m' snapshots (the spatial entry points need m >= 2: m' = 1 runs as two with a zero second column)."""
+        return make_shape(self.n, max(m_out, 2), self.r, self.polyorder, self.nF, self.n_global, self.shape.path, ld=self.ld)
+
+    def temporal_rows_at(self, index=None, times=None) -> torch.Tensor:
+        """z(t) at the instants, (K, m') fp32: forward()'s z_values there, unscaled by the gates, all K terms in K order."""
+        idx, t = _instants(index, times, self.m, self.nF)
+        m_out = (idx if idx is not None else t).size
+        rows = torch.empty(self.K, round_up(m_out, 16), dtype=torch.float32, device=self.device)
+        self._w_at(idx, t, rows.shape[1], rows)
+        return rows[:, :m_out]
+
+    def reconstruct_at(self, index=None, times=None) -> torch.Tensor:
+        """recon at the instants, (m', n) fp32, allocating only m' rows: desmo_build_w_at, then desmo_reconstruct on an m'-snapshot
+        shape.  reconstruct_at(index=k) is bit for bit reconstruct()[k]."""
+        idx, t = _instants(index, times, self.m, self.nF)
+        m_out = (idx if idx is not None else t).size
+        sh = self._shape_at(m_out)
+        W = self._w_at(idx, t, sh.mld)
+        out = torch.empty(sh.m, self.ld, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.lib.desmo_reconstruct(C.byref(sh), _ptr(self.P), _ptr(self.phi), _ptr(self.omega), _ptr(W), _ptr(out), self._stream()),
+                  "desmo_reconstruct")
+        return out[:m_out, :self.n]
+
+    def residual_profile_at(self, snapshots: torch.Tensor, index=None, times=None) -> dict:
+        """residual_profile() for a held-out block: r = recon(t_i) - snapshots[i], snapshots (m', n) fp32, fp64 or bf16, on the host or
+        the device.  The block is stored as U is (snapshot_dtype; fp32 / fp64 into bf16 by desmo_snapshot_to_bf16 in chunks of at
+        most SNAPSHOT_CHUNK_BYTES) in a temporary [m'][ld] buffer.  Returns the four keys of residual_profile(): (m',) snapshot
+        sums, summed over ranks when point-sharded, and this rank's (n,) point sums."""
+        idx, t = _instants(index, times, self.m, self.nF)
+        m_out = (idx if idx is not None else t).size
+        if not torch.is_tensor(snapshots) or tuple(snapshots.shape) != (m_out, self.n):
+            got = tuple(snapshots.shape) if torch.is_tensor(snapshots) else type(snapshots).__name__
+            raise _lib.DesmoError(f"snapshots must be a ({m_out}, {self.n}) tensor, one row per instant, got {got}")
+        if snapshots.dtype not in (torch.float32, torch.float64, torch.bfloat16):
+            raise _lib.DesmoError(f"snapshots must be float32, float64 or bfloat16, got {snapshots.dtype}")
+        sh = self._shape_at(m_out)
+        W = self._w_at(idx, t, sh.mld)
+        U = torch.zeros(sh.m, self.ld, dtype=self.snapshot_dtype, device=self.device)
+        if self.snapshot_dtype == torch.float32 or snapshots.dtype == torch.bfloat16:
+            U[:m_out, :self.n].copy_(snapshots)
+        else:
+            self._snapshot_to_bf16(snapshots, U, sh, False)
+        snap = torch.empty(2, sh.m, dtype=torch.float64, device=self.device)
+        point = torch.empty(2, self.ld, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.lib.desmo_residual_profile(C.byref(sh), _ptr(U), _lib.u_dtype_code(U.dtype), _ptr(self.P), _ptr(self.phi),
+                                                  _ptr(self.omega), _ptr(W), _ptr(snap), _ptr(point), self._stream()), "desmo_residual_profile")
+            if self.n_global != self.n and torch.distributed.is_initialized():
+                torch.distributed.all_reduce(snap, group=self.pg)
+        return {"snapshot_residual2": snap[0, :m_out], "snapshot_norm2": snap[1, :m_out], "point_residual2": point[0, :self.n],
                 "point_norm2": point[1, :self.n]}
 
     def term_norms(self, physical: bool = False) -> torch.Tensor:

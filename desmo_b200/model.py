@@ -210,6 +210,22 @@ class _DesmoBase(nn.Module):
             zv = torch.stack(list(self.z_list), dim=0)  # CYL:550
         return recon, lat, zv
 
+    # ---- evaluation at chosen instants (DesmoEngine; exactly one of index= / times=, no autograd) ---------------------------
+    def time_points(self, index):
+        return self.engine.time_points(index)
+
+    def temporal_rows_at(self, index=None, times=None) -> torch.Tensor:
+        self.sync_parameters()
+        return self.engine.temporal_rows_at(index=index, times=times)
+
+    def reconstruct_at(self, index=None, times=None) -> torch.Tensor:
+        self.sync_parameters()
+        return self.engine.reconstruct_at(index=index, times=times)
+
+    def residual_profile_at(self, snapshots: torch.Tensor, index=None, times=None) -> dict:
+        self.sync_parameters()
+        return self.engine.residual_profile_at(snapshots, index=index, times=times)
+
     def mse_loss(self, snapshot: Optional[torch.Tensor] = None) -> torch.Tensor:
         """criterion(model(snapshot)[0], snapshot) (CYL:711,722) without materialising recon; differentiable w.r.t. every
         parameter of the module (backward = the fused residual+grad kernel)."""

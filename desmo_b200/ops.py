@@ -1,6 +1,6 @@
 """torch custom ops over the C ABI: one ``torch.ops.desmo_b200.*`` op per hot-path entry point of include/desmo_b200.h.
 
-  build_w, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, library_colnorm2, term_norms,
+  build_w, build_w_at, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, library_colnorm2, term_norms,
   pod_gram, pod_eig, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce
 
 They take the packed device tensors of a DesmoEngine (layout: include/desmo_b200.h) plus the shape integers and launch the
@@ -40,6 +40,33 @@ def build_w(gates: torch.Tensor, rows: torch.Tensor, coefs: Optional[torch.Tenso
     with torch.cuda.device(gates.device):
         check(_lib.load().desmo_build_w(C.byref(s), _p(gates), _p(rows), _p(coefs), _p(periods), _p(W), _p(step), _p(workspace),
                                         _stream(gates)), "desmo_build_w")
+
+
+@torch.library.custom_op("desmo_b200::build_w_at", mutates_args=("W_out", "rows_out"))
+def build_w_at(gates: torch.Tensor, rows: torch.Tensor, coefs: Optional[torch.Tensor], periods: Optional[torch.Tensor],
+               index: Optional[torch.Tensor], times: Optional[torch.Tensor], W_out: torch.Tensor, rows_out: Optional[torch.Tensor], n: int,
+               n_global: int, m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """W_out [Kp, mld_out] (and rows_out [K, mld_out]) = diag(gates) z(t_i) at the instants of exactly one of index (int32, training
+    snapshot indices) or times (fp32, Fourier models), both HOST tensors (desmo_build_w_at); m_out = their length, mld_out =
+    W_out.shape[1].  Nothing the model owns is written."""
+    _require_cuda(gates, rows, W_out, rows_out)
+    inst = index if times is None else times
+    if inst is None or (index is not None and times is not None):
+        raise _lib.DesmoError("build_w_at: pass exactly one of index / times")
+    want = torch.int32 if times is None else torch.float32
+    if inst.device.type != "cpu" or inst.dtype != want or inst.dim() != 1 or not inst.is_contiguous():
+        raise _lib.DesmoError(f"build_w_at: {'index' if times is None else 'times'} must be a contiguous 1-D {want} host tensor")
+    if W_out.dtype != torch.float32 or W_out.dim() != 2 or not W_out.is_contiguous() or \
+            (rows_out is not None and (rows_out.dtype != torch.float32 or not rows_out.is_contiguous() or rows_out.shape[-1] != W_out.shape[1])):
+        raise _lib.DesmoError("build_w_at: W_out [Kp, mld_out] and rows_out [K, mld_out] must be contiguous float32")
+    lib = _lib.load()
+    Kp, K = lib.desmo_padded_k(r, polyorder), lib.desmo_num_terms(r, polyorder) + 3 * r
+    if W_out.shape[0] < Kp or (rows_out is not None and rows_out.numel() < K * W_out.shape[1]):
+        raise _lib.DesmoError(f"build_w_at: W_out needs {Kp} rows and rows_out {K}")
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(gates.device):
+        check(lib.desmo_build_w_at(C.byref(s), _p(gates), _p(rows), _p(coefs), _p(periods), inst.numel(), W_out.shape[1],
+                                           _p(index), _p(times), _p(W_out), _p(rows_out), _stream(gates)), "desmo_build_w_at")
 
 
 @torch.library.custom_op("desmo_b200::fused_residual_grad", mutates_args=("dphi", "red", "workspace"))

@@ -91,6 +91,23 @@ int desmo_workspace_bytes(const desmo_shape* s, size_t* bytes);
 int desmo_build_w(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods,
                   float* W, int32_t* step_dev, void* workspace, void* stream);
 
+/* W at chosen instants (evaluation only): W_out[Kp][mld_out] = diag(gates) * z(t_i) for m_out instants, without touching the model's
+ * rows, W, workspace or step counter.  index and times are HOST arrays of m_out entries; exactly one of them is non-NULL.
+ *   index : instant i is training snapshot index[i] (0 <= index[i] < m, any order, repeats allowed).  DESMO gathers rows[k][index[i]];
+ *           DESMOFourier evaluates its series at t_point(index[i], m), the fp32 time desmo_build_w uses, so column i is bit for bit
+ *           column index[i] of desmo_build_w's W.
+ *   times : DESMOFourier only (DESMO_ERR_ARG for DESMO's free rows): instant i is times[i] in the model's own time coordinate (the
+ *           units of t_points, FCYL:485), any finite fp32 value, also before 0 or beyond the training window.  The series is
+ *           evaluated with desmo_build_w's own operations, so times[i] == t_point(k, m) gives column k bit for bit.
+ * rows_out[K][mld_out] (may be NULL) receives z_k(t_i) unscaled (forward()'s z_values).  mld_out >= m_out, mld_out % 16 == 0; pad
+ * columns and rows K..Kp-1 of W_out are zero, as are the pad columns of rows_out.  rows is read for DESMO only (may be NULL for
+ * DESMOFourier).  Every argument, the index range and the finiteness of the times included, is checked on the host before any
+ * launch.  The instants travel as kernel parameters (one launch per 512), so the call allocates nothing, never synchronises and
+ * can be captured in a CUDA graph; the host arrays may be reused as soon as it returns. */
+int desmo_build_w_at(const desmo_shape* s, const float* gates, const float* rows, const float* coefs, const float* periods,
+                     int32_t m_out, int32_t mld_out, const int32_t* index, const float* times, float* W_out, float* rows_out,
+                     void* stream);
+
 /* The fused pass: streams U once and produces, without materialising R = G(Phi) W - U,
  *   red    (see above; overwritten, local-rank partial)
  *   dphi   [r][ld]  d mse / d phi_list (chain rule through POOL_DATA, sin/cos/tanh and phi*POD; ortho term excluded)
