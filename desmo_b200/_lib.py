@@ -66,6 +66,8 @@ SIGNATURES: Dict[str, tuple] = {
     "desmo_pod_project": (C.c_int, [_SP] + [_vp] * 5),
     "desmo_pod_gram_ex": (C.c_int, [_SP, _vp, _i32, _vp, _vp, _vp]),
     "desmo_pod_project_ex": (C.c_int, [_SP, _vp, _i32, _vp, _vp, _vp, _vp]),
+    "desmo_pod_eigh_workspace_bytes": (C.c_int, [_i32, _i32, C.POINTER(C.c_size_t)]),
+    "desmo_pod_eigh": (C.c_int, [_i32, _i32] + [_vp] * 5 + [C.c_size_t, _vp]),
     "desmo_preprocess": (C.c_int, [_SP, _vp, _i32, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
     "desmo_preprocess_ex": (C.c_int, [_SP, _vp, _i32, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _i32, _vp, _vp, _vp]),
     "desmo_snapshot_to_bf16": (C.c_int, [_SP, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),

@@ -497,6 +497,35 @@ int desmo_pod_eig(int32_t m, int32_t r, const float* C, float* V, float* sigma, 
     return pod_eig(m, r, C, V, sigma, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
+static int check_eigh_args(int32_t m, int32_t r, const char* what) {
+    if (m < 1 || r < 1) { set_error("%s: need m >= 1 and r >= 1 (got m=%d r=%d)", what, m, r); return DESMO_ERR_ARG; }
+    if (r > DESMO_MAX_R || m > DESMO_EIGH_MAX_M) {
+        set_error("%s: r=%d, m=%d outside r <= %d, m <= %d", what, r, m, DESMO_MAX_R, DESMO_EIGH_MAX_M);
+        return DESMO_ERR_UNSUPPORTED;
+    }
+    if (r > m) { set_error("%s: r=%d modes of an m=%d Gram", what, r, m); return DESMO_ERR_ARG; }
+    return DESMO_OK;
+}
+
+int desmo_pod_eigh_workspace_bytes(int32_t m, int32_t r, size_t* bytes) {
+    if (!bytes) { set_error("desmo_pod_eigh_workspace_bytes: null pointer"); return DESMO_ERR_ARG; }
+    const int rc = check_eigh_args(m, r, "desmo_pod_eigh_workspace_bytes");
+    if (rc) return rc;
+    *bytes = pod_eigh_workspace_bytes(m, r);
+    return DESMO_OK;
+}
+
+int desmo_pod_eigh(int32_t m, int32_t r, const float* C, double* S, float* V, float* sigma, void* workspace, size_t workspace_bytes,
+                   void* stream) {
+    int rc = check_eigh_args(m, r, "desmo_pod_eigh");
+    if (rc) return rc;
+    if (!C || !S || !V || !sigma || !workspace) { set_error("desmo_pod_eigh: null pointer"); return DESMO_ERR_ARG; }
+    const size_t need = pod_eigh_workspace_bytes(m, r);
+    if (workspace_bytes < need) { set_error("desmo_pod_eigh: workspace too small (%zu < %zu)", workspace_bytes, need); return DESMO_ERR_ARG; }
+    if ((rc = device_ok())) return rc;
+    return pod_eigh(m, r, C, S, V, sigma, workspace, (cudaStream_t)stream);
+}
+
 int desmo_pod_project_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* V, const float* sigma, float* P, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);

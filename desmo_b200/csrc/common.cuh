@@ -108,6 +108,9 @@ int pod_gram_fp32(const desmo_shape* s, const void* U, int u_dtype, float* C, cu
 int pod_gram_tc(const desmo_shape* s, const void* U, int u_dtype, float* C, void* workspace, cudaStream_t st);
 int pod_eig(int m, int r, const float* C, float* V, float* sigma, void* workspace, size_t workspace_bytes, cudaStream_t st);
 int pod_project(const desmo_shape* s, const void* U, int u_dtype, const float* V, const float* sigma, float* P, cudaStream_t st);
+// dense eigensolver (eigh.cu); arguments validated by desmo_pod_eigh
+size_t pod_eigh_workspace_bytes(int m, int r);
+int pod_eigh(int m, int r, const float* C, double* S, float* V, float* sigma, void* workspace, cudaStream_t st);
 // U is written as fp32 or, for u_dtype == DESMO_DTYPE_BF16, as bf16_rn of the fp32 value; qsums (optional, fp64 [2]) accumulates
 // sum (u - q)^2 and sum u^2 over the n real points, u = the fp32 value, q = the stored one
 int preprocess(const desmo_shape* s, const void* V, int v_dtype, long long v_ld, int m_in, int t_stride, int d_in, int d_use, int flags,

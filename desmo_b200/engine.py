@@ -562,18 +562,11 @@ class DesmoEngine:
         eigensolver does not converge (P then holds the projection of the unconverged modes)."""
         ud = self._u_dtype()
         f32 = dict(dtype=torch.float32, device=self.device)
-        Cm = torch.zeros(self.m, self.m, **f32)
         V, sigma = torch.zeros(self.r, self.m, **f32), torch.zeros(self.r, **f32)
         ws = torch.zeros(2 * 8 * 16 * self.m + 1024, dtype=torch.uint8, device=self.device)
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
         with torch.cuda.device(self.device):
-            ev[0].record()
-            check(self.lib.desmo_pod_gram_ex(C.byref(self.shape), _ptr(self.U), ud, _ptr(Cm), _ptr(self.workspace), self._stream()),
-                  "desmo_pod_gram")
-            ev[1].record()
-            if self.n_global != self.n and torch.distributed.is_initialized():
-                torch.distributed.all_reduce(Cm, group=self.pg)
-            trace = Cm.diagonal().sum(dtype=torch.float64)  # = sum of all sigma^2 = ||X||_F^2 (the all-reduced Gram's trace)
+            Cm, trace = self._pod_gram(ev[0], ev[1])
             check(self.lib.desmo_pod_eig(self.m, self.r, _ptr(Cm), _ptr(V), _ptr(sigma), _ptr(ws), ws.numel(), self._stream()), "desmo_pod_eig")
             ev[2].record()
             check(self.lib.desmo_pod_project_ex(C.byref(self.shape), _ptr(self.U), ud, _ptr(V), _ptr(sigma), _ptr(self.P), self._stream()),
@@ -589,6 +582,61 @@ class DesmoEngine:
             raise _lib.DesmoError(f"desmo_pod_eig did not converge in {iterations} sweeps (residual {self.pod_eig_residual:.2e} lambda_1)")
         # POD_analysis' diagnostics (CYL:200-211) without forming X_approx: energy_content = S^2 / sum(S^2) of the r leading modes, its
         # running sum, and err_POD = ||X - X_r|| / ||X|| = sqrt(1 - sum_{i<r} sigma_i^2 / ||X||_F^2) (Eckart-Young)
+        s2 = sigma.double() ** 2
+        self.pod_energy = (s2 / trace).cpu()
+        self.pod_cumulative_energy = torch.cumsum(self.pod_energy, 0)
+        self.pod_error = float(torch.sqrt(torch.clamp(1.0 - s2.sum() / trace, min=0.0)))
+        return sigma
+
+    def _pod_gram(self, ev_start: torch.cuda.Event, ev_gram: torch.cuda.Event):
+        """C = U U^T of the resident snapshot, all-reduced over the ranks when point-sharded, and its fp64 trace (= ||X||_F^2).  The
+        events bracket the Gram kernel (the all-reduce comes after ev_gram).  Call inside torch.cuda.device(self.device)."""
+        Cm = torch.zeros(self.m, self.m, dtype=torch.float32, device=self.device)
+        ev_start.record()
+        check(self.lib.desmo_pod_gram_ex(C.byref(self.shape), _ptr(self.U), self._u_dtype(), _ptr(Cm), _ptr(self.workspace), self._stream()),
+              "desmo_pod_gram")
+        ev_gram.record()
+        if self.n_global != self.n and torch.distributed.is_initialized():
+            torch.distributed.all_reduce(Cm, group=self.pg)
+        return Cm, Cm.diagonal().sum(dtype=torch.float64)
+
+    def _eigh_workspace(self) -> torch.Tensor:
+        nbytes = C.c_size_t(0)
+        check(self.lib.desmo_pod_eigh_workspace_bytes(self.m, self.r, C.byref(nbytes)), "desmo_pod_eigh_workspace_bytes")
+        return torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+
+    def pod_analysis(self) -> torch.Tensor:
+        """POD_analysis (CYL:197-211) of the resident snapshot matrix for any r <= 64: returns the singular values sigma (r,) and
+        fills self.P with the r leading modes.
+
+        The Gram C = U U^T (all-reduced when point-sharded) goes through the dense fp64 eigensolver (desmo_pod_eigh), which also
+        returns the whole spectrum: self.pod_singular_values holds all m singular values (fp64, host, descending), POD_analysis'
+        S for the energy plot and the choice of r.  Sets the attributes pod_from_snapshot sets (pod_V = the temporal coefficients
+        V^T[:r], pod_gram, pod_energy, pod_cumulative_energy, pod_error, pod_timing).  A mode at the rounding level of the fp32 Gram
+        (lambda_i <= 2^-23 trace) comes back as sigma_i = 0 with a zero row of P.  Raises DesmoError, with P untouched, when the
+        solver reports a non-finite result or a residual ||C v_i - lambda_i v_i|| above 2^-27 lambda_1."""
+        f32 = dict(dtype=torch.float32, device=self.device)
+        V, sigma = torch.zeros(self.r, self.m, **f32), torch.zeros(self.r, **f32)
+        S = torch.zeros(self.m, dtype=torch.float64, device=self.device)
+        ws = self._eigh_workspace()
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+        with torch.cuda.device(self.device):
+            Cm, trace = self._pod_gram(ev[0], ev[1])
+            check(self.lib.desmo_pod_eigh(self.m, self.r, _ptr(Cm), _ptr(S), _ptr(V), _ptr(sigma), _ptr(ws), ws.numel(), self._stream()),
+                  "desmo_pod_eigh")
+            ev[2].record()
+            status = int(ws[:4].view(torch.int32).item())
+            residual = float(ws[8:16].view(torch.float64).item())
+            self.pod_eig_residual = residual
+            if status != 0 or not residual <= 2.0 ** -27:
+                raise _lib.DesmoError(f"desmo_pod_eigh failed (status {status}, residual {residual:.2e} lambda_1); P is unchanged")
+            check(self.lib.desmo_pod_project_ex(C.byref(self.shape), _ptr(self.U), self._u_dtype(), _ptr(V), _ptr(sigma), _ptr(self.P),
+                                                self._stream()), "desmo_pod_project")
+            ev[3].record()
+        torch.cuda.synchronize(self.device)
+        self.pod_timing = {"gram_ms": ev[0].elapsed_time(ev[1]), "eig_ms": ev[1].elapsed_time(ev[2]), "project_ms": ev[2].elapsed_time(ev[3])}
+        self.pod_V, self.pod_gram = V, Cm
+        self.pod_singular_values = S.cpu()
         s2 = sigma.double() ** 2
         self.pod_energy = (s2 / trace).cpu()
         self.pod_cumulative_energy = torch.cumsum(self.pod_energy, 0)

@@ -1,7 +1,7 @@
 """torch custom ops over the C ABI: one ``torch.ops.desmo_b200.*`` op per hot-path entry point of include/desmo_b200.h.
 
   build_w, build_w_at, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, library_colnorm2, term_norms,
-  pod_gram, pod_eig, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce
+  pod_gram, pod_eig, pod_eigh, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce
 
 They take the packed device tensors of a DesmoEngine (layout: include/desmo_b200.h) plus the shape integers and launch the
 sm_100a kernels on the current stream.  CUDA only: no CPU implementation is registered and every op checks its tensors, so a call
@@ -187,6 +187,15 @@ def pod_eig(Cm: torch.Tensor, V: torch.Tensor, sigma: torch.Tensor, workspace: t
                                         _stream(Cm)), "desmo_pod_eig")
 
 
+@torch.library.custom_op("desmo_b200::pod_eigh", mutates_args=("S", "V", "sigma", "workspace"))
+def pod_eigh(Cm: torch.Tensor, S: torch.Tensor, V: torch.Tensor, sigma: torch.Tensor, workspace: torch.Tensor, m: int, r: int) -> None:
+    """All m singular values S (fp64) and the top r eigenpairs (V, sigma) of the Gram Cm (desmo_pod_eigh); report in workspace[:16]."""
+    _require_cuda(Cm, S, V, sigma, workspace)
+    with torch.cuda.device(Cm.device):
+        check(_lib.load().desmo_pod_eigh(m, r, _p(Cm), _p(S), _p(V), _p(sigma), _p(workspace), workspace.numel() * workspace.element_size(),
+                                         _stream(Cm)), "desmo_pod_eigh")
+
+
 @torch.library.custom_op("desmo_b200::pod_project", mutates_args=("P",))
 def pod_project(U: torch.Tensor, V: torch.Tensor, sigma: torch.Tensor, P: torch.Tensor, n: int, n_global: int, m: int, r: int,
                 polyorder: int, nF: int, path: int) -> None:
@@ -310,5 +319,25 @@ def engine_pod_via_ops(e) -> torch.Tensor:
     if e.n_global != e.n and torch.distributed.is_initialized():
         torch.distributed.all_reduce(Cm, group=e.pg)
     torch.ops.desmo_b200.pod_eig(Cm, V, sigma, ws, e.m, e.r)
+    torch.ops.desmo_b200.pod_project(e.U, V, sigma, e.P, *sa)
+    return sigma
+
+
+def engine_pod_analysis_via_ops(e) -> torch.Tensor:
+    """DesmoEngine.pod_analysis() through the registered pod_gram / pod_eigh / pod_project ops: returns sigma, fills e.P (untouched when
+    the solver's report is not OK)."""
+    sa = _shape_args(e)
+    f32 = dict(dtype=torch.float32, device=e.device)
+    Cm = torch.zeros(e.m, e.m, **f32)
+    V, sigma = torch.zeros(e.r, e.m, **f32), torch.zeros(e.r, **f32)
+    S = torch.zeros(e.m, dtype=torch.float64, device=e.device)
+    ws = e._eigh_workspace()
+    torch.ops.desmo_b200.pod_gram(e.U, Cm, e.workspace, *sa)
+    if e.n_global != e.n and torch.distributed.is_initialized():
+        torch.distributed.all_reduce(Cm, group=e.pg)
+    torch.ops.desmo_b200.pod_eigh(Cm, S, V, sigma, ws, e.m, e.r)
+    status, residual = int(ws[:4].view(torch.int32).item()), float(ws[8:16].view(torch.float64).item())
+    if status != 0 or not residual <= 2.0 ** -27:
+        raise _lib.DesmoError(f"desmo_pod_eigh failed (status {status}, residual {residual:.2e} lambda_1); P is unchanged")
     torch.ops.desmo_b200.pod_project(e.U, V, sigma, e.P, *sa)
     return sigma

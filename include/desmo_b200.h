@@ -238,6 +238,21 @@ int desmo_pod_project(const desmo_shape* s, const float* U, const float* V, cons
 int desmo_pod_gram_ex(const desmo_shape* s, const void* U, int32_t u_dtype, float* C, void* workspace, void* stream);
 int desmo_pod_project_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* V, const float* sigma, float* P, void* stream);
 
+/* POD eigensolve for any r <= DESMO_MAX_R, with the full spectrum (POD_analysis' S, CYL:197-211): a dense fp64 eigensolver of the
+ * (all-reduced) Gram C[m][m], read as symmetric through its lower triangle.  1 <= r <= min(DESMO_MAX_R, m), m <= DESMO_EIGH_MAX_M.
+ *   S[m]      fp64, all m singular values sqrt(lambda_i), descending; lambda_i <= 2^-23 trace(C) gives 0 (desmo_pod_eig's floor)
+ *   V[r][m]   the top r eigenvectors, orthonormal (floored modes included), largest-|.| entry positive
+ *   sigma[r]  fp32 S[:r]; V and sigma feed desmo_pod_project_ex unchanged
+ * Householder tridiagonalisation, bisection, inverse iteration with re-orthogonalisation inside clusters, back-transformation;
+ * then every emitted pair is checked in fp64 against the fp32 C.  Stream-ordered, no allocation, no synchronisation; the same C
+ * gives the same bits on every call.  workspace_bytes >= desmo_pod_eigh_workspace_bytes(m, r) (8 m^2 + O(r m) bytes).  Its first
+ * 16 bytes receive {int32 status (0: every output finite), int32, double worst ||C v_i - lambda_i v_i|| / lambda_1 over the modes
+ * above the floor}; read them once the stream has passed the call. */
+#define DESMO_EIGH_MAX_M 8192
+int desmo_pod_eigh_workspace_bytes(int32_t m, int32_t r, size_t* bytes);
+int desmo_pod_eigh(int32_t m, int32_t r, const float* C, double* S, float* V, float* sigma, void* workspace, size_t workspace_bytes,
+                   void* stream);
+
 /* Snapshot pre-processing between the reader and POD/training, on the device (reference: numpy on the host).  V is X.T as
  * read: V[m_in][v_ld] with v_ld >= n * d_in, a point's d_in components adjacent.  Replaces convert3Dto2D_data (CYL:88-106:
  * d_in = 3, d_use = 2), convertToMagnitude (CYL:109-133, float64), subtract_mean (CYL:136-149; mean over all m_in snapshots),
