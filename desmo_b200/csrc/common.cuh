@@ -155,6 +155,13 @@ __device__ __forceinline__ float ldg_u(const __nv_bfloat16* p) {
     return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
 }
 
+// Nanosecond clock of the device, common to all SMs: the time base of the watchdogs that trap a wait still open after ~10 s.
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
+    return t;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -31,11 +31,6 @@ __device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p) {
     asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
     return v;
 }
-__device__ __forceinline__ unsigned long long eigh_globaltimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
 
 // Grid-wide barrier of the cooperative tridiagonalisation kernel: a monotonic arrival counter (zeroed before the launch).  A CTA
 // that never arrives fails the launch after ~10 s instead of hanging the GPU.
@@ -45,9 +40,9 @@ __device__ __forceinline__ void grid_barrier(unsigned* counter, unsigned& target
     if (threadIdx.x == 0) {
         __threadfence();
         atomicAdd(counter, 1u);
-        const unsigned long long t0 = eigh_globaltimer_ns();
+        const unsigned long long t0 = globaltimer_ns();
         while ((int)(ld_acquire_gpu(counter) - target) < 0)
-            if (eigh_globaltimer_ns() - t0 > 10000000000ull) __trap();
+            if (globaltimer_ns() - t0 > 10000000000ull) __trap();
         __threadfence();
     }
     __syncthreads();

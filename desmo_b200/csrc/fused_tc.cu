@@ -25,8 +25,10 @@
 #include <type_traits>
 
 #include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace desmo {
+using namespace ptx;
 
 namespace tc {
 constexpr int KP = 32;          // padded library size handled by this kernel
@@ -116,13 +118,9 @@ struct TcArgs {
     MonoTable mt;
 };
 
-// ------------------------------------------------------------------------------------------------- PTX helpers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+// ------------------------------------------------------------------------------------------------- PTX helpers (the rest: tcgen05.cuh)
 __device__ __forceinline__ uint32_t sw128(uint32_t row, uint32_t byte_in_row) {
     return row * 128u + ((((byte_in_row >> 4) ^ (row & 7u)) << 4) | (byte_in_row & 15u));
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
 }
 __device__ unsigned long long* g_tc_dbg = nullptr;  // host-mapped diagnostics buffer (DESMO_TC_DEBUG), survives a trap
 template <bool kDebug>
@@ -131,8 +129,7 @@ __device__ __forceinline__ void mbar_wait_t(uint32_t bar, uint32_t parity, int t
     unsigned spins = 0;
     while (!done) {
         // the suspend-time hint lets the hardware park the thread instead of burning issue slots the epilogue math needs
-        asm volatile("{\n\t.reg .pred q;\n\tmbarrier.try_wait.parity.shared::cta.b64 q, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, q;\n\t}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity), "r"(kDebug ? 2000u : 0x989680u) : "memory");
+        done = mbar_try_wait(bar, parity, kDebug ? 2000u : 0x989680u);
         if (kDebug && !done && ++spins >= (1u << 20)) {
             // debug runs report who was stuck where (production runs rely on the CTA's watchdog lane: a spin counter in every
             // wait loop was measured to cost 6 % of the kernel)
@@ -145,16 +142,6 @@ __device__ __forceinline__ void mbar_wait_t(uint32_t bar, uint32_t parity, int t
         }
     }
 }
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar) : "memory");
-}
 // One non-blocking test of a phase, without a retry loop.  A SYNCS round trip costs a few hundred cycles under this kernel's
 // shared-memory load even when the phase completed long ago; a straight-line probe lets ptxas place independent work (or a second
 // probe) under that latency, which a wait loop (a branch after every attempt) cannot.  test_wait, not try_wait: try_wait may park the
@@ -166,26 +153,10 @@ __device__ __forceinline__ uint32_t mbar_probe(uint32_t bar, uint32_t parity) {
                  : "=r"(done) : "r"(bar), "r"(parity) : "memory");
     return done;
 }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 __device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
     return (uint64_t)((saddr >> 4) & 0x3fff) | ((uint64_t)((lbo_bytes >> 4) & 0x3fff) << 16) |
            ((uint64_t)((sbo_bytes >> 4) & 0x3fff) << 32) | ((uint64_t)1 << 46) | ((uint64_t)2 << 61);  // version 1, SWIZZLE_128B
-}
-__device__ __forceinline__ constexpr uint32_t make_idesc_bf16(int M, int N, int a_mn, int b_mn) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) |
-           ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ void mma_bf16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
 // Collector hints: consecutive MMAs that read the SAME A tile (or, for the weight-stationary form, the same B tile) keep it in the
 // tensor core's operand collector instead of fetching it from shared memory again -- shared-memory bandwidth binds this kernel.
@@ -227,28 +198,13 @@ __device__ __forceinline__ void mma_bf16_ts_wsb(uint32_t d_tmem, uint32_t a_tmem
                      "tcgen05.mma.ws.cta_group::1.kind::f16.collector::b0::discard [%0], [%1], %2, %3, p;\n\t}\n"
                      ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* v) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-                   "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                 : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
 __device__ __forceinline__ void st_shared_u16(uint32_t addr, uint16_t v) {
     asm volatile("st.shared.u16 [%0], %1;" ::"r"(addr), "h"(v) : "memory");
-}
-__device__ __forceinline__ bool elect_one_sync() {
-    uint32_t pred = 0;
-    asm volatile("{\n\t.reg .b32 rx;\n\t.reg .pred px;\n\telect.sync rx|px, %1;\n\t@px mov.s32 %0, 1;\n\t}\n" : "+r"(pred) : "r"(0xffffffffu));
-    return pred != 0;
 }
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t* v) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                  : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]) : "r"(taddr) : "memory");
 }
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_st1(uint32_t taddr, uint32_t v) {
     asm volatile("tcgen05.st.sync.aligned.32x32b.x1.b32 [%0], {%1};" ::"r"(taddr), "r"(v) : "memory");
 }
@@ -270,12 +226,8 @@ __device__ __forceinline__ void split2_pair(float x0, float x1, uint32_t& w1, ui
 }
 
 // The six (a-plane, b-plane) products kept by the 3-way split (i + j <= 4), smallest contributions first.
-// Descriptors: the high word is constant per operand role; the low word is (addr >> 4) | (LBO >> 4) << 16, so stepping through
-// planes / k-steps is ONE 32-bit add of a compile-time constant per operand (smem addresses < 256 KB never carry out of 14 bits).
 #define DESMO_PAIRS(X) X(2, 0) X(0, 2) X(1, 1) X(1, 0) X(0, 1) X(0, 0)
 #define DESMO_GRAD_PAIRS(X) X(1, 0) X(0, 1) X(0, 0)
-__device__ __forceinline__ uint64_t desc_from(uint32_t lo, uint32_t hi) { return ((uint64_t)hi << 32) | lo; }
-constexpr uint32_t kDescHi = (1024u >> 4) | (1u << 14) | (2u << 29);  // SBO = 1024 B, version 1, SWIZZLE_128B
 
 // kSupplied: backward of forward()'s reconstruction for an arbitrary upstream gradient (desmo_recon_backward): the buffer read through
 // the U path holds dL/drecon, R := seed_scale * (that) instead of G W - U, G1 is skipped; G3 / G4 / hand-overs are unchanged.
@@ -327,12 +279,9 @@ __global__ void __launch_bounds__(tc::THREADS, 1) fused_tc_kernel(const TcArgs a
         mbar_init(bar(D_FULL), 1); mbar_init(bar(D_EMPTY), EPI_THREADS);
         for (int i = 0; i < NQ * U_RING; ++i) { mbar_init(bar(U_FULL0 + i), 1); mbar_init(bar(U_EMPTY0 + i), 128); }
         for (int i = 0; i < 4; ++i) mbar_init(bar(R_EMPTYQ0 + i), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbar_init();
     }
-    if (warp == 2) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 2) tmem_alloc<512>(smem_u32(&tmem_base_s));
     if (tid < 4) red_s[tid] = 0.0;
     if (tid == 0) progress_s = 0;
     if (tid < 3 * a.r) omega_s[tid] = a.omega[tid];
@@ -870,7 +819,7 @@ __global__ void __launch_bounds__(tc::THREADS, 1) fused_tc_kernel(const TcArgs a
         a.Spart[(long long)blockIdx.x * kScal + i] = (i == 0) ? (((red_s[0] + red_s[1]) + red_s[2]) + red_s[3]) : 0.0;
     if (warp == 2) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512u) : "memory");
+        tmem_dealloc<512>(tmem);
     }
 }
 
@@ -945,21 +894,6 @@ int tc_debug_read(uint64_t* out, int count) {
     if (!g_dbg_host) return DESMO_ERR_ARG;
     memcpy(out, g_dbg_host, sizeof(uint64_t) * (count < (int)kDbgWords ? count : (int)kDbgWords));
     return DESMO_OK;
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(p);
-    }
-    return fn;
 }
 
 int fused_tc_supported(const desmo_shape* s, int Kp) {

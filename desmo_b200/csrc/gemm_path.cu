@@ -24,9 +24,11 @@
 #include <type_traits>
 
 #include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace desmo {
 namespace gp {
+using namespace ptx;
 
 constexpr int BM = 128, BN = 128, BK = 64;
 constexpr uint32_t PLANE_TILE = 128 * 128;  // bytes of one operand plane tile: 128 rows x 64 bf16 (K-major) or 2 x [64 k-rows x 64 bf16] (MN-major)
@@ -42,59 +44,17 @@ enum { EPI_RESID = 0, EPI_D = 1, EPI_E = 2, EPI_RECON = 3, EPI_RESID_BF16 = 4, E
 constexpr int kProfSlab = 4 * 2 * 4 * 32 + 2 * 128;
 constexpr size_t kProfSmem = 2 * sizeof(float) * kProfSlab;
 
-// ------------------------------------------------------------------------------------------------- PTX helpers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
+// ------------------------------------------------------------------------------------------------- PTX helpers (the rest: tcgen05.cuh)
 // Every wait carries a watchdog: a protocol error traps (the launch fails with an error) instead of hanging the GPU.
+// (Keep this loop's shape: written as while (!mbar_try_wait(...)) it compiles to different register allocations in every GEMM kernel.)
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     uint32_t done = 0;
     unsigned spins = 0;
     while (!done) {
-        asm volatile("{\n\t.reg .pred q;\n\tmbarrier.try_wait.parity.shared::cta.b64 q, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, q;\n\t}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity), "r"(20000u) : "memory");
+        done = mbar_try_wait(bar, parity, 20000u);
         if (!done && ++spins > (1u << 18)) __trap();
     }
 }
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ bool elect_one_sync() {
-    uint32_t pred = 0;
-    asm volatile("{\n\t.reg .b32 rx;\n\t.reg .pred px;\n\telect.sync rx|px, %1;\n\t@px mov.s32 %0, 1;\n\t}\n" : "+r"(pred) : "r"(0xffffffffu));
-    return pred != 0;
-}
-__device__ __forceinline__ void mma_bf16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* v) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-                   "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                 : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-// instruction descriptor, kind::f16 with bf16 operands and fp32 accumulation (same encoding as fused_tc.cu)
-__host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N, int a_mn, int b_mn) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) |
-           ((uint32_t)(M >> 4) << 24);
-}
-constexpr uint32_t kDescHi = (1024u >> 4) | (1u << 14) | (2u << 29);  // SBO = 1024 B, version 1, SWIZZLE_128B
-__device__ __forceinline__ uint64_t desc_from(uint32_t lo, uint32_t hi) { return ((uint64_t)hi << 32) | lo; }
 // K-major operand tile [128 rows][128 B]: LBO unused (1); a k-step of 16 elements advances 32 B inside the swizzled row.
 // MN-major operand tile, two boxes [64 k-rows][128 B = 64 mn]: LBO = 8192 B (next 64-wide mn block); a k-step of 16 rows advances 2048 B.
 template <bool MN>
@@ -162,12 +122,9 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
     if (tid == 32) {
         for (int i = 0; i < NSTAGE; ++i) { mbar_init(bar(FULL0 + i), 1); mbar_init(bar(EMPTY0 + i), 1); }
         for (int i = 0; i < 2; ++i) { mbar_init(bar(ACC_FULL0 + i), 1); mbar_init(bar(ACC_EMPTY0 + i), EPI_WARPS * 32); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbar_init();
     }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(256u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 0) tmem_alloc<256>(smem_u32(&tmem_base_s));
     if (tid < EPI_WARPS) loss_s[tid] = 0.0;
     tc_fence_before();
     __syncthreads();
@@ -413,7 +370,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
     }
     if (warp == 0) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(256u) : "memory");
+        tmem_dealloc<256>(tmem);
     }
 }
 
@@ -677,20 +634,6 @@ __global__ void __launch_bounds__(256) colnorm2_generic_kernel(const float* __re
 }
 
 // ------------------------------------------------------------------------------------------------- host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(p);
-    }
-    return fn;
-}
-
 // 2-D bf16 map over `rows` rows of `inner` contiguous elements; box = [64 inner][box_rows]
 static int make_map(CUtensorMap* tm, const void* base, long long inner, long long rows, int box_rows) {
     EncodeTiledFn enc = encode_fn();

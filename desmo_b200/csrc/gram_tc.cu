@@ -14,9 +14,11 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace desmo {
 namespace gram {
+using namespace ptx;
 
 constexpr int BM = 128;            // rows (snapshots) per tile edge
 constexpr int BK = 64;             // mesh points per chunk (= one 128 B swizzled row of bf16)
@@ -30,36 +32,13 @@ constexpr uint32_t OPERAND = 3 * PLANE;              // 49152
 constexpr uint32_t STAGE = 2 * OPERAND;              // A planes + B planes
 constexpr uint32_t SMEM_BYTES = 2 * STAGE + 1024;    // two stages + alignment slack
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
+// Every wait carries a watchdog: a wait still open after ~10 s (by %globaltimer, read only once the first try has failed) traps,
+// so a protocol error fails the launch instead of hanging the GPU.  The 10 ms suspend hint parks the waiting warps.
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    while (!done)
-        asm volatile("{\n\t.reg .pred q;\n\tmbarrier.try_wait.parity.shared::cta.b64 q, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, q;\n\t}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity), "r"(0x989680u) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ bool elect_one_sync() {
-    uint32_t pred = 0;
-    asm volatile("{\n\t.reg .b32 rx;\n\t.reg .pred px;\n\telect.sync rx|px, %1;\n\t@px mov.s32 %0, 1;\n\t}\n" : "+r"(pred) : "r"(0xffffffffu));
-    return pred != 0;
-}
-__device__ __forceinline__ void mma_bf16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* v) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-                   "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                 : "r"(taddr) : "memory");
+    if (mbar_try_wait(bar, parity, 0x989680u)) return;
+    const unsigned long long t0 = globaltimer_ns();
+    while (!mbar_try_wait(bar, parity, 0x989680u))
+        if (globaltimer_ns() - t0 > 10000000000ull) __trap();
 }
 // volatile: keeps the next chunk's loads BELOW the current chunk's split + stores (hoisted, they double the live registers and spill)
 __device__ __forceinline__ float4 ldg_nc_v4(const float4* p) {
@@ -71,9 +50,6 @@ __device__ __forceinline__ uint4 ldg_nc_u4(const uint4* p) {
     uint4 v;
     asm volatile("ld.global.nc.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
     return v;
-}
-__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
 __device__ __forceinline__ void split3_pair(float x0, float x1, uint32_t& w1, uint32_t& w2, uint32_t& w3) {
     asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(w1) : "f"(x1), "f"(x0));
@@ -109,21 +85,17 @@ __global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const void* __restr
     if (tid == 32) {
         mbar_init(bar(FULL0), CONV_WARPS * 32); mbar_init(bar(FULL1), CONV_WARPS * 32);
         mbar_init(bar(EMPTY0), 1); mbar_init(bar(EMPTY1), 1); mbar_init(bar(ACC_FULL), 1); mbar_init(bar(ACC_EMPTY), CONV_WARPS * 32);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbar_init();
     }
-    if (warp == 2) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(128u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    if (warp == 2) tmem_alloc<128>(smem_u32(&tmem_base_s));
+    tc_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc_fence_after();
     const uint32_t tmem = tmem_base_s;
 
     if (warp == 1) {
         if (elect_one_sync()) {
-            constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BM >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);  // bf16 x bf16 -> f32, K-major both
-            constexpr uint32_t desc_hi = (1024u >> 4) | (1u << 14) | (2u << 29);                                                        // SBO 1024, v1, SWIZZLE_128B
+            constexpr uint32_t idesc = make_idesc_bf16(BM, BM, 0, 0);  // K-major both
             uint32_t acc = 0;
             for (int c = 0; c < nchunks; ++c) {
                 const int st = c & 1;
@@ -132,13 +104,13 @@ __global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const void* __restr
                     acc = 0;
                 }
                 mbar_wait(bar(FULL0 + st), (c >> 1) & 1);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 const uint32_t a_lo = ((sbase + st * STAGE) >> 4) | (1u << 16);
                 const uint32_t b_lo = diag ? a_lo : (((sbase + st * STAGE + OPERAND) >> 4) | (1u << 16));
 #define GRAM_PAIR(PA, PB)                                                                                                   \
     _Pragma("unroll") for (int ks = 0; ks < BK / 16; ++ks) {                                                                 \
-        mma_bf16(tmem, ((uint64_t)desc_hi << 32) | (a_lo + ((PA * PLANE + ks * 32) >> 4)),                                   \
-                 ((uint64_t)desc_hi << 32) | (b_lo + ((PB * PLANE + ks * 32) >> 4)), idesc, acc);                            \
+        mma_bf16(tmem, desc_from(a_lo + ((PA * PLANE + ks * 32) >> 4), kDescHi),                                             \
+                 desc_from(b_lo + ((PB * PLANE + ks * 32) >> 4), kDescHi), idesc, acc);                                      \
         acc = 1;                                                                                                             \
     }
                 if constexpr (kU16) {
@@ -243,13 +215,13 @@ __global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const void* __restr
                 if (!diag) store_planes(sbase + st * STAGE + OPERAND, rb);
             }
             if (c + 1 < nchunks) load_chunk(c + 1);  // next chunk's loads fly while this chunk's MMAs run
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_async_smem();
             mbar_arrive(bar(FULL0 + st));
             if ((c + 1) % FLUSH == 0 || c == nchunks - 1) {
                 // ---- drain the accumulator tile: partial += TMEM (fp32 RN); the last drain goes to C (and its mirror) ----
                 const int f = c / FLUSH;
                 mbar_wait(bar(ACC_FULL), f & 1);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
 #pragma unroll
                 for (int cc = 0; cc < 4; ++cc) {
                     uint32_t v[16];
@@ -259,22 +231,22 @@ __global__ void __launch_bounds__(THREADS, 1) gram_tc_kernel(const void* __restr
 #pragma unroll
                     for (int j = 0; j < 16; ++j) old[j] = (f == 0) ? 0.0f : __ldcg(pp + j * BM);
                     tmem_ld16(tmem + ((uint32_t)(q * 32) << 16) + hcol * 64 + cc * 16, v);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                    tmem_ld_wait();
 #pragma unroll
                     for (int j = 0; j < 16; ++j) {
                         __stcg(pp + j * BM, old[j] + __uint_as_float(v[j]));  // the per-CTA partial tile; summed in a fixed order below
                     }
                 }
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                tc_fence_before();
                 mbar_arrive(bar(ACC_EMPTY));
             }
         }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
     }
     __syncthreads();
     if (warp == 2) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(128u) : "memory");
+        tc_fence_after();
+        tmem_dealloc<128>(tmem);
     }
 }
 

@@ -36,11 +36,6 @@ __device__ __forceinline__ float4 ld_volatile_f4(const float4* p) {
     asm volatile("ld.volatile.global.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p) : "memory");
     return v;
 }
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
 // spins until *flag >= target; a peer that never arrives (crashed rank) fails the launch after ~10 s instead of hanging the GPU
 __device__ __forceinline__ void wait_flag(const unsigned* flag, unsigned target) {
     const unsigned long long t0 = globaltimer_ns();
