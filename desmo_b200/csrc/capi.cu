@@ -393,6 +393,42 @@ int desmo_residual_profile(const desmo_shape* s, const void* U, int32_t u_dtype,
     return residual_profile_gemm_path(s, d.T, d.K, d.Kp, U, u_dtype, P, phi, omega, W, snap, point, (cudaStream_t)stream);
 }
 
+int desmo_pruning_profile(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                          const float* W, int32_t steps, const int32_t* order, double* snap, double* norm, void* stream) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if ((rc = check_u_dtype(u_dtype, "desmo_pruning_profile"))) return rc;
+    if (!U || !P || !phi || !omega || !W || !snap || (steps > 0 && !order)) { set_error("desmo_pruning_profile: null pointer"); return DESMO_ERR_ARG; }
+    if (reinterpret_cast<uintptr_t>(U) % 16 != 0) { set_error("desmo_pruning_profile: U must be 16-byte aligned"); return DESMO_ERR_ARG; }
+    if (steps < 0 || steps > d.K) { set_error("desmo_pruning_profile: steps = %d outside 0 .. K = %d", steps, d.K); return DESMO_ERR_ARG; }
+    std::vector<char> seen((size_t)d.K, 0);
+    for (int i = 0; i < steps; ++i) {  // host array: every index is checked before anything is launched
+        if (order[i] < 0 || order[i] >= d.K) {
+            set_error("desmo_pruning_profile: order[%d] = %d outside 0 .. K-1 = %d", i, order[i], d.K - 1);
+            return DESMO_ERR_ARG;
+        }
+        if (seen[order[i]]) { set_error("desmo_pruning_profile: order[%d] = %d repeats an earlier term", i, order[i]); return DESMO_ERR_ARG; }
+        seen[order[i]] = 1;
+    }
+    if ((rc = device_ok())) return rc;
+    // one route for every library, as desmo_residual_profile: GEMM 1 of the general path, here transposed
+    return pruning_profile_gemm_path(s, d.T, d.K, d.Kp, U, u_dtype, P, phi, omega, W, steps, order, snap, norm, (cudaStream_t)stream);
+}
+
+int desmo_pruning_profile_scratch_bytes(const desmo_shape* s, int32_t steps, int32_t sms, size_t* bytes) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if (!bytes) { set_error("desmo_pruning_profile_scratch_bytes: null pointer"); return DESMO_ERR_ARG; }
+    if (steps < 0 || steps > d.K || sms < 1) {
+        set_error("desmo_pruning_profile_scratch_bytes: need 0 <= steps <= K = %d and sms >= 1 (got steps=%d sms=%d)", d.K, steps, sms);
+        return DESMO_ERR_ARG;
+    }
+    *bytes = pruning_profile_scratch_bytes(s, d.T, d.K, steps, sms);
+    return DESMO_OK;
+}
+
 int desmo_library_colnorm2(const desmo_shape* s, const float* P, const float* phi, const float* omega, float* out_k, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);

@@ -131,6 +131,12 @@ int reconstruct_gemm_path(const desmo_shape* s, int T, int K, int Kp, const floa
 // stream-ordered allocator
 int residual_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
                                const float* omega, const float* W, double* snap, float* point, cudaStream_t st);
+// snap [steps + 1][m] fp64: snap[s][t] = sum_x r_s^2, r_s = r with the terms order[0 .. s) peeled off; norm [m] (may be null) = sum_x u^2.
+// order is a validated host array; scratch from the stream-ordered allocator, pruning_profile_scratch_bytes of it
+int pruning_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
+                              const float* omega, const float* W, int steps, const int32_t* order, double* snap, double* norm,
+                              cudaStream_t st);
+size_t pruning_profile_scratch_bytes(const desmo_shape* s, int T, int K, int steps, int sms);
 int colnorm2_gemm_path(const desmo_shape* s, int T, int K, const float* P, const float* phi, const float* omega, float* out_k, cudaStream_t st);
 int launch_update_phi_generic(const UpdateArgs& a, cudaStream_t st);
 int select_path(const desmo_shape* s, const Dims& d);  // DESMO_PATH_FP32 / _TC / _GEMM actually used, or <0 (error set)

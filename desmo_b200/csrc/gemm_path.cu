@@ -38,11 +38,18 @@ constexpr int kChunkPoints = 16384;
 
 // EPI_RESID_BF16: EPI_RESID reading bf16 snapshots.  EPI_PROFILE (_BF16): r = Rec - U as EPI_RESID forms it, reduced to the two marginals of
 // r^2 and u^2 (per point, per snapshot) instead of being written out (desmo_residual_profile).
-enum { EPI_RESID = 0, EPI_D = 1, EPI_E = 2, EPI_RECON = 3, EPI_RESID_BF16 = 4, EPI_PROFILE = 5, EPI_PROFILE_BF16 = 6 };
+// EPI_PRUNE (_BF16): GEMM 1 transposed (rows = snapshots, columns = points), r = Rec - U as EPI_RESID forms it, then a sequence of
+// library terms peeled off one FFMA at a time, reduced to sum_x r_s^2 per snapshot and step (desmo_pruning_profile).
+enum { EPI_RESID = 0, EPI_D = 1, EPI_E = 2, EPI_RECON = 3, EPI_RESID_BF16 = 4, EPI_PROFILE = 5, EPI_PROFILE_BF16 = 6, EPI_PRUNE = 7,
+       EPI_PRUNE_BF16 = 8 };
 // EPI_PROFILE scratch behind the operand stages (dynamic shared memory), two buffers used by alternate tiles:
 // [4 lane quadrants][2 column halves][4 blocks of 16 columns][32] per-warp column sums, then [2][128] per-point sums of column half 1
 constexpr int kProfSlab = 4 * 2 * 4 * 32 + 2 * 128;
 constexpr size_t kProfSmem = 2 * sizeof(float) * kProfSlab;
+// EPI_PRUNE scratch behind the operand stages: a of one step chunk [kPruneSteps][BN points], then the fp32 partials of the two column
+// halves [2][kPruneSteps + 1][BM snapshots] (row kPruneSteps: sum_x u^2, first chunk only)
+constexpr int kPruneSteps = 16;
+constexpr size_t kPruneSmem = sizeof(float) * (kPruneSteps * 128 + 2 * (kPruneSteps + 1) * 128);
 
 // ------------------------------------------------------------------------------------------------- PTX helpers (the rest: tcgen05.cuh)
 // Every wait carries a watchdog: a protocol error traps (the launch fails with an error) instead of hanging the GPU.
@@ -68,6 +75,26 @@ __device__ __forceinline__ void split2_pair(float x0, float x1, uint32_t& w1, ui
     asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(w2) : "f"(e1), "f"(e0));
 }
 
+// Eight consecutive snapshot values (16-byte aligned) widened exactly to fp32, or zeros when !ok
+__device__ __forceinline__ void ldg8_u(const float* p, bool ok, float* u) {
+    float4 a = make_float4(0.0f, 0.0f, 0.0f, 0.0f), b = a;
+    if (ok) { a = __ldg(reinterpret_cast<const float4*>(p)); b = __ldg(reinterpret_cast<const float4*>(p) + 1); }
+    u[0] = a.x; u[1] = a.y; u[2] = a.z; u[3] = a.w; u[4] = b.x; u[5] = b.y; u[6] = b.z; u[7] = b.w;
+}
+__device__ __forceinline__ void ldg8_u(const __nv_bfloat16* p, bool ok, float* u) {
+    uint4 v = make_uint4(0u, 0u, 0u, 0u);
+    if (ok) v = __ldg(reinterpret_cast<const uint4*>(p));
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) { u[2 * i] = __uint_as_float(w[i] << 16); u[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u); }
+}
+
+__device__ __forceinline__ float4 lds_v4(uint32_t addr) {
+    float4 v;
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
+    return v;
+}
+
 struct GemmArgs {
     int tiles_m, tiles_n;      // output tiles (tn fastest in the work order: neighbouring CTAs share the A tile)
     int nslice, kb_per_slice;  // split of the contraction over work items (EPI_E); kb = k-blocks of 64
@@ -86,6 +113,10 @@ struct GemmArgs {
     long long rows_r;          // rows per plane of Rp (chunk points padded to 128)
     int m, mld, mp, K, Kp;
     int first_chunk;
+    // EPI_PRUNE (appended: the fields above keep their offsets): loss_part = per-CTA partials [gridDim.x][steps + 2][BM]
+    const float* prune_a;      // [steps + 1][rows_r]: row s = library values of term order[s - 1] at the chunk's points, row 0 = 0
+    const float* prune_b;      // [steps + 1][mp]: row s = W[order[s - 1]][t] (0 for t >= m), row 0 = 0
+    int steps;
 };
 
 // the plane pairs kept by the split, smallest contributions first
@@ -108,7 +139,8 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
     static_assert(NPA == NPB, "plane pairs are defined for equal plane counts");
     constexpr bool kResid = EPI == EPI_RESID || EPI == EPI_RESID_BF16;
     constexpr bool kProfile = EPI == EPI_PROFILE || EPI == EPI_PROFILE_BF16;
-    using UT = typename std::conditional<EPI == EPI_RESID_BF16 || EPI == EPI_PROFILE_BF16, __nv_bfloat16, float>::type;
+    constexpr bool kPrune = EPI == EPI_PRUNE || EPI == EPI_PRUNE_BF16;
+    using UT = typename std::conditional<EPI == EPI_RESID_BF16 || EPI == EPI_PROFILE_BF16 || EPI == EPI_PRUNE_BF16, __nv_bfloat16, float>::type;
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bars[2 * NSTAGE + 4];
     __shared__ uint32_t tmem_base_s;
@@ -142,7 +174,8 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
             int cnt = 0;
             for (int w = blockIdx.x; w < items; w += gridDim.x) {
                 const int slice = w / tiles, rem = w - slice * tiles;
-                const int tm = rem / g.tiles_n, tn = rem - tm * g.tiles_n;
+                // EPI_PRUNE: tm fastest -- with gridDim.x a multiple of tiles_m, every tile of a CTA has the same snapshot rows
+                const int tm = kPrune ? rem % g.tiles_m : rem / g.tiles_n, tn = kPrune ? rem / g.tiles_m : rem - tm * g.tiles_n;
                 const int kb0 = slice * g.kb_per_slice, kb1 = min(kb0 + g.kb_per_slice, g.kblocks);
                 for (int kb = kb0; kb < kb1; ++kb, ++cnt) {
                     const int st = cnt % NSTAGE;
@@ -217,7 +250,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
         int job = 0;
         for (int w = blockIdx.x; w < items; w += gridDim.x) {
             const int slice = w / tiles, rem = w - slice * tiles;
-            const int tm = rem / g.tiles_n, tn = rem - tm * g.tiles_n;
+            const int tm = kPrune ? rem % g.tiles_m : rem / g.tiles_n, tn = kPrune ? rem / g.tiles_m : rem - tm * g.tiles_n;
             const int kb0 = slice * g.kb_per_slice, kb1 = min(kb0 + g.kb_per_slice, g.kblocks);
             float sum[64];
 #pragma unroll
@@ -341,6 +374,77 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
                     const int t = tn * BN + ch * 64 + blk * 16 + (l & 15);
                     double* dst = g.loss_part + ((long long)blockIdx.x * 2 + (l >> 4)) * g.mp + t;
                     *dst += sq;
+                }
+            } else if (kPrune) {
+                // GEMM 1 transposed: rows = snapshots, columns = points of the chunk.  r_0 = Rec - U exactly as EPI_RESID forms it; step
+                // s = 1 .. steps peels term order[s - 1] off, r_s = r_{s-1} - a_s(x) b_s(t) (one FFMA), and sum_x r_s^2 over this
+                // thread's 64 points is a running sum in registers: no cross-lane reduction, and a_s(x) is a broadcast read of the warp.
+                const int t = tm * BM + row;
+                const bool tin = t < g.m;
+                const long long xc = g.x0 + (long long)tn * BN + c * 64;  // first point of this thread's columns
+                float* a_s = reinterpret_cast<float*>(smem + NSTAGE * STAGE);
+                float* p_s = a_s + kPruneSteps * BN;
+                const int e = (warp - 2) * 32 + lane;  // 0 .. 255 over the epilogue warps
+                const UT* up = static_cast<const UT*>(g.U) + (long long)t * g.ld + xc;
+                float pu = 0.0f;
+#pragma unroll
+                for (int blk = 0; blk < 8; ++blk) {
+                    float u[8];
+                    ldg8_u(up + blk * 8, tin, u);
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        const bool in = tin && xc + blk * 8 + j < g.n;
+                        const float uu = in ? u[j] : 0.0f;
+                        sum[blk * 8 + j] = in ? sum[blk * 8 + j] - uu : 0.0f;
+                        pu = fmaf(uu, uu, pu);
+                    }
+                }
+                const int nout = g.steps + 1;
+                for (int o0 = 0; o0 < nout; o0 += kPruneSteps) {
+                    const int nc = min(kPruneSteps, nout - o0);
+                    float bv[kPruneSteps];
+#pragma unroll
+                    for (int i = 0; i < kPruneSteps; ++i) bv[i] = i < nc ? __ldg(g.prune_b + (long long)(o0 + i) * g.mp + t) : 0.0f;
+                    // a of the chunk's steps at the tile's 128 points
+#pragma unroll
+                    for (int q4 = 0; q4 < kPruneSteps * BN / 4 / (EPI_WARPS * 32); ++q4) {
+                        const int f = e + q4 * EPI_WARPS * 32, i = f / (BN / 4), x4 = f - i * (BN / 4);
+                        float4 v = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                        if (i < nc) v = __ldg(reinterpret_cast<const float4*>(g.prune_a + (long long)(o0 + i) * g.rows_r + (long long)tn * BN) + x4);
+                        reinterpret_cast<float4*>(a_s)[f] = v;
+                    }
+                    asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");  // the epilogue warps only
+#pragma unroll
+                    for (int i = 0; i < kPruneSteps; ++i) {
+                        if (i < nc) {
+                            const uint32_t a = smem_u32(a_s + i * BN + c * 64);
+                            float acc[8];
+#pragma unroll
+                            for (int j = 0; j < 8; ++j) acc[j] = 0.0f;
+#pragma unroll
+                            for (int j = 0; j < 64; j += 4) {
+                                const float4 av = lds_v4(a + j * 4);  // the same address in every lane: a broadcast
+                                sum[j] = fmaf(-av.x, bv[i], sum[j]);
+                                sum[j + 1] = fmaf(-av.y, bv[i], sum[j + 1]);
+                                sum[j + 2] = fmaf(-av.z, bv[i], sum[j + 2]);
+                                sum[j + 3] = fmaf(-av.w, bv[i], sum[j + 3]);
+#pragma unroll
+                                for (int k = 0; k < 4; ++k) acc[(j + k) & 7] = fmaf(sum[j + k], sum[j + k], acc[(j + k) & 7]);
+                            }
+                            p_s[(c * (kPruneSteps + 1) + i) * BM + row] = ((acc[0] + acc[1]) + (acc[2] + acc[3])) + ((acc[4] + acc[5]) + (acc[6] + acc[7]));
+                        }
+                    }
+                    if (o0 == 0) p_s[(c * (kPruneSteps + 1) + kPruneSteps) * BM + row] = pu;
+                    asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
+                    // fp64: column half 0 + column half 1, added into this CTA's running partial [steps + 2][BM] (row steps + 1: sum_x u^2).
+                    // Each element always falls to the same thread, so the partial needs no atomics.
+                    const int nrow = nc + (o0 == 0 ? 1 : 0);
+                    for (int f = e; f < nrow * BM; f += EPI_WARPS * 32) {
+                        const int i = f / BM, tt = f - i * BM;
+                        const int slot = i < nc ? i : kPruneSteps, o = i < nc ? o0 + i : nout;
+                        double* dst = g.loss_part + ((long long)blockIdx.x * (nout + 1) + o) * BM + tt;
+                        *dst += (double)p_s[slot * BM + tt] + (double)p_s[(kPruneSteps + 1 + slot) * BM + tt];
+                    }
                 }
             } else {  // EPI_E: rows = snapshots, columns = library terms; this slice's partial of E^T, accumulated over the chunks
                 const int t = tm * BM + row;
@@ -653,7 +757,7 @@ template <bool A_MN, bool B_MN, int NPA, int NPB, int EPI>
 static int launch_gemm(const GemmArgs& g, const CUtensorMap& tmA, const CUtensorMap& tmB, int sms, cudaStream_t st) {
     constexpr size_t stage = (size_t)(NPA + NPB) * PLANE_TILE;
     constexpr int nstage = (NPA + NPB) >= 6 ? 2 : 3;
-    constexpr size_t extra = (EPI == EPI_PROFILE || EPI == EPI_PROFILE_BF16) ? kProfSmem : 0;
+    constexpr size_t extra = (EPI == EPI_PROFILE || EPI == EPI_PROFILE_BF16) ? kProfSmem : (EPI == EPI_PRUNE || EPI == EPI_PRUNE_BF16) ? kPruneSmem : 0;
     const size_t smem = nstage * stage + 1024 + extra;
     auto kern = gemm_planes_kernel<A_MN, B_MN, NPA, NPB, EPI>;
     DESMO_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -953,6 +1057,151 @@ int residual_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const
     }
     cudaFreeAsync(scratch, st);
     return rc;
+}
+
+// Pruning profile (desmo_pruning_profile): library planes + the gathered step operands per chunk of points, GEMM 1 transposed with the
+// pruning epilogue, then fixed-order sums of the per-CTA partials.  The term order travels by value (two bytes a term), so the call
+// needs no host-to-device copy and stays capturable.
+struct PruneOrder {
+    uint16_t k[DESMO_MAX_K];
+};
+
+// B [steps + 1][mp]: row s = W[order[s - 1]][t] for t < m; row 0 and the columns t >= m are zero
+__global__ void __launch_bounds__(256) prune_b_kernel(const float* __restrict__ W, int mld, int m, int mp, int steps,
+                                                      const __grid_constant__ PruneOrder ord, float* __restrict__ B) {
+    const long long total = (long long)(steps + 1) * mp;
+    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < total; i += (long long)gridDim.x * 256) {
+        const int o = (int)(i / mp), t = (int)(i - (long long)o * mp);
+        B[i] = (o > 0 && t < m) ? W[(long long)ord.k[o - 1] * mld + t] : 0.0f;
+    }
+}
+
+// A [steps + 1][rows_c]: row s = the fp32 library value of term order[s - 1] at the chunk's points, b1 + (b2 + b3) of its three planes
+// (each addition is exact: the planes are the split of that value); row 0 is zero
+__global__ void __launch_bounds__(256) prune_a_kernel(const __nv_bfloat16* __restrict__ Gp, int Kr, long long rows_c, int steps,
+                                                      const __grid_constant__ PruneOrder ord, float* __restrict__ A) {
+    const long long xl = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (xl >= rows_c) return;
+    const size_t plane = (size_t)Kr * rows_c;
+    for (int o = blockIdx.y; o <= steps; o += gridDim.y) {
+        float v = 0.0f;
+        if (o > 0) {
+            const size_t i = (size_t)ord.k[o - 1] * rows_c + xl;
+            v = __bfloat162float(Gp[i]) + (__bfloat162float(Gp[plane + i]) + __bfloat162float(Gp[2 * plane + i]));
+        }
+        A[(size_t)o * rows_c + xl] = v;
+    }
+}
+
+// snap[o][t] = sum, in CTA order, of the partials of the gpt CTAs that own snapshot tile t / 128; norm[t] the same for row steps + 1
+__global__ void __launch_bounds__(256) prune_snapshots_kernel(const double* __restrict__ part, int tiles_m, int gpt, int steps, int m,
+                                                              double* __restrict__ snap, double* __restrict__ norm) {
+    const int rows = steps + 2;
+    const long long i = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (i >= (long long)rows * m) return;
+    const int o = (int)(i / m), t = (int)(i - (long long)o * m);
+    double s = 0.0;
+    for (int k = 0; k < gpt; ++k) s += part[((long long)(t / gp::BM + k * tiles_m) * rows + o) * gp::BM + (t % gp::BM)];
+    if (o <= steps) snap[(long long)o * m + t] = s;
+    else if (norm) norm[t] = s;
+}
+
+// Scratch layout of the pruning profile.  gpt CTAs share each 128-snapshot tile (tiles_m * gpt ~ the SM count), every CTA keeps one
+// fp64 partial [steps + 2][128], and chunks of points are a multiple of gpt * 128 so that each CTA gets the same number of tiles.
+struct PruneLayout {
+    int Kr, mp, tiles_m, gpt;
+    long long rows_c;
+    size_t o_idx, o_deg, o_gp, o_wp, o_a, o_b, o_part, part_bytes, bytes;
+};
+size_t pruning_profile_layout(const desmo_shape* s, int T, int K, int steps, int sms, PruneLayout* L) {
+    L->Kr = (K + 63) / 64 * 64;  // GEMM 1 reads (K + 63) / 64 k-blocks, as residual_profile_gemm_path
+    L->mp = (s->m + 127) / 128 * 128;
+    L->tiles_m = L->mp / 128;
+    const long long ptiles = s->ld / 128;
+    long long gpt = sms / L->tiles_m;
+    if (gpt < 1) gpt = 1;
+    if (gpt > ptiles) gpt = ptiles;
+    L->gpt = (int)gpt;
+    const size_t per_point = (size_t)3 * L->Kr * 2 + (size_t)(steps + 1) * 4;
+    const long long unit = 128 * gpt;
+    long long rc = (long long)(kProfileChunkBytes / per_point) / unit * unit;
+    if (rc < unit) rc = unit;
+    if (rc > s->ld) rc = s->ld;
+    L->rows_c = rc;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off = align_up_g(off + bytes, 1024); return o; };
+    L->o_idx = take((size_t)T * 8);
+    L->o_deg = take((size_t)T);
+    L->o_gp = take((size_t)3 * L->Kr * rc * 2);
+    L->o_wp = take((size_t)3 * L->Kr * L->mp * 2);
+    L->o_a = take((size_t)(steps + 1) * rc * 4);
+    L->o_b = take((size_t)(steps + 1) * L->mp * 4);
+    L->part_bytes = (size_t)L->tiles_m * L->gpt * (steps + 2) * gp::BM * sizeof(double);
+    L->o_part = take(L->part_bytes);
+    L->bytes = off;
+    return off;
+}
+
+int pruning_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
+                              const float* omega, const float* W, int steps, const int32_t* order, double* snap, double* norm,
+                              cudaStream_t st) {
+    using namespace gp;
+    int dev = 0, sms = 0;
+    DESMO_CUDA(cudaGetDevice(&dev));
+    DESMO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    PruneLayout L;
+    pruning_profile_layout(s, T, K, steps, sms, &L);
+    PruneOrder ord;
+    memset(&ord, 0, sizeof(ord));
+    for (int i = 0; i < steps; ++i) ord.k[i] = (uint16_t)order[i];
+    uint8_t* scratch = nullptr;
+    DESMO_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&scratch), L.bytes, st));
+    __nv_bfloat16* Gp = reinterpret_cast<__nv_bfloat16*>(scratch + L.o_gp);
+    __nv_bfloat16* Wp = reinterpret_cast<__nv_bfloat16*>(scratch + L.o_wp);
+    float* A = reinterpret_cast<float*>(scratch + L.o_a);
+    float* B = reinterpret_cast<float*>(scratch + L.o_b);
+    double* part = reinterpret_cast<double*>(scratch + L.o_part);
+    TermTable tab{scratch + L.o_idx, scratch + L.o_deg};
+    const int Kr = L.Kr, mp = L.mp, grid = L.tiles_m * L.gpt;
+    const long long rows_c = L.rows_c;
+    int rc = check_cuda(cudaMemsetAsync(part, 0, L.part_bytes, st), "cudaMemsetAsync");
+    CUtensorMap tmW_mn, tmG_mn;
+    if (!rc) {
+        term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab);
+        w_planes_kernel<<<Kr, 256, 0, st>>>(W, K, Kr, s->m, s->mld, mp, Wp);
+        const long long nb = ((long long)(steps + 1) * mp + 255) / 256;
+        prune_b_kernel<<<(unsigned)(nb < 4096 ? nb : 4096), 256, 0, st>>>(W, s->mld, s->m, mp, steps, ord, B);
+        rc = check_cuda(cudaGetLastError(), "prune_b_kernel");
+    }
+    // GEMM 1 transposed: Rec^T[t x p] = W^T G^T; A = W planes (MN-major: t contiguous), B = G planes (MN-major: p contiguous)
+    if (!rc && !(rc = make_map(&tmW_mn, Wp, mp, 3LL * Kr, 64))) rc = make_map(&tmG_mn, Gp, rows_c, 3LL * Kr, 64);
+    for (long long x0 = 0; x0 < s->ld && !rc; x0 += rows_c) {
+        const long long pts = (s->ld - x0 < rows_c) ? s->ld - x0 : rows_c;  // multiple of 128
+        const unsigned bx = (unsigned)((rows_c + 255) / 256);
+        library_planes_kernel<<<dim3(bx, 64u), 256, 0, st>>>(P, phi, omega, tab, s->r, T, K, Kr, s->n, s->ld, x0, rows_c, Gp);
+        prune_a_kernel<<<dim3(bx, (unsigned)(steps + 1 < 64 ? steps + 1 : 64)), 256, 0, st>>>(Gp, Kr, rows_c, steps, ord, A);
+        if ((rc = check_cuda(cudaGetLastError(), "prune_a_kernel"))) break;
+        GemmArgs g{};
+        g.U = U; g.loss_part = part; g.prune_a = A; g.prune_b = B; g.steps = steps;
+        g.n = s->n; g.ld = s->ld; g.x0 = x0; g.rows_r = rows_c; g.m = s->m; g.mld = s->mld; g.mp = mp; g.K = K; g.Kp = Kp;
+        g.tiles_m = L.tiles_m; g.tiles_n = (int)(pts / 128); g.nslice = 1; g.kblocks = (K + 63) / 64; g.kb_per_slice = g.kblocks;
+        g.kgroup = 4; g.a_rows = Kr; g.b_rows = Kr; g.first_chunk = 1;
+        // at most `grid` CTAs (a multiple of tiles_m): CTA b owns snapshot tile b % tiles_m and partial slot b in every chunk
+        rc = u_dtype == DESMO_DTYPE_BF16 ? launch_gemm<true, true, 3, 3, EPI_PRUNE_BF16>(g, tmW_mn, tmG_mn, grid, st)
+                                         : launch_gemm<true, true, 3, 3, EPI_PRUNE>(g, tmW_mn, tmG_mn, grid, st);
+    }
+    if (!rc) {
+        const long long total = (long long)(steps + 2) * s->m;
+        prune_snapshots_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(part, L.tiles_m, L.gpt, steps, s->m, snap, norm);
+        rc = check_cuda(cudaGetLastError(), "prune_snapshots_kernel");
+    }
+    cudaFreeAsync(scratch, st);
+    return rc;
+}
+
+size_t pruning_profile_scratch_bytes(const desmo_shape* s, int T, int K, int steps, int sms) {
+    PruneLayout L;
+    return pruning_profile_layout(s, T, K, steps, sms, &L);
 }
 
 int colnorm2_gemm_path(const desmo_shape* s, int T, int K, const float* P, const float* phi, const float* omega, float* out_k, cudaStream_t st) {

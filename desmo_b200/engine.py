@@ -64,6 +64,22 @@ def _instants(index, times, m: int, nF: int):
     return np.ascontiguousarray(k, dtype=np.int32), None
 
 
+def pruning_order(order, K: int) -> np.ndarray:
+    """The term order of desmo_pruning_profile as a contiguous int32 host array: distinct packed indices in 0 .. K-1, at most K of
+    them.  Raises DesmoError before any launch (the C ABI checks the same again)."""
+    raw = order.detach().cpu().numpy() if torch.is_tensor(order) else np.asarray(order)
+    if raw.size and not np.issubdtype(raw.dtype, np.integer):
+        raise _lib.DesmoError(f"order must hold integer term indices, got {raw.dtype}")
+    k = raw.astype(np.int64).reshape(-1)
+    if k.size > K:
+        raise _lib.DesmoError(f"order has {k.size} terms, the library only {K}")
+    if k.size and (int(k.min()) < 0 or int(k.max()) >= K):
+        raise _lib.DesmoError(f"order must hold term indices in 0 .. {K - 1}")
+    if np.unique(k).size != k.size:
+        raise _lib.DesmoError("order must not repeat a term")
+    return np.ascontiguousarray(k, dtype=np.int32)
+
+
 class _PeerDesc(C.Structure):  # desmo_peer (include/desmo_b200.h)
     _fields_ = [("world", C.c_int32), ("rank", C.c_int32), ("red_ptrs", C.c_void_p), ("flag_ptrs", C.c_void_p), ("state", C.c_void_p)]
 
@@ -429,6 +445,30 @@ class DesmoEngine:
                 torch.distributed.all_reduce(snap, group=self.pg)
         return {"snapshot_residual2": snap[0], "snapshot_norm2": snap[1], "point_residual2": point[0, :self.n],
                 "point_norm2": point[1, :self.n]}
+
+    def pruning_profile(self, order) -> dict:
+        """The error of every step of a term-pruning sequence, in one pass over U (desmo_pruning_profile).  Step s removes the terms
+        order[0 .. s) (packed K indices, distinct, at most K): r_s = recon - U with those terms' gates at zero.  Returns
+
+          snapshot_residual2 (S+1, m) fp64  sum_x r_s(x, t)^2   summed over ranks when point-sharded
+          snapshot_norm2     (m,)     fp64  sum_x U(x, t)^2     summed over ranks when point-sharded
+
+        Row 0 is residual_profile()'s snapshot_residual2 up to the order of the sums; row s is what residual_profile() gives with the
+        gates of order[0 .. s) zeroed, up to one fp32 rounding per removed term.  Nothing the model owns is written (gates, rows, the
+        step counter and U stay as they are).  Bit-identical from call to call."""
+        idx = pruning_order(order, self.K)
+        ud = self._u_dtype()
+        snap = torch.empty(idx.size + 1, self.m, dtype=torch.float64, device=self.device)
+        norm = torch.empty(self.m, dtype=torch.float64, device=self.device)
+        with torch.cuda.device(self.device):
+            self.build_w(False)
+            check(self.lib.desmo_pruning_profile(C.byref(self.shape), _ptr(self.U), ud, _ptr(self.P), _ptr(self.phi), _ptr(self.omega),
+                                                 _ptr(self.W), int(idx.size), idx.ctypes.data if idx.size else None, _ptr(snap),
+                                                 _ptr(norm), self._stream()), "desmo_pruning_profile")
+            if self.n_global != self.n and torch.distributed.is_initialized():
+                torch.distributed.all_reduce(snap, group=self.pg)
+                torch.distributed.all_reduce(norm, group=self.pg)
+        return {"snapshot_residual2": snap, "snapshot_norm2": norm}
 
     # ------------------------------------------------------------------ evaluation at chosen instants
     # Each of these takes exactly one of index= (training snapshot indices, any order, repeats allowed) or times= (fp32 times in the

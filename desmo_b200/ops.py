@@ -1,6 +1,6 @@
 """torch custom ops over the C ABI: one ``torch.ops.desmo_b200.*`` op per hot-path entry point of include/desmo_b200.h.
 
-  build_w, build_w_at, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, library_colnorm2, term_norms,
+  build_w, build_w_at, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, pruning_profile, library_colnorm2, term_norms,
   pod_gram, pod_eig, pod_eigh, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce
 
 They take the packed device tensors of a DesmoEngine (layout: include/desmo_b200.h) plus the shape integers and launch the
@@ -149,6 +149,26 @@ def residual_profile(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, omega:
     with torch.cuda.device(U.device):
         check(_lib.load().desmo_residual_profile(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), _p(snap), _p(point), _stream(U)),
               "desmo_residual_profile")
+
+
+@torch.library.custom_op("desmo_b200::pruning_profile", mutates_args=("snap", "norm"))
+def pruning_profile(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, omega: torch.Tensor, W: torch.Tensor, order: torch.Tensor,
+                    snap: torch.Tensor, norm: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """snap (fp64 [S+1, m]) = sum_x r_s^2 with the terms order[0 .. s) removed, norm (fp64 [m]) = sum_x U^2 (desmo_pruning_profile).
+    ``order`` is a host int32 tensor of S distinct term indices."""
+    _require_cuda(U, P, phi, omega, W, snap, norm)
+    ud = _lib.u_dtype_code(U.dtype)
+    if order.device.type != "cpu" or order.dtype != torch.int32 or order.dim() != 1 or not order.is_contiguous():
+        raise _lib.DesmoError("pruning_profile: order must be a contiguous 1-D int32 tensor on the host")
+    S = order.numel()
+    if snap.dtype != torch.float64 or norm.dtype != torch.float64:
+        raise _lib.DesmoError("pruning_profile: snap and norm must be float64")
+    if snap.numel() < (S + 1) * m or norm.numel() < m or not (snap.is_contiguous() and norm.is_contiguous()):
+        raise _lib.DesmoError(f"pruning_profile: need contiguous snap [{S + 1}, {m}] and norm [{m}]")
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(U.device):
+        check(_lib.load().desmo_pruning_profile(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), S, _p(order) if S else None,
+                                                _p(snap), _p(norm), _stream(U)), "desmo_pruning_profile")
 
 
 @torch.library.custom_op("desmo_b200::library_colnorm2", mutates_args=("out",))
@@ -306,6 +326,23 @@ def engine_residual_profile_via_ops(e) -> dict:
     if e.n_global != e.n and torch.distributed.is_initialized():
         torch.distributed.all_reduce(snap, group=e.pg)
     return {"snapshot_residual2": snap[0], "snapshot_norm2": snap[1], "point_residual2": point[0, :e.n], "point_norm2": point[1, :e.n]}
+
+
+def engine_pruning_profile_via_ops(e, order) -> dict:
+    """DesmoEngine.pruning_profile() through the registered build_w / pruning_profile ops (the optimizer's step counter is not moved)."""
+    from .engine import pruning_order
+
+    sa = _shape_args(e)
+    idx = torch.from_numpy(pruning_order(order, e.K))
+    snap = torch.empty(idx.numel() + 1, e.m, dtype=torch.float64, device=e.device)
+    norm = torch.empty(e.m, dtype=torch.float64, device=e.device)
+    scratch_step = e.step_dev.clone()
+    torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, scratch_step, e.workspace, *sa)
+    torch.ops.desmo_b200.pruning_profile(e.U, e.P, e.phi, e.omega, e.W, idx, snap, norm, *sa)
+    if e.n_global != e.n and torch.distributed.is_initialized():
+        torch.distributed.all_reduce(snap, group=e.pg)
+        torch.distributed.all_reduce(norm, group=e.pg)
+    return {"snapshot_residual2": snap, "snapshot_norm2": norm}
 
 
 def engine_pod_via_ops(e) -> torch.Tensor:

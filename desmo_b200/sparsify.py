@@ -1,9 +1,13 @@
 """Post-hoc sparsification (CYL:624-692,1184-1270; TURB:1166-1245): term norms -> threshold sweep -> active mask."""
 from __future__ import annotations
 
-from typing import List, Tuple
+from dataclasses import dataclass
+from typing import List, Optional, Tuple
 
+import numpy as np
 import torch
+
+from ._lib import DesmoError
 
 
 def threshold_sweep(model, snapshot_norm2: float, thresholds=None) -> List[Tuple[float, float, int, torch.Tensor]]:
@@ -52,3 +56,70 @@ def greedy_removal(model, snapshot_norm2: float) -> List[Tuple[int, float, int]]
         out.append((step, float((e.residual_norm2() / snapshot_norm2) ** 0.5), int((e.gates != 0).sum().item())))
     e.gates.copy_(saved)
     return out
+
+
+def threshold_steps(norms, gates, order, threshold: float) -> int:
+    """How many leading terms of ``order`` a threshold removes.  threshold_sweep keeps a term iff norm >= threshold and its gate is
+    non-zero; the removed terms are a prefix of the norm-ascending removal_order (a zero gate has norm 0 and comes first).  Raises
+    DesmoError when the removed set is not a prefix of ``order``."""
+    norms = np.asarray(norms.detach().cpu().numpy() if torch.is_tensor(norms) else norms, dtype=np.float64)
+    gates = np.asarray(gates.detach().cpu().numpy() if torch.is_tensor(gates) else gates)
+    removed = ~((norms >= threshold) & (gates != 0))
+    s = int(removed.sum())
+    if sorted(int(k) for k in order[:s]) != np.flatnonzero(removed).tolist():
+        raise DesmoError(f"threshold {threshold} removes terms that are not the first {s} of this order")
+    return s
+
+
+@dataclass
+class PruningProfile:
+    """One pass over U for a whole pruning sequence.  Step s removes order[:s]; s = 0 .. len(order)."""
+    order: List[int]
+    snapshot_residual2: torch.Tensor  # (S+1, m) fp64: sum_x r_s(x, t)^2
+    snapshot_norm2: torch.Tensor      # (m,) fp64: sum_x U(x, t)^2
+    relative_error: List[float]       # ||X - recon_s|| / ||X|| per step (TURB:1227)
+    nonzero_terms: List[int]          # non-zero gates left per step (TURB:1229-1234)
+    term_norms: torch.Tensor          # (K,) fp64, the norms threshold_sweep compares with a threshold
+    gates: torch.Tensor               # (K,) the gates the profile was taken with
+
+    def steps_for_threshold(self, threshold: float) -> int:
+        """The step whose removed terms are exactly those threshold_sweep removes at ``threshold``."""
+        return threshold_steps(self.term_norms, self.gates, self.order, threshold)
+
+    def active_mask(self, step: int) -> torch.Tensor:
+        """threshold_sweep's mask after ``step`` removals: gate non-zero and not among order[:step]."""
+        mask = self.gates != 0
+        mask[list(self.order[:step])] = False
+        return mask
+
+    def threshold_sweep(self, thresholds) -> List[Tuple[float, float, int, torch.Tensor]]:
+        """threshold_sweep()'s [(threshold, relative_error, n_active, mask)], read off this profile."""
+        out = []
+        for thr in thresholds:
+            s = self.steps_for_threshold(float(thr))
+            out.append((float(thr), self.relative_error[s], self.nonzero_terms[s], self.active_mask(s)))
+        return out
+
+
+def pruning_profile(model, order=None, snapshot_norm2: Optional[float] = None) -> PruningProfile:
+    """Every step of a term-pruning sequence scored in one pass over U (DesmoEngine.pruning_profile): per-snapshot residuals, the
+    relative error ||X - recon_s|| / ||X|| and the non-zero gate count after removing order[:s], for s = 0 .. len(order).  The default
+    order is removal_order(term_norms()), so the result is greedy_removal's curve, and threshold_sweep's points are read off it with
+    steps_for_threshold.  ``snapshot_norm2`` is ||X||^2 (as greedy_removal takes it); by default the sum of the stored U's squares.
+    The gates are not touched."""
+    e = model.engine
+    if hasattr(model, "sync_parameters"):
+        model.sync_parameters()
+    norms = e.term_norms()
+    if order is None:
+        order = removal_order(norms, e.T, e.r)
+    order = [int(k) for k in (order.tolist() if torch.is_tensor(order) else order)]
+    prof = e.pruning_profile(order)
+    total = float(prof["snapshot_norm2"].sum()) if snapshot_norm2 is None else float(snapshot_norm2)
+    rel = (prof["snapshot_residual2"].sum(1) / total).sqrt().tolist()
+    gates = e.gates.clone()
+    nz_host = (gates != 0).cpu().numpy()
+    nonzero = [int(nz_host.sum())]
+    for k in order:
+        nonzero.append(nonzero[-1] - int(nz_host[k]))
+    return PruningProfile(order, prof["snapshot_residual2"], prof["snapshot_norm2"], rel, nonzero, norms, gates)

@@ -176,6 +176,25 @@ int desmo_reconstruct(const desmo_shape* s, const float* P, const float* phi, co
 int desmo_residual_profile(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
                            const float* W, double* snap, float* point, void* stream);
 
+/* Pruning profile: the per-snapshot error of every step of a term-pruning sequence, in one pass over U (evaluation only; writes
+ * nothing else).  order[0 .. steps) is a HOST array of distinct library indices in 0 .. K-1 (steps <= K; checked before any launch,
+ * DESMO_ERR_ARG otherwise).  With r_0 = G(Phi) W - U exactly as desmo_residual_profile forms it (U as stored, u_dtype F32 or BF16, U
+ * 16-byte aligned) and r_s = r_{s-1} - G_{order[s-1]}(x) W[order[s-1]][t] (one fp32 FFMA per step, G the exact fp32 library value):
+ *   snap  [steps + 1][m] fp64: snap[s][t] = sum_x r_s(x, t)^2   (local partial -- all-reduce it across ranks)
+ *   norm  [m]            fp64: norm[t] = sum_x U(x, t)^2        (may be NULL)
+ * Zeroing the gates of order[0 .. s) and calling desmo_residual_profile gives snap[s] up to one FFMA rounding per peeled term and the
+ * split-bf16 GEMM's own rounding of the removed terms.  Greedy removal takes the first s terms of the norm-ascending order, and a
+ * threshold removes a prefix of that same order, so both sweeps are read off one call.  Sums: fp32 over the 64 points a thread holds,
+ * fp64 beyond, in a fixed order with no float atomics -- bit-identical from call to call.  Scratch from the stream-ordered allocator on
+ * `stream` (the call stays capturable), with Kr = 64 ceil(K / 64), mp = 128 ceil(m / 128), tiles_m = mp / 128,
+ * gpt = clamp(floor(sms / tiles_m), 1, ld / 128), rows_c = the point chunk, and A(v) = v rounded up to 1024 bytes:
+ *   A(8T) + A(T) + A(6 Kr rows_c) + A(6 Kr mp) + A(4 (steps+1) rows_c) + A(4 (steps+1) mp) + A(1024 tiles_m gpt (steps+2))
+ * The last term, one fp64 partial [steps + 2][128] per CTA, is about sms * (steps + 2) KB: 97 MB at K = 657 on 148 SMs;
+ * desmo_pruning_profile_scratch_bytes returns the total for a given SM count (host only). */
+int desmo_pruning_profile(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                          const float* W, int32_t steps, const int32_t* order, double* snap, double* norm, void* stream);
+int desmo_pruning_profile_scratch_bytes(const desmo_shape* s, int32_t steps, int32_t sms, size_t* bytes);
+
 /* Post-hoc sparsification inputs: squared column norms of G (K floats, local partial -- all-reduce them across ranks).
  * P == NULL evaluates the library on the raw phi_list, which is what the reference's sweep passes to poly_norm /
  * nonlinear_norm (CYL:1192-1194; the functions, CYL:624-692, never multiply by POD_modes); P != NULL gives the columns of
