@@ -50,6 +50,14 @@ SIGNATURES: Dict[str, tuple] = {
     "desmo_fused_residual_grad_finish_ex": (C.c_int, [_SP, _vp, _i32] + [_vp] * 8),
     "desmo_adamax_update": (C.c_int, [_SP] + [_vp] * 26),
     "desmo_assemble_grads": (C.c_int, [_SP] + [_vp] * 17),
+    "desmo_active_terms_bytes": (C.c_int, [_SP, _i32, C.POINTER(C.c_size_t)]),
+    "desmo_active_terms_prepare": (C.c_int, [_SP, _vp, _i32, _vp, _vp]),
+    "desmo_build_w_active": (C.c_int, [_SP] + [_vp] * 9),
+    "desmo_fused_residual_grad_active": (C.c_int, [_SP, _vp, _i32] + [_vp] * 8 + [_i32, _vp]),
+    "desmo_fused_residual_grad_begin_active": (C.c_int, [_SP, _vp, _i32] + [_vp] * 8 + [_i32, _vp]),
+    "desmo_fused_residual_grad_finish_active": (C.c_int, [_SP, _vp, _i32] + [_vp] * 8 + [_i32, _vp]),
+    "desmo_adamax_update_active": (C.c_int, [_SP] + [_vp] * 27),
+    "desmo_assemble_grads_active": (C.c_int, [_SP] + [_vp] * 18),
     "desmo_reconstruct": (C.c_int, [_SP] + [_vp] * 6),
     "desmo_library_colnorm2": (C.c_int, [_SP] + [_vp] * 5),
     "desmo_residual_profile": (C.c_int, [_SP, _vp, _i32] + [_vp] * 7),

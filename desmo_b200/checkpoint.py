@@ -5,7 +5,8 @@ The reference saves ``model.state_dict()`` only (CYL:781-786,802-805).  A sharde
 the POD modes) as per-rank slabs of mesh points; everything else is replicated.  ``gather_trainer_state`` assembles the full vectors on
 rank 0 (``torch.distributed.gather`` of padded slabs), so that ``checkpoint["model"]`` is exactly the reference's ``state_dict`` for the
 whole mesh -- loadable by the reference scripts -- and ``scatter_trainer_state`` cuts the slab of (rank, world) out of it again,
-for any world size.  Works on any tensor device (the gloo tests run it on CPU tensors with a stand-in engine).
+for any world size.  The active-term mask (``active_terms``, DesmoEngine.set_active_terms) is replicated and passes through as it is.
+Works on any tensor device (the gloo tests run it on CPU tensors with a stand-in engine).
 """
 from __future__ import annotations
 

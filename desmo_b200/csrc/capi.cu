@@ -204,18 +204,68 @@ int desmo_workspace_bytes(const desmo_shape* s, size_t* bytes) {
     return DESMO_OK;
 }
 
-int desmo_build_w(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
-                  int32_t* step_dev, void* workspace, void* stream) {
+int desmo_active_terms_bytes(const desmo_shape* s, int32_t count, size_t* bytes) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if (!bytes) { set_error("desmo_active_terms_bytes: null pointer"); return DESMO_ERR_ARG; }
+    if (count < 1 || count > d.K) { set_error("desmo_active_terms_bytes: count = %d outside 1 .. K = %d", count, d.K); return DESMO_ERR_ARG; }
+    *bytes = sizeof(int32_t) * ((size_t)d.K + (size_t)count);
+    return DESMO_OK;
+}
+
+int desmo_active_terms_prepare(const desmo_shape* s, const int32_t* host_indices, int32_t count, void* table_dev, void* stream) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if (!host_indices || !table_dev) { set_error("desmo_active_terms_prepare: null pointer"); return DESMO_ERR_ARG; }
+    if (count < 1 || count > d.K) {
+        set_error("desmo_active_terms_prepare: an active set holds 1 .. K = %d terms (got %d)", d.K, count);
+        return DESMO_ERR_ARG;
+    }
+    // host array: every index is checked before anything is written; strictly increasing also rules out repeats
+    std::vector<int32_t> table((size_t)d.K + count, -1);
+    for (int i = 0; i < count; ++i) {
+        const int k = host_indices[i];
+        if (k < 0 || k >= d.K) { set_error("desmo_active_terms_prepare: index[%d] = %d outside 0 .. K-1 = %d", i, k, d.K - 1); return DESMO_ERR_ARG; }
+        if (i > 0 && k == host_indices[i - 1]) { set_error("desmo_active_terms_prepare: index[%d] = %d repeats a term", i, k); return DESMO_ERR_ARG; }
+        if (i > 0 && k < host_indices[i - 1]) {
+            set_error("desmo_active_terms_prepare: indices must be strictly increasing (index[%d] = %d after %d)", i, k, host_indices[i - 1]);
+            return DESMO_ERR_ARG;
+        }
+        table[k] = i;
+        table[(size_t)d.K + i] = k;
+    }
+    if ((rc = device_ok())) return rc;
+    // from pageable memory: the copy has consumed `table` when it returns
+    DESMO_CUDA(cudaMemcpyAsync(table_dev, table.data(), sizeof(int32_t) * table.size(), cudaMemcpyHostToDevice, (cudaStream_t)stream));
+    return DESMO_OK;
+}
+
+static int build_w_impl(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
+                        int32_t* step_dev, void* workspace, const int32_t* active, void* stream, const char* who) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
     if ((rc = device_ok())) return rc;
-    if (!gates || !rows || !W || !workspace || (s->nF > 0 && (!coefs || !periods))) { set_error("desmo_build_w: null pointer"); return DESMO_ERR_ARG; }
+    if (!gates || !rows || !W || !workspace || (s->nF > 0 && (!coefs || !periods))) { set_error("%s: null pointer", who); return DESMO_ERR_ARG; }
     Workspace ws;
     if ((rc = carve_workspace(s, d, workspace, &ws))) return rc;
     const bool tc = use_tc_path(s, d);
     return build_w(s, d.K, d.Kp, gates, rows, coefs, periods, W, tc ? ws.tc : nullptr, tc ? ws.tc + (size_t)d.Kp * s->mld : nullptr,
-                   step_dev, ws.l1, (cudaStream_t)stream);
+                   step_dev, ws.l1, (cudaStream_t)stream, active);
+}
+
+int desmo_build_w_active(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
+                         int32_t* step_dev, void* workspace, const void* active, void* stream) {
+    if (!active) { set_error("desmo_build_w_active: null active-term table"); return DESMO_ERR_ARG; }
+    return build_w_impl(s, gates, rows, coefs, periods, W, step_dev, workspace, static_cast<const int32_t*>(active), stream,
+                        "desmo_build_w_active");
+}
+
+int desmo_build_w(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
+                  int32_t* step_dev, void* workspace, void* stream) {
+    return build_w_impl(s, gates, rows, coefs, periods, W, step_dev, workspace, nullptr, stream, "desmo_build_w");
 }
 
 int desmo_build_w_at(const desmo_shape* s, const float* gates, const float* rows, const float* coefs, const float* periods, int32_t m_out,
@@ -247,15 +297,18 @@ int desmo_build_w_at(const desmo_shape* s, const float* gates, const float* rows
     return build_w_at(s, d.K, d.Kp, gates, rows, coefs, periods, m_out, mld_out, index, times, W_out, rows_out, (cudaStream_t)stream);
 }
 
+// active / Ka: an active-term table and its size (null: the whole library).  The fused kernels take the full library and rely on
+// the zero W rows of desmo_build_w_active; the GEMM path builds the active columns only.
 static int fused_dispatch(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
                           const float* W, float* dphi, float* red, void* workspace, void* stream, bool supplied, const char* who,
-                          int phase = 0) {
+                          int phase = 0, const int32_t* active = nullptr, int Ka = 0) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
     if ((rc = check_u_dtype(u_dtype, who))) return rc;
     if ((rc = device_ok())) return rc;
     if (!U || !P || !phi || !omega || !W || !dphi || !red || !workspace) { set_error("%s: null pointer", who); return DESMO_ERR_ARG; }
+    if (active && (Ka < 1 || Ka > d.K)) { set_error("%s: active_count = %d outside 1 .. K = %d", who, Ka, d.K); return DESMO_ERR_ARG; }
     Workspace ws;
     if ((rc = carve_workspace(s, d, workspace, &ws))) return rc;
     switch (select_path(s, d)) {
@@ -265,7 +318,8 @@ static int fused_dispatch(const desmo_shape* s, const void* U, int32_t u_dtype, 
             return fused_fp32(s, d.mt, d.T, d.Kp, U, u_dtype, P, phi, omega, W, dphi, red, ws, (cudaStream_t)stream, supplied);
         case DESMO_PATH_GEMM:
             if (phase == 2) return DESMO_OK;
-            return fused_gemm_path(s, d.T, d.K, d.Kp, U, u_dtype, P, phi, omega, W, dphi, red, ws.Dacc, ws.gemm, (cudaStream_t)stream, supplied);
+            return fused_gemm_path(s, d.T, d.K, d.Kp, U, u_dtype, P, phi, omega, W, dphi, red, ws.Dacc, ws.gemm, (cudaStream_t)stream, supplied,
+                                   active, Ka);
         default: return DESMO_ERR_UNSUPPORTED;
     }
 }
@@ -300,6 +354,34 @@ int desmo_fused_residual_grad_finish_ex(const desmo_shape* s, const void* U, int
     return fused_dispatch(s, U, u_dtype, P, phi, omega, W, dphi, red, workspace, stream, false, "desmo_fused_residual_grad_finish_ex", 2);
 }
 
+static int fused_active(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                        const float* W, float* dphi, float* red, void* workspace, const void* active, int32_t active_count, void* stream,
+                        const char* who, int phase) {
+    if (!active) { set_error("%s: null active-term table", who); return DESMO_ERR_ARG; }
+    return fused_dispatch(s, U, u_dtype, P, phi, omega, W, dphi, red, workspace, stream, false, who, phase, static_cast<const int32_t*>(active),
+                          active_count);
+}
+
+int desmo_fused_residual_grad_active(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                     const float* omega, const float* W, float* dphi, float* red, void* workspace, const void* active,
+                                     int32_t active_count, void* stream) {
+    return fused_active(s, U, u_dtype, P, phi, omega, W, dphi, red, workspace, active, active_count, stream, "desmo_fused_residual_grad_active", 0);
+}
+
+int desmo_fused_residual_grad_begin_active(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                           const float* omega, const float* W, float* dphi, float* red, void* workspace,
+                                           const void* active, int32_t active_count, void* stream) {
+    return fused_active(s, U, u_dtype, P, phi, omega, W, dphi, red, workspace, active, active_count, stream,
+                        "desmo_fused_residual_grad_begin_active", 1);
+}
+
+int desmo_fused_residual_grad_finish_active(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                            const float* omega, const float* W, float* dphi, float* red, void* workspace,
+                                            const void* active, int32_t active_count, void* stream) {
+    return fused_active(s, U, u_dtype, P, phi, omega, W, dphi, red, workspace, active, active_count, stream,
+                        "desmo_fused_residual_grad_finish_active", 2);
+}
+
 int desmo_recon_backward(const desmo_shape* s, const float* grad_recon, const float* P, const float* phi, const float* omega,
                          const float* W, float* dphi, float* red, void* workspace, void* stream) {
     return fused_dispatch(s, grad_recon, DESMO_DTYPE_F32, P, phi, omega, W, dphi, red, workspace, stream, true, "desmo_recon_backward");
@@ -313,11 +395,42 @@ static int fill_update(const desmo_shape* s, const Dims& d, const Workspace& ws,
     return DESMO_OK;
 }
 
+static int desmo_adamax_update_impl(const desmo_shape* s, const float* red, const float* dphi, const float* P, float* phi, float* phi_m,
+                                    float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows, float* rows_m, float* rows_u,
+                                    float* coefs, float* coefs_m, float* coefs_u, float* periods, float* periods_m, float* periods_u,
+                                    float* omega, float* omega_m, float* omega_u, const float* hyper, const int32_t* step_dev,
+                                    float* losses_out, void* workspace, const int32_t* active, void* stream);
+static int assemble_grads_impl(const desmo_shape* s, const float* red, float* dphi, const float* P, const float* phi, const float* gates,
+                               const float* rows, const float* coefs, const float* periods, const float* hyper, float* d_gates,
+                               float* d_rows, float* d_coefs, float* d_periods, float* d_omega, float* losses_out, void* workspace,
+                               const int32_t* active, void* stream);
+
 int desmo_adamax_update(const desmo_shape* s, const float* red, const float* dphi, const float* P, float* phi, float* phi_m,
                         float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows, float* rows_m, float* rows_u,
                         float* coefs, float* coefs_m, float* coefs_u, float* periods, float* periods_m, float* periods_u,
                         float* omega, float* omega_m, float* omega_u, const float* hyper, const int32_t* step_dev,
                         float* losses_out, void* workspace, void* stream) {
+    return desmo_adamax_update_impl(s, red, dphi, P, phi, phi_m, phi_u, gates, gates_m, gates_u, rows, rows_m, rows_u, coefs, coefs_m,
+                                    coefs_u, periods, periods_m, periods_u, omega, omega_m, omega_u, hyper, step_dev, losses_out, workspace,
+                                    nullptr, stream);
+}
+
+int desmo_adamax_update_active(const desmo_shape* s, const float* red, const float* dphi, const float* P, float* phi, float* phi_m,
+                               float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows, float* rows_m, float* rows_u,
+                               float* coefs, float* coefs_m, float* coefs_u, float* periods, float* periods_m, float* periods_u,
+                               float* omega, float* omega_m, float* omega_u, const float* hyper, const int32_t* step_dev,
+                               float* losses_out, void* workspace, const void* active, void* stream) {
+    if (!active) { set_error("desmo_adamax_update_active: null active-term table"); return DESMO_ERR_ARG; }
+    return desmo_adamax_update_impl(s, red, dphi, P, phi, phi_m, phi_u, gates, gates_m, gates_u, rows, rows_m, rows_u, coefs, coefs_m,
+                                    coefs_u, periods, periods_m, periods_u, omega, omega_m, omega_u, hyper, step_dev, losses_out, workspace,
+                                    static_cast<const int32_t*>(active), stream);
+}
+
+static int desmo_adamax_update_impl(const desmo_shape* s, const float* red, const float* dphi, const float* P, float* phi, float* phi_m,
+                                    float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows, float* rows_m, float* rows_u,
+                                    float* coefs, float* coefs_m, float* coefs_u, float* periods, float* periods_m, float* periods_u,
+                                    float* omega, float* omega_m, float* omega_u, const float* hyper, const int32_t* step_dev,
+                                    float* losses_out, void* workspace, const int32_t* active, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
@@ -338,6 +451,7 @@ int desmo_adamax_update(const desmo_shape* s, const float* red, const float* dph
     a.coefs = coefs; a.coefs_m = coefs_m; a.coefs_u = coefs_u; a.periods = periods; a.periods_m = periods_m; a.periods_u = periods_u;
     a.omega = omega; a.omega_m = omega_m; a.omega_u = omega_u; a.hyper = hyper; a.step_dev = step_dev; a.losses_out = losses_out;
     a.apply = 1;
+    a.active_pos = active;
     return launch_update(a, (cudaStream_t)stream);
 }
 
@@ -345,6 +459,23 @@ int desmo_assemble_grads(const desmo_shape* s, const float* red, float* dphi, co
                          const float* rows, const float* coefs, const float* periods, const float* hyper, float* d_gates,
                          float* d_rows, float* d_coefs, float* d_periods, float* d_omega, float* losses_out, void* workspace,
                          void* stream) {
+    return assemble_grads_impl(s, red, dphi, P, phi, gates, rows, coefs, periods, hyper, d_gates, d_rows, d_coefs, d_periods, d_omega,
+                               losses_out, workspace, nullptr, stream);
+}
+
+int desmo_assemble_grads_active(const desmo_shape* s, const float* red, float* dphi, const float* P, const float* phi, const float* gates,
+                                const float* rows, const float* coefs, const float* periods, const float* hyper, float* d_gates,
+                                float* d_rows, float* d_coefs, float* d_periods, float* d_omega, float* losses_out, void* workspace,
+                                const void* active, void* stream) {
+    if (!active) { set_error("desmo_assemble_grads_active: null active-term table"); return DESMO_ERR_ARG; }
+    return assemble_grads_impl(s, red, dphi, P, phi, gates, rows, coefs, periods, hyper, d_gates, d_rows, d_coefs, d_periods, d_omega,
+                               losses_out, workspace, static_cast<const int32_t*>(active), stream);
+}
+
+static int assemble_grads_impl(const desmo_shape* s, const float* red, float* dphi, const float* P, const float* phi, const float* gates,
+                               const float* rows, const float* coefs, const float* periods, const float* hyper, float* d_gates,
+                               float* d_rows, float* d_coefs, float* d_periods, float* d_omega, float* losses_out, void* workspace,
+                               const int32_t* active, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
@@ -364,6 +495,7 @@ int desmo_assemble_grads(const desmo_shape* s, const float* red, float* dphi, co
     a.periods = const_cast<float*>(periods); a.hyper = hyper; a.d_gates = d_gates; a.d_rows = d_rows; a.d_coefs = d_coefs;
     a.d_periods = d_periods; a.d_omega = d_omega; a.losses_out = losses_out;
     a.apply = 0;
+    a.active_pos = active;
     return launch_update(a, (cudaStream_t)stream);
 }
 

@@ -61,6 +61,7 @@ struct UpdateArgs {
     double inv_nm;  // 1 / (n_global * m)
     int m, mld, r, K, Kp, nF;
     int apply;      // 1 = Adamax in place, 0 = write gradients
+    const int32_t* active_pos;  // [K] compact column or -1 (desmo_active_terms_prepare); null = every term active
 };
 
 struct EvalArgs {
@@ -75,8 +76,9 @@ struct EvalArgs {
 };
 
 // host-side launchers (one per translation unit)
+// active_pos: [K] of an active-term table (null = every term active); absent terms get zero W rows and no L1 share
 int build_w(const desmo_shape* s, int K, int Kp, const float* gates, float* rows, const float* coefs, const float* periods,
-            float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st);
+            float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st, const int32_t* active_pos = nullptr);
 // W_out[Kp][mld_out] (and rows_out[K][mld_out] if non-null) at m_out host-given instants, one launch per kAtBatch of them; the
 // arguments are validated by desmo_build_w_at
 constexpr int kAtBatch = 512;
@@ -123,8 +125,10 @@ struct Dims { int T, K, Kp; bool small; MonoTable mt; };  // small: within the f
 int count_terms(int r, int p);  // T = C(r+p, p) for 1 <= r <= DESMO_MAX_R, 0 <= p <= DESMO_MAX_P and T + 3r <= DESMO_MAX_K, else -1
 struct GemmWorkspace;
 size_t gemm_workspace_bytes(const desmo_shape* s, int T, int K, int Kp, uint8_t* base, GemmWorkspace* w);
+// active: device table of desmo_active_terms_prepare with Ka terms (null: the whole library, Ka = K) -- only those columns are built
 int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi, const float* omega,
-                    const float* W, float* dphi, float* red, float* Dacc, void* gemm_ws, cudaStream_t st, bool supplied);
+                    const float* W, float* dphi, float* red, float* Dacc, void* gemm_ws, cudaStream_t st, bool supplied,
+                    const int32_t* active = nullptr, int Ka = 0);
 int reconstruct_gemm_path(const desmo_shape* s, int T, int K, int Kp, const float* P, const float* phi, const float* omega, const float* W,
                           float* out, cudaStream_t st);
 // snap [2][m] fp64 = {sum_x r^2, sum_x u^2}, point [2][ld] fp32 = {sum_t r^2, sum_t u^2} (pad columns 0), r = G W - U; scratch from the

@@ -481,21 +481,27 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
 // ------------------------------------------------------------------------------------------------- library terms for any (r, p)
 // Column order of POOL_DATA (CYL:376-434) = combinations with replacement of range(r), degree by degree, lexicographic.  The index tuple of
 // column j is found by unranking (no table upload, no host state: the kernel is stateless and capturable).
+// Library columns may be a compact list: column c is term cols[c] of the K order (an active set, desmo_active_terms_prepare: strictly
+// increasing, so the polynomial terms come first); cols == null is the whole library, column c = term c.  Entry j of the table then
+// describes column j.
 struct TermTable {
     uint8_t* idx;  // [T][8]: idx[j][0..deg) = mode indices multiplied left to right
     uint8_t* deg;  // [T]
 };
+__device__ __forceinline__ int term_of(const int32_t* __restrict__ cols, int c) { return cols ? cols[c] : c; }
 __device__ __forceinline__ unsigned long long binom_d(int n, int k) {
     if (k < 0 || k > n) return 0ull;
     unsigned long long v = 1;
     for (int i = 1; i <= k; ++i) v = v * (unsigned long long)(n - k + i) / (unsigned long long)i;
     return v;
 }
-__global__ void term_table_kernel(int r, int p, int T, TermTable tab) {
+__global__ void term_table_kernel(int r, int p, int T, TermTable tab, const int32_t* __restrict__ cols, int ncols) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= T) return;
-    // degree of column j: first d with sum_{e<=d} C(r+e-1, e) > j
-    long long rem = j;
+    if (j >= T || j >= ncols) return;
+    const int k = term_of(cols, j);
+    if (k >= T) return;
+    // degree of term k: first d with sum_{e<=d} C(r+e-1, e) > k
+    long long rem = k;
     int d = 0;
     for (; d <= p; ++d) {
         const long long c = (long long)binom_d(r + d - 1, d);
@@ -520,10 +526,11 @@ __global__ void term_table_kernel(int r, int p, int T, TermTable tab) {
 }
 
 // G planes of a chunk: thread <-> point, loop over the K columns.  Gp[plane][k][xl], xl contiguous; rows K..Kr-1 and columns of points >= n are zero.
+// (K here counts the columns: the library's K, or the active set's size with cols its list)
 __global__ void __launch_bounds__(256) library_planes_kernel(const float* __restrict__ P, const float* __restrict__ phi,
-                                                             const float* __restrict__ omega, TermTable tab, int r, int T, int K, int Kr,
-                                                             long long n, long long ld, long long x0, long long rows_c,
-                                                             __nv_bfloat16* __restrict__ Gp) {
+                                                             const float* __restrict__ omega, TermTable tab, const int32_t* __restrict__ cols,
+                                                             int r, int T, int K, int Kr, long long n, long long ld, long long x0,
+                                                             long long rows_c, __nv_bfloat16* __restrict__ Gp) {
     const long long xl = (long long)blockIdx.x * 256 + threadIdx.x;
     if (xl >= rows_c) return;
     const long long x = x0 + xl;
@@ -533,8 +540,9 @@ __global__ void __launch_bounds__(256) library_planes_kernel(const float* __rest
     const size_t plane = (size_t)Kr * rows_c;
     for (int k = blockIdx.y; k < Kr; k += gridDim.y) {
         float v = 0.0f;
+        const int term = k < K ? term_of(cols, k) : K;
         if (xin) {
-            if (k < T) {
+            if (term < T) {
                 const int deg = tab.deg[k];
                 v = 1.0f;
                 for (int q = 0; q < deg; ++q) {
@@ -542,7 +550,7 @@ __global__ void __launch_bounds__(256) library_planes_kernel(const float* __rest
                     v = (q == 0) ? f : v * f;  // left-to-right products, as CYL:390-431
                 }
             } else if (k < K) {
-                const int b = (k - T) / r, i = (k - T) - b * r;
+                const int b = (term - T) / r, i = (term - T) - b * r;
                 const float arg = omega[3 * i + b] * lat[i];
                 v = (b == 0) ? sinf(arg) : (b == 1) ? cosf(arg) : tanhf(arg);
             }
@@ -558,13 +566,14 @@ __global__ void __launch_bounds__(256) library_planes_kernel(const float* __rest
     }
 }
 
-// W planes [3][Kr][mp] from the fp32 W [Kp][mld] of desmo_build_w (rows >= K and columns >= m are zero)
-__global__ void __launch_bounds__(256) w_planes_kernel(const float* __restrict__ W, int K, int Kr, int m, int mld, int mp,
-                                                       __nv_bfloat16* __restrict__ Wp) {
+// W planes [3][Kr][mp] from the fp32 W [Kp][mld] of desmo_build_w (rows >= K and columns >= m are zero); row k is W's row cols[k]
+__global__ void __launch_bounds__(256) w_planes_kernel(const float* __restrict__ W, const int32_t* __restrict__ cols, int K, int Kr, int m,
+                                                       int mld, int mp, __nv_bfloat16* __restrict__ Wp) {
     const int k = blockIdx.x;
     const size_t plane = (size_t)Kr * mp;
+    const size_t src = k < K ? (size_t)term_of(cols, k) * mld : 0;
     for (int t = threadIdx.x; t < mp; t += 256) {
-        const float w = (k < K && t < m) ? W[(size_t)k * mld + t] : 0.0f;
+        const float w = (k < K && t < m) ? W[src + t] : 0.0f;
         const __nv_bfloat16 b1 = __float2bfloat16_rn(w);
         const float e1 = w - __bfloat162float(b1);
         const __nv_bfloat16 b2 = __float2bfloat16_rn(e1);
@@ -578,9 +587,11 @@ __global__ void __launch_bounds__(256) w_planes_kernel(const float* __restrict__
 
 // Chain rule D -> d mse / d phi, d mse / d omega for any (r, p): thread <-> point, one pass over the library columns.  For column
 // j = Phi_{i1} ... Phi_{id}: d L_j / d Phi_v = sum over the positions holding v of the product of the other factors (multiplicity-aware,
-// the same formula as the oracle's pool_data_derivative).  dom_part[cta][3r] are per-CTA partial sums of d omega.
+// the same formula as the oracle's pool_data_derivative).  dom_part[cta][3r] are per-CTA partial sums of d omega.  Dacc row c is library
+// column c: term cols[c] of an active set of Ka terms, pos[k] = the column of term k or -1 (both null: the whole library, Ka = K).
 __global__ void __launch_bounds__(128) chain_rule_generic_kernel(const float* __restrict__ Dacc, const float* __restrict__ P,
                                                                  const float* __restrict__ phi, const float* __restrict__ omega, TermTable tab,
+                                                                 const int32_t* __restrict__ cols, const int32_t* __restrict__ pos, int Ka,
                                                                  int r, int T, long long n, long long ld, float scale, float* __restrict__ dphi,
                                                                  double* __restrict__ dom_part) {
     extern __shared__ double dom_s[];  // [3r]
@@ -597,8 +608,9 @@ __global__ void __launch_bounds__(128) chain_rule_generic_kernel(const float* __
             dl[i] = 0.0f;
         }
         if (xin) {
-            for (int j = 1; j < T; ++j) {
+            for (int j = 0; j < Ka && term_of(cols, j) < T; ++j) {  // the active polynomial columns; the constant has no derivative
                 const int deg = tab.deg[j];
+                if (deg == 0) continue;
                 const float dj = Dacc[(long long)j * ld + x];
                 for (int pos = 0; pos < deg; ++pos) {
                     float rest = 1.0f;
@@ -612,10 +624,11 @@ __global__ void __launch_bounds__(128) chain_rule_generic_kernel(const float* __
             const float ph = lat[i];
             const float ws = omega[3 * i], wc = omega[3 * i + 1], wh = omega[3 * i + 2];
             float ds = 0.0f, dc = 0.0f, dh = 0.0f;
-            if (xin) {
-                ds = Dacc[(long long)(T + i) * ld + x];
-                dc = Dacc[(long long)(T + r + i) * ld + x];
-                dh = Dacc[(long long)(T + 2 * r + i) * ld + x];
+            if (xin) {  // an absent trig term has no column: its dL/dG is zero
+                const int cs_ = pos ? pos[T + i] : T + i, cc_ = pos ? pos[T + r + i] : T + r + i, ch_ = pos ? pos[T + 2 * r + i] : T + 2 * r + i;
+                if (cs_ >= 0) ds = Dacc[(long long)cs_ * ld + x];
+                if (cc_ >= 0) dc = Dacc[(long long)cc_ * ld + x];
+                if (ch_ >= 0) dh = Dacc[(long long)ch_ * ld + x];
             }
             const float cs = cosf(ws * ph), sn = sinf(wc * ph), th = tanhf(wh * ph);
             const float sech2 = 1.0f - th * th;
@@ -673,15 +686,20 @@ __global__ void __launch_bounds__(256) gram_phi_kernel(const float* __restrict__
     }
 }
 
-// Fixed-order sums of all partials into `red` = [E (Kp x mld) | sum r^2 | Phi^T Phi (r x r) | d omega (3r)].
-__global__ void __launch_bounds__(256) reduce_generic_kernel(const float* __restrict__ Epart, int nslice, long long ecount,
+// Fixed-order sums of all partials into `red` = [E (Kp x mld) | sum r^2 | Phi^T Phi (r x r) | d omega (3r)].  The slices of Epart hold
+// the library columns ([nslice][ecount_c / mld][mld]); row k of E is column pos[k] (pos null: column k), zero for an absent term.
+__global__ void __launch_bounds__(256) reduce_generic_kernel(const float* __restrict__ Epart, int nslice, long long ecount, long long ecount_c,
+                                                             const int32_t* __restrict__ pos, int K, int mld,
                                                              const double* __restrict__ loss_part, int nloss, const double* __restrict__ gram_part,
                                                              int ngram, const double* __restrict__ dom_part, int ndom, int r,
                                                              float* __restrict__ red) {
     const long long o = (long long)blockIdx.x * 256 + threadIdx.x;
     if (o < ecount) {
+        const int k = (int)(o / mld), t = (int)(o - (long long)k * mld);
+        const int c = k < K ? (pos ? pos[k] : k) : -1;
         float s = 0.0f;
-        for (int b = 0; b < nslice; ++b) s += Epart[(long long)b * ecount + o];
+        if (c >= 0)
+            for (int b = 0; b < nslice; ++b) s += Epart[(long long)b * ecount_c + (long long)c * mld + t];
         red[o] = s;
     }
     if (blockIdx.x == 0) {
@@ -839,20 +857,27 @@ __global__ void __launch_bounds__(256) supplied_planes_kernel(const float* __res
 }
 
 int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi, const float* omega,
-                    const float* W, float* dphi, float* red, float* Dacc, void* gemm_ws, cudaStream_t st, bool supplied) {
+                    const float* W, float* dphi, float* red, float* Dacc, void* gemm_ws, cudaStream_t st, bool supplied,
+                    const int32_t* active, int Ka) {
     using namespace gp;
     int dev = 0, sms = 0;
     DESMO_CUDA(cudaGetDevice(&dev));
     DESMO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     GemmWorkspace w;
     gemm_workspace_bytes(s, T, K, Kp, static_cast<uint8_t*>(gemm_ws), &w);
+    // Library columns: the active set (pos [K] = column of each term or -1, then cols [Ka] = the terms) or, without one, all K terms.
+    // The workspace is laid out for K; the planes, GEMM extents and partials below use the Ka columns only.
+    const int32_t* pos = active;
+    const int32_t* cols = active ? active + K : nullptr;
+    if (!active) Ka = K;
+    const int Kap = (Ka + 15) / 16 * 16;
     int Kr, mp;
     long long rows_c;
-    gemm_dims(s, K, &Kr, &mp, &rows_c);
+    gemm_dims(s, Ka, &Kr, &mp, &rows_c);
     const int r = s->r;
     TermTable tab{w.tab_idx, w.tab_deg};
-    term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(r, s->polyorder, T, tab);
-    w_planes_kernel<<<Kr, 256, 0, st>>>(W, K, Kr, s->m, s->mld, mp, w.Wp);
+    term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(r, s->polyorder, T, tab, cols, Ka);
+    w_planes_kernel<<<Kr, 256, 0, st>>>(W, cols, Ka, Kr, s->m, s->mld, mp, w.Wp);
     DESMO_CUDA(cudaGetLastError());
 
     CUtensorMap tmG_mn, tmG_k, tmW_mn, tmW_k, tmR_k, tmR_mn;
@@ -867,7 +892,7 @@ int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, i
     if ((rc = make_map(&tmR_k, w.Rp, mp, 2LL * rows_c, 128))) return rc;
     if ((rc = make_map(&tmR_mn, w.Rp, mp, 2LL * rows_c, 64))) return rc;
 
-    const int n_lib16 = (K + 15) / 16 * 16;
+    const int n_lib16 = Kap;
     const float seed = (float)(0.5 * (double)s->n_global * (double)s->m);
     int nslice_used = 1, nloss = 0;
     bool first = true;
@@ -876,16 +901,16 @@ int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, i
         const int tiles_p = (int)(pts / 128);
         {
             dim3 grid((unsigned)((rows_c + 255) / 256), (unsigned)(Kr < 64 ? Kr : 64));
-            library_planes_kernel<<<grid, 256, 0, st>>>(P, phi, omega, tab, r, T, K, Kr, s->n, s->ld, x0, rows_c, w.Gp);
+            library_planes_kernel<<<grid, 256, 0, st>>>(P, phi, omega, tab, cols, r, T, Ka, Kr, s->n, s->ld, x0, rows_c, w.Gp);
             DESMO_CUDA(cudaGetLastError());
         }
         GemmArgs g{};
         g.U = U; g.Rp = w.Rp; g.Dacc = Dacc; g.Epart = w.Epart; g.loss_part = w.loss_part;
-        g.n = s->n; g.ld = s->ld; g.x0 = x0; g.rows_r = rows_c; g.m = s->m; g.mld = s->mld; g.mp = mp; g.K = K; g.Kp = Kp;
+        g.n = s->n; g.ld = s->ld; g.x0 = x0; g.rows_r = rows_c; g.m = s->m; g.mld = s->mld; g.mp = mp; g.K = Ka; g.Kp = Kap;
         g.first_chunk = first ? 1 : 0; g.n_lib16 = n_lib16;
         if (!supplied) {
             // GEMM 1: Rec[p x t] = G W; A = G (MN-major: p contiguous), B = W (MN-major: t contiguous), contraction over the library
-            g.tiles_m = tiles_p; g.tiles_n = mp / 128; g.nslice = 1; g.kblocks = (K + 63) / 64; g.kb_per_slice = g.kblocks; g.kgroup = 4;
+            g.tiles_m = tiles_p; g.tiles_n = mp / 128; g.nslice = 1; g.kblocks = (Ka + 63) / 64; g.kb_per_slice = g.kblocks; g.kgroup = 4;
             g.a_rows = Kr; g.b_rows = Kr;
             rc = u_dtype == DESMO_DTYPE_BF16 ? launch_gemm<true, true, 3, 3, EPI_RESID_BF16>(g, tmG_mn, tmW_mn, sms, st)
                                              : launch_gemm<true, true, 3, 3, EPI_RESID>(g, tmG_mn, tmW_mn, sms, st);
@@ -899,11 +924,11 @@ int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, i
             DESMO_CUDA(cudaGetLastError());
         }
         // GEMM 3: D[p x lib] = R W^T; A = R (K-major: t contiguous), B = W (K-major), contraction over the snapshots
-        g.tiles_m = tiles_p; g.tiles_n = (K + 127) / 128; g.nslice = 1; g.kblocks = mp / 64; g.kb_per_slice = g.kblocks; g.kgroup = 32;
+        g.tiles_m = tiles_p; g.tiles_n = (Ka + 127) / 128; g.nslice = 1; g.kblocks = mp / 64; g.kb_per_slice = g.kblocks; g.kgroup = 32;
         g.a_rows = (int)rows_c; g.b_rows = Kr;
         if ((rc = launch_gemm<false, false, 2, 2, EPI_D>(g, tmR_k, tmW_k, sms, st))) return rc;
         // GEMM 4: E^T[t x lib] = R^T G; A = R (MN-major: t contiguous), B = G (K-major: p contiguous), contraction over the chunk's points
-        g.tiles_m = mp / 128; g.tiles_n = (K + 127) / 128; g.kblocks = (int)(pts / 64);
+        g.tiles_m = mp / 128; g.tiles_n = (Ka + 127) / 128; g.kblocks = (int)(pts / 64);
         {
             const int tiles = g.tiles_m * g.tiles_n;
             int ns = sms / tiles;
@@ -924,15 +949,17 @@ int fused_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, i
     const float scale = (float)(2.0 / ((double)s->n_global * (double)s->m));
     const long long ntiles = (s->ld + 127) / 128;
     const int gc = (int)(ntiles < kChainCtas ? ntiles : kChainCtas);
-    chain_rule_generic_kernel<<<gc, 128, sizeof(double) * 3 * r, st>>>(Dacc, P, phi, omega, tab, r, T, s->n, s->ld, scale, dphi, w.dom_part);
+    chain_rule_generic_kernel<<<gc, 128, sizeof(double) * 3 * r, st>>>(Dacc, P, phi, omega, tab, cols, pos, Ka, r, T, s->n, s->ld, scale, dphi,
+                                                                        w.dom_part);
     const long long gtiles = (s->n + 127) / 128;
     const int gg = (int)(gtiles < kGramCtas ? gtiles : kGramCtas);
     const size_t gsm = sizeof(float) * (size_t)r * 129;
     DESMO_CUDA(cudaFuncSetAttribute(gram_phi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gsm));
     gram_phi_kernel<<<gg, 256, gsm, st>>>(P, phi, r, s->n, s->ld, w.gram_part);
     const long long ecount = (long long)Kp * s->mld;
-    reduce_generic_kernel<<<(unsigned)((ecount + 255) / 256), 256, 0, st>>>(w.Epart, nslice_used, ecount, w.loss_part, supplied ? 0 : nloss, w.gram_part,
-                                                                            gg, w.dom_part, gc, r, red);
+    reduce_generic_kernel<<<(unsigned)((ecount + 255) / 256), 256, 0, st>>>(w.Epart, nslice_used, ecount, (long long)Kap * s->mld, pos, K, s->mld,
+                                                                            w.loss_part, supplied ? 0 : nloss, w.gram_part, gg, w.dom_part, gc, r,
+                                                                            red);
     DESMO_CUDA(cudaGetLastError());
     return DESMO_OK;
 }
@@ -954,15 +981,15 @@ int reconstruct_gemm_path(const desmo_shape* s, int T, int K, int Kp, const floa
     long long rows_c;
     gemm_dims(s, K, &Kr, &mp, &rows_c);
     TermTable tab{w.tab_idx, w.tab_deg};
-    term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab);
-    w_planes_kernel<<<Kr, 256, 0, st>>>(W, K, Kr, s->m, s->mld, mp, w.Wp);
+    term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab, nullptr, K);
+    w_planes_kernel<<<Kr, 256, 0, st>>>(W, nullptr, K, Kr, s->m, s->mld, mp, w.Wp);
     CUtensorMap tmG_mn, tmW_mn;
     int rc;
     if ((rc = make_map(&tmG_mn, w.Gp, rows_c, 3LL * Kr, 64)) || (rc = make_map(&tmW_mn, w.Wp, mp, 3LL * Kr, 64))) { cudaFreeAsync(scratch, st); return rc; }
     for (long long x0 = 0; x0 < s->ld && !rc; x0 += rows_c) {
         const long long pts = (s->ld - x0 < rows_c) ? s->ld - x0 : rows_c;
         dim3 grid((unsigned)((rows_c + 255) / 256), (unsigned)(Kr < 64 ? Kr : 64));
-        library_planes_kernel<<<grid, 256, 0, st>>>(P, phi, omega, tab, s->r, T, K, Kr, s->n, s->ld, x0, rows_c, w.Gp);
+        library_planes_kernel<<<grid, 256, 0, st>>>(P, phi, omega, tab, nullptr, s->r, T, K, Kr, s->n, s->ld, x0, rows_c, w.Gp);
         GemmArgs g{};
         g.out = out; g.n = s->n; g.ld = s->ld; g.x0 = x0; g.rows_r = rows_c; g.m = s->m; g.mld = s->mld; g.mp = mp; g.K = K; g.Kp = Kp;
         g.tiles_m = (int)(pts / 128); g.tiles_n = mp / 128; g.nslice = 1; g.kblocks = (K + 63) / 64; g.kb_per_slice = g.kblocks; g.kgroup = 4;
@@ -1031,15 +1058,15 @@ int residual_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const
     int rc = check_cuda(cudaMemsetAsync(part, 0, (size_t)sms * 2 * mp * sizeof(double), st), "cudaMemsetAsync");
     CUtensorMap tmG_mn, tmW_mn;
     if (!rc) {
-        term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab);
-        w_planes_kernel<<<Kr, 256, 0, st>>>(W, K, Kr, s->m, s->mld, mp, Wp);
+        term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab, nullptr, K);
+        w_planes_kernel<<<Kr, 256, 0, st>>>(W, nullptr, K, Kr, s->m, s->mld, mp, Wp);
         rc = check_cuda(cudaGetLastError(), "w_planes_kernel");
     }
     if (!rc && !(rc = make_map(&tmG_mn, Gp, rows_c, 3LL * Kr, 64))) rc = make_map(&tmW_mn, Wp, mp, 3LL * Kr, 64);
     for (long long x0 = 0; x0 < s->ld && !rc; x0 += rows_c) {
         const long long pts = (s->ld - x0 < rows_c) ? s->ld - x0 : rows_c;  // multiple of 128
         dim3 grid((unsigned)((rows_c + 255) / 256), 64u);
-        library_planes_kernel<<<grid, 256, 0, st>>>(P, phi, omega, tab, s->r, T, K, Kr, s->n, s->ld, x0, rows_c, Gp);
+        library_planes_kernel<<<grid, 256, 0, st>>>(P, phi, omega, tab, nullptr, s->r, T, K, Kr, s->n, s->ld, x0, rows_c, Gp);
         GemmArgs g{};
         g.U = U; g.out = pp; g.loss_part = part;
         g.n = s->n; g.ld = s->ld; g.x0 = x0; g.rows_r = rows_c; g.m = s->m; g.mld = s->mld; g.mp = mp; g.K = K; g.Kp = Kp;
@@ -1167,8 +1194,8 @@ int pruning_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const 
     int rc = check_cuda(cudaMemsetAsync(part, 0, L.part_bytes, st), "cudaMemsetAsync");
     CUtensorMap tmW_mn, tmG_mn;
     if (!rc) {
-        term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab);
-        w_planes_kernel<<<Kr, 256, 0, st>>>(W, K, Kr, s->m, s->mld, mp, Wp);
+        term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab, nullptr, K);
+        w_planes_kernel<<<Kr, 256, 0, st>>>(W, nullptr, K, Kr, s->m, s->mld, mp, Wp);
         const long long nb = ((long long)(steps + 1) * mp + 255) / 256;
         prune_b_kernel<<<(unsigned)(nb < 4096 ? nb : 4096), 256, 0, st>>>(W, s->mld, s->m, mp, steps, ord, B);
         rc = check_cuda(cudaGetLastError(), "prune_b_kernel");
@@ -1178,7 +1205,7 @@ int pruning_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const 
     for (long long x0 = 0; x0 < s->ld && !rc; x0 += rows_c) {
         const long long pts = (s->ld - x0 < rows_c) ? s->ld - x0 : rows_c;  // multiple of 128
         const unsigned bx = (unsigned)((rows_c + 255) / 256);
-        library_planes_kernel<<<dim3(bx, 64u), 256, 0, st>>>(P, phi, omega, tab, s->r, T, K, Kr, s->n, s->ld, x0, rows_c, Gp);
+        library_planes_kernel<<<dim3(bx, 64u), 256, 0, st>>>(P, phi, omega, tab, nullptr, s->r, T, K, Kr, s->n, s->ld, x0, rows_c, Gp);
         prune_a_kernel<<<dim3(bx, (unsigned)(steps + 1 < 64 ? steps + 1 : 64)), 256, 0, st>>>(Gp, Kr, rows_c, steps, ord, A);
         if ((rc = check_cuda(cudaGetLastError(), "prune_a_kernel"))) break;
         GemmArgs g{};
@@ -1210,7 +1237,7 @@ int colnorm2_gemm_path(const desmo_shape* s, int T, int K, const float* P, const
     const size_t bytes = (size_t)T * 9 + 2048;
     DESMO_CUDA(cudaMallocAsync(&scratch, bytes, st));
     TermTable tab{static_cast<uint8_t*>(scratch), static_cast<uint8_t*>(scratch) + align_up_g((size_t)T * 8, 256)};
-    term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab);
+    term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab, nullptr, K);
     DESMO_CUDA(cudaMemsetAsync(out_k, 0, sizeof(float) * K, st));
     colnorm2_generic_kernel<<<(unsigned)((s->n + 255) / 256), 256, 0, st>>>(P, phi, omega, tab, s->r, T, K, s->n, s->ld, out_k);
     DESMO_CUDA(cudaGetLastError());

@@ -32,19 +32,22 @@ __device__ __forceinline__ float fourier_value(const float* __restrict__ c, int 
 // grid = Kp blocks (one library term each), 256 threads over time.
 __global__ void build_w_kernel(int K, int m, int mld, int nF, const float* __restrict__ gates, float* __restrict__ rows,
                                const float* __restrict__ coefs, const float* __restrict__ periods, float* __restrict__ W,
-                               __nv_bfloat16* __restrict__ Wb, int Kp, int32_t* step_dev, float* l1_out) {
-    // Wb: three bf16 planes [3][32][mld] of W for the tcgen05 path (w = b1 + b2 + b3), rows >= K zero
+                               __nv_bfloat16* __restrict__ Wb, int Kp, int32_t* step_dev, float* l1_out,
+                               const int32_t* __restrict__ active_pos) {
+    // Wb: three bf16 planes [3][32][mld] of W for the tcgen05 path (w = b1 + b2 + b3), rows >= K zero.
+    // active_pos (null: every term active): an absent term has a zero W row and no share of the L1 sum.
     const int k = blockIdx.x;
     if (k == 0 && threadIdx.x < 32) {
         float s = 0.0f;
-        for (int j = threadIdx.x; j < K; j += 32) s += fabsf(gates[j]);
+        for (int j = threadIdx.x; j < K; j += 32)
+            if (!active_pos || active_pos[j] >= 0) s += fabsf(gates[j]);
         s = warp_sum(s);
         if (threadIdx.x == 0) {
             *l1_out = s;                       // L1 of the gates before this step's update (CYL:725-731)
             if (step_dev) *step_dev += 1;      // optimizer step counter t (Adamax bias correction)
         }
     }
-    const float gate = (k < K) ? gates[k] : 0.0f;
+    const float gate = (k < K && (!active_pos || active_pos[k] >= 0)) ? gates[k] : 0.0f;
     const float period = (nF > 0 && k < K) ? periods[k] : 1.0f;
     for (int t = threadIdx.x; t < mld; t += blockDim.x) {
         float w = 0.0f;
@@ -72,11 +75,11 @@ __global__ void build_w_kernel(int K, int m, int mld, int nF, const float* __res
 }
 
 int build_w(const desmo_shape* s, int K, int Kp, const float* gates, float* rows, const float* coefs, const float* periods,
-            float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st) {
+            float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st, const int32_t* active_pos) {
     (void)Wlo;
     const int grid = (Whi && Kp < 32) ? 32 : Kp;
     build_w_kernel<<<grid, 256, 0, st>>>(K, s->m, s->mld, s->nF, gates, rows, coefs, periods, W, reinterpret_cast<__nv_bfloat16*>(Whi), Kp,
-                                         step_dev, l1_out);
+                                         step_dev, l1_out, active_pos);
     DESMO_CUDA(cudaGetLastError());
     return DESMO_OK;
 }

@@ -52,6 +52,19 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateArgs a) {
     if (b < a.K) {
         // ---------------- one library term: temporal row + its gate ----------------
         const int k = b;
+        if (a.active_pos && a.active_pos[k] < 0) {
+            // absent from the model (active set): nothing is updated, its gradients are exactly zero
+            if (!a.apply) {
+                if (a.nF == 0) {
+                    for (int t = tid; t < a.m; t += 256) a.d_rows[(long long)k * a.mld + t] = 0.0f;
+                } else {
+                    if (tid < 2 * a.nF + 1) a.d_coefs[(long long)k * (2 * a.nF + 1) + tid] = 0.0f;
+                    if (tid == 0) a.d_periods[k] = 0.0f;
+                }
+                if (tid == 0) a.d_gates[k] = 0.0f;
+            }
+            return;
+        }
         const float gate = a.gates[k];
         const float* E = a.red + (long long)k * a.mld;
         float* row = a.rows + (long long)k * a.mld;
@@ -115,9 +128,14 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateArgs a) {
         // ---------------- omega + the three printed losses ----------------
         const int r = a.r;
         if (tid < 3 * r) {
+            // omega[3i + b] belongs to trig term T + b r + i: frozen when that term is absent
+            const bool frozen = a.active_pos && a.active_pos[a.K - 3 * r + (tid % 3) * r + tid / 3] < 0;
             const float g = a.red[eoff + 1 + r * r + tid];
-            if (a.apply) adamax(a.omega + tid, a.omega_m + tid, a.omega_u + tid, g, clr_of(a.hyper[DESMO_HYP_LR_OMEGA], step));
-            else a.d_omega[tid] = g;
+            if (a.apply) {
+                if (!frozen) adamax(a.omega + tid, a.omega_m + tid, a.omega_u + tid, g, clr_of(a.hyper[DESMO_HYP_LR_OMEGA], step));
+            } else {
+                a.d_omega[tid] = frozen ? 0.0f : g;
+            }
         }
         if (tid == 0 && a.losses_out) {
             const float mse = (float)((double)a.red[eoff] * a.inv_nm);

@@ -80,6 +80,20 @@ def pruning_order(order, K: int) -> np.ndarray:
     return np.ascontiguousarray(k, dtype=np.int32)
 
 
+def active_indices(mask, K: int) -> np.ndarray:
+    """The packed indices (int32, increasing) of an active-term mask: a bool (K,) tensor or array with at least one True.  Raises
+    DesmoError before any launch (desmo_active_terms_prepare checks the indices again)."""
+    raw = mask.detach().cpu().numpy() if torch.is_tensor(mask) else np.asarray(mask)
+    if raw.dtype != np.bool_:
+        raise _lib.DesmoError(f"the active-term mask must be bool, got {raw.dtype}")
+    if raw.shape != (K,):
+        raise _lib.DesmoError(f"the active-term mask must have shape ({K},), got {raw.shape}")
+    idx = np.flatnonzero(raw)
+    if idx.size == 0:
+        raise _lib.DesmoError("the active-term mask keeps no term: an active set holds at least one")
+    return np.ascontiguousarray(idx, dtype=np.int32)
+
+
 class _PeerDesc(C.Structure):  # desmo_peer (include/desmo_b200.h)
     _fields_ = [("world", C.c_int32), ("rank", C.c_int32), ("red_ptrs", C.c_void_p), ("flag_ptrs", C.c_void_p), ("state", C.c_void_p)]
 
@@ -150,6 +164,9 @@ class DesmoEngine:
         self.workspace = torch.zeros(nbytes.value, dtype=torch.uint8, device=self.device)
         self.launches_per_step = 0
         self._side: Optional[torch.cuda.Stream] = None
+        self.active_terms: Optional[torch.Tensor] = None  # bool (K,) on the host; None = every term (set_active_terms)
+        self._active: Optional[torch.Tensor] = None       # its device table (desmo_active_terms_prepare)
+        self._active_count = 0
         self.set_hyper(REFERENCE_LRS, 1e-3, 1e-4)
 
     # ------------------------------------------------------------------ inputs
@@ -242,17 +259,63 @@ class DesmoEngine:
     def _stream(self) -> int:
         return torch.cuda.current_stream(self.device).cuda_stream
 
-    def build_w(self, advance_step: bool = True) -> None:
+    # ------------------------------------------------------------------ active set (training a pruned model)
+    def set_active_terms(self, mask) -> None:
+        """Train on the terms of ``mask`` (bool (K,), packed K order as term_norms; at least one True) from the next step on, or on
+        every term again with ``mask=None``.  A term outside the set is absent from the model: it adds nothing to recon, the losses or
+        any gradient, and its gate, temporal row / Fourier coefficients and period, the omega of a trig term and their Adamax state
+        are frozen (gradients() reports 0 for them).  phi, the active parameters, the ortho term, the step counter and the scheduler
+        train as before -- the reference's loop with the gates multiplied by a fixed 0/1 buffer and the pruned parameters left out of
+        the optimizer.  The gates of absent terms are set to 0, so state_dict(), term_norms(), the sweeps and the evaluation routines
+        see the pruned model without taking the set.  train_step() and gradients() use it; on the GEMM path the step builds the
+        active library columns only.  Point-sharded: every rank must pass the same mask (checked with one all-reduce).  A bad mask
+        raises before anything is written."""
+        if mask is None:
+            self.active_terms, self._active, self._active_count = None, None, 0
+            return
+        idx = active_indices(mask, self.K)
+        host = torch.zeros(self.K, dtype=torch.bool)
+        host[torch.from_numpy(idx).long()] = True
+        if self._sharded():
+            # diverging masks would desynchronise the replicated parameters: sum over ranks == world * own mask on every rank
+            mine = host.to(self.device, torch.float32)
+            tot = mine.clone()
+            torch.distributed.all_reduce(tot, group=self.pg)
+            if not torch.equal(tot, mine * torch.distributed.get_world_size(self.pg)):
+                raise _lib.DesmoError("set_active_terms: the ranks passed different masks (the set is replicated: pass the same one)")
+        nbytes = C.c_size_t(0)
+        check(self.lib.desmo_active_terms_bytes(C.byref(self.shape), int(idx.size), C.byref(nbytes)), "desmo_active_terms_bytes")
+        table = torch.empty(nbytes.value // 4, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.lib.desmo_active_terms_prepare(C.byref(self.shape), idx.ctypes.data, int(idx.size), _ptr(table), self._stream()),
+                  "desmo_active_terms_prepare")
+            self.gates.masked_fill_(~host.to(self.device), 0.0)
+        self.active_terms, self._active, self._active_count = host, table, int(idx.size)
+
+    def build_w(self, advance_step: bool = True, use_active: bool = False) -> None:
+        """W = diag(gates) rows (desmo_build_w); ``use_active``: with the active set, if one is set (absent rows zero)."""
+        if use_active and self._active is not None:
+            check(self.lib.desmo_build_w_active(C.byref(self.shape), _ptr(self.gates), _ptr(self.rows), _ptr(self.coefs), _ptr(self.periods),
+                                                _ptr(self.W), _ptr(self.step_dev) if advance_step else None, _ptr(self.workspace),
+                                                _ptr(self._active), self._stream()), "desmo_build_w_active")
+            return
         check(self.lib.desmo_build_w(C.byref(self.shape), _ptr(self.gates), _ptr(self.rows), _ptr(self.coefs), _ptr(self.periods),
                                      _ptr(self.W), _ptr(self.step_dev) if advance_step else None, _ptr(self.workspace),
                                      self._stream()), "desmo_build_w")
 
-    def fused_residual_grad(self, red: Optional[torch.Tensor] = None) -> None:
+    def fused_residual_grad(self, red: Optional[torch.Tensor] = None, use_active: bool = False, phase: int = 0) -> None:
+        """The fused residual / gradient pass (desmo_fused_residual_grad_ex; phase 1 / 2: its _begin / _finish halves).  ``use_active``:
+        with the active set, if one is set."""
         ud = self._u_dtype()
-        check(self.lib.desmo_fused_residual_grad_ex(C.byref(self.shape), _ptr(self.U), ud, _ptr(self.P), _ptr(self.phi), _ptr(self.omega),
-                                                    _ptr(self.W), _ptr(self.dphi), _ptr(self.red if red is None else red),
-                                                    _ptr(self.workspace), self._stream()),
-              "desmo_fused_residual_grad")
+        args = (C.byref(self.shape), _ptr(self.U), ud, _ptr(self.P), _ptr(self.phi), _ptr(self.omega), _ptr(self.W), _ptr(self.dphi),
+                _ptr(self.red if red is None else red), _ptr(self.workspace))
+        if use_active and self._active is not None:
+            fn = (self.lib.desmo_fused_residual_grad_active, self.lib.desmo_fused_residual_grad_begin_active,
+                  self.lib.desmo_fused_residual_grad_finish_active)[phase]
+            check(fn(*args, _ptr(self._active), self._active_count, self._stream()), fn.__name__)
+            return
+        fn = (self.lib.desmo_fused_residual_grad_ex, self.lib.desmo_fused_residual_grad_begin_ex, self.lib.desmo_fused_residual_grad_finish_ex)[phase]
+        check(fn(*args, self._stream()), fn.__name__)
 
     def enable_peer_allreduce(self, group=None) -> bool:
         """Point-sharded runs on one node: replaces the two NCCL all-reduces of the train step by the one-shot exchange over NVLink /
@@ -306,12 +369,16 @@ class DesmoEngine:
             torch.distributed.all_reduce(self.red, group=self.pg)
 
     def adamax_update(self) -> None:
-        check(self.lib.desmo_adamax_update(
-            C.byref(self.shape), _ptr(self.red), _ptr(self.dphi), _ptr(self.P), _ptr(self.phi), _ptr(self.phi_m), _ptr(self.phi_u),
-            _ptr(self.gates), _ptr(self.gates_m), _ptr(self.gates_u), _ptr(self.rows), _ptr(self.rows_m), _ptr(self.rows_u),
-            _ptr(self.coefs), _ptr(self.coefs_m), _ptr(self.coefs_u), _ptr(self.periods), _ptr(self.periods_m), _ptr(self.periods_u),
-            _ptr(self.omega), _ptr(self.omega_m), _ptr(self.omega_u), _ptr(self.hyper), _ptr(self.step_dev), _ptr(self.losses),
-            _ptr(self.workspace), self._stream()), "desmo_adamax_update")
+        """Losses + Adamax for every parameter (desmo_adamax_update); with the active set (if one is set) the absent terms freeze."""
+        args = (C.byref(self.shape), _ptr(self.red), _ptr(self.dphi), _ptr(self.P), _ptr(self.phi), _ptr(self.phi_m), _ptr(self.phi_u),
+                _ptr(self.gates), _ptr(self.gates_m), _ptr(self.gates_u), _ptr(self.rows), _ptr(self.rows_m), _ptr(self.rows_u),
+                _ptr(self.coefs), _ptr(self.coefs_m), _ptr(self.coefs_u), _ptr(self.periods), _ptr(self.periods_m), _ptr(self.periods_u),
+                _ptr(self.omega), _ptr(self.omega_m), _ptr(self.omega_u), _ptr(self.hyper), _ptr(self.step_dev), _ptr(self.losses),
+                _ptr(self.workspace))
+        if self._active is not None:
+            check(self.lib.desmo_adamax_update_active(*args, _ptr(self._active), self._stream()), "desmo_adamax_update_active")
+        else:
+            check(self.lib.desmo_adamax_update(*args, self._stream()), "desmo_adamax_update")
 
     def _sharded(self) -> bool:
         return self.pg is not None or (torch.distributed.is_available() and torch.distributed.is_initialized() and self.n_global != self.n)
@@ -322,27 +389,25 @@ class DesmoEngine:
         Multi-GPU: the K x m block of `red` (E = G^T R) is final as soon as the dominant kernel has run, so its all-reduce is issued
         on a side stream and overlaps the chain-rule kernel; only the 1 + r^2 + 3r scalars are reduced afterwards."""
         with torch.cuda.device(self.device):
-            self.build_w(True)
+            self.build_w(True, use_active=True)
             if not self._sharded():
-                self.fused_residual_grad()
+                self.fused_residual_grad(use_active=True)
             elif self._peer is not None:
                 # one-shot exchange over NVLink peer memory: no NCCL call, no side stream
                 st = self._stream()
                 check(self.lib.desmo_peer_begin_step(C.byref(self._peer), st), "desmo_peer_begin_step")
-                self.fused_residual_grad(self.red_local)
+                self.fused_residual_grad(self.red_local, use_active=True)
                 check(self.lib.desmo_peer_allreduce(C.byref(self._peer), self._red_pad.numel(), _ptr(self._red_pad), st), "desmo_peer_allreduce")
             else:
-                args = (C.byref(self.shape), _ptr(self.U), self._u_dtype(), _ptr(self.P), _ptr(self.phi), _ptr(self.omega), _ptr(self.W), _ptr(self.dphi),
-                        _ptr(self.red), _ptr(self.workspace))
                 main = torch.cuda.current_stream(self.device)
                 if self._side is None:
                     self._side = torch.cuda.Stream(device=self.device)
                 ecount = self.Kp * self.mld
-                check(self.lib.desmo_fused_residual_grad_begin_ex(*args, main.cuda_stream), "desmo_fused_residual_grad_begin")
+                self.fused_residual_grad(use_active=True, phase=1)
                 self._side.wait_stream(main)
                 with torch.cuda.stream(self._side):
                     torch.distributed.all_reduce(self.red[:ecount], group=self.pg)
-                check(self.lib.desmo_fused_residual_grad_finish_ex(*args, main.cuda_stream), "desmo_fused_residual_grad_finish")
+                self.fused_residual_grad(use_active=True, phase=2)
                 torch.distributed.all_reduce(self.red[ecount:], group=self.pg)
                 main.wait_stream(self._side)
             self.adamax_update()
@@ -363,15 +428,17 @@ class DesmoEngine:
         else:
             g["rows"] = torch.zeros(self.K, self.mld, **f32)
         with torch.cuda.device(self.device):
-            self.build_w(False)
-            self.fused_residual_grad()
+            self.build_w(False, use_active=True)
+            self.fused_residual_grad(use_active=True)
             self.all_reduce()
             g["phi"].copy_(self.dphi)
-            check(self.lib.desmo_assemble_grads(
-                C.byref(self.shape), _ptr(self.red), _ptr(g["phi"]), _ptr(self.P), _ptr(self.phi), _ptr(self.gates), _ptr(self.rows),
-                _ptr(self.coefs), _ptr(self.periods), _ptr(self.hyper), _ptr(g["gates"]), _ptr(g.get("rows")), _ptr(g.get("coefs")),
-                _ptr(g.get("periods")), _ptr(g["omega"]), _ptr(self.losses), _ptr(self.workspace), self._stream()),
-                "desmo_assemble_grads")
+            args = (C.byref(self.shape), _ptr(self.red), _ptr(g["phi"]), _ptr(self.P), _ptr(self.phi), _ptr(self.gates), _ptr(self.rows),
+                    _ptr(self.coefs), _ptr(self.periods), _ptr(self.hyper), _ptr(g["gates"]), _ptr(g.get("rows")), _ptr(g.get("coefs")),
+                    _ptr(g.get("periods")), _ptr(g["omega"]), _ptr(self.losses), _ptr(self.workspace))
+            if self._active is not None:
+                check(self.lib.desmo_assemble_grads_active(*args, _ptr(self._active), self._stream()), "desmo_assemble_grads_active")
+            else:
+                check(self.lib.desmo_assemble_grads(*args, self._stream()), "desmo_assemble_grads")
         if beta is not None or l1_lambda is not None:
             self.set_hyper(saved[:5], saved[5], saved[6])
         g["phi"] = g["phi"][:, :self.n]

@@ -226,6 +226,13 @@ class _DesmoBase(nn.Module):
         self.sync_parameters()
         return self.engine.residual_profile_at(snapshots, index=index, times=times)
 
+    # ---- training a pruned model (DesmoEngine.set_active_terms) ----------------------------------------------------------------
+    def set_active_terms(self, mask) -> None:
+        """Train on the terms of the bool (K,) ``mask`` only (None: every term); see DesmoEngine.set_active_terms.  The set applies to
+        DesmoTrainer's fused step; a torch optimizer stepping this module's Parameters does not know it and would move frozen entries."""
+        self.sync_parameters()
+        self.engine.set_active_terms(mask)
+
     def mse_loss(self, snapshot: Optional[torch.Tensor] = None) -> torch.Tensor:
         """criterion(model(snapshot)[0], snapshot) (CYL:711,722) without materialising recon; differentiable w.r.t. every
         parameter of the module (backward = the fused residual+grad kernel)."""

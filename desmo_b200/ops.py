@@ -1,7 +1,8 @@
 """torch custom ops over the C ABI: one ``torch.ops.desmo_b200.*`` op per hot-path entry point of include/desmo_b200.h.
 
   build_w, build_w_at, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, pruning_profile, library_colnorm2, term_norms,
-  pod_gram, pod_eig, pod_eigh, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce
+  pod_gram, pod_eig, pod_eigh, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce,
+  active_terms_prepare, build_w_active, fused_residual_grad_active, adamax_update_active, assemble_grads_active
 
 They take the packed device tensors of a DesmoEngine (layout: include/desmo_b200.h) plus the shape integers and launch the
 sm_100a kernels on the current stream.  CUDA only: no CPU implementation is registered and every op checks its tensors, so a call
@@ -258,6 +259,86 @@ def snapshot_to_bf16(src: torch.Tensor, U: torch.Tensor, qsums: Optional[torch.T
               "desmo_snapshot_to_bf16")
 
 
+@torch.library.custom_op("desmo_b200::active_terms_prepare", mutates_args=("table",))
+def active_terms_prepare(indices: torch.Tensor, table: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int, nF: int,
+                         path: int) -> None:
+    """The device table of an active set (desmo_active_terms_prepare): ``indices`` a contiguous 1-D int32 HOST tensor of strictly
+    increasing packed term indices, ``table`` an int32 device tensor of desmo_active_terms_bytes / 4 elements."""
+    _require_cuda(table)
+    if indices.device.type != "cpu" or indices.dtype != torch.int32 or indices.dim() != 1 or not indices.is_contiguous():
+        raise _lib.DesmoError("active_terms_prepare: indices must be a contiguous 1-D int32 tensor on the host")
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    nbytes = C.c_size_t(0)
+    check(_lib.load().desmo_active_terms_bytes(C.byref(s), indices.numel(), C.byref(nbytes)), "desmo_active_terms_bytes")
+    if table.dtype != torch.int32 or not table.is_contiguous() or table.numel() * 4 < nbytes.value:
+        raise _lib.DesmoError(f"active_terms_prepare: table must be a contiguous int32 tensor of at least {nbytes.value // 4} elements")
+    with torch.cuda.device(table.device):
+        check(_lib.load().desmo_active_terms_prepare(C.byref(s), _p(indices), indices.numel(), _p(table), _stream(table)),
+              "desmo_active_terms_prepare")
+
+
+@torch.library.custom_op("desmo_b200::build_w_active", mutates_args=("rows", "W", "step", "workspace"))
+def build_w_active(gates: torch.Tensor, rows: torch.Tensor, coefs: Optional[torch.Tensor], periods: Optional[torch.Tensor], W: torch.Tensor,
+                   step: torch.Tensor, workspace: torch.Tensor, active: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int,
+                   nF: int, path: int) -> None:
+    """build_w on an active set (desmo_build_w_active): absent rows of W are zero, the L1 sum takes the active gates."""
+    _require_cuda(gates, rows, W, active)
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(gates.device):
+        check(_lib.load().desmo_build_w_active(C.byref(s), _p(gates), _p(rows), _p(coefs), _p(periods), _p(W), _p(step), _p(workspace),
+                                               _p(active), _stream(gates)), "desmo_build_w_active")
+
+
+@torch.library.custom_op("desmo_b200::fused_residual_grad_active", mutates_args=("dphi", "red", "workspace"))
+def fused_residual_grad_active(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, omega: torch.Tensor, W: torch.Tensor, dphi: torch.Tensor,
+                               red: torch.Tensor, workspace: torch.Tensor, active: torch.Tensor, active_count: int, n: int, n_global: int,
+                               m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """fused_residual_grad on an active set of ``active_count`` terms (desmo_fused_residual_grad_active)."""
+    _require_cuda(U, P, phi, omega, W, dphi, red, active)
+    ud = _lib.u_dtype_code(U.dtype)
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(U.device):
+        check(_lib.load().desmo_fused_residual_grad_active(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), _p(dphi), _p(red),
+                                                           _p(workspace), _p(active), active_count, _stream(U)),
+              "desmo_fused_residual_grad_active")
+
+
+@torch.library.custom_op("desmo_b200::adamax_update_active",
+                         mutates_args=("phi", "phi_m", "phi_u", "gates", "gates_m", "gates_u", "rows", "rows_m", "rows_u", "coefs", "coefs_m",
+                                       "coefs_u", "periods", "periods_m", "periods_u", "omega", "omega_m", "omega_u", "losses", "workspace"))
+def adamax_update_active(red: torch.Tensor, dphi: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, phi_m: torch.Tensor, phi_u: torch.Tensor,
+                         gates: torch.Tensor, gates_m: torch.Tensor, gates_u: torch.Tensor, rows: torch.Tensor, rows_m: torch.Tensor,
+                         rows_u: torch.Tensor, coefs: Optional[torch.Tensor], coefs_m: Optional[torch.Tensor], coefs_u: Optional[torch.Tensor],
+                         periods: Optional[torch.Tensor], periods_m: Optional[torch.Tensor], periods_u: Optional[torch.Tensor],
+                         omega: torch.Tensor, omega_m: torch.Tensor, omega_u: torch.Tensor, hyper: torch.Tensor, step: torch.Tensor,
+                         losses: torch.Tensor, workspace: torch.Tensor, active: torch.Tensor, n: int, n_global: int, m: int, r: int,
+                         polyorder: int, nF: int, path: int) -> None:
+    """adamax_update on an active set (desmo_adamax_update_active): absent terms' parameters and Adamax state are not written."""
+    _require_cuda(red, dphi, P, phi, gates, rows, omega, hyper, step, losses, active)
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(phi.device):
+        check(_lib.load().desmo_adamax_update_active(
+            C.byref(s), _p(red), _p(dphi), _p(P), _p(phi), _p(phi_m), _p(phi_u), _p(gates), _p(gates_m), _p(gates_u), _p(rows), _p(rows_m),
+            _p(rows_u), _p(coefs), _p(coefs_m), _p(coefs_u), _p(periods), _p(periods_m), _p(periods_u), _p(omega), _p(omega_m), _p(omega_u),
+            _p(hyper), _p(step), _p(losses), _p(workspace), _p(active), _stream(phi)), "desmo_adamax_update_active")
+
+
+@torch.library.custom_op("desmo_b200::assemble_grads_active",
+                         mutates_args=("dphi", "d_gates", "d_rows", "d_coefs", "d_periods", "d_omega", "losses", "workspace"))
+def assemble_grads_active(red: torch.Tensor, dphi: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, gates: torch.Tensor, rows: torch.Tensor,
+                          coefs: Optional[torch.Tensor], periods: Optional[torch.Tensor], hyper: torch.Tensor, d_gates: torch.Tensor,
+                          d_rows: Optional[torch.Tensor], d_coefs: Optional[torch.Tensor], d_periods: Optional[torch.Tensor],
+                          d_omega: torch.Tensor, losses: torch.Tensor, workspace: torch.Tensor, active: torch.Tensor, n: int, n_global: int,
+                          m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """assemble_grads on an active set (desmo_assemble_grads_active): absent terms' gradients are exactly 0."""
+    _require_cuda(red, dphi, P, phi, gates, rows, hyper, d_gates, d_omega, losses, active)
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(phi.device):
+        check(_lib.load().desmo_assemble_grads_active(
+            C.byref(s), _p(red), _p(dphi), _p(P), _p(phi), _p(gates), _p(rows), _p(coefs), _p(periods), _p(hyper), _p(d_gates), _p(d_rows),
+            _p(d_coefs), _p(d_periods), _p(d_omega), _p(losses), _p(workspace), _p(active), _stream(phi)), "desmo_assemble_grads_active")
+
+
 @torch.library.custom_op("desmo_b200::plateau_step", mutates_args=("state", "hyper"))
 def plateau_step(state: torch.Tensor, step: torch.Tensor, losses: torch.Tensor, hyper: torch.Tensor) -> None:
     """ReduceLROnPlateau.step(losses[3]) on the device (desmo_plateau_step); ``state`` is the desmo_plateau struct as bytes."""
@@ -294,14 +375,21 @@ def _shape_args(e):
 
 
 def engine_step_via_ops(e) -> None:
-    """One train step of a DesmoEngine routed entirely through the registered ops."""
+    """One train step of a DesmoEngine routed entirely through the registered ops (on its active set, if one is set)."""
     sa = _shape_args(e)
+    opt = (e.red, e.dphi, e.P, e.phi, e.phi_m, e.phi_u, e.gates, e.gates_m, e.gates_u, e.rows, e.rows_m, e.rows_u, e.coefs, e.coefs_m,
+           e.coefs_u, e.periods, e.periods_m, e.periods_u, e.omega, e.omega_m, e.omega_u, e.hyper, e.step_dev, e.losses, e.workspace)
+    if e._active is not None:
+        torch.ops.desmo_b200.build_w_active(e.gates, e.rows, e.coefs, e.periods, e.W, e.step_dev, e.workspace, e._active, *sa)
+        torch.ops.desmo_b200.fused_residual_grad_active(e.U, e.P, e.phi, e.omega, e.W, e.dphi, e.red, e.workspace, e._active,
+                                                        e._active_count, *sa)
+        e.all_reduce()
+        torch.ops.desmo_b200.adamax_update_active(*opt, e._active, *sa)
+        return
     torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, e.step_dev, e.workspace, *sa)
     torch.ops.desmo_b200.fused_residual_grad(e.U, e.P, e.phi, e.omega, e.W, e.dphi, e.red, e.workspace, *sa)
     e.all_reduce()
-    torch.ops.desmo_b200.adamax_update(e.red, e.dphi, e.P, e.phi, e.phi_m, e.phi_u, e.gates, e.gates_m, e.gates_u, e.rows, e.rows_m,
-                                       e.rows_u, e.coefs, e.coefs_m, e.coefs_u, e.periods, e.periods_m, e.periods_u, e.omega, e.omega_m,
-                                       e.omega_u, e.hyper, e.step_dev, e.losses, e.workspace, *sa)
+    torch.ops.desmo_b200.adamax_update(*opt, *sa)
 
 
 def engine_term_norms_via_ops(e, physical: bool = False) -> torch.Tensor:

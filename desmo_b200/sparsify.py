@@ -123,3 +123,37 @@ def pruning_profile(model, order=None, snapshot_norm2: Optional[float] = None) -
     for k in order:
         nonzero.append(nonzero[-1] - int(nz_host[k]))
     return PruningProfile(order, prof["snapshot_residual2"], prof["snapshot_norm2"], rel, nonzero, norms, gates)
+
+
+def _stored_norm2(e) -> float:
+    """||U||_F^2 of the stored snapshot matrix in fp64 (summed over the ranks when point-sharded), a few snapshots at a time."""
+    if e.U is None:
+        raise DesmoError("no snapshot matrix set (call set_snapshot)")
+    tot = torch.zeros((), dtype=torch.float64, device=e.device)
+    for t0 in range(0, e.m, 64):
+        tot += e.U[t0:t0 + 64, :e.n].double().pow(2).sum()
+    if e.n_global != e.n and torch.distributed.is_initialized():
+        torch.distributed.all_reduce(tot, group=e.pg)
+    return float(tot)
+
+
+def sequential_thresholding(trainer, threshold: float, rounds: int, epochs: int,
+                            snapshot_norm2: Optional[float] = None) -> List[Tuple[int, float]]:
+    """Prune, then refit (sequentially thresholded sparse regression) on the engine's resident snapshot.  Each round takes
+    threshold_sweep's mask at ``threshold`` (term norm >= threshold and gate non-zero), intersects it with the current active set,
+    trains on the result (set_active_terms) for ``epochs`` steps of ``trainer`` and records (n_active, ||X - recon|| / ||X||) after
+    the refit.  ``snapshot_norm2`` is ||X||^2; by default the sum of the stored U's squares.  The active set stays in place."""
+    model, e = trainer.model, trainer.engine
+    total = _stored_norm2(e) if snapshot_norm2 is None else float(snapshot_norm2)
+    out = []
+    for _ in range(int(rounds)):
+        if hasattr(model, "sync_parameters"):
+            model.sync_parameters()
+        mask = ((e.term_norms() >= threshold) & (e.gates != 0)).cpu()
+        if e.active_terms is not None:
+            mask &= e.active_terms
+        e.set_active_terms(mask)
+        for _ in range(int(epochs)):
+            trainer.step()
+        out.append((int(mask.sum()), float((e.residual_norm2() / total) ** 0.5)))
+    return out

@@ -66,6 +66,7 @@ class DesmoTrainer:
         self.engine.set_hyper(self.scheduler.lrs, self.beta, self.l1_lambda)
         self.use_cuda_graph = use_cuda_graph
         self._graph: Optional[torch.cuda.CUDAGraph] = None
+        self._graph_active = None  # the engine's active-term table the graph was captured with
         self.device_scheduler, self.log_every = bool(device_scheduler), int(log_every)
         self._plateau_dev: Optional[torch.Tensor] = None
         if self.device_scheduler:
@@ -99,6 +100,8 @@ class DesmoTrainer:
         if not self.use_cuda_graph:
             self.engine.train_step()
             return
+        if self._graph is not None and self._graph_active is not self.engine._active:
+            self._graph = None  # set_active_terms changed the launches: capture again
         if self._graph is None:
             # warm up once outside capture (function attributes, NCCL communicators), then capture the step
             e = self.engine
@@ -117,7 +120,7 @@ class DesmoTrainer:
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
                 e.train_step()
-            self._graph = g
+            self._graph, self._graph_active = g, e._active
             for k, v in snap.items():  # capture does not execute, but keep state exact regardless
                 getattr(e, k).copy_(v)
         self._graph.replay()
@@ -161,6 +164,7 @@ class DesmoTrainer:
                 "scheduler": {"lrs": list(self.scheduler.lrs), "best": self.scheduler.best, "num_bad": self.scheduler.num_bad,
                               "patience": self.scheduler.patience},
                 "epoch": self.epoch, "beta": self.beta, "l1_lambda": self.l1_lambda, "sched_every": self.sched_every,
+                "active_terms": None if e.active_terms is None else e.active_terms.clone(),
                 "shape": {"n": e.n, "m": e.m, "r": e.r, "polyorder": e.polyorder, "nF": e.nF, "n_global": e.n_global}}
 
     def load_state_dict(self, sd: dict) -> None:
@@ -188,6 +192,7 @@ class DesmoTrainer:
         self.sched_every = int(sd.get("sched_every", self.sched_every))
         self.epoch, self.beta, self.l1_lambda = int(sd["epoch"]), float(sd["beta"]), float(sd["l1_lambda"])
         e.set_hyper(self.scheduler.lrs, self.beta, self.l1_lambda)
+        e.set_active_terms(sd.get("active_terms"))  # checkpoints without the key train every term
         if self.device_scheduler:
             self._push_scheduler()
 

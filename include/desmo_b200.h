@@ -133,6 +133,40 @@ int desmo_fused_residual_grad_begin_ex(const desmo_shape* s, const void* U, int3
 int desmo_fused_residual_grad_finish_ex(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
                                         const float* omega, const float* W, float* dphi, float* red, void* workspace, void* stream);
 
+/* Training on an ACTIVE SET of library terms (a pruned model, refitted).  An active set is `count` >= 1 packed term indices in
+ * [0, K), strictly increasing (the K order above, the order desmo_term_norms uses).  A step run with it trains exactly the model in
+ * which every term outside the set is absent -- what a reference loop does when it multiplies the gates by a fixed 0/1 buffer and
+ * leaves the pruned parameters out of the optimizer:
+ *   - an absent term contributes nothing to recon, the MSE, the L1 sum or any gradient (its W row is zero);
+ *   - its gate, its temporal row (DESMOFourier: coefficients and period) and their Adamax state are not written, nor is
+ *     omega[3i+b] when the trig term T + b r + i is absent; desmo_assemble_grads_active reports exactly 0 for all of them;
+ *   - everything else (phi of every mode, the active parameters, the ortho term, the step counter) trains as without a set.
+ * The result does not depend on the path or on the values the frozen entries hold.  The fused kernels (FFMA, tcgen05) keep the full
+ * library and see the zero W rows; the GEMM path builds, multiplies and differentiates the active columns only (Kr = 128
+ * ceil(count / 128) library rows instead of 128 ceil(K / 128)).
+ *
+ * The set lives in a device table made once (host-validated) and passed to every step, so steps stay capturable:
+ *   desmo_active_terms_bytes    table size for `count` terms: 4 (K + count) bytes (host only)
+ *   desmo_active_terms_prepare  checks host_indices[count] (non-empty, in range, strictly increasing -- so no repeats) before
+ *                               anything is written, then copies the table to table_dev (stream-ordered; the host array may be
+ *                               reused when it returns).  Layout: int32 pos[K] (compact column of term k, or -1 when absent),
+ *                               then int32 cols[count] (the indices).
+ * The _active entry points take the table and otherwise the arguments of the calls they extend; active_count must be the count the
+ * table was prepared with (it sizes the GEMM path's launches on the host). */
+int desmo_active_terms_bytes(const desmo_shape* s, int32_t count, size_t* bytes);
+int desmo_active_terms_prepare(const desmo_shape* s, const int32_t* host_indices, int32_t count, void* table_dev, void* stream);
+int desmo_build_w_active(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
+                         int32_t* step_dev, void* workspace, const void* active, void* stream);
+int desmo_fused_residual_grad_active(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                     const float* omega, const float* W, float* dphi, float* red, void* workspace, const void* active,
+                                     int32_t active_count, void* stream);
+int desmo_fused_residual_grad_begin_active(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                           const float* omega, const float* W, float* dphi, float* red, void* workspace,
+                                           const void* active, int32_t active_count, void* stream);
+int desmo_fused_residual_grad_finish_active(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi,
+                                            const float* omega, const float* W, float* dphi, float* red, void* workspace,
+                                            const void* active, int32_t active_count, void* stream);
+
 /* Backward of forward()'s reconstruction for an ARBITRARY upstream gradient (what autograd runs when the reference loop does
  * `recon, _, _ = model(snapshot); loss = criterion(recon, snapshot); total_loss.backward()`, CYL:711,722,766): grad_recon[m][ld]
  * = dL/drecon in the layout of U (pad columns zero).  Same kernels and outputs as desmo_fused_residual_grad with R := (n_global *
@@ -156,6 +190,19 @@ int desmo_assemble_grads(const desmo_shape* s, const float* red, float* dphi, co
                          const float* gates, const float* rows, const float* coefs, const float* periods,
                          const float* hyper, float* d_gates, float* d_rows, float* d_coefs, float* d_periods,
                          float* d_omega, float* losses_out, void* workspace, void* stream);
+
+/* The two calls above on an active set (table of desmo_active_terms_prepare): absent terms' parameters and Adamax state are not
+ * written (update), or their gradients are exactly 0 (assemble); the L1 loss sums the active gates (desmo_build_w_active). */
+int desmo_adamax_update_active(const desmo_shape* s, const float* red, const float* dphi, const float* P, float* phi,
+                               float* phi_m, float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows,
+                               float* rows_m, float* rows_u, float* coefs, float* coefs_m, float* coefs_u, float* periods,
+                               float* periods_m, float* periods_u, float* omega, float* omega_m, float* omega_u,
+                               const float* hyper, const int32_t* step_dev, float* losses_out, void* workspace, const void* active,
+                               void* stream);
+int desmo_assemble_grads_active(const desmo_shape* s, const float* red, float* dphi, const float* P, const float* phi,
+                                const float* gates, const float* rows, const float* coefs, const float* periods,
+                                const float* hyper, float* d_gates, float* d_rows, float* d_coefs, float* d_periods,
+                                float* d_omega, float* losses_out, void* workspace, const void* active, void* stream);
 
 /* Materialise recon (the first element of forward()'s 3-tuple, CYL:576) into out[m][ld] -- evaluation only. */
 int desmo_reconstruct(const desmo_shape* s, const float* P, const float* phi, const float* omega, const float* W,
