@@ -561,6 +561,66 @@ int desmo_pruning_profile_scratch_bytes(const desmo_shape* s, int32_t steps, int
     return DESMO_OK;
 }
 
+// Residual POD: host checks first (shape, u_dtype, pointers, k, scratch against the one-SM size), then the device and the scratch size
+// for its SM count -- all before any launch.
+static int check_residual_pod_args(const desmo_shape* s, Dims* d, const void* U, int32_t u_dtype, const void* scratch, bool ptrs_ok,
+                                   const char* who) {
+    int rc = validate_shape(s, d);
+    if (rc) return rc;
+    if ((rc = check_u_dtype(u_dtype, who))) return rc;
+    if (!U || !scratch || !ptrs_ok) { set_error("%s: null pointer", who); return DESMO_ERR_ARG; }
+    // the planes carved from the scratch are TMA operands: their base must be 16-byte aligned (the carve keeps 1024-byte offsets)
+    if (reinterpret_cast<uintptr_t>(scratch) % 16 != 0) { set_error("%s: scratch must be 16-byte aligned", who); return DESMO_ERR_ARG; }
+    return DESMO_OK;
+}
+
+static int check_residual_scratch(const desmo_shape* s, const Dims& d, size_t scratch_bytes, const char* who) {
+    size_t need = residual_pod_scratch_bytes(s, d.T, d.K, 1);
+    if (scratch_bytes < need) { set_error("%s: scratch too small (%zu < %zu)", who, scratch_bytes, need); return DESMO_ERR_ARG; }
+    int rc = device_ok();
+    if (rc) return rc;
+    int dev = 0, sms = 0;
+    if ((rc = check_cuda(cudaGetDevice(&dev), who))) return rc;
+    if ((rc = check_cuda(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev), who))) return rc;
+    need = residual_pod_scratch_bytes(s, d.T, d.K, sms);
+    if (scratch_bytes < need) { set_error("%s: scratch too small (%zu < %zu for %d SMs)", who, scratch_bytes, need, sms); return DESMO_ERR_ARG; }
+    return DESMO_OK;
+}
+
+int desmo_residual_gram_scratch_bytes(const desmo_shape* s, int32_t sms, size_t* bytes) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if (!bytes) { set_error("desmo_residual_gram_scratch_bytes: null pointer"); return DESMO_ERR_ARG; }
+    if (sms < 1) { set_error("desmo_residual_gram_scratch_bytes: need sms >= 1 (got %d)", sms); return DESMO_ERR_ARG; }
+    *bytes = residual_pod_scratch_bytes(s, d.T, d.K, sms);
+    return DESMO_OK;
+}
+
+int desmo_residual_gram(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                        const float* W, float* C, double* trace, void* scratch, size_t scratch_bytes, void* stream) {
+    Dims d;
+    const char* who = "desmo_residual_gram";
+    int rc = check_residual_pod_args(s, &d, U, u_dtype, scratch, P && phi && omega && W && C && trace, who);
+    if (rc) return rc;
+    if ((rc = check_residual_scratch(s, d, scratch_bytes, who))) return rc;
+    // one route for every library, as desmo_residual_profile: GEMM 1 of the general path, then the Gram GEMM
+    return residual_gram_gemm_path(s, d.T, d.K, d.Kp, U, u_dtype, P, phi, omega, W, C, trace, scratch, (cudaStream_t)stream);
+}
+
+int desmo_residual_modes(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                         const float* W, int32_t k, const float* V, const float* sigma, float* modes, void* scratch, size_t scratch_bytes,
+                         void* stream) {
+    Dims d;
+    const char* who = "desmo_residual_modes";
+    int rc = check_residual_pod_args(s, &d, U, u_dtype, scratch, P && phi && omega && W && V && sigma && modes, who);
+    if (rc) return rc;
+    if (k < 1 || k > s->m) { set_error("%s: need 1 <= k <= m = %d (got k=%d)", who, s->m, k); return DESMO_ERR_ARG; }
+    if (k > DESMO_MAX_R) { set_error("%s: k=%d above %d modes", who, k, DESMO_MAX_R); return DESMO_ERR_UNSUPPORTED; }
+    if ((rc = check_residual_scratch(s, d, scratch_bytes, who))) return rc;
+    return residual_modes_gemm_path(s, d.T, d.K, d.Kp, U, u_dtype, P, phi, omega, W, k, V, sigma, modes, scratch, (cudaStream_t)stream);
+}
+
 int desmo_library_colnorm2(const desmo_shape* s, const float* P, const float* phi, const float* omega, float* out_k, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);

@@ -141,6 +141,13 @@ int pruning_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const 
                               const float* omega, const float* W, int steps, const int32_t* order, double* snap, double* norm,
                               cudaStream_t st);
 size_t pruning_profile_scratch_bytes(const desmo_shape* s, int T, int K, int steps, int sms);
+// residual POD: scratch (residual_pod_scratch_bytes of it) from the caller, arguments validated by desmo_residual_gram / _modes
+size_t residual_pod_scratch_bytes(const desmo_shape* s, int T, int K, int sms);
+int residual_gram_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
+                            const float* omega, const float* W, float* C, double* trace, void* scratch, cudaStream_t st);
+int residual_modes_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
+                             const float* omega, const float* W, int k, const float* V, const float* sigma, float* modes, void* scratch,
+                             cudaStream_t st);
 int colnorm2_gemm_path(const desmo_shape* s, int T, int K, const float* P, const float* phi, const float* omega, float* out_k, cudaStream_t st);
 int launch_update_phi_generic(const UpdateArgs& a, cudaStream_t st);
 int select_path(const desmo_shape* s, const Dims& d);  // DESMO_PATH_FP32 / _TC / _GEMM actually used, or <0 (error set)

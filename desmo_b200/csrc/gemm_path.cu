@@ -40,8 +40,10 @@ constexpr int kChunkPoints = 16384;
 // r^2 and u^2 (per point, per snapshot) instead of being written out (desmo_residual_profile).
 // EPI_PRUNE (_BF16): GEMM 1 transposed (rows = snapshots, columns = points), r = Rec - U as EPI_RESID forms it, then a sequence of
 // library terms peeled off one FFMA at a time, reduced to sum_x r_s^2 per snapshot and step (desmo_pruning_profile).
+// EPI_GRAM: the residual Gram C_R = R^T R of a chunk (rows and columns = snapshots, contraction over the chunk's points), upper tiles
+// only (tn >= tm), per-slice fp64 partials accumulated over the chunks (desmo_residual_gram).
 enum { EPI_RESID = 0, EPI_D = 1, EPI_E = 2, EPI_RECON = 3, EPI_RESID_BF16 = 4, EPI_PROFILE = 5, EPI_PROFILE_BF16 = 6, EPI_PRUNE = 7,
-       EPI_PRUNE_BF16 = 8 };
+       EPI_PRUNE_BF16 = 8, EPI_GRAM = 9 };
 // EPI_PROFILE scratch behind the operand stages (dynamic shared memory), two buffers used by alternate tiles:
 // [4 lane quadrants][2 column halves][4 blocks of 16 columns][32] per-warp column sums, then [2][128] per-point sums of column half 1
 constexpr int kProfSlab = 4 * 2 * 4 * 32 + 2 * 128;
@@ -108,7 +110,8 @@ struct GemmArgs {
     __nv_bfloat16* Rp;         // EPI_RESID: [2][rows_r][mp]
     float* Dacc;               // EPI_D: [K][ld]
     float* Epart;              // EPI_E: [nslice_alloc][Kp][mld]
-    double* loss_part;         // EPI_RESID: [gridDim.x]; EPI_PROFILE: per-CTA snapshot partials [gridDim.x][2][mp], accumulated
+    double* loss_part;         // EPI_RESID: [gridDim.x]; EPI_PROFILE: per-CTA snapshot partials [gridDim.x][2][mp], accumulated;
+                               // EPI_GRAM: per-slice partials of the upper tiles [nslice][tiles_n][128 t2][128 t1], accumulated
     long long n, ld, x0;       // points of this rank, pitch, first point of the chunk
     long long rows_r;          // rows per plane of Rp (chunk points padded to 128)
     int m, mld, mp, K, Kp;
@@ -131,6 +134,17 @@ __host__ __device__ constexpr int pair_b(int q) {
     return NP == 3 ? (q == 0 ? 0 : q == 1 ? 2 : q == 2 ? 1 : q == 3 ? 0 : q == 4 ? 1 : 0) : (q == 1 ? 1 : 0);
 }
 
+// EPI_GRAM's work items: index i of the upper triangle of a T x T tile grid, row by row -> (tm, tn), tn >= tm
+__device__ __forceinline__ int upper_tm(int i, int T) {
+    int a = 0;
+    while (i >= T - a) { i -= T - a; ++a; }
+    return a;
+}
+__device__ __forceinline__ int upper_tn(int i, int T) {
+    const int a = upper_tm(i, T);
+    return i - a * T + a * (a - 1) / 2 + a;
+}
+
 template <bool A_MN, bool B_MN, int NPA, int NPB, int EPI>
 __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs g, const __grid_constant__ CUtensorMap tmA,
                                                                  const __grid_constant__ CUtensorMap tmB) {
@@ -140,6 +154,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
     constexpr bool kResid = EPI == EPI_RESID || EPI == EPI_RESID_BF16;
     constexpr bool kProfile = EPI == EPI_PROFILE || EPI == EPI_PROFILE_BF16;
     constexpr bool kPrune = EPI == EPI_PRUNE || EPI == EPI_PRUNE_BF16;
+    constexpr bool kGram = EPI == EPI_GRAM;
     using UT = typename std::conditional<EPI == EPI_RESID_BF16 || EPI == EPI_PROFILE_BF16 || EPI == EPI_PRUNE_BF16, __nv_bfloat16, float>::type;
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bars[2 * NSTAGE + 4];
@@ -175,7 +190,8 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
             for (int w = blockIdx.x; w < items; w += gridDim.x) {
                 const int slice = w / tiles, rem = w - slice * tiles;
                 // EPI_PRUNE: tm fastest -- with gridDim.x a multiple of tiles_m, every tile of a CTA has the same snapshot rows
-                const int tm = kPrune ? rem % g.tiles_m : rem / g.tiles_n, tn = kPrune ? rem / g.tiles_m : rem - tm * g.tiles_n;
+                const int tm = kGram ? upper_tm(rem, g.mp / BM) : kPrune ? rem % g.tiles_m : rem / g.tiles_n,
+                          tn = kGram ? upper_tn(rem, g.mp / BM) : kPrune ? rem / g.tiles_m : rem - tm * g.tiles_n;
                 const int kb0 = slice * g.kb_per_slice, kb1 = min(kb0 + g.kb_per_slice, g.kblocks);
                 for (int kb = kb0; kb < kb1; ++kb, ++cnt) {
                     const int st = cnt % NSTAGE;
@@ -250,7 +266,8 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
         int job = 0;
         for (int w = blockIdx.x; w < items; w += gridDim.x) {
             const int slice = w / tiles, rem = w - slice * tiles;
-            const int tm = kPrune ? rem % g.tiles_m : rem / g.tiles_n, tn = kPrune ? rem / g.tiles_m : rem - tm * g.tiles_n;
+            const int tm = kGram ? upper_tm(rem, g.mp / BM) : kPrune ? rem % g.tiles_m : rem / g.tiles_n,
+                      tn = kGram ? upper_tn(rem, g.mp / BM) : kPrune ? rem / g.tiles_m : rem - tm * g.tiles_n;
             const int kb0 = slice * g.kb_per_slice, kb1 = min(kb0 + g.kb_per_slice, g.kblocks);
             float sum[64];
 #pragma unroll
@@ -445,6 +462,16 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_planes_kernel(const GemmArgs 
                         double* dst = g.loss_part + ((long long)blockIdx.x * (nout + 1) + o) * BM + tt;
                         *dst += (double)p_s[slot * BM + tt] + (double)p_s[(kPruneSteps + 1 + slot) * BM + tt];
                     }
+                }
+            } else if (kGram) {
+                // rows = snapshots t1 of tile tm, columns = snapshots t2 of tile tn >= tm: this slice's fp64 partial of the tile, accumulated
+                // over the chunks in chunk order.  Stored [t2][t1] so that the 32 lanes of a warp write 32 consecutive doubles; every element
+                // always falls to the same thread (the slice layout is the same for every chunk), so no atomics.
+                double* Co = g.loss_part + ((long long)slice * g.tiles_n + rem) * (BM * BN) + row;
+#pragma unroll
+                for (int j = 0; j < 64; ++j) {
+                    double* dst = Co + (long long)(c * 64 + j) * BM;
+                    *dst = g.first_chunk ? (double)sum[j] : *dst + (double)sum[j];
                 }
             } else {  // EPI_E: rows = snapshots, columns = library terms; this slice's partial of E^T, accumulated over the chunks
                 const int t = tm * BM + row;
@@ -1229,6 +1256,192 @@ int pruning_profile_gemm_path(const desmo_shape* s, int T, int K, int Kp, const 
 size_t pruning_profile_scratch_bytes(const desmo_shape* s, int T, int K, int steps, int sms) {
     PruneLayout L;
     return pruning_profile_layout(s, T, K, steps, sms, &L);
+}
+
+// Residual POD (desmo_residual_gram / desmo_residual_modes): per chunk of points, library planes -> GEMM 1 with the residual epilogue
+// (EPI_RESID / EPI_RESID_BF16, as the training step) -> the residual's two bf16 planes, then
+//   Gram pass:  the Gram GEMM (EPI_GRAM), both operands the R planes read MN-major (snapshots contiguous), upper tiles only, the
+//               contraction split into slices as GEMM 4; then a fixed-order reduce of the slice partials into C_R [m][m] and its trace
+//   modes pass: GEMM 3 (EPI_D) with the planes of V / sigma in place of W: Psi [k][ld] = (R V^T / sigma)^T
+// Points per chunk: the chunk's G and R planes take about kResidChunkBytes.
+constexpr size_t kResidChunkBytes = 64u << 20;
+
+struct ResidLayout {
+    int Kr, mp, T, tiles, nslice;
+    long long rows_c;
+    size_t o_idx, o_deg, o_gp, o_wp, o_rp, o_vp, o_lp, o_part, part_bytes, bytes;
+};
+size_t residual_pod_layout(const desmo_shape* s, int T, int K, int sms, ResidLayout* L) {
+    L->Kr = (K + 63) / 64 * 64;  // GEMM 1 reads (K + 63) / 64 k-blocks, as residual_profile_gemm_path
+    L->mp = (s->m + 127) / 128 * 128;
+    L->T = L->mp / 128;
+    L->tiles = L->T * (L->T + 1) / 2;
+    const size_t per_point = (size_t)3 * L->Kr * 2 + (size_t)2 * L->mp * 2;
+    long long rc = (long long)(kResidChunkBytes / per_point) / 128 * 128;
+    if (rc < 128) rc = 128;
+    if (rc > s->ld) rc = s->ld;
+    L->rows_c = rc;
+    // slices of the contraction: enough work items to fill the SMs, fixed for every chunk (at most one slice per k-block of the first)
+    int ns = sms / L->tiles;
+    if (ns < 1) ns = 1;
+    if (ns > kSliceMax) ns = kSliceMax;
+    if (ns > (int)(rc / 64)) ns = (int)(rc / 64);
+    L->nslice = ns;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off = align_up_g(off + bytes, 1024); return o; };
+    L->o_idx = take((size_t)T * 8);
+    L->o_deg = take((size_t)T);
+    L->o_gp = take((size_t)3 * L->Kr * rc * 2);
+    L->o_wp = take((size_t)3 * L->Kr * L->mp * 2);
+    L->o_rp = take((size_t)2 * rc * L->mp * 2);
+    L->o_vp = take((size_t)2 * 128 * L->mp * 2);
+    L->o_lp = take((size_t)(sms > 0 ? sms : 1) * sizeof(double));
+    L->part_bytes = (size_t)ns * L->tiles * gp::BM * gp::BN * sizeof(double);
+    L->o_part = take(L->part_bytes);
+    L->bytes = off;
+    return off;
+}
+
+size_t residual_pod_scratch_bytes(const desmo_shape* s, int T, int K, int sms) {
+    ResidLayout L;
+    return residual_pod_layout(s, T, K, sms, &L);
+}
+
+// C[i][j] = sum over the slices, in order, of the partial of the upper element (min(i, j), max(i, j)): C is exactly symmetric
+__global__ void __launch_bounds__(256) resid_gram_reduce_kernel(const double* __restrict__ part, int nslice, int tiles, int T, int m,
+                                                                float* __restrict__ C) {
+    const long long e = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (e >= (long long)m * m) return;
+    const int i = (int)(e / m), j = (int)(e - (long long)i * m);
+    const int a = i < j ? i : j, b = i < j ? j : i;
+    const int tm = a / gp::BM, tn = b / gp::BN;
+    const long long tile = (long long)tm * T - (long long)tm * (tm - 1) / 2 + (tn - tm);
+    const long long off = tile * (gp::BM * gp::BN) + (long long)(b % gp::BN) * gp::BM + (a % gp::BM);
+    const long long stride = (long long)tiles * gp::BM * gp::BN;
+    double s = 0.0;
+    for (int q = 0; q < nslice; ++q) s += part[q * stride + off];
+    C[e] = (float)s;
+}
+
+// trace = sum_t C_R[t][t] in fp64 (the slice sums of the diagonal, before the fp32 rounding), one block, fixed order
+__global__ void __launch_bounds__(256) resid_gram_trace_kernel(const double* __restrict__ part, int nslice, int tiles, int T, int m,
+                                                               double* __restrict__ trace) {
+    __shared__ double red[256];
+    const long long stride = (long long)tiles * gp::BM * gp::BN;
+    double acc = 0.0;
+    for (int t = threadIdx.x; t < m; t += 256) {
+        const int tm = t / gp::BM;
+        const long long tile = (long long)tm * T - (long long)tm * (tm - 1) / 2;
+        const long long off = tile * (gp::BM * gp::BN) + (long long)(t % gp::BM) * (gp::BM + 1);
+        double s = 0.0;
+        for (int q = 0; q < nslice; ++q) s += part[q * stride + off];
+        acc += s;
+    }
+    red[threadIdx.x] = acc;
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *trace = red[0];
+}
+
+// planes of V / sigma: Vp [2][128][mp], row i = V[i][t] / sigma[i] for i < k, t < m (a zero row when sigma_i = 0), other entries 0
+__global__ void __launch_bounds__(256) mode_planes_kernel(const float* __restrict__ V, const float* __restrict__ sigma, int k, int m, int mp,
+                                                          __nv_bfloat16* __restrict__ Vp) {
+    const int i = blockIdx.x;
+    const float sg = i < k ? sigma[i] : 0.0f;
+    for (int t = threadIdx.x; t < mp; t += 256) {
+        const float w = (i < k && t < m && sg > 0.0f) ? V[(long long)i * m + t] / sg : 0.0f;
+        const __nv_bfloat16 b1 = __float2bfloat16_rn(w);
+        const __nv_bfloat16 b2 = __float2bfloat16_rn(w - __bfloat162float(b1));
+        Vp[(size_t)i * mp + t] = b1;
+        Vp[(size_t)(128 + i) * mp + t] = b2;
+    }
+}
+
+// Shared by both passes: library planes + GEMM 1 (the residual planes) per chunk, then the pass's own GEMM.  V == nullptr: Gram pass.
+static int residual_pod_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
+                                  const float* omega, const float* W, float* Cout, double* trace, int k, const float* V, const float* sigma,
+                                  float* modes, void* scratch_v, cudaStream_t st) {
+    using namespace gp;
+    int dev = 0, sms = 0;
+    DESMO_CUDA(cudaGetDevice(&dev));
+    DESMO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    ResidLayout L;
+    residual_pod_layout(s, T, K, sms, &L);
+    uint8_t* scratch = static_cast<uint8_t*>(scratch_v);
+    __nv_bfloat16* Gp = reinterpret_cast<__nv_bfloat16*>(scratch + L.o_gp);
+    __nv_bfloat16* Wp = reinterpret_cast<__nv_bfloat16*>(scratch + L.o_wp);
+    __nv_bfloat16* Rp = reinterpret_cast<__nv_bfloat16*>(scratch + L.o_rp);
+    __nv_bfloat16* Vp = reinterpret_cast<__nv_bfloat16*>(scratch + L.o_vp);
+    double* lp = reinterpret_cast<double*>(scratch + L.o_lp);
+    double* part = reinterpret_cast<double*>(scratch + L.o_part);
+    TermTable tab{scratch + L.o_idx, scratch + L.o_deg};
+    const int Kr = L.Kr, mp = L.mp;
+    const long long rows_c = L.rows_c;
+    const bool gram = V == nullptr;
+    term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab, nullptr, K);
+    w_planes_kernel<<<Kr, 256, 0, st>>>(W, nullptr, K, Kr, s->m, s->mld, mp, Wp);
+    if (!gram) mode_planes_kernel<<<128, 256, 0, st>>>(V, sigma, k, s->m, mp, Vp);
+    DESMO_CUDA(cudaGetLastError());
+    CUtensorMap tmG_mn, tmW_mn, tmR_mn, tmR_k, tmV_k;
+    int rc;
+    if ((rc = make_map(&tmG_mn, Gp, rows_c, 3LL * Kr, 64)) || (rc = make_map(&tmW_mn, Wp, mp, 3LL * Kr, 64))) return rc;
+    // R planes [2*rows_c rows][mp]: MN-major A and B of the Gram GEMM (as GEMM 4's A), K-major A of GEMM 3
+    if ((rc = make_map(&tmR_mn, Rp, mp, 2LL * rows_c, 64)) || (rc = make_map(&tmR_k, Rp, mp, 2LL * rows_c, 128))) return rc;
+    if ((rc = make_map(&tmV_k, Vp, mp, 2LL * 128, 128))) return rc;
+    bool first = true;
+    for (long long x0 = 0; x0 < s->ld; x0 += rows_c, first = false) {
+        const long long pts = (s->ld - x0 < rows_c) ? s->ld - x0 : rows_c;  // multiple of 128
+        library_planes_kernel<<<dim3((unsigned)((rows_c + 255) / 256), 64u), 256, 0, st>>>(P, phi, omega, tab, nullptr, s->r, T, K, Kr, s->n,
+                                                                                          s->ld, x0, rows_c, Gp);
+        DESMO_CUDA(cudaGetLastError());
+        GemmArgs g{};
+        g.U = U; g.Rp = Rp; g.loss_part = lp;
+        g.n = s->n; g.ld = s->ld; g.x0 = x0; g.rows_r = rows_c; g.m = s->m; g.mld = s->mld; g.mp = mp; g.K = K; g.Kp = Kp;
+        g.first_chunk = 1;
+        // GEMM 1, as the training step's: Rec[p x t] = G W, epilogue r = Rec - U -> two bf16 planes of r
+        g.tiles_m = (int)(pts / 128); g.tiles_n = mp / 128; g.nslice = 1; g.kblocks = (K + 63) / 64; g.kb_per_slice = g.kblocks; g.kgroup = 4;
+        g.a_rows = Kr; g.b_rows = Kr;
+        rc = u_dtype == DESMO_DTYPE_BF16 ? launch_gemm<true, true, 3, 3, EPI_RESID_BF16>(g, tmG_mn, tmW_mn, sms, st)
+                                         : launch_gemm<true, true, 3, 3, EPI_RESID>(g, tmG_mn, tmW_mn, sms, st);
+        if (rc) return rc;
+        if (gram) {
+            // C_R tiles (tm <= tn) [t1 x t2] = R^T R; A = B = R (MN-major: t contiguous), contraction over the chunk's points in
+            // L.nslice slices; chains of 4 k-blocks (48 MMAs) per TMEM accumulator, summed in fp32 RN, then fp64 across the chunks
+            g.loss_part = part; g.first_chunk = first ? 1 : 0;
+            g.tiles_m = 1; g.tiles_n = L.tiles; g.kblocks = (int)(pts / 64); g.nslice = L.nslice;
+            g.kb_per_slice = (g.kblocks + g.nslice - 1) / g.nslice; g.kgroup = 4;
+            g.a_rows = (int)rows_c; g.b_rows = (int)rows_c;
+            rc = launch_gemm<true, true, 2, 2, EPI_GRAM>(g, tmR_mn, tmR_mn, sms, st);
+        } else {
+            // GEMM 3, as the training step's: Psi^T[p x mode] = R (V / sigma)^T; A = R (K-major), B = V planes (K-major)
+            g.Dacc = modes; g.K = k; g.n_lib16 = (k + 15) / 16 * 16;
+            g.tiles_m = (int)(pts / 128); g.tiles_n = 1; g.nslice = 1; g.kblocks = mp / 64; g.kb_per_slice = g.kblocks; g.kgroup = 32;
+            g.a_rows = (int)rows_c; g.b_rows = 128;
+            rc = launch_gemm<false, false, 2, 2, EPI_D>(g, tmR_k, tmV_k, sms, st);
+        }
+        if (rc) return rc;
+    }
+    if (gram) {
+        const long long total = (long long)s->m * s->m;
+        resid_gram_reduce_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(part, L.nslice, L.tiles, L.T, s->m, Cout);
+        resid_gram_trace_kernel<<<1, 256, 0, st>>>(part, L.nslice, L.tiles, L.T, s->m, trace);
+        DESMO_CUDA(cudaGetLastError());
+    }
+    return DESMO_OK;
+}
+
+int residual_gram_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
+                            const float* omega, const float* W, float* C, double* trace, void* scratch, cudaStream_t st) {
+    return residual_pod_gemm_path(s, T, K, Kp, U, u_dtype, P, phi, omega, W, C, trace, 0, nullptr, nullptr, nullptr, scratch, st);
+}
+
+int residual_modes_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
+                             const float* omega, const float* W, int k, const float* V, const float* sigma, float* modes, void* scratch,
+                             cudaStream_t st) {
+    return residual_pod_gemm_path(s, T, K, Kp, U, u_dtype, P, phi, omega, W, nullptr, nullptr, k, V, sigma, modes, scratch, st);
 }
 
 int colnorm2_gemm_path(const desmo_shape* s, int T, int K, const float* P, const float* phi, const float* omega, float* out_k, cudaStream_t st) {

@@ -636,6 +636,69 @@ class DesmoEngine:
             self.all_reduce()
         return float(self.red[self.Kp * self.mld].item())
 
+    def _residual_pod_scratch(self) -> torch.Tensor:
+        """Scratch of desmo_residual_gram / desmo_residual_modes for this device's SM count (bounded by the point chunk and m, not n)."""
+        sms = torch.cuda.get_device_properties(self.device).multi_processor_count
+        nbytes = C.c_size_t(0)
+        check(self.lib.desmo_residual_gram_scratch_bytes(C.byref(self.shape), sms, C.byref(nbytes)), "desmo_residual_gram_scratch_bytes")
+        return torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+
+    def residual_pod(self, k: int = 8) -> dict:
+        """POD of the residual R = recon - U (the training step's residual for the current parameters; U as stored): what shape the
+        misfit has.  R = sum_i sigma_i v_i psi_i^T from the Gram C_R = R R^T (m x m, desmo_residual_gram: tcgen05 tiles over the GEMM
+        path's residual planes, R itself is never formed), all-reduced when point-sharded, the dense fp64 eigensolver (desmo_pod_eigh)
+        and a second pass for psi_i = R^T v_i / sigma_i (desmo_residual_modes).  1 <= k <= min(64, m).  Returns
+
+          singular_values   (m,) fp64 host   all m singular values of R, descending (lambda_i <= 2^-23 trace(C_R) gives 0)
+          sigma             (k,) fp32        the leading k
+          temporal_modes    (k, m) fp32      v_i, unit norm, largest-|.| entry positive
+          spatial_modes     (k, n) fp32      psi_i at this rank's points, orthonormal over all ranks (a zero row when sigma_i = 0)
+          residual_norm2    float            trace(C_R) = ||R||_F^2 (all ranks)
+          energy, cumulative_energy (k,) fp64 host   sigma_i^2 / ||R||_F^2 and its running sum
+          gram              (m, m) fp32      C_R
+
+        A zero residual returns zeros without calling the eigensolver.  Nothing the model owns is written (parameters, Adamax state, P,
+        the pod_* attributes, step_dev, red, dphi, losses, U); W is rebuilt from the parameters as residual_profile() does.  Raises
+        DesmoError when the eigensolver reports failure.  Bit-identical from call to call."""
+        k = int(k)
+        if not 1 <= k <= min(_lib.MAX_R, self.m):
+            raise _lib.DesmoError(f"residual_pod: need 1 <= k <= min({_lib.MAX_R}, m = {self.m}), got k={k}")
+        ud = self._u_dtype()
+        f32 = dict(dtype=torch.float32, device=self.device)
+        scratch = self._residual_pod_scratch()
+        Cm = torch.empty(self.m, self.m, **f32)
+        tr = torch.empty(1, dtype=torch.float64, device=self.device)
+        V, sigma = torch.zeros(k, self.m, **f32), torch.zeros(k, **f32)
+        S = torch.zeros(self.m, dtype=torch.float64, device=self.device)
+        modes = torch.zeros(k, self.ld, **f32)
+        model_args = (_ptr(self.U), ud, _ptr(self.P), _ptr(self.phi), _ptr(self.omega), _ptr(self.W))
+        with torch.cuda.device(self.device):
+            self.build_w(False)
+            check(self.lib.desmo_residual_gram(C.byref(self.shape), *model_args, _ptr(Cm), _ptr(tr), _ptr(scratch), scratch.numel(),
+                                               self._stream()), "desmo_residual_gram")
+            if self.n_global != self.n and torch.distributed.is_initialized():
+                torch.distributed.all_reduce(Cm, group=self.pg)
+                torch.distributed.all_reduce(tr, group=self.pg)
+            trace = float(tr.item())
+            out = {"singular_values": S.cpu(), "sigma": sigma, "temporal_modes": V, "spatial_modes": modes[:, :self.n],
+                   "residual_norm2": trace, "energy": torch.zeros(k, dtype=torch.float64),
+                   "cumulative_energy": torch.zeros(k, dtype=torch.float64), "gram": Cm}
+            if not trace > 0.0:  # a perfect fit: nothing to decompose
+                return out
+            nbytes = C.c_size_t(0)
+            check(self.lib.desmo_pod_eigh_workspace_bytes(self.m, k, C.byref(nbytes)), "desmo_pod_eigh_workspace_bytes")
+            ws = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+            check(self.lib.desmo_pod_eigh(self.m, k, _ptr(Cm), _ptr(S), _ptr(V), _ptr(sigma), _ptr(ws), ws.numel(), self._stream()),
+                  "desmo_pod_eigh")
+            status, residual = int(ws[:4].view(torch.int32).item()), float(ws[8:16].view(torch.float64).item())
+            if status != 0 or not residual <= 2.0 ** -27:
+                raise _lib.DesmoError(f"residual_pod: desmo_pod_eigh failed (status {status}, residual {residual:.2e} lambda_1)")
+            check(self.lib.desmo_residual_modes(C.byref(self.shape), *model_args, k, _ptr(V), _ptr(sigma), _ptr(modes), _ptr(scratch),
+                                                scratch.numel(), self._stream()), "desmo_residual_modes")
+        energy = (sigma.double() ** 2 / trace).cpu()
+        out.update(singular_values=S.cpu(), energy=energy, cumulative_energy=torch.cumsum(energy, 0))
+        return out
+
     # ------------------------------------------------------------------ POD (method of snapshots)
     def preprocess_snapshot(self, raw: torch.Tensor, d_in: int = 1, d_use: Optional[int] = None, magnitude: bool = True,
                             subtract_mean: bool = True, scale_sqrt_m: bool = False, t_stride: int = 1) -> torch.Tensor:

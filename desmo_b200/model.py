@@ -226,6 +226,11 @@ class _DesmoBase(nn.Module):
         self.sync_parameters()
         return self.engine.residual_profile_at(snapshots, index=index, times=times)
 
+    def residual_pod(self, k: int = 8) -> dict:
+        """POD of the residual recon - U of the current parameters: its singular spectrum and k leading modes (DesmoEngine.residual_pod)."""
+        self.sync_parameters()
+        return self.engine.residual_pod(k)
+
     # ---- training a pruned model (DesmoEngine.set_active_terms) ----------------------------------------------------------------
     def set_active_terms(self, mask) -> None:
         """Train on the terms of the bool (K,) ``mask`` only (None: every term); see DesmoEngine.set_active_terms.  The set applies to

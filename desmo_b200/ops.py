@@ -2,7 +2,8 @@
 
   build_w, build_w_at, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, pruning_profile, library_colnorm2, term_norms,
   pod_gram, pod_eig, pod_eigh, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce,
-  active_terms_prepare, build_w_active, fused_residual_grad_active, adamax_update_active, assemble_grads_active
+  active_terms_prepare, build_w_active, fused_residual_grad_active, adamax_update_active, assemble_grads_active,
+  residual_gram, residual_modes
 
 They take the packed device tensors of a DesmoEngine (layout: include/desmo_b200.h) plus the shape integers and launch the
 sm_100a kernels on the current stream.  CUDA only: no CPU implementation is registered and every op checks its tensors, so a call
@@ -170,6 +171,44 @@ def pruning_profile(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, omega: 
     with torch.cuda.device(U.device):
         check(_lib.load().desmo_pruning_profile(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), S, _p(order) if S else None,
                                                 _p(snap), _p(norm), _stream(U)), "desmo_pruning_profile")
+
+
+def _scratch_ok(scratch: torch.Tensor, who: str) -> None:
+    if scratch.dtype != torch.uint8 or not scratch.is_contiguous():
+        raise _lib.DesmoError(f"{who}: scratch must be a contiguous uint8 tensor (desmo_residual_gram_scratch_bytes)")
+
+
+@torch.library.custom_op("desmo_b200::residual_gram", mutates_args=("C_out", "trace", "scratch"))
+def residual_gram(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, omega: torch.Tensor, W: torch.Tensor, C_out: torch.Tensor,
+                  trace: torch.Tensor, scratch: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """C_out (fp32 [m, m]) = C_R = R R^T of r = G W - U, trace (fp64 [1]) its trace (desmo_residual_gram)."""
+    _require_cuda(U, P, phi, omega, W, C_out, trace, scratch)
+    ud = _lib.u_dtype_code(U.dtype)
+    if C_out.dtype != torch.float32 or trace.dtype != torch.float64 or C_out.numel() < m * m or not C_out.is_contiguous():
+        raise _lib.DesmoError(f"residual_gram: need contiguous float32 C_out [{m}, {m}] and float64 trace [1]")
+    _scratch_ok(scratch, "residual_gram")
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(U.device):
+        check(_lib.load().desmo_residual_gram(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), _p(C_out), _p(trace), _p(scratch),
+                                              scratch.numel(), _stream(U)), "desmo_residual_gram")
+
+
+@torch.library.custom_op("desmo_b200::residual_modes", mutates_args=("modes", "scratch"))
+def residual_modes(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, omega: torch.Tensor, W: torch.Tensor, V: torch.Tensor,
+                   sigma: torch.Tensor, modes: torch.Tensor, scratch: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int,
+                   nF: int, path: int) -> None:
+    """modes (fp32 [k, ld]) row i = R^T V[i] / sigma[i] (zero when sigma_i = 0), k = V.shape[0] (desmo_residual_modes)."""
+    _require_cuda(U, P, phi, omega, W, V, sigma, modes, scratch)
+    ud = _lib.u_dtype_code(U.dtype)
+    k = V.shape[0]
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    if V.dtype != torch.float32 or sigma.dtype != torch.float32 or modes.dtype != torch.float32 or V.numel() != k * m or \
+            sigma.numel() < k or modes.numel() < k * s.ld or not (V.is_contiguous() and modes.is_contiguous()):
+        raise _lib.DesmoError(f"residual_modes: need contiguous float32 V [k, {m}], sigma [k] and modes [k, {s.ld}]")
+    _scratch_ok(scratch, "residual_modes")
+    with torch.cuda.device(U.device):
+        check(_lib.load().desmo_residual_modes(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), k, _p(V), _p(sigma), _p(modes),
+                                               _p(scratch), scratch.numel(), _stream(U)), "desmo_residual_modes")
 
 
 @torch.library.custom_op("desmo_b200::library_colnorm2", mutates_args=("out",))
@@ -466,3 +505,31 @@ def engine_pod_analysis_via_ops(e) -> torch.Tensor:
         raise _lib.DesmoError(f"desmo_pod_eigh failed (status {status}, residual {residual:.2e} lambda_1); P is unchanged")
     torch.ops.desmo_b200.pod_project(e.U, V, sigma, e.P, *sa)
     return sigma
+
+
+def engine_residual_pod_via_ops(e, k: int = 8) -> dict:
+    """DesmoEngine.residual_pod(k) through the registered build_w / residual_gram / pod_eigh / residual_modes ops (the optimizer's step
+    counter is not moved)."""
+    sa = _shape_args(e)
+    f32 = dict(dtype=torch.float32, device=e.device)
+    scratch = e._residual_pod_scratch()
+    Cm, tr = torch.empty(e.m, e.m, **f32), torch.empty(1, dtype=torch.float64, device=e.device)
+    V, sigma, modes = torch.zeros(k, e.m, **f32), torch.zeros(k, **f32), torch.zeros(k, e.ld, **f32)
+    S = torch.zeros(e.m, dtype=torch.float64, device=e.device)
+    scratch_step = e.step_dev.clone()
+    torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, scratch_step, e.workspace, *sa)
+    torch.ops.desmo_b200.residual_gram(e.U, e.P, e.phi, e.omega, e.W, Cm, tr, scratch, *sa)
+    if e.n_global != e.n and torch.distributed.is_initialized():
+        torch.distributed.all_reduce(Cm, group=e.pg)
+        torch.distributed.all_reduce(tr, group=e.pg)
+    if float(tr.item()) > 0.0:
+        nbytes = C.c_size_t(0)
+        check(_lib.load().desmo_pod_eigh_workspace_bytes(e.m, k, C.byref(nbytes)), "desmo_pod_eigh_workspace_bytes")
+        ws = torch.empty(nbytes.value, dtype=torch.uint8, device=e.device)
+        torch.ops.desmo_b200.pod_eigh(Cm, S, V, sigma, ws, e.m, k)
+        status, residual = int(ws[:4].view(torch.int32).item()), float(ws[8:16].view(torch.float64).item())
+        if status != 0 or not residual <= 2.0 ** -27:
+            raise _lib.DesmoError(f"residual_pod: desmo_pod_eigh failed (status {status}, residual {residual:.2e} lambda_1)")
+        torch.ops.desmo_b200.residual_modes(e.U, e.P, e.phi, e.omega, e.W, V, sigma, modes, scratch, *sa)
+    return {"singular_values": S.cpu(), "sigma": sigma, "temporal_modes": V, "spatial_modes": modes[:, :e.n], "residual_norm2": float(tr.item()),
+            "gram": Cm}

@@ -242,6 +242,33 @@ int desmo_pruning_profile(const desmo_shape* s, const void* U, int32_t u_dtype, 
                           const float* W, int32_t steps, const int32_t* order, double* snap, double* norm, void* stream);
 int desmo_pruning_profile_scratch_bytes(const desmo_shape* s, int32_t steps, int32_t sms, size_t* bytes);
 
+/* Residual POD: the singular spectrum and leading modes of R = G(Phi) W - U (the (m, n) residual of the current parameters, U as
+ * stored, u_dtype F32 or BF16), without forming R.  R = sum_i sigma_i v_i psi_i^T, v_i over the m snapshots, psi_i over the points.
+ *   gram   C[m][m] fp32 = C_R, C_R[s][t] = sum_x r(x, s) r(x, t) (local partial -- all-reduce it across ranks); trace[1] fp64 = its trace
+ *          before the fp32 rounding (= ||R||_F^2 up to the split error below; local partial)
+ *   (eigensolve: desmo_pod_eigh(m, k, C, S, V, sigma, ...) on the all-reduced C: C_R v_i = sigma_i^2 v_i)
+ *   modes  modes[k][ld] fp32, row i = psi_i = R^T v_i / sigma_i at this rank's points (pad columns 0; a zero row when sigma_i = 0)
+ *          from V[k][m] and sigma[k] as desmo_pod_eigh writes them; 1 <= k <= min(DESMO_MAX_R, m)
+ * Route, per chunk of points, for every library: the library planes and GEMM 1 with the training step's residual epilogue (r exactly
+ * as desmo_residual_profile forms it, split into two bf16 planes r = b1 + b2 + e), then the tcgen05 Gram GEMM (upper tiles,
+ * b1 b1 + b1 b2 + b2 b1; fp32 chains of 48 MMAs, fp64 across slices and chunks, fixed order, no float atomics: bit-identical from
+ * call to call) or GEMM 3 with the planes of V / sigma.  Entrywise, |C - C_exact| <= 2^-14 sum_x |r(x, s)| |r(x, t)| against the exact
+ * sums of the fp32 r: 3 * 2^-16 from the split residual e and the omitted b2 b2, the rest from the tensor core's truncating adds (48 per
+ * chain), the fp32 sums of the chains and the final rounding.
+ * Both calls are stream-ordered, allocate nothing, write only their outputs and the caller's scratch, and check every argument
+ * (k, pointers, u_dtype, scratch size and 16-byte alignment) before any launch.  Scratch bytes, with Kr = 64 ceil(K / 64), mp = 128 ceil(m / 128),
+ * T = mp / 128, tiles = T (T + 1) / 2, rows_c = clamp(128 floor(2^26 / (6 Kr + 4 mp) / 128), 128, ld) the point chunk,
+ * ns = clamp(floor(sms / tiles), 1, min(32, rows_c / 64)) the slices and A(v) = v rounded up to 1024 bytes:
+ *   A(8T') + A(T') + A(6 Kr rows_c) + A(6 Kr mp) + A(4 rows_c mp) + A(512 mp) + A(8 sms) + A(131072 ns tiles)     (T' = polynomial terms)
+ * bounded by the chunk and by m, never by n: about 90 MB at m = 1000 on 148 SMs.  desmo_residual_gram_scratch_bytes returns it
+ * (host only); both calls take the same scratch. */
+int desmo_residual_gram_scratch_bytes(const desmo_shape* s, int32_t sms, size_t* bytes);
+int desmo_residual_gram(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                        const float* W, float* C, double* trace, void* scratch, size_t scratch_bytes, void* stream);
+int desmo_residual_modes(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                         const float* W, int32_t k, const float* V, const float* sigma, float* modes, void* scratch, size_t scratch_bytes,
+                         void* stream);
+
 /* Post-hoc sparsification inputs: squared column norms of G (K floats, local partial -- all-reduce them across ranks).
  * P == NULL evaluates the library on the raw phi_list, which is what the reference's sweep passes to poly_norm /
  * nonlinear_norm (CYL:1192-1194; the functions, CYL:624-692, never multiply by POD_modes); P != NULL gives the columns of
