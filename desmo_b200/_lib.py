@@ -66,6 +66,9 @@ SIGNATURES: Dict[str, tuple] = {
     "desmo_residual_gram_scratch_bytes": (C.c_int, [_SP, _i32, C.POINTER(C.c_size_t)]),
     "desmo_residual_gram": (C.c_int, [_SP, _vp, _i32] + [_vp] * 7 + [C.c_size_t, _vp]),
     "desmo_residual_modes": (C.c_int, [_SP, _vp, _i32] + [_vp] * 4 + [_i32] + [_vp] * 4 + [C.c_size_t, _vp]),
+    "desmo_elimination_scratch_bytes": (C.c_int, [_SP, _i32, C.POINTER(C.c_size_t)]),
+    "desmo_elimination_pass": (C.c_int, [_SP, _vp, _i32] + [_vp] * 8 + [C.c_size_t, _vp]),
+    "desmo_elimination_greedy": (C.c_int, [_SP] + [_vp] * 4 + [_i32] + [_vp] * 3 + [C.c_size_t, _vp]),
     "desmo_term_norms": (C.c_int, [_SP, _vp, _vp, _vp, _i32, _vp, _vp]),
     "desmo_selftest_tables": (C.c_int, []),
     "desmo_selftest_chain_sweep": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float)]),

@@ -10,7 +10,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdesmo_b200.so")
-SOURCES = ["capi.cu", "library.cu", "fused_fp32.cu", "fused_tc.cu", "gemm_path.cu", "gram_tc.cu", "preprocess.cu", "update.cu", "eval.cu", "pod.cu", "eigh.cu", "host_api.cu", "peer.cu"]
+SOURCES = ["capi.cu", "library.cu", "fused_fp32.cu", "fused_tc.cu", "gemm_path.cu", "gram_tc.cu", "preprocess.cu", "update.cu", "eval.cu", "pod.cu", "eigh.cu", "host_api.cu", "peer.cu",
+           "elimination.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr", "-Xptxas", "-v"]
 

@@ -621,6 +621,51 @@ int desmo_residual_modes(const desmo_shape* s, const void* U, int32_t u_dtype, c
     return residual_modes_gemm_path(s, d.T, d.K, d.Kp, U, u_dtype, P, phi, omega, W, k, V, sigma, modes, scratch, (cudaStream_t)stream);
 }
 
+// Backward elimination: host checks first (shape, u_dtype, pointers, steps, scratch alignment and its size against the one-SM formula),
+// then the device and the scratch size for its SM count -- all before any launch.
+int desmo_elimination_scratch_bytes(const desmo_shape* s, int32_t sms, size_t* bytes) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if (!bytes) { set_error("desmo_elimination_scratch_bytes: null pointer"); return DESMO_ERR_ARG; }
+    if (sms < 1) { set_error("desmo_elimination_scratch_bytes: need sms >= 1 (got %d)", sms); return DESMO_ERR_ARG; }
+    *bytes = elimination_scratch_bytes(s, d.T, d.K, sms);
+    return DESMO_OK;
+}
+
+int desmo_elimination_pass(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                           const float* W, double* A, double* F, double* r2, void* scratch, size_t scratch_bytes, void* stream) {
+    Dims d;
+    const char* who = "desmo_elimination_pass";
+    int rc = check_residual_pod_args(s, &d, U, u_dtype, scratch, P && phi && omega && W && A && F && r2, who);
+    if (rc) return rc;
+    size_t need = elimination_scratch_bytes(s, d.T, d.K, 1);
+    if (scratch_bytes < need) { set_error("%s: scratch too small (%zu < %zu)", who, scratch_bytes, need); return DESMO_ERR_ARG; }
+    if ((rc = device_ok())) return rc;
+    int dev = 0, sms = 0;
+    if ((rc = check_cuda(cudaGetDevice(&dev), who))) return rc;
+    if ((rc = check_cuda(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev), who))) return rc;
+    need = elimination_scratch_bytes(s, d.T, d.K, sms);
+    if (scratch_bytes < need) { set_error("%s: scratch too small (%zu < %zu for %d SMs)", who, scratch_bytes, need, sms); return DESMO_ERR_ARG; }
+    // one route for every library, as desmo_residual_profile: GEMM 1 of the general path, then GEMM 4 and the library Gram GEMM
+    return elimination_pass_gemm_path(s, d.T, d.K, U, u_dtype, P, phi, omega, W, A, F, r2, scratch, (cudaStream_t)stream);
+}
+
+int desmo_elimination_greedy(const desmo_shape* s, const double* A, double* F, const double* r2, const float* W, int32_t steps,
+                             int32_t* order, double* predicted, void* scratch, size_t scratch_bytes, void* stream) {
+    Dims d;
+    const char* who = "desmo_elimination_greedy";
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if (!A || !F || !r2 || !W || !predicted || !scratch || (steps > 0 && !order)) { set_error("%s: null pointer", who); return DESMO_ERR_ARG; }
+    if (steps < 0 || steps > d.K) { set_error("%s: steps = %d outside 0 .. K = %d", who, steps, d.K); return DESMO_ERR_ARG; }
+    if (reinterpret_cast<uintptr_t>(scratch) % 16 != 0) { set_error("%s: scratch must be 16-byte aligned", who); return DESMO_ERR_ARG; }
+    const size_t need = elimination_greedy_scratch_bytes(d.K);
+    if (scratch_bytes < need) { set_error("%s: scratch too small (%zu < %zu)", who, scratch_bytes, need); return DESMO_ERR_ARG; }
+    if ((rc = device_ok())) return rc;
+    return elimination_greedy(d.K, s->m, s->mld, A, F, r2, W, steps, order, predicted, scratch, (cudaStream_t)stream);
+}
+
 int desmo_library_colnorm2(const desmo_shape* s, const float* P, const float* phi, const float* omega, float* out_k, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);

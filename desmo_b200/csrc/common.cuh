@@ -148,6 +148,14 @@ int residual_gram_gemm_path(const desmo_shape* s, int T, int K, int Kp, const vo
 int residual_modes_gemm_path(const desmo_shape* s, int T, int K, int Kp, const void* U, int u_dtype, const float* P, const float* phi,
                              const float* omega, const float* W, int k, const float* V, const float* sigma, float* modes, void* scratch,
                              cudaStream_t st);
+// backward elimination: scratch (elimination_scratch_bytes of it) from the caller, arguments validated by desmo_elimination_pass /
+// desmo_elimination_greedy; the greedy uses the first elimination_greedy_scratch_bytes(K) of the same scratch (elimination.cu)
+size_t elimination_scratch_bytes(const desmo_shape* s, int T, int K, int sms);
+int elimination_pass_gemm_path(const desmo_shape* s, int T, int K, const void* U, int u_dtype, const float* P, const float* phi,
+                               const float* omega, const float* W, double* A, double* F, double* r2, void* scratch, cudaStream_t st);
+size_t elimination_greedy_scratch_bytes(int K);
+int elimination_greedy(int K, int m, int mld, const double* A, double* F, const double* r2, const float* W, int steps, int32_t* order,
+                       double* predicted, void* scratch, cudaStream_t st);
 int colnorm2_gemm_path(const desmo_shape* s, int T, int K, const float* P, const float* phi, const float* omega, float* out_k, cudaStream_t st);
 int launch_update_phi_generic(const UpdateArgs& a, cudaStream_t st);
 int select_path(const desmo_shape* s, const Dims& d);  // DESMO_PATH_FP32 / _TC / _GEMM actually used, or <0 (error set)

@@ -1444,6 +1444,163 @@ int residual_modes_gemm_path(const desmo_shape* s, int T, int K, int Kp, const v
     return residual_pod_gemm_path(s, T, K, Kp, U, u_dtype, P, phi, omega, W, nullptr, nullptr, k, V, sigma, modes, scratch, st);
 }
 
+// Backward elimination pass (desmo_elimination_pass): per chunk of points, library planes -> GEMM 1 with the residual epilogue (EPI_RESID
+// / EPI_RESID_BF16, as the training step: r's two bf16 planes and sum r^2) -> then
+//   GEMM 4 (EPI_E, as the training step): this chunk's slices of F^T = R^T G, added in slice order into the fp64 F [K][mld]
+//   the library Gram GEMM (EPI_GRAM): both operands the three G planes read K-major through GEMM 4's B map, upper tiles only, the
+//               contraction over the chunk's points split into slices fixed for every chunk, fp64 slice partials accumulated over the
+//               chunks; then a fixed-order reduce into the fp64 A [K][K], mirrored.
+// Points per chunk: the chunk's G and R planes take about kElimChunkBytes.
+constexpr size_t kElimChunkBytes = 64u << 20;
+
+struct ElimLayout {
+    int Kr, Kp16, mp, TK, tiles, nslice_g, nslice_e;
+    long long rows_c;
+    size_t o_idx, o_deg, o_gp, o_wp, o_rp, o_ep, o_lp, o_part, part_bytes, bytes;
+};
+size_t elimination_layout(const desmo_shape* s, int T, int K, int sms, ElimLayout* L) {
+    L->Kr = (K + 127) / 128 * 128;  // GEMM 4 and the Gram GEMM read tiles of 128 library rows
+    L->Kp16 = (K + 15) / 16 * 16;
+    L->mp = (s->m + 127) / 128 * 128;
+    L->TK = L->Kr / 128;
+    L->tiles = L->TK * (L->TK + 1) / 2;
+    const size_t per_point = (size_t)3 * L->Kr * 2 + (size_t)2 * L->mp * 2;
+    long long rc = (long long)(kElimChunkBytes / per_point) / 128 * 128;
+    if (rc < 128) rc = 128;
+    if (rc > s->ld) rc = s->ld;
+    L->rows_c = rc;
+    // slices of the two contractions over the points: enough work items to fill the SMs, the same for every chunk
+    auto slices = [&](int tiles) {
+        int ns = sms / tiles;
+        if (ns < 1) ns = 1;
+        if (ns > kSliceMax) ns = kSliceMax;
+        if (ns > (int)(rc / 64)) ns = (int)(rc / 64);
+        return ns;
+    };
+    L->nslice_g = slices(L->tiles);
+    L->nslice_e = slices((L->mp / 128) * L->TK);
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off = align_up_g(off + bytes, 1024); return o; };
+    L->o_idx = take((size_t)T * 8);
+    L->o_deg = take((size_t)T);
+    L->o_gp = take((size_t)3 * L->Kr * rc * 2);
+    L->o_wp = take((size_t)3 * L->Kr * L->mp * 2);
+    L->o_rp = take((size_t)2 * rc * L->mp * 2);
+    L->o_ep = take((size_t)L->nslice_e * L->Kp16 * s->mld * 4);
+    L->o_lp = take((size_t)(sms > 0 ? sms : 1) * sizeof(double));
+    L->part_bytes = (size_t)L->nslice_g * L->tiles * gp::BM * gp::BN * sizeof(double);
+    L->o_part = take(L->part_bytes);
+    L->bytes = off;
+    return off;
+}
+
+size_t elimination_scratch_bytes(const desmo_shape* s, int T, int K, int sms) {
+    ElimLayout L;
+    return elimination_layout(s, T, K, sms, &L);
+}
+
+// F [K][mld] fp64: the first chunk stores, later chunks add, the sum of this chunk's E slices [nslice][Kp16][mld] in slice order
+__global__ void __launch_bounds__(256) elim_f_accum_kernel(const float* __restrict__ Ep, int nslice, int K, int Kp16, int mld, int first,
+                                                           double* __restrict__ F) {
+    const long long e = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (e >= (long long)K * mld) return;
+    const long long slice = (long long)Kp16 * mld;
+    double s = 0.0;
+    for (int q = 0; q < nslice; ++q) s += (double)Ep[q * slice + e];
+    F[e] = first ? s : F[e] + s;
+}
+
+// A[i][j] = sum over the slices, in order, of the partial of the upper element (min(i, j), max(i, j)): A is exactly symmetric.
+// Block 0 also writes r2 = the GEMM 1 loss partials summed in CTA order.
+__global__ void __launch_bounds__(256) elim_gram_reduce_kernel(const double* __restrict__ part, int nslice, int tiles, int TK, int K,
+                                                               const double* __restrict__ lp, int nloss, double* __restrict__ A,
+                                                               double* __restrict__ r2) {
+    const long long e = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (e == 0) {
+        double s = 0.0;
+        for (int b = 0; b < nloss; ++b) s += lp[b];
+        *r2 = s;
+    }
+    if (e >= (long long)K * K) return;
+    const int i = (int)(e / K), j = (int)(e - (long long)i * K);
+    const int a = i < j ? i : j, b = i < j ? j : i;
+    const int tm = a / gp::BM, tn = b / gp::BN;
+    const long long tile = (long long)tm * TK - (long long)tm * (tm - 1) / 2 + (tn - tm);
+    const long long off = tile * (gp::BM * gp::BN) + (long long)(b % gp::BN) * gp::BM + (a % gp::BM);
+    const long long stride = (long long)tiles * gp::BM * gp::BN;
+    double s = 0.0;
+    for (int q = 0; q < nslice; ++q) s += part[q * stride + off];
+    A[e] = s;
+}
+
+int elimination_pass_gemm_path(const desmo_shape* s, int T, int K, const void* U, int u_dtype, const float* P, const float* phi,
+                               const float* omega, const float* W, double* A, double* F, double* r2, void* scratch_v, cudaStream_t st) {
+    using namespace gp;
+    int dev = 0, sms = 0;
+    DESMO_CUDA(cudaGetDevice(&dev));
+    DESMO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    ElimLayout L;
+    elimination_layout(s, T, K, sms, &L);
+    uint8_t* scratch = static_cast<uint8_t*>(scratch_v);
+    __nv_bfloat16* Gp = reinterpret_cast<__nv_bfloat16*>(scratch + L.o_gp);
+    __nv_bfloat16* Wp = reinterpret_cast<__nv_bfloat16*>(scratch + L.o_wp);
+    __nv_bfloat16* Rp = reinterpret_cast<__nv_bfloat16*>(scratch + L.o_rp);
+    float* Ep = reinterpret_cast<float*>(scratch + L.o_ep);
+    double* lp = reinterpret_cast<double*>(scratch + L.o_lp);
+    double* part = reinterpret_cast<double*>(scratch + L.o_part);
+    TermTable tab{scratch + L.o_idx, scratch + L.o_deg};
+    const int Kr = L.Kr, mp = L.mp;
+    const long long rows_c = L.rows_c;
+    term_table_kernel<<<(T + 127) / 128, 128, 0, st>>>(s->r, s->polyorder, T, tab, nullptr, K);
+    w_planes_kernel<<<Kr, 256, 0, st>>>(W, nullptr, K, Kr, s->m, s->mld, mp, Wp);
+    DESMO_CUDA(cudaGetLastError());
+    CUtensorMap tmG_mn, tmG_k, tmW_mn, tmR_mn;
+    int rc;
+    // G planes [3*Kr rows][rows_c]: MN-major A of GEMM 1, K-major B of GEMM 4 and both operands of the Gram GEMM
+    if ((rc = make_map(&tmG_mn, Gp, rows_c, 3LL * Kr, 64)) || (rc = make_map(&tmG_k, Gp, rows_c, 3LL * Kr, 128))) return rc;
+    if ((rc = make_map(&tmW_mn, Wp, mp, 3LL * Kr, 64)) || (rc = make_map(&tmR_mn, Rp, mp, 2LL * rows_c, 64))) return rc;
+    int nloss = 0;
+    bool first = true;
+    for (long long x0 = 0; x0 < s->ld; x0 += rows_c, first = false) {
+        const long long pts = (s->ld - x0 < rows_c) ? s->ld - x0 : rows_c;  // multiple of 128
+        library_planes_kernel<<<dim3((unsigned)((rows_c + 255) / 256), 64u), 256, 0, st>>>(P, phi, omega, tab, nullptr, s->r, T, K, Kr, s->n,
+                                                                                          s->ld, x0, rows_c, Gp);
+        DESMO_CUDA(cudaGetLastError());
+        GemmArgs g{};
+        g.U = U; g.Rp = Rp; g.Epart = Ep; g.loss_part = lp;
+        g.n = s->n; g.ld = s->ld; g.x0 = x0; g.rows_r = rows_c; g.m = s->m; g.mld = s->mld; g.mp = mp; g.K = K; g.Kp = L.Kp16;
+        g.n_lib16 = L.Kp16;
+        // GEMM 1, as the training step's: Rec[p x t] = G W, epilogue r = Rec - U -> two bf16 planes of r, sum r^2 per CTA over the chunks
+        g.first_chunk = first ? 1 : 0;
+        g.tiles_m = (int)(pts / 128); g.tiles_n = mp / 128; g.nslice = 1; g.kblocks = (K + 63) / 64; g.kb_per_slice = g.kblocks; g.kgroup = 4;
+        g.a_rows = Kr; g.b_rows = Kr;
+        rc = u_dtype == DESMO_DTYPE_BF16 ? launch_gemm<true, true, 3, 3, EPI_RESID_BF16>(g, tmG_mn, tmW_mn, sms, st)
+                                         : launch_gemm<true, true, 3, 3, EPI_RESID>(g, tmG_mn, tmW_mn, sms, st);
+        if (rc) return rc;
+        if (first) nloss = g.tiles_m * g.tiles_n < sms ? g.tiles_m * g.tiles_n : sms;  // the first chunk is the largest
+        // GEMM 4, as the training step's: E^T[t x lib] = R^T G; A = R (MN-major), B = G (K-major), this chunk's points in slices
+        g.first_chunk = 1;
+        g.tiles_m = mp / 128; g.tiles_n = L.TK; g.kblocks = (int)(pts / 64); g.nslice = L.nslice_e;
+        g.kb_per_slice = (g.kblocks + g.nslice - 1) / g.nslice; g.kgroup = 32;
+        g.a_rows = (int)rows_c; g.b_rows = Kr;
+        if ((rc = launch_gemm<true, false, 2, 2, EPI_E>(g, tmR_mn, tmG_k, sms, st))) return rc;
+        const long long fcount = (long long)K * s->mld;
+        elim_f_accum_kernel<<<(unsigned)((fcount + 255) / 256), 256, 0, st>>>(Ep, L.nslice_e, K, L.Kp16, s->mld, first ? 1 : 0, F);
+        DESMO_CUDA(cudaGetLastError());
+        // Gram GEMM: A tiles (tm <= tn) [k1 x k2] = G^T G; A = B = G (K-major: p contiguous), the six products of GEMM 1, chains of 2
+        // k-blocks (48 MMAs) per TMEM accumulator, summed in fp32 RN within a slice, fp64 across slices and chunks
+        g.loss_part = part; g.first_chunk = first ? 1 : 0; g.mp = Kr;
+        g.tiles_m = 1; g.tiles_n = L.tiles; g.kblocks = (int)(pts / 64); g.nslice = L.nslice_g;
+        g.kb_per_slice = (g.kblocks + g.nslice - 1) / g.nslice; g.kgroup = 2;
+        g.a_rows = Kr; g.b_rows = Kr;
+        if ((rc = launch_gemm<false, false, 3, 3, EPI_GRAM>(g, tmG_k, tmG_k, sms, st))) return rc;
+    }
+    const long long total = (long long)K * K;
+    elim_gram_reduce_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(part, L.nslice_g, L.tiles, L.TK, K, lp, nloss, A, r2);
+    DESMO_CUDA(cudaGetLastError());
+    return DESMO_OK;
+}
+
 int colnorm2_gemm_path(const desmo_shape* s, int T, int K, const float* P, const float* phi, const float* omega, float* out_k, cudaStream_t st) {
     using namespace gp;
     void* scratch = nullptr;

@@ -699,6 +699,49 @@ class DesmoEngine:
         out.update(singular_values=S.cpu(), energy=energy, cumulative_energy=torch.cumsum(energy, 0))
         return out
 
+    def _elimination_scratch(self) -> torch.Tensor:
+        """Scratch of desmo_elimination_pass / desmo_elimination_greedy for this device's SM count (bounded by the chunk, K and m)."""
+        sms = torch.cuda.get_device_properties(self.device).multi_processor_count
+        nbytes = C.c_size_t(0)
+        check(self.lib.desmo_elimination_scratch_bytes(C.byref(self.shape), sms, C.byref(nbytes)), "desmo_elimination_scratch_bytes")
+        return torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+
+    def backward_elimination(self, steps: Optional[int] = None) -> dict:
+        """Backward elimination by error at fixed coefficients: the order in which removing one term at a time raises ||U - recon||_F^2
+        the least, for the current parameters (no refit; U as stored).  One pass over U gives the library Gram A = G^T G, F = G^T R
+        and ||R||_F^2 (desmo_elimination_pass; all-reduced in fp64 when point-sharded); the greedy then runs on the device from those
+        alone (desmo_elimination_greedy): terms with a zero W row (zero gates, terms outside an active set) first in index order, then
+        at each step the term of least increment, ties to the lowest index.  ``steps`` (default K) terms are removed.  Returns
+
+          order                (S,) int64 host    packed K indices in removal order
+          predicted_residual2  (S+1,) fp64        ||R_s||_F^2 predicted from A and F (all ranks): a ranking quantity, see below
+          gram                 (K, K) fp64        A = G^T G (all ranks)
+
+        A and F carry the split-bf16 GEMMs' rounding (include/desmo_b200.h), so candidates whose increments differ by less than that
+        may be ranked either way, and predicted_residual2 is not an exact error: pruning_profile(order) scores the order exactly.
+        Nothing the model owns is written (parameters, Adamax state, red, dphi, losses, step_dev, U); W is rebuilt from the
+        parameters as residual_profile() does.  The same inputs give the same order on every call and every rank."""
+        S = self.K if steps is None else int(steps)
+        if not 0 <= S <= self.K:
+            raise _lib.DesmoError(f"backward_elimination: need 0 <= steps <= K = {self.K}, got {steps}")
+        ud = self._u_dtype()
+        f64 = dict(dtype=torch.float64, device=self.device)
+        scratch = self._elimination_scratch()
+        A, F, r2 = torch.empty(self.K, self.K, **f64), torch.empty(self.K, self.mld, **f64), torch.empty(1, **f64)
+        order = torch.empty(max(S, 1), dtype=torch.int32, device=self.device)
+        pred = torch.empty(S + 1, **f64)
+        with torch.cuda.device(self.device):
+            self.build_w(False)
+            check(self.lib.desmo_elimination_pass(C.byref(self.shape), _ptr(self.U), ud, _ptr(self.P), _ptr(self.phi), _ptr(self.omega),
+                                                  _ptr(self.W), _ptr(A), _ptr(F), _ptr(r2), _ptr(scratch), scratch.numel(), self._stream()),
+                  "desmo_elimination_pass")
+            if self.n_global != self.n and torch.distributed.is_initialized():
+                for t in (A, F, r2):
+                    torch.distributed.all_reduce(t, group=self.pg)
+            check(self.lib.desmo_elimination_greedy(C.byref(self.shape), _ptr(A), _ptr(F), _ptr(r2), _ptr(self.W), S, _ptr(order), _ptr(pred),
+                                                    _ptr(scratch), scratch.numel(), self._stream()), "desmo_elimination_greedy")
+        return {"order": order[:S].cpu().long(), "predicted_residual2": pred, "gram": A}
+
     # ------------------------------------------------------------------ POD (method of snapshots)
     def preprocess_snapshot(self, raw: torch.Tensor, d_in: int = 1, d_use: Optional[int] = None, magnitude: bool = True,
                             subtract_mean: bool = True, scale_sqrt_m: bool = False, t_stride: int = 1) -> torch.Tensor:

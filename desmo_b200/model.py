@@ -231,6 +231,11 @@ class _DesmoBase(nn.Module):
         self.sync_parameters()
         return self.engine.residual_pod(k)
 
+    def backward_elimination(self, steps=None) -> dict:
+        """The removal order by error at fixed coefficients, chosen on the device (DesmoEngine.backward_elimination)."""
+        self.sync_parameters()
+        return self.engine.backward_elimination(steps)
+
     # ---- training a pruned model (DesmoEngine.set_active_terms) ----------------------------------------------------------------
     def set_active_terms(self, mask) -> None:
         """Train on the terms of the bool (K,) ``mask`` only (None: every term); see DesmoEngine.set_active_terms.  The set applies to

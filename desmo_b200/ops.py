@@ -3,7 +3,7 @@
   build_w, build_w_at, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, pruning_profile, library_colnorm2, term_norms,
   pod_gram, pod_eig, pod_eigh, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce,
   active_terms_prepare, build_w_active, fused_residual_grad_active, adamax_update_active, assemble_grads_active,
-  residual_gram, residual_modes
+  residual_gram, residual_modes, elimination_pass, elimination_greedy
 
 They take the packed device tensors of a DesmoEngine (layout: include/desmo_b200.h) plus the shape integers and launch the
 sm_100a kernels on the current stream.  CUDA only: no CPU implementation is registered and every op checks its tensors, so a call
@@ -209,6 +209,41 @@ def residual_modes(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, omega: t
     with torch.cuda.device(U.device):
         check(_lib.load().desmo_residual_modes(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), k, _p(V), _p(sigma), _p(modes),
                                                _p(scratch), scratch.numel(), _stream(U)), "desmo_residual_modes")
+
+
+@torch.library.custom_op("desmo_b200::elimination_pass", mutates_args=("A", "F", "r2", "scratch"))
+def elimination_pass(U: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, omega: torch.Tensor, W: torch.Tensor, A: torch.Tensor,
+                     F: torch.Tensor, r2: torch.Tensor, scratch: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int,
+                     nF: int, path: int) -> None:
+    """A (fp64 [K, K]) = G^T G, F (fp64 [K, mld]) = G^T R, r2 (fp64 [1]) = ||R||_F^2 of R = G W - U (desmo_elimination_pass)."""
+    _require_cuda(U, P, phi, omega, W, A, F, r2, scratch)
+    ud = _lib.u_dtype_code(U.dtype)
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    K = _lib.load().desmo_num_terms(r, polyorder) + 3 * r
+    if any(t.dtype != torch.float64 or not t.is_contiguous() for t in (A, F, r2)) or A.numel() < K * K or F.numel() < K * s.mld or \
+            r2.numel() < 1:
+        raise _lib.DesmoError(f"elimination_pass: need contiguous float64 A [{K}, {K}], F [{K}, {s.mld}] and r2 [1]")
+    _scratch_ok(scratch, "elimination_pass")
+    with torch.cuda.device(U.device):
+        check(_lib.load().desmo_elimination_pass(C.byref(s), _p(U), ud, _p(P), _p(phi), _p(omega), _p(W), _p(A), _p(F), _p(r2),
+                                                 _p(scratch), scratch.numel(), _stream(U)), "desmo_elimination_pass")
+
+
+@torch.library.custom_op("desmo_b200::elimination_greedy", mutates_args=("F", "order", "predicted", "scratch"))
+def elimination_greedy(A: torch.Tensor, F: torch.Tensor, r2: torch.Tensor, W: torch.Tensor, order: torch.Tensor, predicted: torch.Tensor,
+                       scratch: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """order (int32 [S]) and predicted (fp64 [S+1]) of the greedy on A, F (consumed), r2 and W, S = predicted.numel() - 1
+    (desmo_elimination_greedy)."""
+    _require_cuda(A, F, r2, W, order, predicted, scratch)
+    S = predicted.numel() - 1
+    if order.dtype != torch.int32 or predicted.dtype != torch.float64 or order.numel() < S or S < 0 or \
+            not (order.is_contiguous() and predicted.is_contiguous()):
+        raise _lib.DesmoError("elimination_greedy: need contiguous int32 order [S] and float64 predicted [S + 1]")
+    _scratch_ok(scratch, "elimination_greedy")
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(A.device):
+        check(_lib.load().desmo_elimination_greedy(C.byref(s), _p(A), _p(F), _p(r2), _p(W), S, _p(order), _p(predicted), _p(scratch),
+                                                   scratch.numel(), _stream(A)), "desmo_elimination_greedy")
 
 
 @torch.library.custom_op("desmo_b200::library_colnorm2", mutates_args=("out",))
@@ -533,3 +568,22 @@ def engine_residual_pod_via_ops(e, k: int = 8) -> dict:
         torch.ops.desmo_b200.residual_modes(e.U, e.P, e.phi, e.omega, e.W, V, sigma, modes, scratch, *sa)
     return {"singular_values": S.cpu(), "sigma": sigma, "temporal_modes": V, "spatial_modes": modes[:, :e.n], "residual_norm2": float(tr.item()),
             "gram": Cm}
+
+
+def engine_backward_elimination_via_ops(e, steps=None) -> dict:
+    """DesmoEngine.backward_elimination() through the registered build_w / elimination_pass / elimination_greedy ops (the optimizer's
+    step counter is not moved)."""
+    sa = _shape_args(e)
+    S = e.K if steps is None else int(steps)
+    f64 = dict(dtype=torch.float64, device=e.device)
+    scratch = e._elimination_scratch()
+    A, F, r2 = torch.empty(e.K, e.K, **f64), torch.empty(e.K, e.mld, **f64), torch.empty(1, **f64)
+    order, pred = torch.empty(max(S, 1), dtype=torch.int32, device=e.device), torch.empty(S + 1, **f64)
+    scratch_step = e.step_dev.clone()
+    torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, scratch_step, e.workspace, *sa)
+    torch.ops.desmo_b200.elimination_pass(e.U, e.P, e.phi, e.omega, e.W, A, F, r2, scratch, *sa)
+    if e.n_global != e.n and torch.distributed.is_initialized():
+        for t in (A, F, r2):
+            torch.distributed.all_reduce(t, group=e.pg)
+    torch.ops.desmo_b200.elimination_greedy(A, F, r2, e.W, order, pred, scratch, *sa)
+    return {"order": order[:S].cpu().long(), "predicted_residual2": pred, "gram": A}

@@ -83,7 +83,9 @@ class PruningProfile:
     gates: torch.Tensor               # (K,) the gates the profile was taken with
 
     def steps_for_threshold(self, threshold: float) -> int:
-        """The step whose removed terms are exactly those threshold_sweep removes at ``threshold``."""
+        """The step whose removed terms are exactly those threshold_sweep removes at ``threshold``.  Raises DesmoError when no step
+        of this order removes exactly that set, as for most thresholds on backward_elimination()'s order (a threshold removes a
+        prefix of the norm order)."""
         return threshold_steps(self.term_norms, self.gates, self.order, threshold)
 
     def active_mask(self, step: int) -> torch.Tensor:
@@ -123,6 +125,21 @@ def pruning_profile(model, order=None, snapshot_norm2: Optional[float] = None) -
     for k in order:
         nonzero.append(nonzero[-1] - int(nz_host[k]))
     return PruningProfile(order, prof["snapshot_residual2"], prof["snapshot_norm2"], rel, nonzero, norms, gates)
+
+
+def backward_elimination(model, steps: Optional[int] = None, snapshot_norm2: Optional[float] = None) -> PruningProfile:
+    """Backward elimination by error at fixed coefficients: greedy_removal's experiment (no refit, one term per step) with the term
+    whose removal raises ||X - recon|| least taken at each step instead of the smallest-norm one.  The order comes from the device
+    greedy (DesmoEngine.backward_elimination: one pass over U, then A = G^T G and F = G^T R alone); the errors, per-snapshot
+    residuals and non-zero counts come from pruning_profile(model, order), so they are exact and on the same axes as the norm order's
+    pruning_profile(model).  active_mask(step) feeds set_active_terms for a refit; steps_for_threshold raises for this order (see
+    there).  ``steps`` defaults to K; ``snapshot_norm2`` as in pruning_profile.  The gates, rows, step counter and any active set are
+    left as they are."""
+    e = model.engine
+    if hasattr(model, "sync_parameters"):
+        model.sync_parameters()
+    order = e.backward_elimination(steps)["order"].tolist()
+    return pruning_profile(model, order, snapshot_norm2)
 
 
 def _stored_norm2(e) -> float:

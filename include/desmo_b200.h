@@ -269,6 +269,32 @@ int desmo_residual_modes(const desmo_shape* s, const void* U, int32_t u_dtype, c
                          const float* W, int32_t k, const float* V, const float* sigma, float* modes, void* scratch, size_t scratch_bytes,
                          void* stream);
 
+/* Backward elimination by error at fixed coefficients: the removal order that raises ||U - recon||_F^2 least at every step, chosen on
+ * the device without a residual pass per candidate.  With R = G(Phi) W - U (U as stored, u_dtype F32 or BF16) and the library G:
+ *   pass    A[K][K] fp64 = G^T G (exactly symmetric), F[K][mld] fp64 = G^T R (columns t >= m are 0), r2[1] fp64 = ||R||_F^2 -- local
+ *           partials: all-reduce all three across ranks.  Route, per chunk of points, for every library: the library planes and GEMM 1
+ *           with the training step's residual epilogue (r's two bf16 planes and sum r^2), GEMM 4 as in the training step (two planes,
+ *           three products) for F, and a tcgen05 Gram GEMM of the three library planes (the six products of GEMM 1, upper tiles, chains
+ *           of 48 MMAs) for A.  fp64 across slices and chunks, fixed order, no float atomics: bit-identical from call to call.
+ *           Entrywise, |A - A_exact| <= 2^-15 sum_x |G_i||G_j| and |F - F_exact| <= 2^-14 sum_x |G_k| (|r| + |G||W|) (DESIGN.md 3.4).
+ *   greedy  order[steps] int32 (device) and predicted[steps + 1] fp64 from A, F, r2 and W (the [Kp][mld] fp32 W of desmo_build_w):
+ *           terms with a zero W row first, in index order; then at each step the remaining k of least sum_t Delta_k(t),
+ *           Delta_k(t) = W_k(t) (A_kk W_k(t) - 2 F_k(t)), ties to the lowest index, and F_l <- F_l - A_lk W_k for the remaining l.
+ *           predicted[s] = r2 + the increments of the first s choices.  F is overwritten (consumed).  One launch per step on `stream`;
+ *           fp64 sums in a fixed order: the same inputs give the same order on every call and every rank.  0 <= steps <= K.
+ * Both calls allocate nothing, write only their outputs and the caller's scratch, and check every argument (pointers, u_dtype, steps,
+ * scratch size and 16-byte alignment) before any launch.  Scratch bytes, with Kr = 128 ceil(K / 128), Kp16 = 16 ceil(K / 16),
+ * mp = 128 ceil(m / 128), TK = Kr / 128, tiles = TK (TK + 1) / 2, rows_c = clamp(128 floor(2^26 / (6 Kr + 4 mp) / 128), 128, ld) the
+ * point chunk, ns(x) = clamp(floor(sms / x), 1, min(32, rows_c / 64)), nsg = ns(tiles), nse = ns(TK mp / 128), A(v) = v rounded up to 1024:
+ *   A(8T') + A(T') + A(6 Kr rows_c) + A(6 Kr mp) + A(4 rows_c mp) + A(4 nse Kp16 mld) + A(8 sms) + A(131072 nsg tiles)  (T' = polynomial terms)
+ * bounded by the chunk, K and m, never by n: about 99 MB at K = 657, m = 1000 on 148 SMs.  desmo_elimination_scratch_bytes returns it
+ * (host only); the greedy takes the same scratch and uses its first 256 + 2 A256(4K) + A256(8K) bytes (A256: rounded up to 256). */
+int desmo_elimination_scratch_bytes(const desmo_shape* s, int32_t sms, size_t* bytes);
+int desmo_elimination_pass(const desmo_shape* s, const void* U, int32_t u_dtype, const float* P, const float* phi, const float* omega,
+                           const float* W, double* A, double* F, double* r2, void* scratch, size_t scratch_bytes, void* stream);
+int desmo_elimination_greedy(const desmo_shape* s, const double* A, double* F, const double* r2, const float* W, int32_t steps,
+                             int32_t* order, double* predicted, void* scratch, size_t scratch_bytes, void* stream);
+
 /* Post-hoc sparsification inputs: squared column norms of G (K floats, local partial -- all-reduce them across ranks).
  * P == NULL evaluates the library on the raw phi_list, which is what the reference's sweep passes to poly_norm /
  * nonlinear_norm (CYL:1192-1194; the functions, CYL:624-692, never multiply by POD_modes); P != NULL gives the columns of
