@@ -58,6 +58,10 @@ SIGNATURES: Dict[str, tuple] = {
     "desmo_fused_residual_grad_finish_active": (C.c_int, [_SP, _vp, _i32] + [_vp] * 8 + [_i32, _vp]),
     "desmo_adamax_update_active": (C.c_int, [_SP] + [_vp] * 27),
     "desmo_assemble_grads_active": (C.c_int, [_SP] + [_vp] * 18),
+    "desmo_time_points_prepare": (C.c_int, [_SP, _vp, _i32, _vp, _vp]),
+    "desmo_build_w_times": (C.c_int, [_SP] + [_vp] * 10),
+    "desmo_adamax_update_times": (C.c_int, [_SP] + [_vp] * 28),
+    "desmo_assemble_grads_times": (C.c_int, [_SP] + [_vp] * 19),
     "desmo_reconstruct": (C.c_int, [_SP] + [_vp] * 6),
     "desmo_library_colnorm2": (C.c_int, [_SP] + [_vp] * 5),
     "desmo_residual_profile": (C.c_int, [_SP, _vp, _i32] + [_vp] * 7),

@@ -242,18 +242,54 @@ int desmo_active_terms_prepare(const desmo_shape* s, const int32_t* host_indices
     return DESMO_OK;
 }
 
-static int build_w_impl(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
-                        int32_t* step_dev, void* workspace, const int32_t* active, void* stream, const char* who) {
+int desmo_time_points_prepare(const desmo_shape* s, const float* host_times, int32_t count, void* table_dev, void* stream) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
+    if (!host_times || !table_dev) { set_error("desmo_time_points_prepare: null pointer"); return DESMO_ERR_ARG; }
+    if (s->nF <= 0) {
+        set_error("desmo_time_points_prepare: time points need a Fourier model (nF > 0); DESMO's free rows have no time coordinate");
+        return DESMO_ERR_ARG;
+    }
+    if (count != s->m) { set_error("desmo_time_points_prepare: need one time per snapshot, count = m = %d (got %d)", s->m, count); return DESMO_ERR_ARG; }
+    // host array: every value is checked before anything is written
+    for (int i = 0; i < count; ++i)
+        if (!isfinite(host_times[i])) { set_error("desmo_time_points_prepare: times[%d] is not finite", i); return DESMO_ERR_ARG; }
+    if ((rc = device_ok())) return rc;
+    // from pageable memory: the copy has consumed host_times when it returns
+    DESMO_CUDA(cudaMemcpyAsync(table_dev, host_times, sizeof(float) * (size_t)count, cudaMemcpyHostToDevice, (cudaStream_t)stream));
+    return DESMO_OK;
+}
+
+// a time table belongs to a Fourier model only
+static int check_times(const desmo_shape* s, const float* t_points, const char* who) {
+    if (t_points && s->nF <= 0) {
+        set_error("%s: time points need a Fourier model (nF > 0); DESMO's free rows have no time coordinate", who);
+        return DESMO_ERR_ARG;
+    }
+    return DESMO_OK;
+}
+
+static int build_w_impl(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
+                        int32_t* step_dev, void* workspace, const int32_t* active, void* stream, const char* who,
+                        const float* t_points = nullptr) {
+    Dims d;
+    int rc = validate_shape(s, &d);
+    if (rc) return rc;
+    if ((rc = check_times(s, t_points, who))) return rc;
     if ((rc = device_ok())) return rc;
     if (!gates || !rows || !W || !workspace || (s->nF > 0 && (!coefs || !periods))) { set_error("%s: null pointer", who); return DESMO_ERR_ARG; }
     Workspace ws;
     if ((rc = carve_workspace(s, d, workspace, &ws))) return rc;
     const bool tc = use_tc_path(s, d);
     return build_w(s, d.K, d.Kp, gates, rows, coefs, periods, W, tc ? ws.tc : nullptr, tc ? ws.tc + (size_t)d.Kp * s->mld : nullptr,
-                   step_dev, ws.l1, (cudaStream_t)stream, active);
+                   step_dev, ws.l1, (cudaStream_t)stream, active, t_points);
+}
+
+int desmo_build_w_times(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
+                        int32_t* step_dev, void* workspace, const void* active, const float* t_points, void* stream) {
+    return build_w_impl(s, gates, rows, coefs, periods, W, step_dev, workspace, static_cast<const int32_t*>(active), stream,
+                        "desmo_build_w_times", t_points);
 }
 
 int desmo_build_w_active(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
@@ -399,11 +435,12 @@ static int desmo_adamax_update_impl(const desmo_shape* s, const float* red, cons
                                     float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows, float* rows_m, float* rows_u,
                                     float* coefs, float* coefs_m, float* coefs_u, float* periods, float* periods_m, float* periods_u,
                                     float* omega, float* omega_m, float* omega_u, const float* hyper, const int32_t* step_dev,
-                                    float* losses_out, void* workspace, const int32_t* active, void* stream);
+                                    float* losses_out, void* workspace, const int32_t* active, void* stream,
+                                    const float* t_points = nullptr);
 static int assemble_grads_impl(const desmo_shape* s, const float* red, float* dphi, const float* P, const float* phi, const float* gates,
                                const float* rows, const float* coefs, const float* periods, const float* hyper, float* d_gates,
                                float* d_rows, float* d_coefs, float* d_periods, float* d_omega, float* losses_out, void* workspace,
-                               const int32_t* active, void* stream);
+                               const int32_t* active, void* stream, const float* t_points = nullptr);
 
 int desmo_adamax_update(const desmo_shape* s, const float* red, const float* dphi, const float* P, float* phi, float* phi_m,
                         float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows, float* rows_m, float* rows_u,
@@ -426,14 +463,25 @@ int desmo_adamax_update_active(const desmo_shape* s, const float* red, const flo
                                     static_cast<const int32_t*>(active), stream);
 }
 
+int desmo_adamax_update_times(const desmo_shape* s, const float* red, const float* dphi, const float* P, float* phi, float* phi_m,
+                              float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows, float* rows_m, float* rows_u,
+                              float* coefs, float* coefs_m, float* coefs_u, float* periods, float* periods_m, float* periods_u,
+                              float* omega, float* omega_m, float* omega_u, const float* hyper, const int32_t* step_dev,
+                              float* losses_out, void* workspace, const void* active, const float* t_points, void* stream) {
+    return desmo_adamax_update_impl(s, red, dphi, P, phi, phi_m, phi_u, gates, gates_m, gates_u, rows, rows_m, rows_u, coefs, coefs_m,
+                                    coefs_u, periods, periods_m, periods_u, omega, omega_m, omega_u, hyper, step_dev, losses_out, workspace,
+                                    static_cast<const int32_t*>(active), stream, t_points);
+}
+
 static int desmo_adamax_update_impl(const desmo_shape* s, const float* red, const float* dphi, const float* P, float* phi, float* phi_m,
                                     float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows, float* rows_m, float* rows_u,
                                     float* coefs, float* coefs_m, float* coefs_u, float* periods, float* periods_m, float* periods_u,
                                     float* omega, float* omega_m, float* omega_u, const float* hyper, const int32_t* step_dev,
-                                    float* losses_out, void* workspace, const int32_t* active, void* stream) {
+                                    float* losses_out, void* workspace, const int32_t* active, void* stream, const float* t_points) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
+    if ((rc = check_times(s, t_points, "desmo_adamax_update_times"))) return rc;
     if ((rc = device_ok())) return rc;
     const bool f = s->nF > 0;
     if (!red || !dphi || !P || !phi || !phi_m || !phi_u || !gates || !gates_m || !gates_u || !rows || !omega || !omega_m || !omega_u ||
@@ -452,6 +500,7 @@ static int desmo_adamax_update_impl(const desmo_shape* s, const float* red, cons
     a.omega = omega; a.omega_m = omega_m; a.omega_u = omega_u; a.hyper = hyper; a.step_dev = step_dev; a.losses_out = losses_out;
     a.apply = 1;
     a.active_pos = active;
+    a.t_points = t_points;
     return launch_update(a, (cudaStream_t)stream);
 }
 
@@ -472,13 +521,22 @@ int desmo_assemble_grads_active(const desmo_shape* s, const float* red, float* d
                                losses_out, workspace, static_cast<const int32_t*>(active), stream);
 }
 
+int desmo_assemble_grads_times(const desmo_shape* s, const float* red, float* dphi, const float* P, const float* phi, const float* gates,
+                               const float* rows, const float* coefs, const float* periods, const float* hyper, float* d_gates,
+                               float* d_rows, float* d_coefs, float* d_periods, float* d_omega, float* losses_out, void* workspace,
+                               const void* active, const float* t_points, void* stream) {
+    return assemble_grads_impl(s, red, dphi, P, phi, gates, rows, coefs, periods, hyper, d_gates, d_rows, d_coefs, d_periods, d_omega,
+                               losses_out, workspace, static_cast<const int32_t*>(active), stream, t_points);
+}
+
 static int assemble_grads_impl(const desmo_shape* s, const float* red, float* dphi, const float* P, const float* phi, const float* gates,
                                const float* rows, const float* coefs, const float* periods, const float* hyper, float* d_gates,
                                float* d_rows, float* d_coefs, float* d_periods, float* d_omega, float* losses_out, void* workspace,
-                               const int32_t* active, void* stream) {
+                               const int32_t* active, void* stream, const float* t_points) {
     Dims d;
     int rc = validate_shape(s, &d);
     if (rc) return rc;
+    if ((rc = check_times(s, t_points, "desmo_assemble_grads_times"))) return rc;
     if ((rc = device_ok())) return rc;
     const bool f = s->nF > 0;
     if (!red || !dphi || !P || !phi || !gates || !rows || !hyper || !d_gates || !d_omega || !workspace || (!f && !d_rows) ||
@@ -496,6 +554,7 @@ static int assemble_grads_impl(const desmo_shape* s, const float* red, float* dp
     a.d_periods = d_periods; a.d_omega = d_omega; a.losses_out = losses_out;
     a.apply = 0;
     a.active_pos = active;
+    a.t_points = t_points;
     return launch_update(a, (cudaStream_t)stream);
 }
 

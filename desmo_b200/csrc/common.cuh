@@ -62,6 +62,7 @@ struct UpdateArgs {
     int m, mld, r, K, Kp, nF;
     int apply;      // 1 = Adamax in place, 0 = write gradients
     const int32_t* active_pos;  // [K] compact column or -1 (desmo_active_terms_prepare); null = every term active
+    const float* t_points;      // [m] times of the snapshot columns (desmo_time_points_prepare); null = the grid t_point(t, m)
 };
 
 struct EvalArgs {
@@ -77,8 +78,10 @@ struct EvalArgs {
 
 // host-side launchers (one per translation unit)
 // active_pos: [K] of an active-term table (null = every term active); absent terms get zero W rows and no L1 share
+// t_points: [m] fp32 times of a Fourier model's columns (desmo_time_points_prepare; null = the grid t_point(t, m))
 int build_w(const desmo_shape* s, int K, int Kp, const float* gates, float* rows, const float* coefs, const float* periods,
-            float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st, const int32_t* active_pos = nullptr);
+            float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st, const int32_t* active_pos = nullptr,
+            const float* t_points = nullptr);
 // W_out[Kp][mld_out] (and rows_out[K][mld_out] if non-null) at m_out host-given instants, one launch per kAtBatch of them; the
 // arguments are validated by desmo_build_w_at
 constexpr int kAtBatch = 512;

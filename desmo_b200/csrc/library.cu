@@ -29,11 +29,14 @@ __device__ __forceinline__ float fourier_value(const float* __restrict__ c, int 
     return z;
 }
 
-// grid = Kp blocks (one library term each), 256 threads over time.
+// grid = Kp blocks (one library term each), 256 threads over time.  kTimes: column t of a Fourier model is evaluated at
+// t_points[t] (desmo_time_points_prepare) instead of t_point(t, m); the table is read by address at every launch.  The parameter
+// comes last, so the instantiation without a table compiles to the kernel it was before the table existed.
+template <bool kTimes>
 __global__ void build_w_kernel(int K, int m, int mld, int nF, const float* __restrict__ gates, float* __restrict__ rows,
                                const float* __restrict__ coefs, const float* __restrict__ periods, float* __restrict__ W,
                                __nv_bfloat16* __restrict__ Wb, int Kp, int32_t* step_dev, float* l1_out,
-                               const int32_t* __restrict__ active_pos) {
+                               const int32_t* __restrict__ active_pos, const float* __restrict__ t_points) {
     // Wb: three bf16 planes [3][32][mld] of W for the tcgen05 path (w = b1 + b2 + b3), rows >= K zero.
     // active_pos (null: every term active): an absent term has a zero W row and no share of the L1 sum.
     const int k = blockIdx.x;
@@ -54,7 +57,7 @@ __global__ void build_w_kernel(int K, int m, int mld, int nF, const float* __res
         if (k < K && t < m) {
             float z;
             if (nF > 0) {
-                z = fourier_value(coefs + (size_t)k * (2 * nF + 1), nF, t_point(t, m), period);
+                z = fourier_value(coefs + (size_t)k * (2 * nF + 1), nF, kTimes ? t_points[t] : t_point(t, m), period);
                 rows[(size_t)k * mld + t] = z;
             } else {
                 z = rows[(size_t)k * mld + t];
@@ -75,11 +78,16 @@ __global__ void build_w_kernel(int K, int m, int mld, int nF, const float* __res
 }
 
 int build_w(const desmo_shape* s, int K, int Kp, const float* gates, float* rows, const float* coefs, const float* periods,
-            float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st, const int32_t* active_pos) {
+            float* W, float* Whi, float* Wlo, int32_t* step_dev, float* l1_out, cudaStream_t st, const int32_t* active_pos,
+            const float* t_points) {
     (void)Wlo;
     const int grid = (Whi && Kp < 32) ? 32 : Kp;
-    build_w_kernel<<<grid, 256, 0, st>>>(K, s->m, s->mld, s->nF, gates, rows, coefs, periods, W, reinterpret_cast<__nv_bfloat16*>(Whi), Kp,
-                                         step_dev, l1_out, active_pos);
+    if (t_points)
+        build_w_kernel<true><<<grid, 256, 0, st>>>(K, s->m, s->mld, s->nF, gates, rows, coefs, periods, W,
+                                                   reinterpret_cast<__nv_bfloat16*>(Whi), Kp, step_dev, l1_out, active_pos, t_points);
+    else
+        build_w_kernel<false><<<grid, 256, 0, st>>>(K, s->m, s->mld, s->nF, gates, rows, coefs, periods, W,
+                                                    reinterpret_cast<__nv_bfloat16*>(Whi), Kp, step_dev, l1_out, active_pos, nullptr);
     DESMO_CUDA(cudaGetLastError());
     return DESMO_OK;
 }

@@ -38,6 +38,9 @@ __device__ __forceinline__ float t_point_u(int t, int m) {
     return (t < m / 2) ? __fmul_rn(step, (float)t) : __fsub_rn((float)m, __fmul_rn(step, (float)(m - 1 - t)));
 }
 
+// kTimes: the Fourier gradients take column t at a.t_points[t] (desmo_time_points_prepare) instead of t_point_u(t, m); without a
+// table the instantiation is the kernel it was before the table existed (a.t_points is the last field of UpdateArgs).
+template <bool kTimes>
 __global__ void __launch_bounds__(256) update_kernel(const UpdateArgs a) {
     __shared__ float sh[8];
     __shared__ float gsign[kMaxR * kMaxR];
@@ -96,7 +99,7 @@ __global__ void __launch_bounds__(256) update_kernel(const UpdateArgs a) {
                 const float ah = c[2 * h - 1], bh = c[2 * h];
                 for (int t = tid; t < a.m; t += 256) {
                     const float dz = gate * (scale * E[t]);
-                    const float th = __fdiv_rn(__fmul_rn(two_pi_h, t_point_u(t, a.m)), period);
+                    const float th = __fdiv_rn(__fmul_rn(two_pi_h, kTimes ? a.t_points[t] : t_point_u(t, a.m)), period);
                     const float cs = cosf(th), sn = sinf(th);
                     ca = fmaf(dz, cs, ca);
                     sa = fmaf(dz, sn, sa);
@@ -266,7 +269,8 @@ int launch_update(const UpdateArgs& a, cudaStream_t st) {
         if (rc) return rc;
         nb = 0;
     }
-    update_kernel<<<(unsigned)(a.K + 1 + nb), 256, 0, st>>>(a);
+    if (a.t_points) update_kernel<true><<<(unsigned)(a.K + 1 + nb), 256, 0, st>>>(a);
+    else update_kernel<false><<<(unsigned)(a.K + 1 + nb), 256, 0, st>>>(a);
     DESMO_CUDA(cudaGetLastError());
     return DESMO_OK;
 }

@@ -40,8 +40,26 @@ def time_points(index, m: int) -> np.ndarray:
     return np.where((k < m // 2) | (k >= m), up, down).astype(np.float32)
 
 
-def _instants(index, times, m: int, nF: int):
-    """Host arrays for desmo_build_w_at: (int32 index or None, fp32 times or None).  Raises DesmoError before any launch."""
+def time_table(t_points, m: int, nF: int) -> np.ndarray:
+    """The time table of a Fourier model as a contiguous fp32 host array: m finite values, t_points[t] the time of snapshot row t
+    (any order, repeats allowed).  A tensor, an array or a sequence; fp64 input is rounded to nearest once.  Raises DesmoError
+    before any launch (desmo_time_points_prepare checks the same again)."""
+    if not nF:
+        raise _lib.DesmoError("t_points needs a Fourier model (DESMOFourier, nF > 0): DESMO's free temporal rows have no time coordinate")
+    raw = t_points.detach().cpu().numpy() if torch.is_tensor(t_points) else np.asarray(t_points)
+    if raw.dtype == np.bool_ or not (np.issubdtype(raw.dtype, np.floating) or np.issubdtype(raw.dtype, np.integer)):
+        raise _lib.DesmoError(f"t_points must hold real numbers, got {raw.dtype}")
+    t = np.ascontiguousarray(raw, dtype=np.float32)
+    if t.shape != (m,):
+        raise _lib.DesmoError(f"t_points must hold one time per snapshot, shape ({m},), got {t.shape}")
+    if not np.isfinite(t).all():
+        raise _lib.DesmoError("t_points must be finite")
+    return t
+
+
+def _instants(index, times, m: int, nF: int, table: Optional[np.ndarray] = None):
+    """Host arrays for desmo_build_w_at: (int32 index or None, fp32 times or None).  With a time table, index k is the instant
+    table[k] and comes back as times.  Raises DesmoError before any launch."""
     if (index is None) == (times is None):
         raise _lib.DesmoError("pass exactly one of index= (training snapshot indices) or times= (Fourier model times)")
     if times is not None:
@@ -61,6 +79,8 @@ def _instants(index, times, m: int, nF: int):
     k = raw.astype(np.int64).reshape(-1)
     if int(k.min()) < 0 or int(k.max()) >= m:
         raise _lib.DesmoError(f"index= must lie in 0 .. {m - 1} (training snapshots; use times= to evaluate elsewhere)")
+    if table is not None:
+        return None, np.ascontiguousarray(table[k], dtype=np.float32)
     return np.ascontiguousarray(k, dtype=np.int32), None
 
 
@@ -106,7 +126,7 @@ class DesmoEngine:
 
     def __init__(self, n: int, m: int, polyorder: int, r: int, omega_init: float = 10000.0, nF: Optional[int] = None,
                  period_init: float = 60.0, device: Optional[torch.device] = None, n_global: Optional[int] = None,
-                 path: int = _lib.PATH_AUTO, process_group=None, snapshot_dtype: torch.dtype = torch.float32):
+                 path: int = _lib.PATH_AUTO, process_group=None, snapshot_dtype: torch.dtype = torch.float32, t_points=None):
         if snapshot_dtype not in (torch.float32, torch.bfloat16):
             raise _lib.DesmoError(f"snapshot_dtype must be torch.float32 or torch.bfloat16, got {snapshot_dtype}")
         self.snapshot_dtype = snapshot_dtype
@@ -167,7 +187,12 @@ class DesmoEngine:
         self.active_terms: Optional[torch.Tensor] = None  # bool (K,) on the host; None = every term (set_active_terms)
         self._active: Optional[torch.Tensor] = None       # its device table (desmo_active_terms_prepare)
         self._active_count = 0
+        self.t_points: Optional[np.ndarray] = None        # fp32 (m,) host copy of the time table; None = the grid (set_time_points)
+        self._times: Optional[torch.Tensor] = None        # the device table the steps read, or None
+        self._times_buf: Optional[torch.Tensor] = None    # its storage, rewritten in place by every set_time_points
         self.set_hyper(REFERENCE_LRS, 1e-3, 1e-4)
+        if t_points is not None:
+            self.set_time_points(t_points)
 
     # ------------------------------------------------------------------ inputs
     def set_pod_modes(self, pod_modes) -> None:
@@ -292,8 +317,46 @@ class DesmoEngine:
             self.gates.masked_fill_(~host.to(self.device), 0.0)
         self.active_terms, self._active, self._active_count = host, table, int(idx.size)
 
+    # ------------------------------------------------------------------ time points (Fourier models)
+    def set_time_points(self, t_points) -> None:
+        """Train and evaluate a Fourier model at caller-given times: ``t_points`` holds m finite values (tensor, array or sequence;
+        stored as fp32, fp64 rounded to nearest once), t_points[t] the time of snapshot row t in the model's time coordinate -- the
+        reference's module global t_points (FCYL:485), which its scripts set to torch.linspace(0, m, m).  Order and repeats are free.
+        ``None`` goes back to that grid.  Column t of the model is evaluated at t_points[t] in the rows, W and the coefficient and
+        period gradients, so everything downstream (reconstruct, losses, term_norms, the sweeps and profiles) follows; a table equal
+        to the grid gives every step bit for bit what no table gives.  index=k of the evaluation routines means t_points[k].
+        The device table is rewritten in place, so a step captured with a table follows later tables.  Point-sharded: every rank must
+        pass the same table (checked with one all-reduce).  A bad table raises before anything is written; DESMO raises always."""
+        if t_points is None:
+            if not self.nF:
+                return
+            self.t_points, self._times = None, None
+            return
+        t = time_table(t_points, self.m, self.nF)
+        if self._sharded():
+            # diverging tables would desynchronise the replicated parameters: compare the bit patterns through max(b) and max(-b)
+            bits = torch.from_numpy(t.view(np.int32).astype(np.int64)).to(self.device)
+            mine = torch.cat([bits, -bits])
+            tot = mine.clone()
+            torch.distributed.all_reduce(tot, op=torch.distributed.ReduceOp.MAX, group=self.pg)
+            if not torch.equal(tot, mine):
+                raise _lib.DesmoError("set_time_points: the ranks passed different tables (the table is replicated: pass the same one)")
+        if self._times_buf is None:
+            self._times_buf = torch.empty(self.m, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.lib.desmo_time_points_prepare(C.byref(self.shape), t.ctypes.data, self.m, _ptr(self._times_buf), self._stream()),
+                  "desmo_time_points_prepare")
+        self.t_points, self._times = t.copy(), self._times_buf
+
     def build_w(self, advance_step: bool = True, use_active: bool = False) -> None:
-        """W = diag(gates) rows (desmo_build_w); ``use_active``: with the active set, if one is set (absent rows zero)."""
+        """W = diag(gates) rows (desmo_build_w); ``use_active``: with the active set, if one is set (absent rows zero).  A Fourier
+        model with a time table evaluates its rows there (desmo_build_w_times)."""
+        if self._times is not None:
+            active = self._active if use_active else None
+            check(self.lib.desmo_build_w_times(C.byref(self.shape), _ptr(self.gates), _ptr(self.rows), _ptr(self.coefs), _ptr(self.periods),
+                                               _ptr(self.W), _ptr(self.step_dev) if advance_step else None, _ptr(self.workspace),
+                                               _ptr(active), _ptr(self._times), self._stream()), "desmo_build_w_times")
+            return
         if use_active and self._active is not None:
             check(self.lib.desmo_build_w_active(C.byref(self.shape), _ptr(self.gates), _ptr(self.rows), _ptr(self.coefs), _ptr(self.periods),
                                                 _ptr(self.W), _ptr(self.step_dev) if advance_step else None, _ptr(self.workspace),
@@ -375,7 +438,9 @@ class DesmoEngine:
                 _ptr(self.coefs), _ptr(self.coefs_m), _ptr(self.coefs_u), _ptr(self.periods), _ptr(self.periods_m), _ptr(self.periods_u),
                 _ptr(self.omega), _ptr(self.omega_m), _ptr(self.omega_u), _ptr(self.hyper), _ptr(self.step_dev), _ptr(self.losses),
                 _ptr(self.workspace))
-        if self._active is not None:
+        if self._times is not None:
+            check(self.lib.desmo_adamax_update_times(*args, _ptr(self._active), _ptr(self._times), self._stream()), "desmo_adamax_update_times")
+        elif self._active is not None:
             check(self.lib.desmo_adamax_update_active(*args, _ptr(self._active), self._stream()), "desmo_adamax_update_active")
         else:
             check(self.lib.desmo_adamax_update(*args, self._stream()), "desmo_adamax_update")
@@ -435,7 +500,10 @@ class DesmoEngine:
             args = (C.byref(self.shape), _ptr(self.red), _ptr(g["phi"]), _ptr(self.P), _ptr(self.phi), _ptr(self.gates), _ptr(self.rows),
                     _ptr(self.coefs), _ptr(self.periods), _ptr(self.hyper), _ptr(g["gates"]), _ptr(g.get("rows")), _ptr(g.get("coefs")),
                     _ptr(g.get("periods")), _ptr(g["omega"]), _ptr(self.losses), _ptr(self.workspace))
-            if self._active is not None:
+            if self._times is not None:
+                check(self.lib.desmo_assemble_grads_times(*args, _ptr(self._active), _ptr(self._times), self._stream()),
+                      "desmo_assemble_grads_times")
+            elif self._active is not None:
                 check(self.lib.desmo_assemble_grads_active(*args, _ptr(self._active), self._stream()), "desmo_assemble_grads_active")
             else:
                 check(self.lib.desmo_assemble_grads(*args, self._stream()), "desmo_assemble_grads")
@@ -470,10 +538,13 @@ class DesmoEngine:
                   "desmo_recon_backward")
             self.all_reduce()
             g["phi"].copy_(self.dphi)
-            check(self.lib.desmo_assemble_grads(
-                C.byref(self.shape), _ptr(self.red), _ptr(g["phi"]), _ptr(self.P), _ptr(self.phi), _ptr(self.gates), _ptr(self.rows),
-                _ptr(self.coefs), _ptr(self.periods), _ptr(self.hyper), _ptr(g["gates"]), _ptr(g.get("rows")), _ptr(g.get("coefs")),
-                _ptr(g.get("periods")), _ptr(g["omega"]), _ptr(losses), _ptr(self.workspace), self._stream()), "desmo_assemble_grads")
+            args = (C.byref(self.shape), _ptr(self.red), _ptr(g["phi"]), _ptr(self.P), _ptr(self.phi), _ptr(self.gates), _ptr(self.rows),
+                    _ptr(self.coefs), _ptr(self.periods), _ptr(self.hyper), _ptr(g["gates"]), _ptr(g.get("rows")), _ptr(g.get("coefs")),
+                    _ptr(g.get("periods")), _ptr(g["omega"]), _ptr(losses), _ptr(self.workspace))
+            if self._times is not None:
+                check(self.lib.desmo_assemble_grads_times(*args, None, _ptr(self._times), self._stream()), "desmo_assemble_grads_times")
+            else:
+                check(self.lib.desmo_assemble_grads(*args, self._stream()), "desmo_assemble_grads")
         self.set_hyper(saved[:5], saved[5], saved[6])
         g["phi"] = g["phi"][:, :self.n]
         if "rows" in g:
@@ -539,12 +610,19 @@ class DesmoEngine:
 
     # ------------------------------------------------------------------ evaluation at chosen instants
     # Each of these takes exactly one of index= (training snapshot indices, any order, repeats allowed) or times= (fp32 times in the
-    # model's own time coordinate, Fourier models only, any finite value: between grid points, before 0, beyond the window).  They
-    # write nothing the model owns: parameters, optimizer state, rows, W, red, dphi, losses, step_dev and U stay as they are.
+    # model's own time coordinate, Fourier models only, any finite value: between grid points, before 0, beyond the window).  With a
+    # time table (set_time_points), index=k is the instant t_points[k].  They write nothing the model owns: parameters, optimizer
+    # state, rows, W, red, dphi, losses, step_dev and U stay as they are.
     def time_points(self, index) -> np.ndarray:
         """fp32 times of the given snapshot indices (k >= m continues the grid): times=time_points(range(m, 2 * m)) is the next
-        window at the training spacing, and times=time_points(index) gives the same bits as index=index."""
-        return time_points(index, self.m)
+        window at the training spacing, and times=time_points(index) gives the same bits as index=index.  With a time table the
+        times are t_points[index] and k >= m raises: there is no grid to continue."""
+        if self.t_points is None:
+            return time_points(index, self.m)
+        k = np.asarray(index.detach().cpu().numpy() if torch.is_tensor(index) else index).astype(np.int64).reshape(-1)
+        if k.size and (int(k.min()) < 0 or int(k.max()) >= self.m):
+            raise _lib.DesmoError(f"time_points: with a time table the snapshot indices lie in 0 .. {self.m - 1}")
+        return self.t_points[k].copy()
 
     def _w_at(self, idx: Optional[np.ndarray], t: Optional[np.ndarray], mld_out: int, rows_out: Optional[torch.Tensor] = None):
         """W' [Kp][mld_out] at the instants _instants() validated (desmo_build_w_at); rows_out [K][mld_out] receives z(t_i)."""
@@ -562,7 +640,7 @@ class DesmoEngine:
 
     def temporal_rows_at(self, index=None, times=None) -> torch.Tensor:
         """z(t) at the instants, (K, m') fp32: forward()'s z_values there, unscaled by the gates, all K terms in K order."""
-        idx, t = _instants(index, times, self.m, self.nF)
+        idx, t = _instants(index, times, self.m, self.nF, self.t_points)
         m_out = (idx if idx is not None else t).size
         rows = torch.empty(self.K, round_up(m_out, 16), dtype=torch.float32, device=self.device)
         self._w_at(idx, t, rows.shape[1], rows)
@@ -571,7 +649,7 @@ class DesmoEngine:
     def reconstruct_at(self, index=None, times=None) -> torch.Tensor:
         """recon at the instants, (m', n) fp32, allocating only m' rows: desmo_build_w_at, then desmo_reconstruct on an m'-snapshot
         shape.  reconstruct_at(index=k) is bit for bit reconstruct()[k]."""
-        idx, t = _instants(index, times, self.m, self.nF)
+        idx, t = _instants(index, times, self.m, self.nF, self.t_points)
         m_out = (idx if idx is not None else t).size
         sh = self._shape_at(m_out)
         W = self._w_at(idx, t, sh.mld)
@@ -586,7 +664,7 @@ class DesmoEngine:
         the device.  The block is stored as U is (snapshot_dtype; fp32 / fp64 into bf16 by desmo_snapshot_to_bf16 in chunks of at
         most SNAPSHOT_CHUNK_BYTES) in a temporary [m'][ld] buffer.  Returns the four keys of residual_profile(): (m',) snapshot
         sums, summed over ranks when point-sharded, and this rank's (n,) point sums."""
-        idx, t = _instants(index, times, self.m, self.nF)
+        idx, t = _instants(index, times, self.m, self.nF, self.t_points)
         m_out = (idx if idx is not None else t).size
         if not torch.is_tensor(snapshots) or tuple(snapshots.shape) != (m_out, self.n):
             got = tuple(snapshots.shape) if torch.is_tensor(snapshots) else type(snapshots).__name__

@@ -6,7 +6,7 @@ unchanged, and the shipped ``.pt`` files load with ``strict=True``).  Every ``nn
 packed device buffers, so kernel-side updates are visible through the module and vice versa.
 
 The reference reads ``POD_modes`` / ``device`` / ``t_points`` / ``period_init`` from module globals; here they are explicit
-keyword arguments (``pod_modes=...``).  ``forward(X)`` keeps the reference signature and returns the same 3-tuple; ``recon`` is
+keyword arguments (``pod_modes=...``, ``DESMOFourier(..., t_points=...)``; ``t_points=None`` is the scripts' torch.linspace(0, m, m)).  ``forward(X)`` keeps the reference signature and returns the same 3-tuple; ``recon`` is
 materialised and carries a ``grad_fn`` whose backward runs the fused kernels on the upstream gradient (``desmo_recon_backward``),
 so the reference loop ``recon, lat, _ = model(snapshot); loss = criterion(recon, snapshot); total.backward(); optimizer.step()``
 (CYL:711-768) runs unmodified.  The fast paths are ``DesmoTrainer.step()`` (fully fused, no m x n tensor besides the snapshot)
@@ -87,9 +87,9 @@ def _slice_grad(eng: DesmoEngine, g: dict, kind: str, idx) -> torch.Tensor:
 
 class _DesmoBase(nn.Module):
     def _build(self, n, m, polyorder, r_DESMO, omega_init, nF, period_init, pod_modes, device, n_global, path, process_group,
-               snapshot_dtype):
+               snapshot_dtype, t_points=None):
         self.engine = DesmoEngine(n, m, polyorder, r_DESMO, omega_init, nF, period_init, device=device, n_global=n_global,
-                                  path=path, process_group=process_group, snapshot_dtype=snapshot_dtype)
+                                  path=path, process_group=process_group, snapshot_dtype=snapshot_dtype, t_points=t_points)
         e = self.engine
         T, r = e.T, e.r
         print('Number of terms in polynomial library:', T)  # CYL:510
@@ -236,6 +236,16 @@ class _DesmoBase(nn.Module):
         self.sync_parameters()
         return self.engine.backward_elimination(steps)
 
+    # ---- caller-given times (DesmoEngine.set_time_points) --------------------------------------------------------------------
+    @property
+    def t_points(self):
+        """The fp32 (m,) host time table of the snapshot rows, or None for the grid torch.linspace(0, m, m)."""
+        return self.engine.t_points
+
+    def set_time_points(self, t_points) -> None:
+        """Train and evaluate at ``t_points`` (m finite times, one per snapshot row; None: the grid); see DesmoEngine.set_time_points."""
+        self.engine.set_time_points(t_points)
+
     # ---- training a pruned model (DesmoEngine.set_active_terms) ----------------------------------------------------------------
     def set_active_terms(self, mask) -> None:
         """Train on the terms of the bool (K,) ``mask`` only (None: every term); see DesmoEngine.set_active_terms.  The set applies to
@@ -254,19 +264,24 @@ class _DesmoBase(nn.Module):
 
 
 class DESMO(_DesmoBase):
-    """``snapshot_dtype=torch.bfloat16`` stores the snapshot matrix in bf16 (see DesmoEngine)."""
+    """``snapshot_dtype=torch.bfloat16`` stores the snapshot matrix in bf16 (see DesmoEngine).  Free temporal rows have no time
+    coordinate: ``t_points`` other than None raises DesmoError."""
 
     def __init__(self, n, m, polyorder, r_DESMO, omega_init=10000, *, pod_modes=None, device=None, n_global=None,
-                 path=_lib.PATH_AUTO, process_group=None, snapshot_dtype=torch.float32):
+                 path=_lib.PATH_AUTO, process_group=None, snapshot_dtype=torch.float32, t_points=None):
+        if t_points is not None:
+            raise _lib.DesmoError("DESMO has free temporal rows and no time coordinate: t_points needs DESMOFourier")
         super().__init__()
         self._build(n, m, polyorder, r_DESMO, omega_init, None, 0.0, pod_modes, device, n_global, path, process_group, snapshot_dtype)
 
 
 class DESMOFourier(_DesmoBase):
-    """``snapshot_dtype=torch.bfloat16`` stores the snapshot matrix in bf16 (see DesmoEngine)."""
+    """``snapshot_dtype=torch.bfloat16`` stores the snapshot matrix in bf16 (see DesmoEngine).  ``t_points``: the times of the m
+    snapshot rows (tensor, array or sequence; the reference's module global t_points, FCYL:485), or None for its default
+    torch.linspace(0, m, m).  See DesmoEngine.set_time_points."""
 
     def __init__(self, n, m, polyorder, r_DESMO, omega_init=10000, nF=10, *, period_init=60.0, pod_modes=None, device=None,
-                 n_global=None, path=_lib.PATH_AUTO, process_group=None, snapshot_dtype=torch.float32):
+                 n_global=None, path=_lib.PATH_AUTO, process_group=None, snapshot_dtype=torch.float32, t_points=None):
         super().__init__()
         self._build(n, m, polyorder, r_DESMO, omega_init, nF, period_init, pod_modes, device, n_global, path, process_group,
-                    snapshot_dtype)
+                    snapshot_dtype, t_points)

@@ -3,7 +3,8 @@
   build_w, build_w_at, fused_residual_grad, recon_backward, adamax_update, assemble_grads, reconstruct, residual_profile, pruning_profile, library_colnorm2, term_norms,
   pod_gram, pod_eig, pod_eigh, pod_project, preprocess, snapshot_to_bf16, plateau_step, peer_begin_step, peer_allreduce,
   active_terms_prepare, build_w_active, fused_residual_grad_active, adamax_update_active, assemble_grads_active,
-  residual_gram, residual_modes, elimination_pass, elimination_greedy
+  residual_gram, residual_modes, elimination_pass, elimination_greedy,
+  time_points_prepare, build_w_times, adamax_update_times, assemble_grads_times
 
 They take the packed device tensors of a DesmoEngine (layout: include/desmo_b200.h) plus the shape integers and launch the
 sm_100a kernels on the current stream.  CUDA only: no CPU implementation is registered and every op checks its tensors, so a call
@@ -413,6 +414,71 @@ def assemble_grads_active(red: torch.Tensor, dphi: torch.Tensor, P: torch.Tensor
             _p(d_coefs), _p(d_periods), _p(d_omega), _p(losses), _p(workspace), _p(active), _stream(phi)), "desmo_assemble_grads_active")
 
 
+@torch.library.custom_op("desmo_b200::time_points_prepare", mutates_args=("table",))
+def time_points_prepare(times: torch.Tensor, table: torch.Tensor, n: int, n_global: int, m: int, r: int, polyorder: int, nF: int,
+                        path: int) -> None:
+    """The device time table of a Fourier model (desmo_time_points_prepare): ``times`` a contiguous 1-D float32 HOST tensor of m finite
+    values, ``table`` a float32 device tensor of m elements."""
+    _require_cuda(table)
+    if times.device.type != "cpu" or times.dtype != torch.float32 or times.dim() != 1 or not times.is_contiguous():
+        raise _lib.DesmoError("time_points_prepare: times must be a contiguous 1-D float32 tensor on the host")
+    if table.dtype != torch.float32 or not table.is_contiguous() or table.numel() < m:
+        raise _lib.DesmoError(f"time_points_prepare: table must be a contiguous float32 tensor of at least {m} elements")
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(table.device):
+        check(_lib.load().desmo_time_points_prepare(C.byref(s), _p(times), times.numel(), _p(table), _stream(table)),
+              "desmo_time_points_prepare")
+
+
+@torch.library.custom_op("desmo_b200::build_w_times", mutates_args=("rows", "W", "step", "workspace"))
+def build_w_times(gates: torch.Tensor, rows: torch.Tensor, coefs: Optional[torch.Tensor], periods: Optional[torch.Tensor], W: torch.Tensor,
+                  step: torch.Tensor, workspace: torch.Tensor, active: Optional[torch.Tensor], t_points: Optional[torch.Tensor], n: int,
+                  n_global: int, m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """build_w with an optional active set and an optional time table (desmo_build_w_times)."""
+    _require_cuda(gates, rows, W)
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(gates.device):
+        check(_lib.load().desmo_build_w_times(C.byref(s), _p(gates), _p(rows), _p(coefs), _p(periods), _p(W), _p(step), _p(workspace),
+                                              _p(active), _p(t_points), _stream(gates)), "desmo_build_w_times")
+
+
+@torch.library.custom_op("desmo_b200::adamax_update_times",
+                         mutates_args=("phi", "phi_m", "phi_u", "gates", "gates_m", "gates_u", "rows", "rows_m", "rows_u", "coefs", "coefs_m",
+                                       "coefs_u", "periods", "periods_m", "periods_u", "omega", "omega_m", "omega_u", "losses", "workspace"))
+def adamax_update_times(red: torch.Tensor, dphi: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, phi_m: torch.Tensor, phi_u: torch.Tensor,
+                        gates: torch.Tensor, gates_m: torch.Tensor, gates_u: torch.Tensor, rows: torch.Tensor, rows_m: torch.Tensor,
+                        rows_u: torch.Tensor, coefs: Optional[torch.Tensor], coefs_m: Optional[torch.Tensor], coefs_u: Optional[torch.Tensor],
+                        periods: Optional[torch.Tensor], periods_m: Optional[torch.Tensor], periods_u: Optional[torch.Tensor],
+                        omega: torch.Tensor, omega_m: torch.Tensor, omega_u: torch.Tensor, hyper: torch.Tensor, step: torch.Tensor,
+                        losses: torch.Tensor, workspace: torch.Tensor, active: Optional[torch.Tensor], t_points: Optional[torch.Tensor],
+                        n: int, n_global: int, m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """adamax_update with an optional active set and an optional time table (desmo_adamax_update_times)."""
+    _require_cuda(red, dphi, P, phi, gates, rows, omega, hyper, step, losses)
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(phi.device):
+        check(_lib.load().desmo_adamax_update_times(
+            C.byref(s), _p(red), _p(dphi), _p(P), _p(phi), _p(phi_m), _p(phi_u), _p(gates), _p(gates_m), _p(gates_u), _p(rows), _p(rows_m),
+            _p(rows_u), _p(coefs), _p(coefs_m), _p(coefs_u), _p(periods), _p(periods_m), _p(periods_u), _p(omega), _p(omega_m), _p(omega_u),
+            _p(hyper), _p(step), _p(losses), _p(workspace), _p(active), _p(t_points), _stream(phi)), "desmo_adamax_update_times")
+
+
+@torch.library.custom_op("desmo_b200::assemble_grads_times",
+                         mutates_args=("dphi", "d_gates", "d_rows", "d_coefs", "d_periods", "d_omega", "losses", "workspace"))
+def assemble_grads_times(red: torch.Tensor, dphi: torch.Tensor, P: torch.Tensor, phi: torch.Tensor, gates: torch.Tensor, rows: torch.Tensor,
+                         coefs: Optional[torch.Tensor], periods: Optional[torch.Tensor], hyper: torch.Tensor, d_gates: torch.Tensor,
+                         d_rows: Optional[torch.Tensor], d_coefs: Optional[torch.Tensor], d_periods: Optional[torch.Tensor],
+                         d_omega: torch.Tensor, losses: torch.Tensor, workspace: torch.Tensor, active: Optional[torch.Tensor],
+                         t_points: Optional[torch.Tensor], n: int, n_global: int, m: int, r: int, polyorder: int, nF: int, path: int) -> None:
+    """assemble_grads with an optional active set and an optional time table (desmo_assemble_grads_times)."""
+    _require_cuda(red, dphi, P, phi, gates, rows, hyper, d_gates, d_omega, losses)
+    s = make_shape(n, m, r, polyorder, nF, n_global, path)
+    with torch.cuda.device(phi.device):
+        check(_lib.load().desmo_assemble_grads_times(
+            C.byref(s), _p(red), _p(dphi), _p(P), _p(phi), _p(gates), _p(rows), _p(coefs), _p(periods), _p(hyper), _p(d_gates), _p(d_rows),
+            _p(d_coefs), _p(d_periods), _p(d_omega), _p(losses), _p(workspace), _p(active), _p(t_points), _stream(phi)),
+            "desmo_assemble_grads_times")
+
+
 @torch.library.custom_op("desmo_b200::plateau_step", mutates_args=("state", "hyper"))
 def plateau_step(state: torch.Tensor, step: torch.Tensor, losses: torch.Tensor, hyper: torch.Tensor) -> None:
     """ReduceLROnPlateau.step(losses[3]) on the device (desmo_plateau_step); ``state`` is the desmo_plateau struct as bytes."""
@@ -448,11 +514,29 @@ def _shape_args(e):
     return (e.n, e.n_global, e.m, e.r, e.polyorder, e.nF, e.shape.path)
 
 
+def _build_w_op(e, step, sa) -> None:
+    """W of the engine's current parameters through the build_w op, or build_w_times at the engine's time table."""
+    if e._times is not None:
+        torch.ops.desmo_b200.build_w_times(e.gates, e.rows, e.coefs, e.periods, e.W, step, e.workspace, None, e._times, *sa)
+    else:
+        torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, step, e.workspace, *sa)
+
+
 def engine_step_via_ops(e) -> None:
-    """One train step of a DesmoEngine routed entirely through the registered ops (on its active set, if one is set)."""
+    """One train step of a DesmoEngine routed entirely through the registered ops (on its active set and at its time table, if set)."""
     sa = _shape_args(e)
     opt = (e.red, e.dphi, e.P, e.phi, e.phi_m, e.phi_u, e.gates, e.gates_m, e.gates_u, e.rows, e.rows_m, e.rows_u, e.coefs, e.coefs_m,
            e.coefs_u, e.periods, e.periods_m, e.periods_u, e.omega, e.omega_m, e.omega_u, e.hyper, e.step_dev, e.losses, e.workspace)
+    if e._times is not None:
+        torch.ops.desmo_b200.build_w_times(e.gates, e.rows, e.coefs, e.periods, e.W, e.step_dev, e.workspace, e._active, e._times, *sa)
+        if e._active is not None:
+            torch.ops.desmo_b200.fused_residual_grad_active(e.U, e.P, e.phi, e.omega, e.W, e.dphi, e.red, e.workspace, e._active,
+                                                            e._active_count, *sa)
+        else:
+            torch.ops.desmo_b200.fused_residual_grad(e.U, e.P, e.phi, e.omega, e.W, e.dphi, e.red, e.workspace, *sa)
+        e.all_reduce()
+        torch.ops.desmo_b200.adamax_update_times(*opt, e._active, e._times, *sa)
+        return
     if e._active is not None:
         torch.ops.desmo_b200.build_w_active(e.gates, e.rows, e.coefs, e.periods, e.W, e.step_dev, e.workspace, e._active, *sa)
         torch.ops.desmo_b200.fused_residual_grad_active(e.U, e.P, e.phi, e.omega, e.W, e.dphi, e.red, e.workspace, e._active,
@@ -471,7 +555,7 @@ def engine_term_norms_via_ops(e, physical: bool = False) -> torch.Tensor:
     g2 = torch.zeros(e.K, dtype=torch.float32, device=e.device)
     out = torch.zeros(e.K, dtype=torch.float64, device=e.device)
     scratch_step = e.step_dev.clone()  # build_w advances the counter it is given; the optimizer's own one must not move
-    torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, scratch_step, e.workspace, *sa)
+    _build_w_op(e, scratch_step, sa)
     torch.ops.desmo_b200.library_colnorm2(e.P if physical else None, e.phi, e.omega, g2, *sa)
     torch.ops.desmo_b200.term_norms(g2, e.gates, e.rows, 1 if (e.nF and not physical) else 0, out, *sa)
     return out
@@ -483,7 +567,7 @@ def engine_residual_profile_via_ops(e) -> dict:
     snap = torch.empty(2, e.m, dtype=torch.float64, device=e.device)
     point = torch.empty(2, e.ld, dtype=torch.float32, device=e.device)
     scratch_step = e.step_dev.clone()
-    torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, scratch_step, e.workspace, *sa)
+    _build_w_op(e, scratch_step, sa)
     torch.ops.desmo_b200.residual_profile(e.U, e.P, e.phi, e.omega, e.W, snap, point, *sa)
     if e.n_global != e.n and torch.distributed.is_initialized():
         torch.distributed.all_reduce(snap, group=e.pg)
@@ -499,7 +583,7 @@ def engine_pruning_profile_via_ops(e, order) -> dict:
     snap = torch.empty(idx.numel() + 1, e.m, dtype=torch.float64, device=e.device)
     norm = torch.empty(e.m, dtype=torch.float64, device=e.device)
     scratch_step = e.step_dev.clone()
-    torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, scratch_step, e.workspace, *sa)
+    _build_w_op(e, scratch_step, sa)
     torch.ops.desmo_b200.pruning_profile(e.U, e.P, e.phi, e.omega, e.W, idx, snap, norm, *sa)
     if e.n_global != e.n and torch.distributed.is_initialized():
         torch.distributed.all_reduce(snap, group=e.pg)
@@ -552,7 +636,7 @@ def engine_residual_pod_via_ops(e, k: int = 8) -> dict:
     V, sigma, modes = torch.zeros(k, e.m, **f32), torch.zeros(k, **f32), torch.zeros(k, e.ld, **f32)
     S = torch.zeros(e.m, dtype=torch.float64, device=e.device)
     scratch_step = e.step_dev.clone()
-    torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, scratch_step, e.workspace, *sa)
+    _build_w_op(e, scratch_step, sa)
     torch.ops.desmo_b200.residual_gram(e.U, e.P, e.phi, e.omega, e.W, Cm, tr, scratch, *sa)
     if e.n_global != e.n and torch.distributed.is_initialized():
         torch.distributed.all_reduce(Cm, group=e.pg)
@@ -580,7 +664,7 @@ def engine_backward_elimination_via_ops(e, steps=None) -> dict:
     A, F, r2 = torch.empty(e.K, e.K, **f64), torch.empty(e.K, e.mld, **f64), torch.empty(1, **f64)
     order, pred = torch.empty(max(S, 1), dtype=torch.int32, device=e.device), torch.empty(S + 1, **f64)
     scratch_step = e.step_dev.clone()
-    torch.ops.desmo_b200.build_w(e.gates, e.rows, e.coefs, e.periods, e.W, scratch_step, e.workspace, *sa)
+    _build_w_op(e, scratch_step, sa)
     torch.ops.desmo_b200.elimination_pass(e.U, e.P, e.phi, e.omega, e.W, A, F, r2, scratch, *sa)
     if e.n_global != e.n and torch.distributed.is_initialized():
         for t in (A, F, r2):

@@ -9,8 +9,9 @@ from __future__ import annotations
 
 import ctypes
 import math
-from typing import List, Optional, Sequence
+from typing import List, NamedTuple, Optional, Sequence
 
+import numpy as np
 import torch
 
 from .engine import REFERENCE_LRS, DesmoEngine
@@ -41,6 +42,15 @@ class PlateauScheduler:
         return changed
 
 
+class Validation(NamedTuple):
+    """A held-out validation entry of ``DesmoTrainer.history`` (fit(validation=...)): after ``epoch`` epochs, the relative error
+    sqrt(residual2 / norm2) of the held-out block, with residual2 = sum r^2 and norm2 = sum u^2 over the block (residual_profile_at)."""
+    epoch: int
+    rel_error: float
+    residual2: float
+    norm2: float
+
+
 class _PlateauState(ctypes.Structure):  # desmo_plateau (include/desmo_b200.h)
     _fields_ = [("best", ctypes.c_double), ("lrs", ctypes.c_double * 5), ("threshold", ctypes.c_double), ("factor", ctypes.c_double),
                 ("min_lr", ctypes.c_double), ("eps", ctypes.c_double), ("num_bad", ctypes.c_int32), ("patience", ctypes.c_int32),
@@ -67,6 +77,7 @@ class DesmoTrainer:
         self.use_cuda_graph = use_cuda_graph
         self._graph: Optional[torch.cuda.CUDAGraph] = None
         self._graph_active = None  # the engine's active-term table the graph was captured with
+        self._graph_times = None   # ... and its time table (None: the grid)
         self.device_scheduler, self.log_every = bool(device_scheduler), int(log_every)
         self._plateau_dev: Optional[torch.Tensor] = None
         if self.device_scheduler:
@@ -100,8 +111,9 @@ class DesmoTrainer:
         if not self.use_cuda_graph:
             self.engine.train_step()
             return
-        if self._graph is not None and self._graph_active is not self.engine._active:
-            self._graph = None  # set_active_terms changed the launches: capture again
+        if self._graph is not None and (self._graph_active is not self.engine._active or
+                                        self._graph_times is not getattr(self.engine, "_times", None)):
+            self._graph = None  # set_active_terms / set_time_points(None <-> table) changed the launches: capture again
         if self._graph is None:
             # warm up once outside capture (function attributes, NCCL communicators), then capture the step
             e = self.engine
@@ -120,7 +132,7 @@ class DesmoTrainer:
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
                 e.train_step()
-            self._graph, self._graph_active = g, e._active
+            self._graph, self._graph_active, self._graph_times = g, e._active, getattr(e, "_times", None)
             for k, v in snap.items():  # capture does not execute, but keep state exact regardless
                 getattr(e, k).copy_(v)
         self._graph.replay()
@@ -165,6 +177,7 @@ class DesmoTrainer:
                               "patience": self.scheduler.patience},
                 "epoch": self.epoch, "beta": self.beta, "l1_lambda": self.l1_lambda, "sched_every": self.sched_every,
                 "active_terms": None if e.active_terms is None else e.active_terms.clone(),
+                "t_points": None if getattr(e, "t_points", None) is None else torch.from_numpy(e.t_points.copy()),
                 "shape": {"n": e.n, "m": e.m, "r": e.r, "polyorder": e.polyorder, "nF": e.nF, "n_global": e.n_global}}
 
     def load_state_dict(self, sd: dict) -> None:
@@ -193,14 +206,36 @@ class DesmoTrainer:
         self.epoch, self.beta, self.l1_lambda = int(sd["epoch"]), float(sd["beta"]), float(sd["l1_lambda"])
         e.set_hyper(self.scheduler.lrs, self.beta, self.l1_lambda)
         e.set_active_terms(sd.get("active_terms"))  # checkpoints without the key train every term
+        t_points = sd.get("t_points")  # checkpoints without the key train on the grid
+        if t_points is not None or getattr(e, "t_points", None) is not None:
+            e.set_time_points(t_points)
         if self.device_scheduler:
             self._push_scheduler()
 
-    def fit(self, snapshot: torch.Tensor, epochs: int, log_every: int = 0):
+    def validate(self, snapshots: torch.Tensor, instants) -> Validation:
+        """The held-out relative error of the current parameters on ``snapshots`` (m', n) at ``instants``: integer snapshot indices
+        (index=, the model's own times t_points[k] when it has a table) or float times (times=, Fourier models).  One
+        residual_profile_at pass; nothing the model owns is written."""
+        raw = instants.detach().cpu().numpy() if torch.is_tensor(instants) else np.asarray(instants)
+        kw = {"index": raw} if np.issubdtype(raw.dtype, np.integer) else {"times": raw}
+        prof = self.engine.residual_profile_at(snapshots, **kw)
+        r2, u2 = float(prof["snapshot_residual2"].sum()), float(prof["snapshot_norm2"].sum())
+        return Validation(self.epoch, math.sqrt(r2 / u2) if u2 > 0 else math.inf, r2, u2)
+
+    def fit(self, snapshot: torch.Tensor, epochs: int, log_every: int = 0, validation=None, val_every: int = 1):
+        """``epochs`` steps on ``snapshot``.  ``validation=(snapshots, times_or_index)``: a held-out block (m', n) and its instants (see
+        validate()); every ``val_every`` epochs a Validation entry (held-out relative error sqrt(sum r^2 / sum u^2)) is appended to
+        ``history`` after the loss entries of that epoch.  Validation is measurement only: it does not change the training."""
+        if validation is not None:
+            if int(val_every) < 1:
+                raise ValueError(f"val_every must be >= 1, got {val_every}")
+            val_snap, val_at = validation
         self.engine.set_snapshot(snapshot)
         for _ in range(epochs):
             vals = self.step()
             if log_every and vals is not None and (self.epoch - 1) % log_every == 0:
                 print(f"Epoch [{self.epoch}/{epochs}], Rec Loss: {vals[0]:.12f}, Spatial ortho loss: {vals[1]:.8f}, "
                       f"L1 loss: {vals[2]:.4f} ", flush=True)  # CYL:777
+            if validation is not None and self.epoch % int(val_every) == 0:
+                self.history.append(self.validate(val_snap, val_at))
         return self.history

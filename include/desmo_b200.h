@@ -167,6 +167,33 @@ int desmo_fused_residual_grad_finish_active(const desmo_shape* s, const void* U,
                                             const float* omega, const float* W, float* dphi, float* red, void* workspace,
                                             const void* active, int32_t active_count, void* stream);
 
+/* Training a DESMOFourier model on CALLER-GIVEN TIMES (the reference's t_points, FCYL:485, which the scripts set to
+ * torch.linspace(0, m, m)).  A time table holds m finite fp32 values, t_points[t] the time of snapshot row t of U in the model's
+ * time coordinate (any order, repeats allowed).  Column t of the model is evaluated at t_points[t] wherever the grid entry points
+ * use t_point(t, m): the Fourier rows and W (build_w), and the coefficient and period gradients (update / assemble).  Everything
+ * downstream of rows and W (losses, reconstruct, residual_profile, term norms, the sweeps, the residual POD, elimination) follows.
+ * A table equal to the grid gives every step bit for bit what the grid entry points give.  DESMO's free rows have no time
+ * coordinate: a table with nF == 0 is DESMO_ERR_ARG.
+ *   desmo_time_points_prepare  checks host_times[count] (nF > 0, count == m, every value finite) before anything is written, then
+ *                              copies it to table_dev (m floats; stream-ordered, the host array may be reused when it returns).
+ *                              Steps read the table by address, so a captured step follows a table rewritten in place.
+ * The _times entry points take a nullable active-term table (desmo_active_terms_prepare; NULL = every term) and a nullable time
+ * table (NULL = the grid), and otherwise the arguments of the calls they extend. */
+int desmo_time_points_prepare(const desmo_shape* s, const float* host_times, int32_t count, void* table_dev, void* stream);
+int desmo_build_w_times(const desmo_shape* s, const float* gates, float* rows, const float* coefs, const float* periods, float* W,
+                        int32_t* step_dev, void* workspace, const void* active, const float* t_points, void* stream);
+int desmo_adamax_update_times(const desmo_shape* s, const float* red, const float* dphi, const float* P, float* phi,
+                              float* phi_m, float* phi_u, float* gates, float* gates_m, float* gates_u, float* rows,
+                              float* rows_m, float* rows_u, float* coefs, float* coefs_m, float* coefs_u, float* periods,
+                              float* periods_m, float* periods_u, float* omega, float* omega_m, float* omega_u,
+                              const float* hyper, const int32_t* step_dev, float* losses_out, void* workspace, const void* active,
+                              const float* t_points, void* stream);
+int desmo_assemble_grads_times(const desmo_shape* s, const float* red, float* dphi, const float* P, const float* phi,
+                               const float* gates, const float* rows, const float* coefs, const float* periods,
+                               const float* hyper, float* d_gates, float* d_rows, float* d_coefs, float* d_periods,
+                               float* d_omega, float* losses_out, void* workspace, const void* active, const float* t_points,
+                               void* stream);
+
 /* Backward of forward()'s reconstruction for an ARBITRARY upstream gradient (what autograd runs when the reference loop does
  * `recon, _, _ = model(snapshot); loss = criterion(recon, snapshot); total_loss.backward()`, CYL:711,722,766): grad_recon[m][ld]
  * = dL/drecon in the layout of U (pad columns zero).  Same kernels and outputs as desmo_fused_residual_grad with R := (n_global *
